@@ -1,7 +1,7 @@
 #!/usr/bin/env python
 """bench.py — Gibbs sweep throughput of the mmseq hot path on B200, with its correctness gates.
 
-  python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference]
+  python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference] [--dump-outputs DIR]
 
 Workload (config.workload "C2-collapsed"): BASELINE.json configs[1] — a synthetic Ensembl-sized
 sample, 180k transcripts / 30M paired fragments per GPU, in the REFERENCE'S OWN REPRESENTATION:
@@ -81,7 +81,11 @@ def parse():
     ap.add_argument("--batch-per-gpu", type=int, default=4, help="samples in flight per GPU")
     ap.add_argument("--batch-sweeps", type=int, default=16384, help="Gibbs sweeps per sample (the reference's default -gibbs_iter)")
     ap.add_argument("--batch-out", default="/tmp/mmq_batch", help="directory of the per-sample summary tables")
+    ap.add_argument("--dump-outputs", metavar="DIR", help="after the timed steps, write what the last one computed as DIR/<name>.npy "
+                                                          "(float64; rank 0): mu.npy, and trace_last_step.npy, the trace slot it recorded")
     args = ap.parse_args()
+    if args.dump_outputs and (args.impl == "reference" or args.batch > 0):
+        ap.error("--dump-outputs writes the outputs of the timed Gibbs steps on the GPU: not with --impl reference or --batch")
     if args.weights:
         args.layout = "perfragment"
     return args
@@ -466,9 +470,10 @@ def posterior_gate(args, H, w, mu_em, cpu_sweeps, threads):
 
 # ----------------------------------------------------------------------------- ours
 
-def timed_run(args, H, w, stream, dev, barrier, K, W, flush_buf, flags):
+def timed_run(args, H, w, stream, dev, barrier, K, W, flush_buf, flags, outputs=None):
     """W warm-up steps, K timed steps through mmq_gibbs (the production launch path), then the same K steps once more
-    with per-launch events for the kernel shares.  Returns (ms, alloc_ms, alloc_n, gamma_ms, gamma_n, launches, clocks)."""
+    with per-launch events for the kernel shares.  Returns (ms, alloc_ms, alloc_n, gamma_ms, gamma_n, launches, clocks).
+    `outputs` (a dict): receives what a caller of the timed steps reads back after the last one, before the repetition."""
     import torch
     from mmseq_b200 import capi
     S = SWEEPS_PER_STEP
@@ -506,11 +511,31 @@ def timed_run(args, H, w, stream, dev, barrier, K, W, flush_buf, flags):
     sampler.join()
     launches = capi.launch_count() - launches0
     ms = float(sum(a.elapsed_time(b) for a, b in evs))
+    if outputs is not None:
+        outputs["mu"] = H.get_mu()
+        outputs["trace_last_step"] = H.get_trace()[:, W + K - 1]   # step j stores its first sweep's mu into slot j
     H.kernel_times()   # drop anything pending
     for _ in range(K):
         step(flags | capi.MMQ_GIBBS_TIME_KERNELS)
     alloc_ms, alloc_n, gamma_ms, gamma_n = H.kernel_times()
     return ms, alloc_ms, alloc_n, gamma_ms, gamma_n, launches, sampler.result()
+
+
+DUMP_BYTES = 64 << 20
+
+
+def dump_outputs(path, arrays):
+    """Each array (one row per transcript) as path/<name>.npy in float64.  Above DUMP_BYTES in all, every array keeps the
+    same fixed, seeded sample of rows: two builds run with the same arguments still compare output for output."""
+    os.makedirs(path, exist_ok=True)
+    arrays = {name: np.asarray(a, np.float64) for name, a in arrays.items()}
+    total = sum(a.nbytes for a in arrays.values())
+    rows = None
+    if total > DUMP_BYTES:
+        n = len(next(iter(arrays.values())))
+        rows = np.sort(np.random.default_rng(SEED).choice(n, n * DUMP_BYTES // total, replace=False))
+    for name, a in arrays.items():
+        np.save(os.path.join(path, name + ".npy"), a if rows is None else a[rows])
 
 
 def extra_weighted_line(args, dev, stream, peak):
@@ -792,7 +817,10 @@ def main():
     rows = None
 
     K, W, S = args.steps, args.warmup, SWEEPS_PER_STEP
-    ms, alloc_ms, alloc_n, gamma_ms, gamma_n, launches, clocks = timed_run(args, H, w, stream, dev, barrier, K, W, flush_buf, flags)
+    outputs = {} if args.dump_outputs and rank == 0 else None
+    ms, alloc_ms, alloc_n, gamma_ms, gamma_n, launches, clocks = timed_run(args, H, w, stream, dev, barrier, K, W, flush_buf, flags, outputs)
+    if outputs is not None:
+        dump_outputs(args.dump_outputs, outputs)
     t = torch.tensor([ms], dtype=torch.float64, device=dev)
     per_rank = None
     if world > 1:

@@ -189,3 +189,27 @@ def test_config1_host_program_against_the_references_own_main(tmp_path):
         z = compare_with_reference(tables.read_table(str(tmp_path / "ref") + ext), tables.read_table(str(tmp_path / "ours") + ext), kind,
                                    z_max=6.0, frac=0.95)
         assert len(z) > 100
+
+
+def test_config1_host_program_against_stored_outputs(tmp_path):
+    """BASELINE config 1 with default flags: `mmseq` on the GPU against tests/golden/c1 (tools/make_golden_c1.py), the
+    outputs of this host program recorded after it agreed with the reference's own main() on the same input
+    (profiles/r02_c1_compare.txt).  .k / .M byte for byte (SHA-256), .identical.mmseq byte for byte, deterministic
+    columns equal, log_mu of the observed features within the two runs' combined Monte-Carlo standard error."""
+    import hashlib
+    import json
+    from tests.test_reference_run import compare_with_reference
+    gold = os.path.join(ROOT, "tests", "golden", "c1")
+    path = str(tmp_path / "c1.hits")
+    synth.Synth(20260101 + 1, 1000, 100000).write_hits_fast(path, True)
+    base = str(tmp_path / "ours")
+    r = subprocess.run([BIN, "-notraces", path, base], capture_output=True, text=True, timeout=600)
+    assert r.returncode == 0, r.stderr[-2000:]
+    digests = json.load(open(os.path.join(gold, "c1_digests.json")))
+    for ext in (".k", ".M"):
+        assert hashlib.sha256(open(base + ext, "rb").read()).hexdigest() == digests[ext], ext
+    assert open(base + ".identical.mmseq").read() == open(os.path.join(gold, "c1.identical.mmseq")).read()
+    for ext, kind in ((".mmseq", "mmseq"), (".gene.mmseq", "gene")):
+        z = compare_with_reference(tables.read_table(os.path.join(gold, "c1" + ext)), tables.read_table(base + ext), kind,
+                                   z_max=6.0, frac=0.95)
+        assert len(z) > 100
