@@ -23,7 +23,7 @@ build/%.o: $(CSRC)/%.cu $(CSRC)/mmq_internal.h $(CSRC)/mmq_device.cuh $(CSRC)/mm
 	@mkdir -p build
 	$(NVCC) $(NVCCFLAGS) -c $< -o $@
 
-$(LIB): build/mmq_core.o build/mmq_post.o build/mmq_seg.o build/mmq_cls.o build/mmq_rows.o build/mmq_cov.o
+$(LIB): build/mmq_core.o build/mmq_post.o build/mmq_seg.o build/mmq_cls.o build/mmq_cov.o
 	$(NVCC) $(ARCH) -shared -o $@ $^ -ldl
 
 $(SYNTH): $(CSRC)/mmq_synth.cpp

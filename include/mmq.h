@@ -140,8 +140,6 @@ int mmq_em(mmq_handle* h, int max_iter, double eps, int* iters_out, double* logl
                                   (same results; for tests and comparison)   */
 #define MMQ_GIBBS_RAGGED_KERNEL 16 /* k == 1 shards: use the row-pointer driven (TMA-staged)
                                   kernel even when the by-length segment plan exists */
-#define MMQ_GIBBS_ROWS_KERNEL 64 /* by-length k == 1 shards: the row plan (columns once per run of identical rows, member-major
-                                  weights: 1.6x fewer bytes than the default segment kernel, measured no faster); same results */
 int mmq_gibbs(mmq_handle* h, uint32_t seed, int64_t first_sweep, int64_t n_sweeps, int stride,
               int trace_len, int flags);
 
@@ -154,18 +152,11 @@ int mmq_gibbs(mmq_handle* h, uint32_t seed, int64_t first_sweep, int64_t n_sweep
  * their packed column slots.  Used by bench.py for the algorithmic-bytes figure. */
 int mmq_cls_stats(const mmq_handle* h, int64_t out[8]);
 
-/* What the row plan of a by-length k == 1 shard holds (mmq_rows.cu; built by this call if no sweep has asked for it yet):
- * out[0] 1 if in use, out[1] rows with >= 2 members, out[2] runs of identical rows ("sets"), out[3] set
- * column entries, out[4] weight slots (0 without weights), out[5] chunks of 128 rows, out[6] bytes streamed
- * per sweep (4 B per weight slot and set column, 32 B per chunk), out[7] single-member rows (not visited). */
-int mmq_rows_stats(mmq_handle* h, int64_t out[8]);
-
-/* Launch-geometry knobs of the class-plan sweep, for measurements (tools/gpu_tune_cls.py); value 0 restores the
- * default.  knob 0: bit mask of pieces NOT launched (1 k >= 2 small classes, 2 rest, 4 k >= 2 large classes, 8 chain,
- * 16 single-fragment classes: timing experiments only, the chain is then wrong); knobs 1..4: resident CTAs per SM the
- * grid of the chain / large / small / single-fragment kernel is capped at; knob 5: launch order variant; knob 6: 1 =
- * the multi-GPU count exchange as reduce-scatter + all-gather (k_gamma_rs) instead of the all-reduce inside the Gamma
- * kernel (all ranks must set it alike).  Results do not depend on knobs 1..6. */
+/* Measurement switches; value 0 restores the default, any knob other than 0 and 6 is MMQ_ERR_ARG.
+ * knob 0: bit mask of pieces of the class-plan sweep NOT launched (1 k >= 2 small classes, 2 rest, 4 k >= 2 large
+ * classes, 8 chain, 16 single-fragment classes), to time the others alone (tools/gpu_tune_cls.py); the chain is then
+ * wrong.  knob 6: 1 = the multi-GPU count exchange as reduce-scatter + all-gather (k_gamma_rs) instead of the all-reduce
+ * inside the Gamma kernel (all ranks must set it alike); results do not depend on it. */
 int mmq_tune(mmq_handle* h, int knob, int value);
 
 /* Device time of the launches made under MMQ_GIBBS_TIME_KERNELS since the last

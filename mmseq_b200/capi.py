@@ -15,7 +15,6 @@ MMQ_GIBBS_NO_GRAPH = 2
 MMQ_GIBBS_TIME_KERNELS = 4
 MMQ_GIBBS_GENERIC_KERNEL = 8
 MMQ_GIBBS_RAGGED_KERNEL = 16
-MMQ_GIBBS_ROWS_KERNEL = 64
 MMQ_GROUP_IDENTICAL = 0
 MMQ_GROUP_GENE = 1
 
@@ -65,7 +64,6 @@ def _load():
         "mmq_sweep_debug": (i32, [vp, u32, i64, i32, vp, vp, vp]),
         "mmq_kernel_times": (i32, [vp, C.POINTER(dbl), C.POINTER(i64), C.POINTER(dbl), C.POINTER(i64)]),
         "mmq_cls_stats": (i32, [vp, C.POINTER(i64)]),
-        "mmq_rows_stats": (i32, [vp, C.POINTER(i64)]),
         "mmq_tune": (i32, [vp, i32, i32]),
         "mmq_get_trace": (i32, [vp, vp]),
         "mmq_trace_len": (i32, [vp]),
@@ -107,7 +105,7 @@ def lib():
 EXPORTS = [
     "mmq_create", "mmq_destroy", "mmq_last_error", "mmq_set_stream", "mmq_get_stream", "mmq_synchronize",
     "mmq_device_bytes", "mmq_comm_id", "mmq_comm_init", "mmq_comm_move", "mmq_p2p_export", "mmq_p2p_attach", "mmq_p2p_attach_local", "mmq_p2p_attached", "mmq_init_mu", "mmq_set_mu", "mmq_get_mu",
-    "mmq_loglik", "mmq_em", "mmq_gibbs", "mmq_sweep_debug", "mmq_kernel_times", "mmq_cls_stats", "mmq_rows_stats", "mmq_tune", "mmq_get_trace", "mmq_trace_len",
+    "mmq_loglik", "mmq_em", "mmq_gibbs", "mmq_sweep_debug", "mmq_kernel_times", "mmq_cls_stats", "mmq_tune", "mmq_get_trace", "mmq_trace_len",
     "mmq_set_groups", "mmq_summarize", "mmq_get_group_trace", "mmq_prop_summaries",
     "mmq_unique_hits_sets", "mmq_sokal_batch", "mmq_prior_draws", "mmq_trace_cov", "mmq_trace_cov_workspace_bytes", "mmq_trace_cov_dev",
     "mmq_handle_trace_cov", "mmq_mean_corrs", "mmq_mean_corrs_dev", "mmq_release_cache", "mmq_launch_count", "mmq_warmup", "mmq_version",
@@ -333,12 +331,6 @@ class Handle:
 
     def tune(self, knob, value):
         self._check(lib().mmq_tune(self._h, knob, value), "mmq_tune")
-
-    def rows_stats(self):
-        """Row plan of a by-length k == 1 shard (mmq_rows.cu)."""
-        out = (C.c_int64 * 8)()
-        self._check(lib().mmq_rows_stats(self._h, out), "mmq_rows_stats")
-        return dict(zip(["in_use", "rows", "sets", "set_columns", "weight_slots", "chunks", "bytes_per_sweep", "singleton_rows"], [int(v) for v in out]))
 
     def sweep_debug(self, seed, sweep, flags=MMQ_GIBBS_TRANSPOSED, want_x=True):
         x = np.zeros(self.nnz, np.int32) if (want_x and (flags & MMQ_GIBBS_TRANSPOSED)) else None

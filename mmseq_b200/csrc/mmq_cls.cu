@@ -805,8 +805,7 @@ static int cls_plan_device(mmq_handle* h, const mmq_problem* p) {
 
 int mmq_cls_plan(mmq_handle* h, const mmq_problem* p) {
   h->cls_ready = false;
-  static const bool off = [] { const char* e = getenv("MMQ_CLS_OFF"); return e && atoi(e) != 0; }();
-  if (off || !h->has_k || h->has_w || h->m == 0) return MMQ_OK;
+  if (!h->has_k || h->has_w || h->m == 0) return MMQ_OK;
   const char* hp_env = getenv("MMQ_CLS_HOST_PLAN"); /* once per mmq_create: the host builder instead of the device one (tests compare the two) */
   const bool host_plan = hp_env && atoi(hp_env) != 0;
   if (!h->stream2) {
@@ -906,40 +905,29 @@ extern "C" int mmq_cls_stats(const mmq_handle* h, int64_t out[8]) {
 int mmq_cls_launch(mmq_handle* h, uint32_t seed, uint32_t sweep, const uint32_t* sweep_base) {
   int rc = mmq_seg_add_base(h, true);
   if (rc) return rc;
-  const int skip = h->tune[0];
+  const int skip = h->skip_mask;
   const bool do_one = h->cls_chunks > h->cls_chunks_gen && !(skip & 16);
   const bool do_chain = h->cls_c_chunks > 0 && !(skip & 8);
   const bool do_rest = h->cls_rest > 0 && !(skip & 2);
   const bool do_hi = h->cls_chunks_gen > h->cls_chunks_lo && !(skip & 4);
   const bool do_lo = h->cls_chunks_lo > 0 && !(skip & 1);
-  auto cap = [&](int knob, int dflt) { return (int64_t)h->num_sms * (h->tune[knob] > 0 ? h->tune[knob] : dflt); };
+  /* grids are capped at this many resident CTAs per SM */
+  constexpr int CHAIN_CTAS = 3, LARGE_CTAS = 5, SMALL_CTAS = 8, SINGLE_CTAS = 9;
   /* up to five independent pieces, concurrently on the handle's side streams; the main stream takes the last
    * one and waits for the others */
   MMQ_CUDA(h, cudaEventRecord(h->ev_fork, h->stream));
 #define MMQ_CLS_ARGS(c0, c1) (int)(c0), (int)(c1), h->cls_pcol, h->cls_pk, h->cls_pcid, h->cls_cdesc, h->cls_cid_hi, h->mu, h->counts, seed, sweep, sweep_base
-  auto launch_one = [&](cudaStream_t st) {
-    const int64_t c0 = h->cls_chunks_gen, c1 = h->cls_chunks;
-    const int grid = (int)std::min<int64_t>((c1 - c0 + MMQ_CLS_WARPS - 1) / MMQ_CLS_WARPS, cap(4, 9));
-    k_alloc_cls1<<<grid, MMQ_CLS_WARPS * 32, 0, st>>>(MMQ_CLS_ARGS(c0, c1));
-  };
-  const bool one_first = h->tune[5] == 1; /* variant: the bulk kernel goes out first (on its own stream) */
-  if (do_one && one_first) {
-    MMQ_CUDA(h, cudaStreamWaitEvent(h->stream2, h->ev_fork, 0));
-    launch_one(h->stream2);
-    MMQ_LAUNCHED(h);
-    MMQ_CUDA(h, cudaEventRecord(h->ev_join, h->stream2));
-  }
   if (do_chain) { /* the longest dependent chains: first in */
     MMQ_CUDA(h, cudaStreamWaitEvent(h->stream4, h->ev_fork, 0));
     constexpr int CW = MMQ_CHAIN_CLASSES / 32;
-    const int grid = (int)std::min<int64_t>((h->cls_c_chunks + CW - 1) / CW, cap(1, 3));
+    const int grid = (int)std::min<int64_t>((h->cls_c_chunks + CW - 1) / CW, (int64_t)h->num_sms * CHAIN_CTAS);
     MMQ_CUDA(h, cudaFuncSetAttribute(k_alloc_chain, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)sizeof(chain_smem)));
     k_alloc_chain<<<grid, MMQ_CHAIN_THREADS, sizeof(chain_smem), h->stream4>>>((int)h->cls_c_chunks, h->cls_c_pcol, h->cls_c_k, h->cls_c_cid, h->cls_c_desc, h->cls_cid_hi,
                                                               h->mu, h->counts, seed, sweep, sweep_base);
     MMQ_LAUNCHED(h);
     MMQ_CUDA(h, cudaEventRecord(h->ev_join4, h->stream4));
   }
-  if (do_rest && !one_first) {
+  if (do_rest) {
     MMQ_CUDA(h, cudaStreamWaitEvent(h->stream2, h->ev_fork, 0));
     const int grid = (int)std::min<int64_t>((h->cls_rest_tiles + MMQ_ALLOC_WARPS - 1) / MMQ_ALLOC_WARPS, (int64_t)h->num_sms * 3);
     mmq_launch_alloc_general(h, h->stream2, grid, h->cls_o_rp, h->cls_o_col, h->cls_o_k, h->cls_rest, h->cls_o_tiles, h->cls_rest_tiles,
@@ -950,7 +938,7 @@ int mmq_cls_launch(mmq_handle* h, uint32_t seed, uint32_t sweep, const uint32_t*
   if (do_hi) { /* 96 registers, no spills */
     MMQ_CUDA(h, cudaStreamWaitEvent(h->stream3, h->ev_fork, 0));
     const int64_t c0 = h->cls_chunks_lo, c1 = h->cls_chunks_gen;
-    const int grid = (int)std::min<int64_t>((c1 - c0 + MMQ_CLS_WARPS - 1) / MMQ_CLS_WARPS, cap(2, 5));
+    const int grid = (int)std::min<int64_t>((c1 - c0 + MMQ_CLS_WARPS - 1) / MMQ_CLS_WARPS, (int64_t)h->num_sms * LARGE_CTAS);
     k_alloc_cls<false, 5><<<grid, MMQ_CLS_WARPS * 32, 0, h->stream3>>>(MMQ_CLS_ARGS(c0, c1));
     MMQ_LAUNCHED(h);
     MMQ_CUDA(h, cudaEventRecord(h->ev_join3, h->stream3));
@@ -958,25 +946,21 @@ int mmq_cls_launch(mmq_handle* h, uint32_t seed, uint32_t sweep, const uint32_t*
   if (do_lo) { /* 64 registers, no spills, 32 warps per SM */
     MMQ_CUDA(h, cudaStreamWaitEvent(h->stream5, h->ev_fork, 0));
     const int64_t c0 = 0, c1 = h->cls_chunks_lo;
-    const int grid = (int)std::min<int64_t>((c1 - c0 + MMQ_CLS_WARPS - 1) / MMQ_CLS_WARPS, cap(3, 8));
+    const int grid = (int)std::min<int64_t>((c1 - c0 + MMQ_CLS_WARPS - 1) / MMQ_CLS_WARPS, (int64_t)h->num_sms * SMALL_CTAS);
     k_alloc_cls<true, 8><<<grid, MMQ_CLS_WARPS * 32, 0, h->stream5>>>(MMQ_CLS_ARGS(c0, c1));
     MMQ_LAUNCHED(h);
     MMQ_CUDA(h, cudaEventRecord(h->ev_join5, h->stream5));
   }
-  if (do_one && !one_first) { /* the bulk of the entries, on the main stream */
-    launch_one(h->stream);
-    MMQ_LAUNCHED(h);
-  }
-  if (do_rest && one_first) { /* (variant) the few > 64-member classes on the main stream */
-    const int grid = (int)std::min<int64_t>((h->cls_rest_tiles + MMQ_ALLOC_WARPS - 1) / MMQ_ALLOC_WARPS, (int64_t)h->num_sms * 3);
-    mmq_launch_alloc_general(h, h->stream, grid, h->cls_o_rp, h->cls_o_col, h->cls_o_k, h->cls_rest, h->cls_o_tiles, h->cls_rest_tiles,
-                             h->cls_o_cid, seed, sweep, sweep_base);
+  if (do_one) { /* the bulk of the entries, on the main stream */
+    const int64_t c0 = h->cls_chunks_gen, c1 = h->cls_chunks;
+    const int grid = (int)std::min<int64_t>((c1 - c0 + MMQ_CLS_WARPS - 1) / MMQ_CLS_WARPS, (int64_t)h->num_sms * SINGLE_CTAS);
+    k_alloc_cls1<<<grid, MMQ_CLS_WARPS * 32, 0, h->stream>>>(MMQ_CLS_ARGS(c0, c1));
     MMQ_LAUNCHED(h);
   }
 #undef MMQ_CLS_ARGS
   if (do_lo) MMQ_CUDA(h, cudaStreamWaitEvent(h->stream, h->ev_join5, 0));
   if (do_hi) MMQ_CUDA(h, cudaStreamWaitEvent(h->stream, h->ev_join3, 0));
-  if ((do_rest && !one_first) || (do_one && one_first)) MMQ_CUDA(h, cudaStreamWaitEvent(h->stream, h->ev_join, 0));
+  if (do_rest) MMQ_CUDA(h, cudaStreamWaitEvent(h->stream, h->ev_join, 0));
   if (do_chain) MMQ_CUDA(h, cudaStreamWaitEvent(h->stream, h->ev_join4, 0));
   return MMQ_OK;
 }

@@ -1490,8 +1490,7 @@ static int prepare_sweep(mmq_handle* h, int flags) {
     if ((rc = build_transpose(h))) return rc;
   }
   const bool fast = !transposed && !(flags & (MMQ_GIBBS_GENERIC_KERNEL | MMQ_GIBBS_RAGGED_KERNEL));
-  if (fast && (flags & MMQ_GIBBS_ROWS_KERNEL) && !h->rows_ready && !h->rows_tried && (rc = mmq_rows_plan(h))) return rc; /* built on first use */
-  if (fast && h->seg_ready && !((flags & MMQ_GIBBS_ROWS_KERNEL) && h->rows_ready) && (rc = mmq_seg_pack(h))) return rc; /* allocations: not inside a capture */
+  if (fast && h->seg_ready && (rc = mmq_seg_pack(h))) return rc; /* allocations: not inside a capture */
   return MMQ_OK;
 }
 
@@ -1522,9 +1521,7 @@ static int enqueue_sweep(mmq_handle* h, uint32_t seed, uint32_t sweep, int flags
       MMQ_LAUNCHED(h);
     } else {
       mark(h->ev_alloc);
-      if (h->rows_ready && (flags & MMQ_GIBBS_ROWS_KERNEL) && !(flags & (MMQ_GIBBS_GENERIC_KERNEL | MMQ_GIBBS_RAGGED_KERNEL))) {
-        if ((rc = mmq_rows_launch(h, seed, sweep, sweep_base))) return rc;
-      } else if (h->seg_ready && !(flags & (MMQ_GIBBS_GENERIC_KERNEL | MMQ_GIBBS_RAGGED_KERNEL))) {
+      if (h->seg_ready && !(flags & (MMQ_GIBBS_GENERIC_KERNEL | MMQ_GIBBS_RAGGED_KERNEL))) {
         if ((rc = mmq_seg_launch(h, seed, sweep, sweep_base))) return rc;
       } else if (h->cls_ready && !(flags & (MMQ_GIBBS_GENERIC_KERNEL | MMQ_GIBBS_RAGGED_KERNEL))) {
         if ((rc = mmq_cls_launch(h, seed, sweep, sweep_base))) return rc;
@@ -1565,7 +1562,7 @@ static int enqueue_sweep(mmq_handle* h, uint32_t seed, uint32_t sweep, int flags
     a.epoch = epoch_base ? (int32_t)(h->p2p_epoch - h->graph_epoch0) : (int32_t)h->p2p_epoch;
     a.epoch_base = epoch_base;
     mark(h->ev_gamma);
-    if (counts_copy || h->tune[6] != 1) {
+    if (counts_copy || h->exchange_rs != 1) {
       /* default: every rank reads the count vectors of all ranks and draws every Gamma variate — ONE barrier per sweep.
        * (The Gamma kernel is bound by the latency of one pass, not by throughput, so drawing n / N variates instead of
        * n saves nothing, while the reduce-scatter variant below pays a second barrier and the peer stores: measured at
@@ -1744,11 +1741,12 @@ int mmq_kernel_times(mmq_handle* h, double* alloc_ms, int64_t* alloc_launches, d
 int mmq_trace_len(const mmq_handle* h) { return h ? h->trace_len : 0; }
 
 int mmq_tune(mmq_handle* h, int knob, int value) {
-  if (!h || knob < 0 || knob >= 8) return mmq_fail(h, MMQ_ERR_ARG, "mmq_tune: bad knob");
+  if (!h || (knob != 0 && knob != 6)) return mmq_fail(h, MMQ_ERR_ARG, "mmq_tune: bad knob");
   MMQ_CUDA(h, cudaSetDevice(h->device));
   MMQ_CUDA(h, cudaStreamSynchronize(h->stream));
-  drop_graph(h); /* a captured graph has the old geometry baked in */
-  h->tune[knob] = value;
+  drop_graph(h); /* a captured graph has the old launches baked in */
+  if (knob == 0) h->skip_mask = value;
+  else h->exchange_rs = value;
   return MMQ_OK;
 }
 

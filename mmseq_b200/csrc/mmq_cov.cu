@@ -11,39 +11,35 @@
  *   k_cov_prep   one block per feature: mean and centred sum of squares in fp64, z = (x - mean) / sqrt(ssq)
  *                (so that the Gram matrix of z IS the correlation matrix, |z| <= 1), split into 1..3 bf16 terms
  *                z = z0 + z1 + z2 with fp64 residuals, stored K-major: Z[c][split * L + s];
- *   k_cov_gemm   the 128 x 256 tiles of Z Z^T that touch the upper triangle, on the 5th-generation tensor cores.  Persistent,
- *                one CTA per SM, warp-specialised: warp 0 = TMA producer (cp.async.bulk.tensor, 128-byte swizzle, SASS
- *                UTMALDG) into a 3-stage shared-memory ring; warp 1 = one thread issuing tcgen05.mma (kind::f16, bf16 x
- *                bf16 -> fp32, M 128 x N 256 x K 16, SASS UTCHMMA) into one of TWO 256-column TMEM accumulators, stage
- *                release and accumulator hand-over through tcgen05.commit on mbarriers; warps 2..9 = epilogue of the
- *                previous tile while the next one accumulates: tcgen05.ld (SASS LDTM), back to covariance in fp64
- *                (r * sd_i * sd_j), a 32 x 32 transposition through shared memory so that BOTH triangles are stored with
- *                full 256-byte warp stores (streaming), the diagonal exactly var_i, exactly symmetric.  The split terms
- *                z_a z_b with a + b < nsplit are extra K-segments of the same accumulation (smallest terms first).
+ *   k_cov_gemm2  the 256 x 256 tiles of Z Z^T on or above the diagonal, on the 5th-generation tensor cores, one tile per
+ *                CTA PAIR.  Persistent, clusters of two CTAs, warp-specialised: warp 0 = TMA producer (cp.async.bulk.tensor,
+ *                128-byte swizzle, SASS UTMALDG.2D.2CTA; each CTA loads its 128 rows of both operands, both signalling the
+ *                leader's mbarrier) into a 4-stage shared-memory ring; warp 1 of the leader = one thread issuing
+ *                tcgen05.mma.cta_group::2 (kind::f16, bf16 x bf16 -> fp32, M 256 x N 256 x K 16 per pair, SASS UTCHMMA.2CTA)
+ *                into one of TWO 256-column TMEM accumulators per SM, stage release and accumulator hand-over through
+ *                tcgen05.commit multicast to both CTAs (UTCBAR.2CTA.MULTICAST); warps 2..9 = epilogue of the previous tile
+ *                while the next one accumulates: tcgen05.ld (SASS LDTM), back to covariance in fp64 (r * sd_i * sd_j), a
+ *                32 x 32 transposition through shared memory so that BOTH triangles are stored with full 256-byte warp
+ *                stores (streaming), the diagonal exactly var_i, exactly symmetric; the accumulator goes back to the leader
+ *                by a remote mbarrier arrive from the epilogue warps of both CTAs.  The split terms z_a z_b with
+ *                a + b < nsplit are extra K-segments of the same accumulation (smallest terms first).
  *   k_mean_corrs the scan over samples, one thread per (row of ts, column) pair.
  *
  * Accuracy (measured, correlation units |cov_gpu - cov_fp64| / (sd_i sd_j), L = 1024): nsplit = 1: 3e-4, 2: 5e-6 (the
  * default), 3: 2e-6 (the floor of fp32 accumulation) — against a Monte-Carlo error of a correlation estimated from 1024
  * draws of >= 1e-2.  The tests state the tolerances.
  *
- * What bounds it (C = 16384, nsplit = 2: 0.99 ms, 0.83 PFLOP/s algorithmic = 0.50 of the measured cuBLAS bf16 peak, tensor
- * pipe 52 % active; profiles/r02_k_cov_gemm_ncu_summary.txt): shared-memory bandwidth.  A single-CTA 128 x 256 x 16 MMA reads
- * 12 KB of operands from shared memory per 1 MFLOP (66 B/clk at the measured peak rate), TMA writes 48 KB per four of them
- * (64 B/clk) and the epilogue's transposition adds 40 B/clk: more than the 128 B/clk an SM has.  Loading every tile once
- * for all split products (64-byte swizzle, 1.5x less L2 traffic) was measured: same time, so it is not the L2.
- *   k_cov_gemm2 (the default; MMQ_COV_PAIR=0 selects k_cov_gemm) is the same pipeline on CTA PAIRS: clusters of two CTAs,
- *                tcgen05.mma.cta_group::2 (M 256 x N 256 x K 16 per pair; SASS UTCHMMA.2CTA), each CTA loading its 128 rows
- *                of both operands (UTMALDG.2D.2CTA, both signalling the leader's mbarrier), tcgen05.commit multicast to both
- *                CTAs (UTCBAR.2CTA.MULTICAST), accumulators handed back by the epilogue warps of both CTAs (remote mbarrier
- *                arrive): 8 KB of operand reads per MMA and SM instead of 12, 32 KB of TMA writes per stage instead of 48.
- *                0.91-0.93 ms at C = 16384, nsplit = 2 (0.54 of the measured peak; 0.66 with nsplit = 3).  Taken apart with
- *                the stores and / or the MMAs switched off (same pipeline otherwise): neither 0.45 ms, stores only 0.78,
- *                MMAs only 0.76, both 0.93-0.96.  The floor is the operand traffic: 6.4 GB of tiles from the L2-resident Z
- *                per launch at the L2's ~12 TB/s (131 flop per byte for a 256 x 256 pair tile caps the MMAs at 1.5 PFLOP/s,
- *                which is what each further split product costs: 0.18 ms), plus the epilogue's own work (TMEM loads, the
- *                fp64 scaling, the transposition: ~0.25 ms) and the 2.1 GB of stores.  Both split terms of a K block in one
- *                stage (every operand tile loaded once: 1.5x less L2 traffic, but only two stages fit) measured 0.90 against
- *                0.94 ms: not kept.  Next: clusters of two pairs with the shared operand multicast.
+ * What bounds it: 0.91-0.93 ms at C = 16384, nsplit = 2 (0.54 of the measured cuBLAS bf16 peak; 0.66 with nsplit = 3).
+ * Per MMA an SM reads 8 KB of operands from shared memory and receives 32 KB of TMA writes per stage, where one CTA alone
+ * (M 128) needs 12 KB and 48 KB: together with the epilogue's transposition that is more than the 128 B/clk of
+ * shared-memory bandwidth an SM has (a single-CTA version measured 0.99 ms; removed).  Taken apart with the stores and / or
+ * the MMAs switched off (same pipeline otherwise): neither 0.45 ms, stores only 0.78, MMAs only 0.76, both 0.93-0.96.
+ * The floor is the operand
+ * traffic: 6.4 GB of tiles from the L2-resident Z per launch at the L2's ~12 TB/s (131 flop per byte for a 256 x 256 pair
+ * tile caps the MMAs at 1.5 PFLOP/s, which is what each further split product costs: 0.18 ms), plus the epilogue's own
+ * work (TMEM loads, the fp64 scaling, the transposition: ~0.25 ms) and the 2.1 GB of stores.  Both split terms of a K block
+ * in one stage (every operand tile loaded once: 1.5x less L2 traffic, but only two stages fit) measured 0.90 against
+ * 0.94 ms: not kept.  Next: clusters of two pairs with the shared operand multicast.
  */
 #include <cuda.h>
 #include <cuda_bf16.h>
@@ -61,16 +57,13 @@
 
 namespace {
 
-constexpr int COV_BM = 128, COV_BN = 256, COV_BK = 64; /* tile: 128 x 256 outputs (UMMA M = 128, N = 256), 64 bf16 (= one 128-byte swizzle row) of K per stage */
-constexpr int COV_STAGES = 3;
+constexpr int COV_BM = 128, COV_BN = 256, COV_BK = 64; /* one SM's part of a tile: 128 x 256 outputs, 64 bf16 (= one 128-byte swizzle row) of K per stage */
 constexpr int COV_UMMA_K = 16;
-constexpr int COV_A_BYTES = COV_BM * COV_BK * 2, COV_B_BYTES = COV_BN * COV_BK * 2;
-constexpr int COV_STAGE_BYTES = COV_A_BYTES + COV_B_BYTES;
+constexpr int COV_A_BYTES = COV_BM * COV_BK * 2;
 constexpr int COV_TMEM_COLS = 2 * COV_BN; /* two fp32 accumulators of COV_BN columns: all 512 columns, one CTA per SM */
 constexpr int COV_THREADS = 320; /* warp 0: TMA producer, warp 1: MMA issuer + TMEM owner, warps 2..9: epilogue (two per TMEM lane quarter) */
 constexpr int COV_EPI_WARPS = 8;
 constexpr int COV_EPI_BYTES = (33 * 32 + 32) * 8; /* per epilogue warp: 33 x 32 transposition buffer + sd of 32 columns */
-constexpr int COV_SMEM = COV_STAGES * COV_STAGE_BYTES + COV_EPI_WARPS * COV_EPI_BYTES + 256 /* barriers, TMEM slot */ + 1024 /* alignment */;
 
 /* ---- small PTX wrappers (tcgen05 / TMA tensor copies; the mbarrier basics are in mmq_device.cuh) ---- */
 __device__ __forceinline__ void mbar_wait_trap(uint64_t* b, uint32_t parity) {
@@ -85,35 +78,14 @@ __device__ __forceinline__ void mbar_wait_trap(uint64_t* b, uint32_t parity) {
     if (spin > (1u << 22)) __trap();
   }
 }
-__device__ __forceinline__ void tma_load_2d(void* dst, const CUtensorMap* map, int c0, int c1, uint64_t* bar) {
-  asm volatile("cp.async.bulk.tensor.2d.shared::cluster.global.mbarrier::complete_tx::bytes [%0], [%1, {%3, %4}], [%2];" ::"r"(smem_u32(dst)),
-               "l"(map), "r"(smem_u32(bar)), "r"(c0), "r"(c1)
-               : "memory");
-}
 __device__ __forceinline__ void tc_fence_before() { asm volatile("tcgen05.fence::before_thread_sync;" ::: "memory"); }
 __device__ __forceinline__ void tc_fence_after() { asm volatile("tcgen05.fence::after_thread_sync;" ::: "memory"); }
-__device__ __forceinline__ void tc_commit(uint64_t* bar) {
-  asm volatile("tcgen05.commit.cta_group::1.mbarrier::arrive::one.shared::cluster.b64 [%0];" ::"r"(smem_u32(bar)) : "memory");
-}
-/* D[tmem] (+)= A[smem] * B[smem]^T, both operands K-major, bf16 in, fp32 out */
-__device__ __forceinline__ void tc_mma_bf16(uint32_t tmem_d, uint64_t desc_a, uint64_t desc_b, uint32_t idesc, uint32_t accumulate) {
-  asm volatile(
-      "{\n\t"
-      ".reg .pred p;\n\t"
-      "setp.ne.b32 p, %4, 0;\n\t"
-      "tcgen05.mma.cta_group::1.kind::f16 [%0], %1, %2, %3, p;\n\t"
-      "}\n" ::"r"(tmem_d),
-      "l"(desc_a), "l"(desc_b), "r"(idesc), "r"(accumulate)
-      : "memory");
-}
 /* shared-memory matrix descriptor of a K-major tile whose rows are 128 bytes, 128-byte swizzle (what TMA wrote):
  * start address >> 4 | leading byte offset (unused with swizzle: 1) << 16 | stride byte offset (8 rows = 1024 B) >> 4 << 32 |
  * descriptor version 1 (sm_100) << 46 | layout type 2 (SWIZZLE_128B) << 61 */
 __device__ __forceinline__ uint64_t smem_desc_sw128(uint32_t saddr) {
   return (uint64_t)((saddr & 0x3FFFFu) >> 4) | (1ull << 16) | ((uint64_t)(1024 >> 4) << 32) | (1ull << 46) | (2ull << 61);
 }
-/* instruction descriptor: fp32 accumulator (1 << 4), A and B bf16 (1 << 7, 1 << 10), both K-major (bits 15, 16 zero), N >> 3 at bit 17, M >> 4 at bit 24 */
-constexpr uint32_t COV_IDESC = (1u << 4) | (1u << 7) | (1u << 10) | ((uint32_t)(COV_BN >> 3) << 17) | ((uint32_t)(COV_BM >> 4) << 24);
 
 __device__ __forceinline__ void tmem_ld32(uint32_t taddr, uint32_t (&v)[32]) {
   asm volatile(
@@ -172,203 +144,20 @@ __global__ void __launch_bounds__(256) k_cov_prep(const double* __restrict__ src
   }
 }
 
-/* ---- k_cov_gemm ---- */
-__device__ __forceinline__ void cov_tile_of(int64_t t, int64_t& mb, int64_t& nb) {
-  /* tiles that hold an element on or above the diagonal: column block nb (256 wide) pairs with the row blocks mb <= 2 nb + 1 (128 high);
-   * linear index nb (nb + 1) + mb */
-  nb = (int64_t)((sqrt(4.0 * (double)t + 1.0) - 1.0) * 0.5);
-  while (nb * (nb + 1) > t) --nb;
-  while ((nb + 1) * (nb + 2) <= t) ++nb;
-  mb = t - nb * (nb + 1);
-}
-
-/* Persistent: one CTA per SM walks the tiles blockIdx.x, + gridDim.x, ...  Three pipelines: the shared-memory ring
- * (TMA producer <-> MMA issuer), two TMEM accumulators (MMA issuer <-> epilogue: the epilogue of tile n drains one
- * while the MMAs of tile n + 1 fill the other), and the tile walk itself. */
-__global__ void __launch_bounds__(COV_THREADS, 1)
-    k_cov_gemm(const __grid_constant__ CUtensorMap zmap, const double* __restrict__ sd, double* __restrict__ R, int64_t C, int L, int nsplit,
-               int64_t tiles) {
-  extern __shared__ uint8_t cov_smem_raw[];
-  uint8_t* smem = cov_smem_raw + ((1024u - (smem_u32(cov_smem_raw) & 1023u)) & 1023u); /* 1024-byte aligned (128-byte swizzle), still provably shared */
-  uint8_t* epi = smem + COV_STAGES * COV_STAGE_BYTES;
-  uint64_t* full = (uint64_t*)(epi + COV_EPI_WARPS * COV_EPI_BYTES);
-  uint64_t* empty = full + COV_STAGES;
-  uint64_t* tfull = empty + COV_STAGES; /* [2] accumulator b complete */
-  uint64_t* tempty = tfull + 2;         /* [2] accumulator b drained by all epilogue warps */
-  uint32_t* tmem_slot = (uint32_t*)(tempty + 2);
-
-  const int warp = threadIdx.x >> 5, lane = threadIdx.x & 31;
-
-  if (warp == 0 && lane == 0) {
-    asm volatile("prefetch.tensormap [%0];" ::"l"(&zmap) : "memory");
-    for (int s = 0; s < COV_STAGES; ++s) {
-      mbar_init(full + s, 1);
-      mbar_init(empty + s, 1);
-    }
-    for (int b = 0; b < 2; ++b) {
-      mbar_init(tfull + b, 1);
-      mbar_init(tempty + b, COV_EPI_WARPS);
-    }
-    asm volatile("fence.mbarrier_init.release.cluster;" ::: "memory");
-  }
-  if (warp == 1) {
-    asm volatile("tcgen05.alloc.cta_group::1.sync.aligned.shared::cta.b32 [%0], %1;" ::"r"(smem_u32(tmem_slot)), "r"(COV_TMEM_COLS) : "memory");
-    asm volatile("tcgen05.relinquish_alloc_permit.cta_group::1.sync.aligned;" ::: "memory");
-  }
-  tc_fence_before();
-  __syncthreads();
-  tc_fence_after();
-  const uint32_t tmem = *tmem_slot;
-
-  const int kb_per_seg = L / COV_BK;
-  const int iters = (nsplit * (nsplit + 1) / 2) * kb_per_seg;
-
-  if (warp == 0) {
-    if (lane == 0) {
-      int it = 0;
-      for (int64_t t = blockIdx.x; t < tiles; t += gridDim.x) {
-        int64_t mb, nb;
-        cov_tile_of(t, mb, nb);
-        const int row_a = (int)(mb * COV_BM), row_b = (int)(nb * COV_BN);
-        if (row_a >= C) continue; /* the last column block may have one row block less */
-        /* segments (a, b), a + b < nsplit, smallest products first: a + b descending */
-        for (int sum = nsplit - 1; sum >= 0; --sum)
-          for (int a = 0; a <= sum; ++a) {
-            const int b = sum - a;
-            for (int kb = 0; kb < kb_per_seg; ++kb, ++it) {
-              const int stage = it % COV_STAGES;
-              const uint32_t phase = (uint32_t)(it / COV_STAGES) & 1u;
-              mbar_wait_trap(empty + stage, phase ^ 1u);
-              uint8_t* dst = smem + stage * COV_STAGE_BYTES;
-              mbar_expect_tx(full + stage, COV_STAGE_BYTES);
-              tma_load_2d(dst, &zmap, a * L + kb * COV_BK, row_a, full + stage);
-              tma_load_2d(dst + COV_A_BYTES, &zmap, b * L + kb * COV_BK, row_b, full + stage); /* two boxes of 128 rows: contiguous 8-row groups */
-              tma_load_2d(dst + COV_A_BYTES + COV_B_BYTES / 2, &zmap, b * L + kb * COV_BK, row_b + 128, full + stage);
-            }
-          }
-      }
-    }
-  } else if (warp == 1) {
-    if (lane == 0) {
-      int it = 0, n = 0;
-      for (int64_t t = blockIdx.x; t < tiles; t += gridDim.x) {
-        int64_t mb, nb;
-        cov_tile_of(t, mb, nb);
-        if (mb * COV_BM >= C) continue;
-        const int buf = n & 1;
-        mbar_wait_trap(tempty + buf, ((uint32_t)(n >> 1) & 1u) ^ 1u); /* the epilogue has drained this accumulator (tile n - 2) */
-        tc_fence_after();
-        const uint32_t acc = tmem + (uint32_t)(buf * COV_BN);
-        for (int i = 0; i < iters; ++i, ++it) {
-          const int stage = it % COV_STAGES;
-          const uint32_t phase = (uint32_t)(it / COV_STAGES) & 1u;
-          mbar_wait_trap(full + stage, phase);
-          tc_fence_after();
-          const uint32_t a0 = smem_u32(smem + stage * COV_STAGE_BYTES), b0 = a0 + COV_A_BYTES;
-#pragma unroll
-          for (int k = 0; k < COV_BK / COV_UMMA_K; ++k) {
-            /* 16 bf16 = 32 bytes further along K inside the 128-byte swizzle row */
-            tc_mma_bf16(acc, smem_desc_sw128(a0 + k * COV_UMMA_K * 2), smem_desc_sw128(b0 + k * COV_UMMA_K * 2), COV_IDESC, (uint32_t)((i | k) != 0));
-          }
-          tc_commit(empty + stage); /* the stage is free once these MMAs have read it */
-        }
-        tc_commit(tfull + buf); /* accumulator complete */
-        ++n;
-      }
-    }
-    __syncwarp();
-  } else {
-    /* epilogue: warp w may read the TMEM lanes 32 (w % 4) .. +31 = rows of the tile; the two warps of a lane quarter split the columns */
-    const int q = warp & 3, half = (warp - 2) >> 2;
-    const int row = q * 32 + lane;
-    double* tp = (double*)(epi + (warp - 2) * COV_EPI_BYTES); /* 33 x 32 transposition buffer: the stores of BOTH triangles are coalesced */
-    double* sdw = tp + 33 * 32;                               /* sd of the chunk's 32 columns */
-    int n = 0;
-    for (int64_t t = blockIdx.x; t < tiles; t += gridDim.x) {
-      int64_t mb, nb;
-      cov_tile_of(t, mb, nb);
-      const int64_t row_a = mb * COV_BM, row_b = nb * COV_BN;
-      if (row_a >= C) continue;
-      const int64_t gi = row_a + row, gi0 = row_a + q * 32;
-      const double si = gi < C ? sd[gi] : 0.0;
-      const bool diag_tile = (mb >> 1) == nb; /* holds elements below the diagonal */
-      const bool edge = diag_tile || row_a + COV_BM > C || row_b + COV_BN > C;
-      const int buf = n & 1;
-      mbar_wait_trap(tfull + buf, (uint32_t)(n >> 1) & 1u);
-      tc_fence_after();
-      for (int c0 = half * (COV_BN / 2); c0 < (half + 1) * (COV_BN / 2); c0 += 32) {
-        uint32_t v[32];
-        tmem_ld32(tmem + ((uint32_t)(q * 32) << 16) + (uint32_t)(buf * COV_BN + c0), v);
-        if (c0 + 32 == (half + 1) * (COV_BN / 2)) {
-          /* this warp's last read of the accumulator: hand it back to the MMA issuer */
-          tc_fence_before();
-          if (lane == 0) asm volatile("mbarrier.arrive.shared::cta.b64 _, [%0];" ::"r"(smem_u32(tempty + buf)) : "memory");
-        }
-        const int64_t gj0 = row_b + c0;
-        sdw[lane] = gj0 + lane < C ? sd[gj0 + lane] : 0.0;
-        __syncwarp();
-        if (!edge) {
-          /* interior tile: no bounds, no diagonal */
-          double* dp = R + gi + C * gj0; /* column gj0 + j, consecutive lanes = consecutive rows */
-#pragma unroll
-          for (int j = 0; j < 32; ++j) {
-            const double val = (double)__uint_as_float(v[j]) * (si * sdw[j]);
-            tp[j * 33 + lane] = val;
-            __stcs(dp, val);
-            dp += C;
-          }
-          __syncwarp();
-          double* mp = R + gj0 + lane + C * gi0; /* mirror: row gj0 + lane of column gi0 + ii */
-#pragma unroll
-          for (int ii = 0; ii < 32; ++ii) {
-            __stcs(mp, tp[lane * 33 + ii]);
-            mp += C;
-          }
-        } else {
-#pragma unroll
-          for (int j = 0; j < 32; ++j) {
-            const int64_t gj = gj0 + j;
-            const double val = gi == gj ? si * si : (double)__uint_as_float(v[j]) * (si * sdw[j]);
-            tp[j * 33 + lane] = val;
-            /* upper triangle and the diagonal of a diagonal tile; its lower triangle comes from the mirror: exactly symmetric */
-            if (gi < C && gj < C && !(diag_tile && gj < gi)) __stcs(R + gi + C * gj, val);
-          }
-          __syncwarp();
-          const int64_t gj = gj0 + lane;
-          if (gj < C) {
-#pragma unroll 8
-            for (int ii = 0; ii < 32; ++ii) {
-              const int64_t gr = gi0 + ii;
-              if (gr >= C) break;
-              if (diag_tile ? gj > gr : true) __stcs(R + gj + C * gr, tp[lane * 33 + ii]);
-            }
-          }
-        }
-        __syncwarp();
-      }
-      ++n;
-    }
-  }
-  tc_fence_before();
-  __syncthreads();
-  if (warp == 1) {
-    tc_fence_after();
-    asm volatile("tcgen05.dealloc.cta_group::1.sync.aligned.b32 %0, %1;" ::"r"(tmem), "r"(COV_TMEM_COLS) : "memory");
-  }
-}
-
-/* ---- k_cov_gemm2: the same product on CTA PAIRS (tcgen05.mma.cta_group::2) ----
+/* ---- k_cov_gemm2: Z Z^T on CTA PAIRS (tcgen05.mma.cta_group::2) ----
  * A cluster of two CTAs (two SMs of one TPC) computes one 256 x 256 tile: CTA r of the pair holds rows 128 r .. of the A
  * operand and rows 128 r .. of the B operand (each loaded by its own TMA producer, both signalling the LEADER's mbarrier),
  * the leader's elected thread issues M 256 x N 256 x K 16 MMAs for both SMs, every SM accumulates its own 128 x 256 half in
  * its own TMEM and drains it with its own epilogue warps.  Per MMA an SM reads 8 KB of operands from shared memory instead
- * of 12 KB and receives 32 KB per stage instead of 48 KB: the single-CTA kernel above is bound by exactly that (DESIGN.md).
- * Stage release and accumulator hand-over: tcgen05.commit with .multicast::cluster to both CTAs; the accumulator is handed
- * back to the leader by the epilogue warps of BOTH CTAs (remote mbarrier arrive through mapa). */
+ * of the 12 KB of a single-CTA M 128 MMA, and receives 32 KB per stage instead of 48 KB: shared-memory bandwidth is what
+ * bounds a single CTA (DESIGN.md).  Persistent: pair p walks the tiles p, p + pairs, ...  Stage release and accumulator
+ * hand-over: tcgen05.commit with .multicast::cluster to both CTAs; the accumulator is handed back to the leader by the
+ * epilogue warps of BOTH CTAs (remote mbarrier arrive through mapa). */
 constexpr int COV2_STAGES = 4;
 constexpr int COV2_STAGE_BYTES = 2 * COV_A_BYTES; /* this CTA's 128 rows of A and its 128 rows of B */
-constexpr int COV2_SMEM = COV2_STAGES * COV2_STAGE_BYTES + COV_EPI_WARPS * COV_EPI_BYTES + 256 + 1024;
-/* instruction descriptor of the pair: M = 256 */
+constexpr int COV2_SMEM = COV2_STAGES * COV2_STAGE_BYTES + COV_EPI_WARPS * COV_EPI_BYTES + 256 /* barriers, TMEM slot */ + 1024 /* alignment */;
+/* instruction descriptor of the pair: fp32 accumulator (1 << 4), A and B bf16 (1 << 7, 1 << 10), both K-major (bits 15,
+ * 16 zero), N >> 3 at bit 17, M >> 4 at bit 24; M = 256 */
 constexpr uint32_t COV2_IDESC = (1u << 4) | (1u << 7) | (1u << 10) | ((uint32_t)(256 >> 3) << 17) | ((uint32_t)(256 >> 4) << 24);
 
 __device__ __forceinline__ uint32_t cluster_rank() {
@@ -654,7 +443,7 @@ int cov_run(const double* src_dev, const int64_t* off_dev, int64_t off_step, int
   if (!enc) return cov_fail(MMQ_ERR_CUDA, "mmq_trace_cov: cuTensorMapEncodeTiled not available from the driver");
   static std::once_flag attr_once;
   static cudaError_t attr_err = cudaSuccess;
-  std::call_once(attr_once, [] { attr_err = cudaFuncSetAttribute(k_cov_gemm, cudaFuncAttributeMaxDynamicSharedMemorySize, COV_SMEM); });
+  std::call_once(attr_once, [] { attr_err = cudaFuncSetAttribute(k_cov_gemm2, cudaFuncAttributeMaxDynamicSharedMemorySize, COV2_SMEM); });
   if (attr_err != cudaSuccess) return cov_fail(MMQ_ERR_CUDA, std::string("mmq_trace_cov: shared-memory attribute: ") + cudaGetErrorString(attr_err));
   __nv_bfloat16* Z = (__nv_bfloat16*)ws_dev;
   const size_t zbytes = ((size_t)C * (size_t)nsplit * (size_t)L * 2 + 255) & ~(size_t)255;
@@ -671,28 +460,12 @@ int cov_run(const double* src_dev, const int64_t* off_dev, int64_t off_step, int
                           CU_TENSOR_MAP_SWIZZLE_128B, CU_TENSOR_MAP_L2_PROMOTION_L2_256B, CU_TENSOR_MAP_FLOAT_OOB_FILL_NONE);
   if (cr != CUDA_SUCCESS) return cov_fail(MMQ_ERR_CUDA, "mmq_trace_cov: cuTensorMapEncodeTiled failed (" + std::to_string((int)cr) + ")");
   const int64_t T = (C + COV_BN - 1) / COV_BN;
-  const char* pair_env = getenv("MMQ_COV_PAIR"); /* 0: the single-CTA kernel (k_cov_gemm); default: CTA pairs (k_cov_gemm2) */
-  const int use_pair = pair_env ? atoi(pair_env) : 1;
-  if (use_pair) {
-    static std::once_flag attr2_once;
-    static cudaError_t attr2_err = cudaSuccess;
-    std::call_once(attr2_once, [] { attr2_err = cudaFuncSetAttribute(k_cov_gemm2, cudaFuncAttributeMaxDynamicSharedMemorySize, COV2_SMEM); });
-    if (attr2_err != cudaSuccess) return cov_fail(MMQ_ERR_CUDA, std::string("mmq_trace_cov: shared-memory attribute: ") + cudaGetErrorString(attr2_err));
-    const int64_t tiles2 = T * (T + 1) / 2; /* 256 x 256 tiles of the upper triangle, one per CTA pair */
-    int dev2 = 0, sms2 = 148;
-    COV_CUDA(cudaGetDevice(&dev2));
-    COV_CUDA(cudaDeviceGetAttribute(&sms2, cudaDevAttrMultiProcessorCount, dev2));
-    const int64_t pairs = std::max<int64_t>(1, std::min<int64_t>(tiles2, sms2 / 2));
-    k_cov_gemm2<<<(unsigned)(2 * pairs), COV_THREADS, COV2_SMEM, st>>>(map, sd, R_dev, C, L, nsplit, tiles2);
-    g_mmq_launches.fetch_add(1, std::memory_order_relaxed);
-    COV_CUDA(cudaGetLastError());
-    return MMQ_OK;
-  }
-  const int64_t tiles = T * (T + 1);
+  const int64_t tiles = T * (T + 1) / 2; /* 256 x 256 tiles of the upper triangle, one per CTA pair */
   int dev = 0, sms = 148;
   COV_CUDA(cudaGetDevice(&dev));
   COV_CUDA(cudaDeviceGetAttribute(&sms, cudaDevAttrMultiProcessorCount, dev));
-  k_cov_gemm<<<(unsigned)std::min<int64_t>(tiles, sms), COV_THREADS, COV_SMEM, st>>>(map, sd, R_dev, C, L, nsplit, tiles);
+  const int64_t pairs = std::max<int64_t>(1, std::min<int64_t>(tiles, sms / 2));
+  k_cov_gemm2<<<(unsigned)(2 * pairs), COV_THREADS, COV2_SMEM, st>>>(map, sd, R_dev, C, L, nsplit, tiles);
   g_mmq_launches.fetch_add(1, std::memory_order_relaxed);
   COV_CUDA(cudaGetLastError());
   return MMQ_OK;

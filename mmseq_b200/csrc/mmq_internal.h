@@ -106,15 +106,6 @@ struct mmq_handle {
   int64_t seg_entries = 0, seg_rows = 0, seg_singletons = 0, seg_packed = 0;
   std::vector<mmq_seg> seg_host; /* the table, kept for the lazy packing (mmq_seg_pack) */
 
-  /* row plan for by-length k == 1 shards (mmq_rows.cu): columns once per run of identical rows, weights member-major */
-  bool rows_ready = false, rows_tried = false;
-  void* rows_runs = nullptr; /* mmq_rows_run[] */
-  void* rows_meta = nullptr; /* mmq_rows_meta[] */
-  int32_t* rows_set_col = nullptr;
-  float* rows_w = nullptr;
-  int rows_nruns = 0;
-  int64_t rows_chunks = 0, rows_chunks_small = 0, rows_rows = 0, rows_sets = 0, rows_set_cols = 0, rows_wslots = 0;
-
   /* class plan for collapsed shards (mmq_cls.cu): the classes with few fragments packed in
    * member-major chunks of 32, the rest as a sub-CSR for the general kernel on stream2 */
   bool cls_ready = false;
@@ -167,8 +158,9 @@ struct mmq_handle {
   /* MMQ_GIBBS_TIME_KERNELS: (start, stop) event pairs around each launch */
   std::vector<cudaEvent_t> ev_alloc, ev_gamma;
 
-  /* launch-geometry knobs of the class-plan sweep (mmq_tune; 0 = the measured default) */
-  int tune[8] = {0, 0, 0, 0, 0, 0, 0, 0};
+  /* mmq_tune: knob 0, pieces of the class-plan sweep not launched (bit mask); knob 6, 1 = the reduce-scatter exchange */
+  int skip_mask = 0;
+  int exchange_rs = 0;
 
   int64_t bytes = 0;
   std::string err;
@@ -200,8 +192,6 @@ int mmq_seg_scan(mmq_handle* h, const int64_t* row_ptr_host);
 int mmq_seg_plan(mmq_handle* h);
 int mmq_seg_launch(mmq_handle* h, uint32_t seed, uint32_t sweep, const uint32_t* sweep_base);
 int mmq_seg_pack(mmq_handle* h);
-int mmq_rows_plan(mmq_handle* h);
-int mmq_rows_launch(mmq_handle* h, uint32_t seed, uint32_t sweep, const uint32_t* sweep_base);
 int mmq_seg_add_base(mmq_handle* h, bool want_in_counts);
 int mmq_cls_plan(mmq_handle* h, const mmq_problem* p);
 int mmq_cls_launch(mmq_handle* h, uint32_t seed, uint32_t sweep, const uint32_t* sweep_base);

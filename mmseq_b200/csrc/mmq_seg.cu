@@ -488,9 +488,8 @@ int mmq_seg_plan(mmq_handle* h) {
   return MMQ_OK;
 }
 
-/* The packed, aligned copies of col / weight the segment kernel streams: made on first use (the row plan of
- * mmq_rows.cu is the default for these shards; k_alloc_seg4 stays as MMQ_GIBBS_SEG_KERNEL and for shards the row plan
- * declines). */
+/* The packed, aligned copies of col / weight the segment kernel streams: made by the first sweep that runs it, so a
+ * handle that is only swept with MMQ_GIBBS_GENERIC_KERNEL, RAGGED_KERNEL or TRANSPOSED never holds them. */
 int mmq_seg_pack(mmq_handle* h) {
   if (h->seg_col || h->seg_count == 0) return MMQ_OK;
   const int64_t packed = h->seg_packed;
@@ -519,8 +518,6 @@ int mmq_seg_launch(mmq_handle* h, uint32_t seed, uint32_t sweep, const uint32_t*
   if (rc) return rc;
   if ((rc = mmq_seg_pack(h))) return rc;
   if (h->seg_count == 0) return MMQ_OK; /* only singletons: nothing random to do */
-  /* geometry (tuning knob): 0 = the measured best */
-  static const int geo = [] { const char* e = getenv("MMQ_SEG_GEO"); return e ? atoi(e) : 0; }();
   const int chunks = (int)h->seg_chunks;
   /* W weights, ST largest staged class size, NW warps per CTA, MINB CTAs per SM (=> register budget) */
 #define MMQ_SEG4_GO(W, ST, NW, MINB)                                                                                        \
@@ -532,14 +529,8 @@ int mmq_seg_launch(mmq_handle* h, uint32_t seed, uint32_t sweep, const uint32_t*
                                                                     grid * NW, h->seg_col, h->seg_w, h->mu, h->counts, seed, \
                                                                     sweep, sweep_base);                                 \
   } while (0)
-  if (h->has_w) {
-    if (geo == 1) MMQ_SEG4_GO(true, 8, 4, 6);
-    else MMQ_SEG4_GO(true, 12, 4, 4); /* 12 KB per warp: 16 warps per SM, no spills */
-  } else {
-    if (geo == 1) MMQ_SEG4_GO(false, 12, 4, 7);
-    else if (geo == 2) MMQ_SEG4_GO(false, 12, 8, 4);
-    else MMQ_SEG4_GO(false, 12, 4, 6); /* 80 registers, no spills, 24 warps per SM */
-  }
+  if (h->has_w) MMQ_SEG4_GO(true, 12, 4, 4); /* 12 KB per warp: 16 warps per SM, no spills */
+  else MMQ_SEG4_GO(false, 12, 4, 6);         /* 80 registers, no spills, 24 warps per SM */
 #undef MMQ_SEG4_GO
   return MMQ_OK;
 }

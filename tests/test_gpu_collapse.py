@@ -34,15 +34,6 @@ def test_cov_matches_oracle(L, C):
         assert abs(R[0, C - 1] / (d[0] * d[C - 1]) - 1.0) < TOL[3]     # duplicated feature
 
 
-def test_single_cta_kernel_gives_the_same_matrix(monkeypatch):
-    """k_cov_gemm2 (CTA pairs, the default) and k_cov_gemm (MMQ_COV_PAIR=0) accumulate the same products in the same order."""
-    M = make_traces(1024, 700, seed=31)
-    R2 = capi.trace_cov(M, nsplit=2)
-    monkeypatch.setenv("MMQ_COV_PAIR", "0")
-    R1 = capi.trace_cov(M, nsplit=2)
-    assert np.array_equal(R1, R1.T) and corr_err(R1, R2) < 1e-6
-
-
 def test_cov_full_size_tile_grid():
     """Several tiles per side incl. a ragged last tile; every tile of the upper triangle and its mirror written."""
     L, C = 1024, 5 * 128 + 77

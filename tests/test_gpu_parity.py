@@ -104,7 +104,7 @@ def test_categorical_fast_path_edges(weighted, cid_base):
 
 @pytest.mark.parametrize("weighted", [False, True])
 @pytest.mark.parametrize("cid_base", [0, 5, 2, 7])
-def test_by_length_layout_segment_kernel(small_synth, weighted, cid_base):
+def test_by_length_layout_kernels_match_replay(small_synth, weighted, cid_base):
     """The loader's by-length layout: runs of equal class size, singletons skipped, no row
     pointers read — same integers and the same chain as the CPU replay and as the other kernels."""
     s = small_synth
@@ -117,13 +117,10 @@ def test_by_length_layout_segment_kernel(small_synth, weighted, cid_base):
     P = orc.Problem(h.row_ptr, h.col, None, h.len, weight=h.w)
     mu, _, _ = P.init_mu()
     with capi.Handle(h.row_ptr, h.col, None, h.len, weight=h.w, class_id_base=cid_base) as H:
-        st = H.rows_stats()   # the row plan (mmq_rows.cu, MMQ_GIBBS_ROWS_KERNEL): columns once per run of identical rows
-        assert st["in_use"] == 1 and st["rows"] + st["singleton_rows"] == h.m and 0 < st["sets"] < st["rows"]
-        assert (st["weight_slots"] > 0) == weighted and st["bytes_per_sweep"] < (8 if weighted else 4) * h.nnz
         for sweep in range(3):
             _, c_o, mu_o = P.sweep_replay(mu, SEED, sweep, class_id_base=cid_base)
-            for flags in (capi.MMQ_GIBBS_DEFAULT, capi.MMQ_GIBBS_ROWS_KERNEL, capi.MMQ_GIBBS_RAGGED_KERNEL, capi.MMQ_GIBBS_GENERIC_KERNEL,
-                          capi.MMQ_GIBBS_TRANSPOSED, capi.MMQ_GIBBS_DEFAULT):
+            for flags in (capi.MMQ_GIBBS_DEFAULT, capi.MMQ_GIBBS_RAGGED_KERNEL, capi.MMQ_GIBBS_GENERIC_KERNEL, capi.MMQ_GIBBS_TRANSPOSED,
+                          capi.MMQ_GIBBS_DEFAULT):
                 H.set_mu(mu)
                 _, c, mu_g = H.sweep_debug(SEED, sweep, flags, want_x=False)
                 assert np.array_equal(c, c_o), (sweep, flags)
@@ -137,8 +134,9 @@ def test_by_length_layout_segment_kernel(small_synth, weighted, cid_base):
             assert np.array_equal(H.get_mu(), mu_end) and np.array_equal(H.get_trace()[:, 1:], tr_o[:, 1:])
 
 
-def test_row_plan_zero_weights(small_synth):
-    """Weights of exactly 0 are legal (a hit that cannot have produced the fragment): such a member is never chosen."""
+def test_zero_weights_never_chosen(small_synth):
+    """Weights of exactly 0 are legal (a hit that cannot have produced the fragment): such a member is never chosen, by
+    the segment kernel (the default for this layout) and by every other kernel."""
     s = small_synth
     rng = np.random.default_rng(12)
     w = np.exp(0.5 * rng.standard_normal(len(s.frag_tid))).astype(np.float32)
@@ -147,12 +145,12 @@ def test_row_plan_zero_weights(small_synth):
     P = orc.Problem(h.row_ptr, h.col, None, h.len, weight=h.w)
     mu = np.random.default_rng(1).gamma(0.5, 10.0, h.n)
     with capi.Handle(h.row_ptr, h.col, None, h.len, weight=h.w) as H:
-        assert H.rows_stats()["in_use"] == 1
         for sweep in range(2):
-            H.set_mu(mu)
             _, c_o, mu_o = P.sweep_replay(mu, SEED, sweep)
-            _, c, mu_g = H.sweep_debug(SEED, sweep, capi.MMQ_GIBBS_ROWS_KERNEL, want_x=False)
-            assert np.array_equal(c, c_o) and np.array_equal(mu_g, mu_o)
+            for flags in (capi.MMQ_GIBBS_DEFAULT, capi.MMQ_GIBBS_RAGGED_KERNEL, capi.MMQ_GIBBS_GENERIC_KERNEL, capi.MMQ_GIBBS_TRANSPOSED):
+                H.set_mu(mu)
+                _, c, mu_g = H.sweep_debug(SEED, sweep, flags, want_x=False)
+                assert np.array_equal(c, c_o) and np.array_equal(mu_g, mu_o), (sweep, flags)
 
 
 def test_weighted_rows_bit_exact(small_synth):
@@ -386,6 +384,8 @@ def test_errors_are_reported_not_fatal(small_problem):
             H.get_trace()                                          # no trace yet
         with pytest.raises(capi.MmqError):
             H.gibbs(SEED, 0, 4, stride=0, trace_len=8)
+        with pytest.raises(capi.MmqError):
+            H.tune(3, 1)                                           # not a knob
     with pytest.raises(capi.MmqError):
         capi.Handle(h.row_ptr, np.where(np.arange(h.nnz) == 5, h.n + 3, h.col), h.k, h.len)   # column out of range
     with pytest.raises(capi.MmqError):

@@ -1,4 +1,4 @@
-"""One k_cov_gemm launch at C = 16384, L = 1024, nsplit = 2 for ncu."""
+"""k_cov_gemm2 launches at C = 16384, L = 1024, nsplit = 2 for ncu."""
 import sys
 import torch
 sys.path.insert(0, ".")

@@ -1,4 +1,4 @@
-"""Launch-geometry experiments on the class-plan sweep (collapsed C2 sample): one workload, one handle, mmq_tune knobs.
+"""Time the pieces of the class-plan sweep alone (collapsed C2 sample): one workload, one handle, mmq_tune knob 0.
    python tools/gpu_tune_cls.py            (on the GPU box)"""
 import os, sys, time
 import numpy as np
@@ -16,11 +16,8 @@ H.init_mu()
 mu0 = H.get_mu()
 flush = torch.empty(256 << 20, dtype=torch.uint8, device="cuda")
 
-def run(label, knobs, steps=8):
-    for k in range(8):
-        H.tune(k, 0)
-    for k, v in knobs.items():
-        H.tune(k, v)
+def run(label, skip, steps=8):
+    H.tune(0, skip)
     H.set_mu(mu0)
     sweep = 0
     for _ in range(2):
@@ -38,19 +35,7 @@ def run(label, knobs, steps=8):
         tot += a.elapsed_time(b)
     print(f"{label:44s} {1000 * tot / (steps * 16):8.2f} us per sweep", flush=True)
 
-run("default", {})
+run("default", 0)
 for name, m in (("no chain", 8), ("no large (HI)", 4), ("no small k>=2 (LO)", 1), ("no single-fragment (cls1)", 16), ("only cls1", 1 | 2 | 4 | 8),
                 ("only LO", 2 | 4 | 8 | 16), ("only HI", 1 | 2 | 8 | 16), ("only chain", 1 | 2 | 4 | 16), ("none (gamma only)", 31)):
-    run("skip: " + name, {0: m})
-for c in (1, 2):
-    run(f"chain grid cap {c}/SM", {1: c})
-for c in (1, 2, 3):
-    run(f"HI grid cap {c}/SM", {2: c})
-for c in (4, 6):
-    run(f"LO grid cap {c}/SM", {3: c})
-for c in (6, 12):
-    run(f"cls1 grid cap {c}/SM", {4: c})
-run("cls1 first", {5: 1})
-run("cls1 first, HI cap 1, chain cap 2", {5: 1, 2: 1, 1: 2})
-run("HI cap 1, chain cap 2", {2: 1, 1: 2})
-run("HI cap 2, LO cap 4", {2: 2, 3: 4})
+    run("skip: " + name, m)
