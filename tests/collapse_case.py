@@ -47,3 +47,26 @@ def mean_corrs_numpy(R, S, ts, sdpenalty=0.0):
                 V[t, v] = V[v, t] = mean + sdpenalty * sd
                 W[t, v] = W[v, t] = sd
     return V, W
+
+
+def make_gene_problem(n=12000, G=5000, n_ident=5000, m=30000, seed=0):
+    """A hand-built collapsed problem with a gene structure: n transcripts in G non-empty genes (1..~6 isoforms), m
+    classes of 1..6 members drawn among neighbouring isoforms, counts k in 1..49, and n_ident disjoint identical-transcript
+    sets of two.  Returns (row_ptr, col, k, len, gene_of, ident_ptr, ident_members)."""
+    rng = np.random.default_rng(seed)
+    gene_of = np.concatenate([np.arange(G), rng.integers(0, G, n - G)])
+    rng.shuffle(gene_of)
+    by_gene = np.argsort(gene_of, kind="stable").astype(np.int32)     # isoforms of a gene are neighbours here
+    d = rng.integers(1, 7, m)
+    start = rng.integers(0, n - 6, m)
+    pos = np.repeat(start, d) + (np.arange(int(d.sum())) - np.repeat(np.cumsum(d) - d, d))
+    row = np.repeat(np.arange(m), d)
+    col = by_gene[pos]
+    o = np.lexsort((col, row))                                          # members ascending within a class
+    col = col[o]
+    row_ptr = np.concatenate([[0], np.cumsum(d)]).astype(np.int64)
+    k = rng.integers(1, 50, m).astype(np.int32)
+    length = rng.uniform(1e-6, 1e-2, n)
+    ident_mem = rng.permutation(n)[:2 * n_ident].astype(np.int32)
+    ident_ptr = np.arange(0, 2 * n_ident + 1, 2, dtype=np.int64)
+    return row_ptr, col, k, length, gene_of.astype(np.int32), ident_ptr, ident_mem

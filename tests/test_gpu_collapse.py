@@ -7,7 +7,7 @@ import pytest
 
 from mmseq_b200 import capi
 from oracle import oracle as orc
-from tests.collapse_case import make_traces
+from tests.collapse_case import make_gene_problem, make_traces
 
 pytestmark = pytest.mark.gpu
 TOL = {1: 1e-2, 2: 3e-5, 3: 1e-5}
@@ -19,8 +19,23 @@ def corr_err(R, ref):
     return np.max(np.abs(R - ref) / (d[:, None] * d[None, :]))
 
 
-@pytest.mark.parametrize("L,C", [(64, 1), (64, 5), (1024, 37), (1024, 128), (1024, 129), (1024, 300), (512, 1000), (2048, 257)])
+def _pair_tiles(C, sms):
+    """k_cov_gemm2's work (mmq_cov.cu:467-468): T (T + 1) / 2 upper-triangle tiles of 256 x 256, T = ceil(C / 256), swept
+    by min(tiles, sms / 2) CTA pairs."""
+    T = -(-C // 256)
+    return T * (T + 1) // 2, sms // 2
+
+
+# C = 5197: 21 tiles a side (the last one ragged), 231 tiles, more than 3 x 74 CTA pairs on 148 SMs: every pair takes three
+# or more tiles, so each reuses TMEM accumulator 0 at least twice and the mbarrier phases wrap.  L = 64, 192 and 1024: one,
+# three and sixteen MMA iterations per tile (nsplit 1) against the 4-stage ring.
+@pytest.mark.parametrize("L,C", [(64, 1), (64, 5), (1024, 37), (1024, 128), (1024, 129), (1024, 300), (512, 1000), (2048, 257),
+                                 (64, 5197), (192, 5197), (1024, 5197)])
 def test_cov_matches_oracle(L, C):
+    import torch
+    if C > 5000:
+        tiles, pairs = _pair_tiles(C, torch.cuda.get_device_properties(0).multi_processor_count)
+        assert tiles > 3 * pairs, (tiles, pairs)
     M = make_traces(L, C, seed=L + C)
     ref = orc.trace_cov(M)
     for nsplit in (1, 2, 3):
@@ -98,9 +113,29 @@ def test_cov_from_a_handles_trace(small_problem):
     H.close()
 
 
-def test_mean_corrs_matches_oracle():
+def test_cov_from_a_handles_trace_many_tiles():
+    """The gather path (features picked from the handle's trace on the device) with more tiles than CTA pairs."""
+    import torch
+    row_ptr, col, k, length, _, _, _ = make_gene_problem()
+    C, L = 4200, 1024
+    tiles, pairs = _pair_tiles(C, torch.cuda.get_device_properties(0).multi_processor_count)
+    assert tiles > 2 * pairs, (tiles, pairs)
+    feats = np.random.default_rng(3).permutation(len(length))[:C].astype(np.int32)
+    with capi.Handle(row_ptr, col, k, length) as H:
+        H.init_mu()
+        H.em(50, 0.1)
+        H.gibbs(7, 0, L, stride=1, trace_len=L)
+        tr = H.get_trace()
+        R = H.trace_cov(feats, nsplit=3)
+    assert np.array_equal(R, capi.trace_cov(tr[feats].T, nsplit=3))     # the gather path is the host-matrix path
+    ref = orc.trace_cov(tr[feats].T)
+    assert np.array_equal(R, R.T)
+    assert np.allclose(np.diag(R), np.diag(ref), rtol=1e-12, atol=0.0)
+    assert corr_err(R, ref) < TOL[3]
+
+
+def _check_mean_corrs(ns, C):
     rng = np.random.default_rng(7)
-    ns, C = 6, 150
     R = np.stack([capi.trace_cov(make_traces(256, C, seed=20 + s), nsplit=2) for s in range(ns)])
     S = (rng.random((C, ns)) < 0.8).astype(np.uint8)
     S[1, :] = 0
@@ -117,3 +152,15 @@ def test_mean_corrs_matches_oracle():
     V1, W1 = capi.mean_corrs(R, S, [4, 9], 0.0, V0.copy() + 1.0, W0.copy())
     Vo, Wo = orc.mean_corrs(R, S, [4, 9], 0.0, V0.copy() + 1.0, W0.copy())
     assert np.allclose(V1, Vo, rtol=1e-12, atol=1e-14, equal_nan=True)
+
+
+def test_mean_corrs_matches_oracle():
+    _check_mean_corrs(6, 150)
+
+
+def test_mean_corrs_many_pairs_matches_oracle():
+    """C = 1600: C^2 = 2.56 M (row, column) pairs, more than twice what one pass of k_mean_corrs covers: min(pairs / 256,
+    148 * 32) CTAs of 256 threads (mmq_cov.cu:587)."""
+    C = 1600
+    assert C * C > 2 * 148 * 32 * 256
+    _check_mean_corrs(4, C)

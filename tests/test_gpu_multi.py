@@ -74,8 +74,12 @@ def test_two_ranks_reproduce_single_gpu_chain(use_p2p):
         assert np.array_equal(r[6], tr) and np.array_equal(r[7], c) and np.array_equal(r[8], mu_dbg)
 
 
-@pytest.mark.parametrize("weighted", [False, True])
-def test_single_process_peer_attach_matches_single_gpu(weighted):
+# padded: the length array has 3 x 189,440 + 77 transcripts, most of them without hits, so that the fused Gamma kernels
+# loop: k_gamma_p2p runs min(n / 256, 5 sms) CTAs and k_gamma_rs min(max(n / ranks, n / 8) / 256, 4 sms) CTAs of 256
+# threads (mmq_core.cu:1570,1575).  rs: mmq_tune knob 6, the reduce-scatter exchange (k_gamma_rs + k_trace_capture).
+@pytest.mark.parametrize("weighted,padded,rs", [(False, False, False), (True, False, False), (False, True, False), (True, True, True)],
+                         ids=["False", "True", "padded", "padded-rs"])
+def test_single_process_peer_attach_matches_single_gpu(weighted, padded, rs):
     """mmq_p2p_attach_local (what the host program uses for -gpus N): two handles in one process,
     sweeps issued from two threads; the fused peer-memory Gamma kernel gives the single-GPU chain.
     weighted = BASELINE config 4 at parity-test size: per-fragment shards with fp32 per-hit weights
@@ -89,14 +93,22 @@ def test_single_process_peer_attach_matches_single_gpu(weighted):
     h = hostlib.from_records(s.T, s.efflen, s.frag_ptr, s.frag_tid, frag_w=s.frag_w if weighted else None,
                              layout=hostlib.LAYOUT_PER_FRAGMENT_BY_LENGTH | hostlib.LAYOUT_HEADER_ORDER_COLUMNS)
     assert (h.w is not None) == weighted
+    length = h.len
+    if padded:
+        sms = torch.cuda.get_device_properties(0).multi_processor_count
+        length = np.concatenate([h.len, np.random.default_rng(1).uniform(1e-6, 1e-2, 3 * 189_440 + 77 - h.n)])
+        assert len(length) > 2.5 * sms * 5 * 256
     cut = [0, (h.m // 2) & ~1, h.m]
-    mu0 = np.random.default_rng(0).gamma(0.5, 50.0, h.n)
+    mu0 = np.random.default_rng(0).gamma(0.5, 50.0, len(length))
     hs = []
     for r in range(2):
         a, b = cut[r], cut[r + 1]
         lo, hi = h.row_ptr[a], h.row_ptr[b]
-        hs.append(capi.Handle(h.row_ptr[a:b + 1] - lo, h.col[lo:hi], None, h.len, weight=None if h.w is None else h.w[lo:hi], class_id_base=a, device=r))
+        hs.append(capi.Handle(h.row_ptr[a:b + 1] - lo, h.col[lo:hi], None, length, weight=None if h.w is None else h.w[lo:hi], class_id_base=a, device=r))
     capi.p2p_attach_local(hs)
+    if rs:
+        for H in hs:
+            H.tune(6, 1)
     out = [None, None]
 
     def run(r):
@@ -111,7 +123,7 @@ def test_single_process_peer_attach_matches_single_gpu(weighted):
         t.join()
     for H in hs:
         H.close()
-    with capi.Handle(h.row_ptr, h.col, None, h.len, weight=h.w) as H:
+    with capi.Handle(h.row_ptr, h.col, None, length, weight=h.w) as H:
         H.set_mu(mu0)
         H.gibbs(1234, 0, 40, stride=4, trace_len=10)
         tr, mu = H.get_trace(), H.get_mu()

@@ -8,6 +8,7 @@ from scipy import special
 
 from mmseq_b200 import capi
 from oracle import oracle as orc
+from tests.collapse_case import make_gene_problem
 
 pytestmark = pytest.mark.gpu
 GOLD = os.path.join(os.path.dirname(__file__), "golden", "sokal_golden.npz")
@@ -28,30 +29,31 @@ def test_sokal_kernel_matches_reference_golden():
 
 
 def test_sokal_batch_many_rows_vs_oracle():
+    """Every row, with more rows than one pass of the grid: mmq_sokal_batch runs k_row_sokal on min(rows, 148 * 8) CTAs,
+    one row per CTA and pass (mmq_post.cu:272)."""
+    rows = 4000
+    assert rows > 3 * 148 * 8
     rng = np.random.default_rng(2)
-    x = np.cumsum(rng.standard_normal((500, 1024)), axis=1) * 0.02 + rng.standard_normal((500, 1024))
+    x = np.cumsum(rng.standard_normal((rows, 1024)), axis=1) * 0.02 + rng.standard_normal((rows, 1024))
     var, tau, win, st = capi.sokal_batch(x)
-    for r in range(0, 500, 7):
+    for r in range(rows):
         rc, v, t, m = orc.sokal(x[r])
-        assert st[r] == rc == 0 and win[r] == m
-        assert np.isclose(var[r], v, rtol=1e-10) and np.isclose(tau[r], t, rtol=1e-9)
+        assert st[r] == rc == 0 and win[r] == m, r
+        assert np.isclose(var[r], v, rtol=1e-10) and np.isclose(tau[r], t, rtol=1e-9), r
 
 
-def test_summaries_groups_props_uh(small_problem, small_synth):
-    h, s = small_problem, small_synth
-    n, L, stride = h.n, 256, 2
-    P = orc.Problem(h.row_ptr, h.col, h.k, h.len)
+def _check_summaries_groups_props_uh(row_ptr, col, k, length, gene_of_col, G, ident_ptr, ident_mem, L, stride):
+    """Group traces, per-row summaries of transcripts, identical sets and genes, proportions and uh() of one handle against
+    the numpy/oracle restatements.  Genes are over observed columns, with an "extra" (prior-simulated) term for gene 3."""
+    n = len(length)
+    P = orc.Problem(row_ptr, col, k, length)
     mu0, _, _ = P.init_mu()
-    # genes over observed columns, plus an "extra" (prior-simulated) term for one gene
-    gene_of_col = s.gene_of[h.col2hdr]
-    G = s.G
     order = np.argsort(gene_of_col, kind="stable")
     gptr = np.concatenate([[0], np.cumsum(np.bincount(gene_of_col, minlength=G))])
     members = order.astype(np.int32)
     rng = np.random.default_rng(4)
     extra = np.zeros((G, L)); extra[3] = rng.gamma(0.1, 5.0, L)
-    ident_ptr = np.array([0, 2, 5]); ident_mem = np.array([0, 1, 4, 5, 6], np.int32)
-    with capi.Handle(h.row_ptr, h.col, h.k, h.len) as H:
+    with capi.Handle(row_ptr, col, k, length) as H:
         H.set_mu(mu0)
         H.gibbs(1234, 0, L * stride, stride=stride, trace_len=L)
         tr = H.get_trace()
@@ -70,7 +72,8 @@ def test_summaries_groups_props_uh(small_problem, small_synth):
     # group traces
     gt_o = np.zeros((G, L)); np.add.at(gt_o, gene_of_col, tr); gt_o += extra
     assert np.allclose(gt, gt_o, rtol=1e-13)
-    assert np.allclose(it[0], tr[0] + tr[1], rtol=1e-14) and np.allclose(it[1], tr[4] + tr[5] + tr[6], rtol=1e-14)
+    it_o = np.zeros((len(ident_ptr) - 1, L)); np.add.at(it_o, np.repeat(np.arange(len(ident_ptr) - 1), np.diff(ident_ptr)), tr[ident_mem])
+    assert np.allclose(it, it_o, rtol=1e-14)
     # per-row summaries vs the numpy/oracle restatement
     for S, trace in ((S0, tr), (S1, it), (S2, gt)):
         O = orc.summaries_transcripts(trace)
@@ -92,8 +95,28 @@ def test_summaries_groups_props_uh(small_problem, small_synth):
     assert np.all(np.isinf(PR["sum_probit"][~m]))                  # single-isoform genes: +inf (src/mmseq.cpp:1252)
     assert np.array_equal(PR["pct"], np.sort(prop, axis=1)[:, pct_idx])
     # uh(): literal restatement of src/uh.cpp on the same sets
-    uh_o = orc.uh_literal(h.row_ptr, h.col, h.k, gptr, members)
+    uh_o = orc.uh_literal(row_ptr, col, k, gptr, members)
     assert np.array_equal(uh, uh_o)
+
+
+def test_summaries_groups_props_uh(small_problem, small_synth):
+    h, s = small_problem, small_synth
+    _check_summaries_groups_props_uh(h.row_ptr, h.col, h.k, h.len, s.gene_of[h.col2hdr], s.G,
+                                     np.array([0, 2, 5]), np.array([0, 1, 4, 5, 6], np.int32), L=256, stride=2)
+
+
+@pytest.mark.parametrize("L", [4, 2048])
+def test_summaries_groups_props_uh_many_rows(L):
+    """The checks of test_summaries_groups_props_uh with more transcripts, genes and identical sets than one pass of each
+    grid covers, at the shortest and the longest trace mmq_summarize accepts (4 and MMQ_MAX_ROW_LEN = 2048)."""
+    import torch
+    sms = torch.cuda.get_device_properties(0).multi_processor_count
+    row_ptr, col, k, length, gene_of, ident_ptr, ident_mem = make_gene_problem()
+    n, G, I = len(length), int(gene_of.max()) + 1, len(ident_ptr) - 1
+    assert min(n, G, I) > 4 * 148 * 8        # k_row_sokal, k_row_percentiles (mmq_post.cu:272,283): min(rows, 148 * 8) CTAs
+    assert n > 4 * sms * 8                   # k_prop (mmq_post.cu:386): min(n, sms * 8) CTAs, one transcript per CTA pass
+    assert min(G, I) > 2 * sms * 16          # k_group_trace (mmq_post.cu:248): min(groups, sms * 16) CTAs
+    _check_summaries_groups_props_uh(row_ptr, col, k, length, gene_of, G, ident_ptr, ident_mem, L=L, stride=2 if L == 4 else 1)
 
 
 def test_prior_draws_bit_exact_and_distributed():
