@@ -821,6 +821,8 @@ void ClassBuilder::finish(HitClasses& out) {
   out.hdr2col = P.hdr2col;
   out.doublehits = P.doublehits;
   out.w.clear();
+  out.set_ptr.clear(); out.set_col.clear(); out.set_k.clear();
+  out.first_zero_weight_record = -1;
   if (P.layout == LAYOUT_COLLAPSED) {
     out.m = out.n_classes;
     out.row_ptr.swap(P.cls_ptr);
@@ -894,21 +896,32 @@ void ClassBuilder::finish(HitClasses& out) {
   if (P.weighted) out.w.resize((size_t)total);
   {
     const int W = (int)std::max(1u, std::min(16u, std::thread::hardware_concurrency()));
+    std::vector<int64_t> zero_rec((size_t)W, R); /* per thread: first record whose weights are all zero */
     auto copy = [&](int w) {
       for (int64_t i = R * w / W; i < R * (w + 1) / W; ++i) {
         const int64_t r = order[(size_t)i];
         const int32_t c = P.rec_class[(size_t)r];
         const int64_t b = P.cls_ptr[(size_t)c], d = P.cls_ptr[(size_t)c + 1] - b;
         std::memcpy(out.col.data() + out.row_ptr[(size_t)i], P.cls_col.data() + b, sizeof(int32_t) * (size_t)d);
-        if (P.weighted) std::memcpy(out.w.data() + out.row_ptr[(size_t)i], P.rec_w.data() + P.rec_wptr[(size_t)r], sizeof(float) * (size_t)d);
+        if (P.weighted) {
+          const float* wr = P.rec_w.data() + P.rec_wptr[(size_t)r];
+          std::memcpy(out.w.data() + out.row_ptr[(size_t)i], wr, sizeof(float) * (size_t)d);
+          if (r < zero_rec[(size_t)w] && std::all_of(wr, wr + d, [](float x) { return x == 0.f; })) zero_rec[(size_t)w] = r;
+        }
       }
     };
     std::vector<std::thread> th;
     for (int w = 1; w < W; ++w) th.emplace_back(copy, w);
     copy(0);
     for (auto& t : th) t.join();
+    const int64_t z = *std::min_element(zero_rec.begin(), zero_rec.end());
+    if (z < R) out.first_zero_weight_record = z;
   }
   tick("rows copied");
+  /* the sets the rows were built from, for what is defined per set (.k, .M, unique hits) */
+  out.set_ptr.swap(P.cls_ptr);
+  out.set_col.swap(P.cls_col);
+  out.set_k.swap(P.cls_k);
 }
 
 /* ------------------------------------------------------------------ header */
@@ -1011,7 +1024,7 @@ double parse_double_like_istream(const std::string& s) { /* string_to_double, sr
 
 }  // namespace
 
-int load_hits_file(const std::string& path, int layout, HitsHeader& hdr, HitClasses& cls, std::string& err) {
+int load_hits_file(const std::string& path, int layout, HitsHeader& hdr, HitClasses& cls, std::string& err, int weighted_layout) {
   ByteSource src;
   const double t_open0 = std::chrono::duration<double>(std::chrono::steady_clock::now().time_since_epoch()).count();
   if (!src.open(path)) { err = "Error reading hits file \"" + path + "\"."; return 1; }
@@ -1108,6 +1121,7 @@ int load_hits_file(const std::string& path, int layout, HitsHeader& hdr, HitClas
   auto now = [] { return std::chrono::duration<double>(std::chrono::steady_clock::now().time_since_epoch()).count(); };
   const double t_hdr = now();
   if (timing) fprintf(stderr, "[loader] open%s + header %.2f s\n", src.whole() ? " (file inflated on all threads)" : "", t_hdr - t_open0);
+  if (hdr.schema == 2 && weighted_layout >= 0) layout = weighted_layout;
   if (hdr.schema == 2 && (layout & 15) == LAYOUT_COLLAPSED) {
     err = "Error: \"" + path + "\" carries per-hit weights (schema 2): it needs a per-fragment layout.";
     return 1;
@@ -1350,6 +1364,8 @@ int64_t mmqh_dim(const mmqh_hits* H, int which) {
     case 6: return (int64_t)H->cls.col.size();
     case 7: return H->cls.n_classes;
     case 8: return H->hdr.schema;
+    case 9: return (int64_t)H->cls.set_col.size();
+    case 10: return H->cls.first_zero_weight_record;
     default: return -1;
   }
 }
@@ -1357,6 +1373,9 @@ const int64_t* mmqh_row_ptr(const mmqh_hits* H) { return H->cls.row_ptr.data(); 
 const int32_t* mmqh_col(const mmqh_hits* H) { return H->cls.col.data(); }
 const int32_t* mmqh_k(const mmqh_hits* H) { return H->cls.k.empty() ? nullptr : H->cls.k.data(); }
 const float* mmqh_w(const mmqh_hits* H) { return H->cls.w.empty() ? nullptr : H->cls.w.data(); }
+const int64_t* mmqh_set_ptr(const mmqh_hits* H) { return H->cls.set_ptr.empty() ? nullptr : H->cls.set_ptr.data(); }
+const int32_t* mmqh_set_col(const mmqh_hits* H) { return H->cls.set_ptr.empty() ? nullptr : H->cls.set_col.data(); }
+const int32_t* mmqh_set_k(const mmqh_hits* H) { return H->cls.set_ptr.empty() ? nullptr : H->cls.set_k.data(); }
 const int32_t* mmqh_col2hdr(const mmqh_hits* H) { return H->cls.col2hdr.data(); }
 const int32_t* mmqh_hdr2col(const mmqh_hits* H) { return H->cls.hdr2col.data(); }
 const int32_t* mmqh_doublehits(const mmqh_hits* H) { return H->cls.doublehits.data(); }

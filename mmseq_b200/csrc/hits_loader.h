@@ -60,10 +60,23 @@ struct HitClasses {
   std::vector<int32_t> k;      /* empty in the per-fragment layouts */
   std::vector<float> w;        /* empty without per-hit weights */
   std::vector<int32_t> col2hdr, hdr2col, doublehits;
+  /* per-fragment layouts: the distinct sets behind the rows, in first-appearance order — what a
+   * LAYOUT_COLLAPSED load of the same records returns as row_ptr / col / k (.k, .M, unique hits).
+   * Empty in the collapsed layout, whose rows are the sets. */
+  std::vector<int64_t> set_ptr;
+  std::vector<int32_t> set_col;
+  std::vector<int32_t> set_k;
+  /* weighted per-fragment layouts: the first record (0-based, record order) whose weights are all
+   * zero — its likelihood is 0 under every mu — or -1 */
+  int64_t first_zero_weight_record = -1;
 };
 
-/* Both return 0 on success; on failure err holds the reference's message where it has one. */
-int load_hits_file(const std::string& path, int layout, HitsHeader& hdr, HitClasses& cls, std::string& err);
+/* Both return 0 on success; on failure err holds the reference's message where it has one.
+ * weighted_layout >= 0: the layout a file with per-hit weights (schema 2) is loaded in instead of
+ * `layout`; hdr.schema tells the caller which one it got.  -1: such a file is loaded in `layout`,
+ * which must then be a per-fragment one. */
+int load_hits_file(const std::string& path, int layout, HitsHeader& hdr, HitClasses& cls, std::string& err,
+                   int weighted_layout = -1);
 int validate_header(const HitsHeader& hdr, std::string& err);
 
 /* Streaming class builder (also the in-memory entry point used by the harness). */

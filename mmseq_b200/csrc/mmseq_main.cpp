@@ -251,14 +251,21 @@ static void run_sample(const Options& o, const string& hits_file, const string& 
   /* the CUDA contexts come up (1-2 s) while the hits file is being parsed */
   thread warmup([ngpus, first_device] { for (int g = 0; g < ngpus; ++g) mmq_warmup(first_device + g); });
 
-  /* ---- load: header + records -> hit classes (src/hitsio.cpp, src/mmseq.cpp:312-441) */
+  /* ---- load: header + records -> hit classes (src/hitsio.cpp, src/mmseq.cpp:312-441).  A file with per-hit
+   * weights (schema 2) cannot be collapsed: two fragments with the same transcript set differ in their weights.
+   * It is loaded one row per fragment, grouped by set size and set (the segment kernel's layout), and the loader
+   * also returns the distinct sets, from which .k, .M and the debug files are written as for an unweighted file. */
   mmq::HitsHeader hdr;
   mmq::HitClasses cls;
   {
     string err;
-    if (mmq::load_hits_file(hits_file, mmq::LAYOUT_COLLAPSED, hdr, cls, err)) { warmup.join(); die(err); }
+    if (mmq::load_hits_file(hits_file, mmq::LAYOUT_COLLAPSED, hdr, cls, err, mmq::LAYOUT_PER_FRAGMENT_BY_LENGTH)) { warmup.join(); die(err); }
   }
   warmup.join();
+  const bool weighted = hdr.schema == 2;
+  if (cls.first_zero_weight_record >= 0) /* its likelihood term is log 0: EM would turn mu into NaN */
+    die("Error: fragment record " + to_string(cls.first_zero_weight_record + 1) + " of \"" + hits_file +
+        "\" has per-hit weights that are all zero: its likelihood is zero whatever the abundances.");
   out << "Running mmseq with parameters:\n"
        << "  alpha:         " << alpha << endl
        << "  beta:          " << beta << endl
@@ -270,13 +277,18 @@ static void run_sample(const Options& o, const string& hits_file, const string& 
        << "  debug:         " << debug << endl
        << "  threads:       " << ngpus << " GPU(s)" << endl;
   const int64_t T = (int64_t)hdr.names.size();
-  const int64_t n = cls.n, m = cls.m;
+  const int64_t n = cls.n, m = cls.m; /* m: rows on the GPUs (sets, or fragments of a weighted file) */
   const int64_t N = cls.N;
   const int64_t G = (int64_t)hdr.gene_names.size(), I = (int64_t)hdr.identical.size();
   const int L = trace_length;
+  /* the distinct transcript sets in first-appearance order, with their fragment counts */
+  const vector<int64_t>& set_ptr = weighted ? cls.set_ptr : cls.row_ptr;
+  const vector<int32_t>& set_col = weighted ? cls.set_col : cls.col;
+  const vector<int32_t>& set_k = weighted ? cls.set_k : cls.k;
+  const int64_t n_sets = weighted ? cls.n_classes : m;
   phase("hits file loaded");
-  out << "Found " << n << " transcripts in " << m << " transcript combinations.\r" << endl;
-  if (n == 0 || m == 0) die("Error: no mapped fragments in the hits file.");
+  out << "Found " << n << " transcripts in " << n_sets << " transcript combinations.\r" << endl;
+  if (n == 0 || n_sets == 0) die("Error: no mapped fragments in the hits file.");
 
   vector<double> l;
   {
@@ -288,7 +300,10 @@ static void run_sample(const Options& o, const string& hits_file, const string& 
    * host hands them over as they are: one GPU takes the loader's arrays in place; several GPUs take
    * every ngpus-th class (first-appearance order is unrelated to the cost of a class, so the deal is
    * an equal mix).  The Philox counter of a class is its first-appearance index either way
-   * (mmq_problem.class_id): the chain does not depend on the number of GPUs. */
+   * (mmq_problem.class_id): the chain does not depend on the number of GPUs.
+   * The fragment rows of a weighted file (k = NULL, where explicit class ids are not accepted) are cut
+   * into contiguous ranges with equal numbers of hits instead; the Philox counter of a row is its index
+   * in the whole row order (mmq_problem.class_id_base), so again the chain does not depend on the cut. */
   vector<Shard> shards((size_t)ngpus);
   vector<vector<int64_t>> shard_rp((size_t)ngpus), shard_id((size_t)ngpus);
   vector<vector<int32_t>> shard_col((size_t)ngpus), shard_k((size_t)ngpus);
@@ -298,7 +313,24 @@ static void run_sample(const Options& o, const string& hits_file, const string& 
     mmq_problem p;
     memset(&p, 0, sizeof p);
     p.n = n;
-    if (ngpus == 1) {
+    if (weighted) {
+      const int64_t nnz = cls.row_ptr[(size_t)m];
+      auto row_at = [&](int64_t gi) { /* first row whose hits start at or after gi/ngpus of all hits */
+        if (gi == ngpus) return m;
+        return (int64_t)(lower_bound(cls.row_ptr.begin(), cls.row_ptr.begin() + m, nnz * gi / ngpus) - cls.row_ptr.begin());
+      };
+      const int64_t r0 = row_at(g), r1 = row_at(g + 1), q0 = cls.row_ptr[(size_t)r0];
+      auto& rp = shard_rp[(size_t)g];
+      rp.resize((size_t)(r1 - r0 + 1));
+      for (int64_t i = r0; i <= r1; ++i) rp[(size_t)(i - r0)] = cls.row_ptr[(size_t)i] - q0;
+      p.m = r1 - r0; p.nnz = rp.back();
+      p.row_ptr = rp.data();
+      p.col = cls.col.data() + q0;
+      p.weight = cls.w.data() + q0;
+      p.k = nullptr;
+      p.class_id = nullptr;
+      p.class_id_base = r0;
+    } else if (ngpus == 1) {
       p.m = m; p.nnz = cls.row_ptr[(size_t)m];
       p.row_ptr = cls.row_ptr.data();
       p.col = cls.col.data();
@@ -323,9 +355,8 @@ static void run_sample(const Options& o, const string& hits_file, const string& 
       p.class_id = id.data();
     }
     S.row0 = 0; S.row1 = p.m;
-    p.weight = nullptr;
     p.len = l.data();
-    p.alpha = alpha; p.beta = beta; p.class_id_base = 0;
+    p.alpha = alpha; p.beta = beta;
     int rc = mmq_create(&p, S.device, &S.h);
     if (rc) die(string("Error: mmq_create: ") + mmq_last_error(nullptr));
   }
@@ -395,13 +426,13 @@ static void run_sample(const Options& o, const string& hits_file, const string& 
       for (const string& blk : part) fwrite(blk.data(), 1, blk.size(), f);
       fclose(f);
     };
-    write_blocks(output_base + ".k", "", m, [&](string& out, int64_t i) { put_int(out, cls.k[(size_t)i]); out.push_back('\n'); });
+    write_blocks(output_base + ".k", "", n_sets, [&](string& out, int64_t i) { put_int(out, set_k[(size_t)i]); out.push_back('\n'); });
     string head = "#";
     for (int64_t t = 0; t < n; t++) { head += "\t"; head += hdr.names[(size_t)cls.col2hdr[(size_t)t]]; }
     head += "\n";
-    write_blocks(output_base + ".M", head, m, [&](string& out, int64_t i) {
-      for (int64_t q = cls.row_ptr[(size_t)i]; q < cls.row_ptr[(size_t)i + 1]; ++q) {
-        put_int(out, i); out.push_back('\t'); put_int(out, cls.col[(size_t)q]); out.push_back('\n');
+    write_blocks(output_base + ".M", head, n_sets, [&](string& out, int64_t i) {
+      for (int64_t q = set_ptr[(size_t)i]; q < set_ptr[(size_t)i + 1]; ++q) {
+        put_int(out, i); out.push_back('\t'); put_int(out, set_col[(size_t)q]); out.push_back('\n');
       }
     });
   }
@@ -410,10 +441,10 @@ static void run_sample(const Options& o, const string& hits_file, const string& 
   phase(".k and .M written");
   if (debug) { /* src/mmseq.cpp:697-731 */
     vector<vector<int>> counts_shared((size_t)n, vector<int>(100, 0));
-    for (int64_t i = 0; i < m; ++i) {
-      const int64_t d = cls.row_ptr[(size_t)i + 1] - cls.row_ptr[(size_t)i];
-      for (int64_t q = cls.row_ptr[(size_t)i]; q < cls.row_ptr[(size_t)i + 1]; ++q)
-        counts_shared[(size_t)cls.col[(size_t)q]][(size_t)min<int64_t>(d, 100) - 1] += cls.k[(size_t)i];
+    for (int64_t i = 0; i < n_sets; ++i) {
+      const int64_t d = set_ptr[(size_t)i + 1] - set_ptr[(size_t)i];
+      for (int64_t q = set_ptr[(size_t)i]; q < set_ptr[(size_t)i + 1]; ++q)
+        counts_shared[(size_t)set_col[(size_t)q]][(size_t)min<int64_t>(d, 100) - 1] += set_k[(size_t)i];
     }
     ofs.open((output_base + ".sharedcounts").c_str());
     for (int64_t hI = 0; hI < T; ++hI) {
@@ -428,8 +459,8 @@ static void run_sample(const Options& o, const string& hits_file, const string& 
     ofs.close(); ofs.clear();
     /* Mt rows (transcripts) equal to the previous row are listed in .dupIDs, the others dumped */
     vector<vector<int32_t>> Mt((size_t)n);
-    for (int64_t i = 0; i < m; ++i)
-      for (int64_t q = cls.row_ptr[(size_t)i]; q < cls.row_ptr[(size_t)i + 1]; ++q) Mt[(size_t)cls.col[(size_t)q]].push_back((int32_t)i);
+    for (int64_t i = 0; i < n_sets; ++i)
+      for (int64_t q = set_ptr[(size_t)i]; q < set_ptr[(size_t)i + 1]; ++q) Mt[(size_t)set_col[(size_t)q]].push_back((int32_t)i);
     ofs.open((output_base + ".Mt-nodups").c_str());
     ofstream ofs2((output_base + ".dupIDs").c_str());
     for (int64_t t = 0; t < n; ++t) {
@@ -495,7 +526,7 @@ static void run_sample(const Options& o, const string& hits_file, const string& 
     out << endl;
     const double sec = chrono::duration<double>(chrono::steady_clock::now() - t0).count();
     err << "Gibbs: " << gibbs_iter << " sweeps in " << sec << " s (" << gibbs_iter / sec << " sweeps/s, " << (double)m * gibbs_iter / sec
-         << " hit-class allocations/s)" << endl;
+         << (weighted ? " fragment allocations/s)" : " hit-class allocations/s)") << endl;
   }
 
   phase("EM + Gibbs");

@@ -42,7 +42,7 @@ def lib():
         L.mmqh_free.argtypes = [vp]
         L.mmqh_dim.restype = i64
         L.mmqh_dim.argtypes = [vp, i32]
-        for nm in ["row_ptr", "col", "k", "w", "col2hdr", "hdr2col", "doublehits", "efflen", "truelen", "gene_of",
+        for nm in ["row_ptr", "col", "k", "w", "set_ptr", "set_col", "set_k", "col2hdr", "hdr2col", "doublehits", "efflen", "truelen", "gene_of",
                    "gene_ptr", "gene_members", "ident_ptr", "ident_members"]:
             f = getattr(L, "mmqh_" + nm)
             f.restype = vp
@@ -75,6 +75,13 @@ class Hits:
         self.col = _arr(L.mmqh_col(handle), self.nnz, np.int32)
         self.k = _arr(L.mmqh_k(handle), self.m, np.int32)
         self.w = _arr(L.mmqh_w(handle), self.nnz, np.float32)
+        # per-fragment layouts: the distinct sets behind the rows, as a LAYOUT_COLLAPSED load returns
+        # them in row_ptr / col / k (None in the collapsed layout)
+        self.set_ptr = _arr(L.mmqh_set_ptr(handle), self.n_classes + 1, np.int64)
+        self.set_col = _arr(L.mmqh_set_col(handle), d(9), np.int32)
+        self.set_k = _arr(L.mmqh_set_k(handle), self.n_classes, np.int32)
+        # weighted per-fragment layouts: first record (0-based) whose weights are all zero, or -1
+        self.first_zero_weight_record = d(10)
         self.col2hdr = _arr(L.mmqh_col2hdr(handle), self.n, np.int32)
         self.hdr2col = _arr(L.mmqh_hdr2col(handle), self.T, np.int32)
         self.doublehits = _arr(L.mmqh_doublehits(handle), self.n, np.int32)
