@@ -226,8 +226,16 @@ int mmq_sokal_batch(int device, int64_t rows, int len, const double* x, double* 
 
 /* ---- the consumer of the traces: mmcollapse's covariance step (src/mmcollapse.cpp:483-561) ----------
  * The one dense contraction of the package: tensor cores (tcgen05, bf16 split products, fp32 accumulation in
- * TMEM), everything around it fp64.  nsplit = bf16 terms per value: 1 (|dr| <~ 4e-3 in correlation units),
- * 2 (<~ 2e-5, the default of the callers here), 3 (<~ 2e-6). */
+ * TMEM), everything around it fp64.  nsplit = bf16 terms per value (2: the default of the callers here).  Error in
+ * correlation units, |cov - cov_exact| / (sd_i sd_j), for traces of length L: at most A + 1.5e-8 L with A = 6e-3 /
+ * 1.2e-5 / 2e-7 for nsplit = 1 / 2 / 3.  A is the bf16 split; 1.5e-8 L is the fp32 accumulation, which truncates
+ * towards zero (|r| comes out a little small) and so grows linearly with L.  At L = 1024: 6e-3 / 2.7e-5 / 1.6e-5; at
+ * the longest L, 65536: 7e-3 / 1e-3 / 1e-3.  (Fitted with a margin of 1.5x or more over the largest error measured on
+ * a B200, tests/collapse_case.py.)
+ * A feature whose centred sum of squares is not finite (a non-finite value, or |x - mean| of ~1e154 and more) gets a
+ * zero row and column, its variance included.  Armadillo's cov() keeps the finite off-diagonal entries of such a
+ * feature, but mmcollapse divides them by its variance, which :556-558 sets to 0: its correlations are not finite
+ * either way. */
 
 /* get_corrs()'s per-sample step, src/mmcollapse.cpp:553-558: R = cov(M) of the L x C trace matrix (column c =
  * the L posterior draws of feature c, contiguous: Armadillo's layout of myM and the layout of mmq_get_trace),

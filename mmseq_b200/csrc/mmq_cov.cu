@@ -25,9 +25,13 @@
  *                a + b < nsplit are extra K-segments of the same accumulation (smallest terms first).
  *   k_mean_corrs the scan over samples, one thread per (row of ts, column) pair.
  *
- * Accuracy (measured, correlation units |cov_gpu - cov_fp64| / (sd_i sd_j), L = 1024): nsplit = 1: 3e-4, 2: 5e-6 (the
- * default), 3: 2e-6 (the floor of fp32 accumulation) — against a Monte-Carlo error of a correlation estimated from 1024
- * draws of >= 1e-2.  The tests state the tolerances.
+ * Accuracy, in correlation units |cov_gpu - cov_exact| / (sd_i sd_j), for traces of length L: at most A + 1.5e-8 L, A =
+ * 6e-3 / 1.2e-5 / 2e-7 for nsplit = 1 / 2 (the default) / 3 (include/mmq.h; tests/test_gpu_cov_accuracy.py asserts it
+ * at L = 64 .. 65536).  A is the bf16 split, each term keeping 8 significant bits of what the previous ones left.  The
+ * L term is the fp32 accumulation in TMEM: the tensor cores truncate the running sum towards zero, L / 16 times per
+ * split product, so the error is a bias towards r = 0 that grows linearly with L, largest for a near-collinear pair
+ * whose sum reaches |r| ~ 1 early.  At mmcollapse's L = 1024 that is 2.7e-5 for nsplit = 2, against a Monte-Carlo
+ * error of a correlation estimated from 1024 draws of >= 1e-2.
  *
  * What bounds it: 0.91-0.93 ms at C = 16384, nsplit = 2 (0.54 of the measured cuBLAS bf16 peak; 0.66 with nsplit = 3).
  * Per MMA an SM reads 8 KB of operands from shared memory and receives 32 KB of TMA writes per stage, where one CTA alone

@@ -1,8 +1,69 @@
 """Shared inputs of the mmcollapse-covariance tests: trace matrices shaped like the posterior traces of collapse candidates
 (raw-scale mu: log-normal levels over several orders of magnitude, blocks of anti-correlated features as unidentifiable
-transcripts produce, a few exactly duplicated and a few tiny-variance columns) and a literal numpy transcription of
-src/mmcollapse.cpp:483-511."""
+transcripts produce, a few exactly duplicated and a few tiny-variance columns), a literal numpy transcription of
+src/mmcollapse.cpp:483-511, an exact fp64 covariance and the covariance kernel's error bound."""
+import math
+
 import numpy as np
+
+# k_cov_gemm2's error bound in correlation units, |cov_gpu - cov_exact| / (sd_i sd_j), for nsplit bf16 terms per value
+# and trace length L; include/mmq.h states the same.  COV_A[nsplit] is the bf16 split: each term keeps 8 significant bits
+# of what the previous ones left.  COV_B * L is the fp32 accumulation in TMEM, which truncates towards zero: the error is
+# a bias towards r = 0 that grows linearly with L (L / 16 MMA steps per split product).  Fitted on one B200 (1000 W) to
+# the largest error of tests/test_gpu_cov_accuracy.py at each (nsplit, L), L = 64 .. 65536, and to 2.0e-5 measured on chain
+# traces at nsplit = 3, L = 2048: at least 1.5x that error everywhere (nsplit = 1 at L = 1024: 4.0e-3 on chain traces;
+# nsplit = 2 at L = 1024: 1.66e-5 on chain traces, L = 64: 7.5e-6 at C = 47104; at L = 65536 about 3.4e-4, 2.9x).
+COV_A = {1: 6e-3, 2: 1.2e-5, 3: 2e-7}
+COV_B = 1.5e-8
+
+
+def cov_bound(nsplit, L):
+    return COV_A[nsplit] + COV_B * L
+
+
+def corr_err(R, ref):
+    """max |R - ref| / (sd_i sd_j), sd from the reference's diagonal (1 where it is 0)."""
+    d = np.sqrt(np.diag(ref))
+    d = np.where(d > 0, d, 1.0)
+    return np.max(np.abs(R - ref) / (d[:, None] * d[None, :]))
+
+
+def exact_cov(M, fsum_mean=False):
+    """Two-pass centred fp64 covariance of the L x C matrix M (column = feature), non-finite entries -> 0 as
+    src/mmcollapse.cpp:556-558.  The centring of x against an fp64 mean is exact wherever |x - mean| <= |mean| (Sterbenz),
+    so what is left is the fp64 dot products: ~1e-13 relative to sd_i sd_j at L = 65536.  fsum_mean: the means by
+    math.fsum (correctly rounded), for columns whose mean is many orders above their spread."""
+    M = np.asarray(M, np.float64)
+    L = M.shape[0]
+    if fsum_mean:
+        mean = np.array([math.fsum(M[:, c]) / L for c in range(M.shape[1])])
+    else:
+        mean = M.mean(axis=0)
+    X = M - mean
+    with np.errstate(all="ignore"):
+        R = (X.T @ X) / max(L - 1, 1)
+    R[~np.isfinite(R)] = 0.0
+    return R
+
+
+def mean_corrs_rows(Rt, D, S, ts, sdpenalty=0.0):
+    """mean_corrs_numpy for the rows ts only, vectorised: Rt[s, i, v] = R[s, ts[i], v], D[s, v] = R[s, v, v].  Returns the
+    rows V[ts, :], W[ts, :]."""
+    ns = Rt.shape[0]
+    ts = np.asarray(ts)
+    with np.errstate(all="ignore"):
+        r = Rt / np.sqrt(D[:, ts])[:, :, None]
+        r = r / np.sqrt(D)[:, None, :]
+        u = (S[ts, :].T.astype(np.int64)[:, :, None] * S.T.astype(np.int64)[:, None, :]).astype(np.float64)
+        r = np.where(u == 0, 0.0, r)
+        n = u.sum(axis=0)
+        mean = (u * r).sum(axis=0) / n
+        if ns > 1:
+            sd = np.sqrt((n / (n - 1.0)) * ((u * r * r).sum(axis=0) / n - mean * mean))
+            sd = np.where(np.isfinite(sd), sd, 0.0)
+        else:
+            sd = np.zeros_like(mean)
+    return mean + sdpenalty * sd, sd
 
 
 def make_traces(L, C, seed=0, blocks=True):

@@ -4,7 +4,7 @@ src/mmcollapse.cpp:483-511.  CPU only."""
 import numpy as np
 
 from oracle import oracle as orc
-from tests.collapse_case import make_traces, mean_corrs_numpy
+from tests.collapse_case import exact_cov, make_traces, mean_corrs_numpy, mean_corrs_rows
 
 
 def test_cov_matches_numpy_cov():
@@ -68,3 +68,37 @@ def test_single_sample_has_zero_sd():
     V, W = orc.mean_corrs(R, np.ones((6, 1), np.uint8), np.arange(6))
     d = np.sqrt(np.diag(R[0]))
     assert np.allclose(V, R[0] / d[:, None] / d[None, :], rtol=1e-13) and np.all(W == 0)
+
+
+def test_exact_cov_matches_the_oracle():
+    """exact_cov, the reference of tests/test_gpu_cov_accuracy.py, is cov() with non-finite entries 0; its fsum means agree
+    with numpy's where the mean is 1e8 times the spread."""
+    M = make_traces(1024, 61, seed=3)
+    M[3, 5] = np.nan
+    R = exact_cov(M)
+    ref = orc.trace_cov(M)
+    d = np.sqrt(np.diag(ref))
+    d = np.where(d > 0, d, 1.0)
+    assert np.max(np.abs(R - ref) / (d[:, None] * d[None, :])) < 1e-13
+    assert np.all(R[5, :] == 0) and np.all(R[:, 5] == 0)
+    G = M[:, :4] - M[:, :4].mean(axis=0)
+    Rb = exact_cov(G + 1e8 * G.std(axis=0), fsum_mean=True)
+    d = np.sqrt(np.diag(Rb))
+    assert np.max(np.abs(Rb - exact_cov(G)) / (d[:, None] * d[None, :])) < 1e-9
+
+
+def test_mean_corrs_rows_matches_the_literal_transcription():
+    rng = np.random.default_rng(8)
+    ns, C = 4, 19
+    R = np.stack([orc.trace_cov(make_traces(256, C, seed=30 + s)) for s in range(ns)])
+    S = (rng.random((C, ns)) < 0.7).astype(np.uint8)
+    S[1, :] = 0
+    S[2, :] = 0
+    S[2, 3] = 1
+    ts = np.array([0, 1, 2, 7, C - 1])
+    D = np.stack([np.diag(R[s]) for s in range(ns)])
+    for pen in (0.0, 0.5):
+        V, W = mean_corrs_numpy(R, S, ts, pen)
+        Vr, Wr = mean_corrs_rows(R[:, ts, :], D, S, ts, pen)
+        assert np.allclose(Vr, V[ts], rtol=1e-13, atol=1e-15, equal_nan=True)
+        assert np.allclose(Wr, W[ts], rtol=1e-12, atol=1e-15, equal_nan=True)
