@@ -173,6 +173,28 @@ int mmq_kernel_times(mmq_handle* h, double* alloc_ms, int64_t* alloc_launches, d
 int mmq_sweep_debug(mmq_handle* h, uint32_t seed, int64_t sweep, int flags, int32_t* x_out,
                     int32_t* counts_out, double* mu_out);
 
+/* ---- posterior fragment counts per transcript, identical set and gene ----------------------------------
+ * (none — the reference reports log_mu and unique hits only; these are the counts Salmon's NumReads, kallisto's
+ * est_counts and RSEM's expected_count give.)  c_t(s) is the count of transcript t that the Gamma step of sweep s
+ * uses (Xcolsum, src/mmseq.cpp:895-899, singleton classes and all shards included); a group's count is the sum of its
+ * members' counts within the sweep, so its variance is not derived from theirs.
+ *
+ * Start (or restart) accumulating: zeroes the accumulators; every later sweep (mmq_gibbs, graph or not, and
+ * mmq_sweep_debug) adds c and c^2 of every row, as exact integers.  ident_of / gene_of: int32[n], the identical set /
+ * gene of each observed transcript or -1 (may be NULL when the group count is 0).  Call it with the same arguments on
+ * every rank; no communication is added.  mmq_gibbs refuses to accumulate under mmq_tune knob 6 (MMQ_ERR_STATE). */
+int mmq_count_moments_begin(mmq_handle* h, const int32_t* ident_of, int64_t n_ident, const int32_t* gene_of, int64_t n_gene);
+/* Stop accumulating and free the accumulators. */
+int mmq_count_moments_end(mmq_handle* h);
+/* which: 0 transcripts (n rows), 1 identical sets, 2 genes.  sweeps: sweeps accumulated (S); sum u64[rows] = sum_s c;
+ * sumsq_lo / sumsq_hi u64[rows]: the low and high words of the 128-bit sum_s c^2.  Any output may be NULL.
+ * Posterior mean sum / S; sd sqrt((S sumsq - sum^2) / (S (S - 1))) (the S - 1 of src/sokal.cc:63), 0 when S < 2. */
+int mmq_get_count_moments(mmq_handle* h, int which, int64_t* sweeps, uint64_t* sum, uint64_t* sumsq_lo, uint64_t* sumsq_hi);
+/* EM expected counts: one E-step at the current mu, src/mmseq.cpp:781-794: out[t] = mu[t] * sum_{i containing t}
+ * k[i] w[i,t] / D_i with D_i = sum_{s in i} mu[s] w[i,s] (w = 1 without weights), summed over all shards (the fp64
+ * all-reduce of mmq_em).  sum_t out[t] = N up to rounding.  out fp64[n].  Leaves mu unchanged. */
+int mmq_expected_counts(mmq_handle* h, double* out);
+
 /* trace_out[t*trace_len + s] = mu[t] at slot s — the layout of mu_trace,
  * src/mmseq.cpp:827, :914. */
 int mmq_get_trace(mmq_handle* h, double* trace_out);

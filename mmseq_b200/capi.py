@@ -65,6 +65,10 @@ def _load():
         "mmq_kernel_times": (i32, [vp, C.POINTER(dbl), C.POINTER(i64), C.POINTER(dbl), C.POINTER(i64)]),
         "mmq_cls_stats": (i32, [vp, C.POINTER(i64)]),
         "mmq_tune": (i32, [vp, i32, i32]),
+        "mmq_count_moments_begin": (i32, [vp, vp, i64, vp, i64]),
+        "mmq_count_moments_end": (i32, [vp]),
+        "mmq_get_count_moments": (i32, [vp, i32, C.POINTER(i64), vp, vp, vp]),
+        "mmq_expected_counts": (i32, [vp, vp]),
         "mmq_get_trace": (i32, [vp, vp]),
         "mmq_trace_len": (i32, [vp]),
         "mmq_set_groups": (i32, [vp, i32, i64, vp, vp, vp]),
@@ -106,6 +110,7 @@ EXPORTS = [
     "mmq_create", "mmq_destroy", "mmq_last_error", "mmq_set_stream", "mmq_get_stream", "mmq_synchronize",
     "mmq_device_bytes", "mmq_comm_id", "mmq_comm_init", "mmq_comm_move", "mmq_p2p_export", "mmq_p2p_attach", "mmq_p2p_attach_local", "mmq_p2p_attached", "mmq_init_mu", "mmq_set_mu", "mmq_get_mu",
     "mmq_loglik", "mmq_em", "mmq_gibbs", "mmq_sweep_debug", "mmq_kernel_times", "mmq_cls_stats", "mmq_tune", "mmq_get_trace", "mmq_trace_len",
+    "mmq_count_moments_begin", "mmq_count_moments_end", "mmq_get_count_moments", "mmq_expected_counts",
     "mmq_set_groups", "mmq_summarize", "mmq_get_group_trace", "mmq_prop_summaries",
     "mmq_unique_hits_sets", "mmq_sokal_batch", "mmq_prior_draws", "mmq_trace_cov", "mmq_trace_cov_workspace_bytes", "mmq_trace_cov_dev",
     "mmq_handle_trace_cov", "mmq_mean_corrs", "mmq_mean_corrs_dev", "mmq_release_cache", "mmq_launch_count", "mmq_warmup", "mmq_version",
@@ -341,6 +346,31 @@ class Handle:
 
     def trace_len(self):
         return int(lib().mmq_trace_len(self._h))
+
+    def count_moments_begin(self, ident_of=None, n_ident=0, gene_of=None, n_gene=0):
+        """Start accumulating posterior fragment counts; ident_of / gene_of: int32[n] group of each transcript or -1."""
+        ident_of = _c(ident_of, np.int32); gene_of = _c(gene_of, np.int32)
+        self._cnt_rows = [self.n, int(n_ident), int(n_gene)]
+        self._check(lib().mmq_count_moments_begin(self._h, _ptr(ident_of), int(n_ident), _ptr(gene_of), int(n_gene)),
+                    "mmq_count_moments_begin")
+
+    def count_moments_end(self):
+        self._check(lib().mmq_count_moments_end(self._h), "mmq_count_moments_end")
+
+    def count_moments(self, which=0):
+        """(sweeps, sum, sumsq_lo, sumsq_hi) of transcripts (0), identical sets (1) or genes (2); uint64 arrays,
+        sum of squares = sumsq_hi * 2**64 + sumsq_lo."""
+        rows = self._cnt_rows[which] if 0 <= which <= 2 else 0
+        sweeps = C.c_int64()
+        s = np.zeros(rows, np.uint64); lo = np.zeros(rows, np.uint64); hi = np.zeros(rows, np.uint64)
+        self._check(lib().mmq_get_count_moments(self._h, which, C.byref(sweeps), _ptr(s), _ptr(lo), _ptr(hi)), "mmq_get_count_moments")
+        return sweeps.value, s, lo, hi
+
+    def expected_counts(self):
+        """One E-step at the current mu: mu[t] * sum_{i containing t} k[i] w[i,t] / D_i over all shards."""
+        out = np.zeros(self.n)
+        self._check(lib().mmq_expected_counts(self._h, _ptr(out)), "mmq_expected_counts")
+        return out
 
     def get_trace(self, out=None):
         """trace[t, slot]; `out`: a caller-provided (n, trace_len) float64 buffer (e.g. pinned memory)."""

@@ -302,6 +302,12 @@ __global__ void k_em_apply(const double* __restrict__ mu, const double* __restri
   if (threadIdx.x == 0) partial[blockIdx.x] = s;
 }
 
+/* out[t] = a[t] * b[t]: the expected counts mu * acc of one E-step (mmq_expected_counts). */
+__global__ void k_mul(const double* __restrict__ a, const double* __restrict__ b, double* __restrict__ out, int64_t n) {
+  for (int64_t t = blockIdx.x * (int64_t)blockDim.x + threadIdx.x; t < n; t += (int64_t)gridDim.x * blockDim.x)
+    out[t] = a[t] * b[t];
+}
+
 __global__ void k_mul_sum(const double* __restrict__ a, const double* __restrict__ b,
                           double* __restrict__ partial, int64_t n) {
   double s = 0.0;
@@ -711,15 +717,60 @@ __device__ __forceinline__ double gamma_block(gamma_smem& S, int64_t t, int32_t 
   return S.boost[tid] * par.d * S.v[tid] / rate;
 }
 
+/* ---- posterior fragment-count moments (mmq_count_moments_begin) ----
+ * Rows [0, n) of the accumulators are the transcripts, [n, n + groups) the identical sets and then the genes.  Every
+ * sweep adds each row's count c to sum (u64) and c^2 to sq (u128): integer sums, so the result does not depend on the
+ * order of the additions (GPU count, launch geometry, graph or not).  A group's count is summed within the sweep first
+ * (gsum, int32, warp-aggregated atomics), since its square is not the sum of its members' squares. */
+struct mmq_cnt_acc {
+  unsigned long long* sum; /* [rows] */
+  unsigned __int128* sq;   /* [rows] */
+  const int2* group;       /* [n] (identical set, n_ident + gene) of each transcript, -1 = none; null: no groups */
+  int32_t* gsum;           /* [groups] this sweep's group counts, zero between sweeps */
+};
+
+/* a group's share of the warp's counts: one atomic per distinct group in the warp.  All 32 lanes call it. */
+__device__ __forceinline__ void count_group_add(int32_t* gsum, int key, int32_t c) {
+  const unsigned peers = __match_any_sync(0xffffffffu, key);
+  const int s = __reduce_add_sync(peers, c);
+  if (key >= 0 && s != 0 && (int)(threadIdx.x & 31) == __ffs(peers) - 1) atomicAdd(gsum + key, s);
+}
+
+/* Every thread of the block calls this with its transcript t (t < 0: none) and the count the Gamma step uses. */
+__device__ __forceinline__ void count_acc(const mmq_cnt_acc& A, int64_t t, int32_t c) {
+  if (t >= 0) {
+    A.sum[t] += (unsigned long long)c;
+    A.sq[t] += (unsigned __int128)((unsigned long long)c * (unsigned long long)c);
+  }
+  if (A.group) {
+    const int2 g = t >= 0 ? A.group[t] : make_int2(-1, -1);
+    count_group_add(A.gsum, g.x, c);
+    count_group_add(A.gsum, g.y, c);
+  }
+}
+
+/* The per-sweep group step: each group's sweep count and its square into rows n + g; gsum back to zero. */
+__global__ void k_count_groups(mmq_cnt_acc A, int64_t n, int64_t groups) {
+  for (int64_t g = blockIdx.x * (int64_t)blockDim.x + threadIdx.x; g < groups; g += (int64_t)gridDim.x * blockDim.x) {
+    const int32_t c = A.gsum[g];
+    if (c == 0) continue;
+    A.gsum[g] = 0;
+    A.sum[n + g] += (unsigned long long)c;
+    A.sq[n + g] += (unsigned __int128)((unsigned long long)c * (unsigned long long)c);
+  }
+}
+
 /* K4 (+K5 capture): mu[t] ~ Gamma(alpha + counts[t], rate beta + l[t]); counts
  * are cleared for the next sweep; trace_col (= trace + slot, or null) receives
- * mu at stride trace_len.  src/mmseq.cpp:904-917. */
-__global__ void __launch_bounds__(MMQ_GAMMA_THREADS, 5)
-k_gamma(int32_t* __restrict__ counts, const int32_t* __restrict__ counts_base, const double* __restrict__ len,
-        double* __restrict__ mu, double* __restrict__ trace, int stride, int trace_len, int64_t n,
-        double alpha, double beta, uint32_t seed, uint32_t sweep, int32_t* __restrict__ counts_copy,
-        const uint32_t* __restrict__ sweep_base) {
-  __shared__ gamma_smem S;
+ * mu at stride trace_len.  src/mmseq.cpp:904-917.
+ * ACC: also add the counts into the moment accumulators (k_gamma_acc).  A compile-time variant: k_gamma is bound by
+ * the latency of one pass and stays the same machine code. */
+template <bool ACC>
+__device__ __forceinline__ void gamma_sweep(gamma_smem& S, int32_t* __restrict__ counts, const int32_t* __restrict__ counts_base,
+                                            const double* __restrict__ len, double* __restrict__ mu, double* __restrict__ trace,
+                                            int stride, int trace_len, int64_t n, double alpha, double beta, uint32_t seed,
+                                            uint32_t sweep, int32_t* __restrict__ counts_copy, const uint32_t* __restrict__ sweep_base,
+                                            const mmq_cnt_acc& A) {
   if (sweep_base) sweep += *sweep_base;
   /* sweep s with s % stride == 0 is recorded in slot s / stride (src/mmseq.cpp:911-917) */
   double* trace_col = nullptr;
@@ -734,12 +785,32 @@ k_gamma(int32_t* __restrict__ counts, const int32_t* __restrict__ counts_base, c
       if (counts_copy) counts_copy[t] = c;
       rate = beta + len[t];
     }
+    if (ACC) count_acc(A, t, c);
     const double v = gamma_block(S, t, c, rate, alpha, seed, sweep);
     if (t >= 0) {
       mu[t] = v;
       if (trace_col) trace_col[t * (int64_t)trace_len] = v;
     }
   }
+}
+
+__global__ void __launch_bounds__(MMQ_GAMMA_THREADS, 5)
+k_gamma(int32_t* __restrict__ counts, const int32_t* __restrict__ counts_base, const double* __restrict__ len,
+        double* __restrict__ mu, double* __restrict__ trace, int stride, int trace_len, int64_t n,
+        double alpha, double beta, uint32_t seed, uint32_t sweep, int32_t* __restrict__ counts_copy,
+        const uint32_t* __restrict__ sweep_base) {
+  __shared__ gamma_smem S;
+  gamma_sweep<false>(S, counts, counts_base, len, mu, trace, stride, trace_len, n, alpha, beta, seed, sweep, counts_copy, sweep_base,
+                     mmq_cnt_acc{});
+}
+
+__global__ void __launch_bounds__(MMQ_GAMMA_THREADS, 5)
+k_gamma_acc(int32_t* __restrict__ counts, const int32_t* __restrict__ counts_base, const double* __restrict__ len,
+            double* __restrict__ mu, double* __restrict__ trace, int stride, int trace_len, int64_t n,
+            double alpha, double beta, uint32_t seed, uint32_t sweep, int32_t* __restrict__ counts_copy,
+            const uint32_t* __restrict__ sweep_base, mmq_cnt_acc A) {
+  __shared__ gamma_smem S;
+  gamma_sweep<true>(S, counts, counts_base, len, mu, trace, stride, trace_len, n, alpha, beta, seed, sweep, counts_copy, sweep_base, A);
 }
 
 /* ---- K3 + K4 fused over NVLink peer memory -------------------------------------------------------
@@ -764,13 +835,14 @@ struct mmq_p2p_args {
 };
 
 /* Debug / parity variant (mmq_sweep_debug): a full all-reduce — every rank reads the count vectors of
- * ALL ranks, draws every Gamma variate and keeps the summed counts.  One barrier. */
-__global__ void __launch_bounds__(MMQ_GAMMA_THREADS, 5)
-k_gamma_p2p(mmq_p2p_args a, const int32_t* __restrict__ counts_base, const double* __restrict__ len,
-            double* __restrict__ mu, double* __restrict__ trace, int stride, int trace_len, int64_t n,
-            double alpha, double beta, uint32_t seed, uint32_t sweep, int32_t* __restrict__ counts_copy,
-            const uint32_t* __restrict__ sweep_base) {
-  __shared__ gamma_smem S;
+ * ALL ranks, draws every Gamma variate and keeps the summed counts.  One barrier.
+ * ACC (k_gamma_p2p_acc): every rank adds the summed counts into its own accumulators. */
+template <bool ACC>
+__device__ __forceinline__ void gamma_p2p_sweep(gamma_smem& S, mmq_p2p_args a, const int32_t* __restrict__ counts_base,
+                                                const double* __restrict__ len, double* __restrict__ mu, double* __restrict__ trace,
+                                                int stride, int trace_len, int64_t n, double alpha, double beta, uint32_t seed,
+                                                uint32_t sweep, int32_t* __restrict__ counts_copy, const uint32_t* __restrict__ sweep_base,
+                                                const mmq_cnt_acc& A) {
   if (sweep_base) sweep += *sweep_base;
   const int32_t epoch = a.epoch + (a.epoch_base ? *a.epoch_base : 0);
   int32_t* own = reinterpret_cast<int32_t*>(a.base[a.rank]);
@@ -799,6 +871,7 @@ k_gamma_p2p(mmq_p2p_args a, const int32_t* __restrict__ counts_base, const doubl
       if (counts_copy) counts_copy[t] = c;
       rate = beta + len[t];
     }
+    if (ACC) count_acc(A, t, c);
     const double v = gamma_block(S, t, c, rate, alpha, seed, sweep);
     if (t >= 0) {
       mu[t] = v;
@@ -809,6 +882,25 @@ k_gamma_p2p(mmq_p2p_args a, const int32_t* __restrict__ counts_base, const doubl
    * wrote its own mu, nothing to wait for */
   if (blockIdx.x == 0 && threadIdx.x < a.nranks)
     p2p_publish(reinterpret_cast<int32_t*>(a.base[threadIdx.x]) + MMQ_P2P_FLAG_MU + 8 * a.rank, epoch);
+}
+
+__global__ void __launch_bounds__(MMQ_GAMMA_THREADS, 5)
+k_gamma_p2p(mmq_p2p_args a, const int32_t* __restrict__ counts_base, const double* __restrict__ len,
+            double* __restrict__ mu, double* __restrict__ trace, int stride, int trace_len, int64_t n,
+            double alpha, double beta, uint32_t seed, uint32_t sweep, int32_t* __restrict__ counts_copy,
+            const uint32_t* __restrict__ sweep_base) {
+  __shared__ gamma_smem S;
+  gamma_p2p_sweep<false>(S, a, counts_base, len, mu, trace, stride, trace_len, n, alpha, beta, seed, sweep, counts_copy, sweep_base,
+                         mmq_cnt_acc{});
+}
+
+__global__ void __launch_bounds__(MMQ_GAMMA_THREADS, 5)
+k_gamma_p2p_acc(mmq_p2p_args a, const int32_t* __restrict__ counts_base, const double* __restrict__ len,
+                double* __restrict__ mu, double* __restrict__ trace, int stride, int trace_len, int64_t n,
+                double alpha, double beta, uint32_t seed, uint32_t sweep, int32_t* __restrict__ counts_copy,
+                const uint32_t* __restrict__ sweep_base, mmq_cnt_acc A) {
+  __shared__ gamma_smem S;
+  gamma_p2p_sweep<true>(S, a, counts_base, len, mu, trace, stride, trace_len, n, alpha, beta, seed, sweep, counts_copy, sweep_base, A);
 }
 
 /* Production variant: reduce-scatter + Gamma + all-gather in ONE kernel.  Rank r owns the transcripts
@@ -1477,6 +1569,17 @@ void mmq_launch_alloc_general(mmq_handle* h, cudaStream_t stream, int grid, cons
   k_alloc<false, true, false><<<grid, MMQ_ALLOC_WARPS * 32, 0, stream>>>(row_ptr, col, k, nullptr, h->mu, h->counts, nullptr, m, tile_start, n_tiles,
                                                                         seed, sweep, 0, class_id, sweep_base);
 }
+static mmq_cnt_acc count_args(const mmq_handle* h) { return mmq_cnt_acc{h->cnt_sum, h->cnt_sq, h->cnt_group, h->cnt_gsum}; }
+/* After the Gamma kernel of a sweep that accumulates count moments: the group step, and the sweep counted (a graph
+ * capture launches nothing now: mmq_gibbs counts its replays). */
+static int count_groups_step(mmq_handle* h, const uint32_t* sweep_base) {
+  if (!h->cnt_block) return MMQ_OK;
+  if (!sweep_base) ++h->cnt_sweeps;
+  if (h->cnt_groups == 0) return MMQ_OK;
+  k_count_groups<<<mmq_grid_for(h->cnt_groups, 256, h->num_sms * 4), 256, 0, h->stream>>>(count_args(h), h->n, h->cnt_groups);
+  MMQ_LAUNCHED(h);
+  return MMQ_OK;
+}
 extern "C" {
 
 /* State a sweep builds on first use (synchronising copies, allocations): done ahead of a graph capture. */
@@ -1567,9 +1670,15 @@ static int enqueue_sweep(mmq_handle* h, uint32_t seed, uint32_t sweep, int flags
        * (The Gamma kernel is bound by the latency of one pass, not by throughput, so drawing n / N variates instead of
        * n saves nothing, while the reduce-scatter variant below pays a second barrier and the peer stores: measured at
        * N = 2, 36 us against 24 us per sweep.) */
-      k_gamma_p2p<<<mmq_grid_for(h->n, MMQ_GAMMA_THREADS, h->num_sms * 5), MMQ_GAMMA_THREADS, 0, h->stream>>>(a, h->seg_base, h->len, h->mu, stride > 0 ? h->trace : nullptr, stride,
-                                                                                h->trace_len, h->n, h->alpha, h->beta, seed, sweep, counts_copy, sweep_base);
+      const int ggrid = mmq_grid_for(h->n, MMQ_GAMMA_THREADS, h->num_sms * 5);
+      if (h->cnt_block)
+        k_gamma_p2p_acc<<<ggrid, MMQ_GAMMA_THREADS, 0, h->stream>>>(a, h->seg_base, h->len, h->mu, stride > 0 ? h->trace : nullptr, stride,
+                                                                    h->trace_len, h->n, h->alpha, h->beta, seed, sweep, counts_copy, sweep_base, count_args(h));
+      else
+        k_gamma_p2p<<<ggrid, MMQ_GAMMA_THREADS, 0, h->stream>>>(a, h->seg_base, h->len, h->mu, stride > 0 ? h->trace : nullptr, stride,
+                                                                h->trace_len, h->n, h->alpha, h->beta, seed, sweep, counts_copy, sweep_base);
       MMQ_LAUNCHED(h);
+      if ((rc = count_groups_step(h, sweep_base))) return rc;
     } else { /* mmq_tune(h, 6, 1): reduce-scatter + Gamma + all-gather */
       const int64_t slice = (h->n + h->p2p_n - 1) / h->p2p_n;
       k_gamma_rs<<<mmq_grid_for(std::max<int64_t>(slice, h->n / 8), MMQ_GAMMA_THREADS, h->num_sms * 4), MMQ_GAMMA_THREADS, 0, h->stream>>>(a, h->seg_base, h->len, h->n, h->alpha, h->beta, seed, sweep, sweep_base);
@@ -1590,9 +1699,15 @@ static int enqueue_sweep(mmq_handle* h, uint32_t seed, uint32_t sweep, int flags
   }
   if ((rc = mmq_allreduce(h, h->counts, (size_t)h->n, 0))) return rc;
   mark(h->ev_gamma);
-  k_gamma<<<mmq_grid_for(h->n, MMQ_GAMMA_THREADS, h->num_sms * 5), MMQ_GAMMA_THREADS, 0, h->stream>>>(h->counts, h->seg_base, h->len, h->mu, stride > 0 ? h->trace : nullptr, stride, h->trace_len, h->n,
-                                                                          h->alpha, h->beta, seed, sweep, counts_copy, sweep_base);
+  const int ggrid = mmq_grid_for(h->n, MMQ_GAMMA_THREADS, h->num_sms * 5);
+  if (h->cnt_block)
+    k_gamma_acc<<<ggrid, MMQ_GAMMA_THREADS, 0, h->stream>>>(h->counts, h->seg_base, h->len, h->mu, stride > 0 ? h->trace : nullptr, stride, h->trace_len, h->n,
+                                                            h->alpha, h->beta, seed, sweep, counts_copy, sweep_base, count_args(h));
+  else
+    k_gamma<<<ggrid, MMQ_GAMMA_THREADS, 0, h->stream>>>(h->counts, h->seg_base, h->len, h->mu, stride > 0 ? h->trace : nullptr, stride, h->trace_len, h->n,
+                                                        h->alpha, h->beta, seed, sweep, counts_copy, sweep_base);
   MMQ_LAUNCHED(h);
+  if ((rc = count_groups_step(h, sweep_base))) return rc;
   mark(h->ev_gamma);
   if (h->seg_base) h->seg_base_in_counts = true; /* k_gamma restarted counts[] from seg_base */
   return MMQ_OK;
@@ -1659,6 +1774,9 @@ int mmq_gibbs(mmq_handle* h, uint32_t seed, int64_t first_sweep, int64_t n_sweep
   if (!h) return MMQ_ERR_ARG;
   if (first_sweep < 0 || n_sweeps < 0 || first_sweep + n_sweeps > (int64_t)0xffffffffll) return mmq_fail(h, MMQ_ERR_ARG, "mmq_gibbs: sweep range out of bounds");
   if (trace_len > 0 && stride <= 0) return mmq_fail(h, MMQ_ERR_ARG, "mmq_gibbs: stride must be > 0");
+  if (h->cnt_block && h->p2p_n > 1 && h->exchange_rs == 1)
+    return mmq_fail(h, MMQ_ERR_STATE, "mmq_gibbs: count moments are not accumulated under the reduce-scatter exchange (mmq_tune knob 6), "
+                                      "where each rank sums only its own slice of the counts; set knob 6 back to 0");
   MMQ_CUDA(h, cudaSetDevice(h->device));
   int rc = ensure_trace(h, trace_len);
   if (rc) return rc;
@@ -1689,6 +1807,7 @@ int mmq_gibbs(mmq_handle* h, uint32_t seed, int64_t first_sweep, int64_t n_sweep
       if (p2p && st > 0 && (int)(s % st) != h->graph_phase) break; /* stride does not divide the graph length: plain launches */
       MMQ_CUDA(h, cudaGraphLaunch(h->graph_exec, h->stream));
       g_mmq_launches.fetch_add(h->graph_launches, std::memory_order_relaxed);
+      if (h->cnt_block) h->cnt_sweeps += MMQ_GRAPH_SWEEPS;
       s += MMQ_GRAPH_SWEEPS;
       if (p2p) h->p2p_epoch += MMQ_GRAPH_SWEEPS;
     }
@@ -1760,6 +1879,122 @@ int mmq_get_trace(mmq_handle* h, double* out) {
   if (!h->trace) return mmq_fail(h, MMQ_ERR_STATE, "mmq_get_trace: no trace recorded (run mmq_gibbs with trace_len > 0)");
   MMQ_CUDA(h, cudaSetDevice(h->device));
   MMQ_CUDA(h, cudaMemcpyAsync(out, h->trace, sizeof(double) * (size_t)h->n * (size_t)h->trace_len, cudaMemcpyDeviceToHost, h->stream));
+  MMQ_CUDA(h, cudaStreamSynchronize(h->stream));
+  return MMQ_OK;
+}
+
+/* ---- posterior fragment counts ---- */
+
+/* bytes of the accumulator block: sq, sum, group map, group sums (mmq_internal.h) */
+static void count_layout(int64_t n, int64_t groups, size_t b[4]) {
+  b[0] = sizeof(unsigned __int128) * (size_t)(n + groups);
+  b[1] = sizeof(unsigned long long) * (size_t)(n + groups);
+  b[2] = groups > 0 ? sizeof(int2) * (size_t)n : 0;
+  b[3] = sizeof(int32_t) * (size_t)groups;
+}
+
+static void count_free(mmq_handle* h) {
+  if (!h->cnt_block) return;
+  size_t b[4];
+  count_layout(h->n, h->cnt_groups, b);
+  h->bytes -= (int64_t)(b[0] + b[1] + b[2] + b[3]);
+  mmq_dev_free(h, h->cnt_block); /* synchronises the stream first */
+  h->cnt_block = nullptr; h->cnt_sq = nullptr; h->cnt_sum = nullptr; h->cnt_group = nullptr; h->cnt_gsum = nullptr;
+  h->cnt_ident = h->cnt_groups = 0;
+  h->cnt_sweeps = 0;
+}
+
+int mmq_count_moments_begin(mmq_handle* h, const int32_t* ident_of, int64_t n_ident, const int32_t* gene_of, int64_t n_gene) {
+  if (!h) return MMQ_ERR_ARG;
+  if (n_ident < 0 || n_gene < 0 || n_ident + n_gene > INT32_MAX)
+    return mmq_fail(h, MMQ_ERR_ARG, "mmq_count_moments_begin: group counts out of range");
+  if ((n_ident > 0 && !ident_of) || (n_gene > 0 && !gene_of))
+    return mmq_fail(h, MMQ_ERR_ARG, "mmq_count_moments_begin: ident_of / gene_of is NULL but its group count is not 0");
+  const int64_t n = h->n, groups = n_ident + n_gene;
+  std::vector<int2> grp;
+  if (groups > 0) {
+    grp.resize((size_t)n);
+    for (int64_t t = 0; t < n; ++t) {
+      const int32_t i = n_ident > 0 ? ident_of[t] : -1, g = n_gene > 0 ? gene_of[t] : -1;
+      if (i < -1 || i >= n_ident || g < -1 || g >= n_gene)
+        return mmq_fail(h, MMQ_ERR_ARG, "mmq_count_moments_begin: transcript " + std::to_string(t) + " names a group out of range");
+      grp[(size_t)t] = make_int2(i, g < 0 ? -1 : (int)(n_ident + g));
+    }
+  }
+  MMQ_CUDA(h, cudaSetDevice(h->device));
+  MMQ_CUDA(h, cudaStreamSynchronize(h->stream));
+  drop_graph(h); /* a captured graph has the other Gamma kernel baked in */
+  count_free(h);
+  size_t b[4];
+  count_layout(n, groups, b);
+  const size_t b_sq = b[0], b_sum = b[1], b_grp = b[2], bytes = b[0] + b[1] + b[2] + b[3];
+  /* from the block cache, not the arena: a handle that never asks for counts pays nothing */
+  void* blk = nullptr;
+  MMQ_CUDA(h, mmq_cache_malloc(&blk, bytes));
+  h->allocs.push_back(blk);
+  h->bytes += (int64_t)bytes;
+  h->cnt_block = blk;
+  char* p = static_cast<char*>(blk);
+  h->cnt_sq = reinterpret_cast<unsigned __int128*>(p);
+  h->cnt_sum = reinterpret_cast<unsigned long long*>(p + b_sq);
+  h->cnt_group = groups > 0 ? reinterpret_cast<int2*>(p + b_sq + b_sum) : nullptr;
+  h->cnt_gsum = reinterpret_cast<int32_t*>(p + b_sq + b_sum + b_grp);
+  h->cnt_ident = n_ident;
+  h->cnt_groups = groups;
+  h->cnt_sweeps = 0;
+  MMQ_CUDA(h, cudaMemsetAsync(blk, 0, bytes, h->stream));
+  if (groups > 0) MMQ_CUDA(h, cudaMemcpyAsync(h->cnt_group, grp.data(), b_grp, cudaMemcpyHostToDevice, h->stream));
+  MMQ_CUDA(h, cudaStreamSynchronize(h->stream));
+  return MMQ_OK;
+}
+
+int mmq_count_moments_end(mmq_handle* h) {
+  if (!h) return MMQ_ERR_ARG;
+  MMQ_CUDA(h, cudaSetDevice(h->device));
+  MMQ_CUDA(h, cudaStreamSynchronize(h->stream));
+  drop_graph(h);
+  count_free(h);
+  return MMQ_OK;
+}
+
+int mmq_get_count_moments(mmq_handle* h, int which, int64_t* sweeps, uint64_t* sum, uint64_t* sumsq_lo, uint64_t* sumsq_hi) {
+  if (!h) return MMQ_ERR_ARG;
+  if (!h->cnt_block) return mmq_fail(h, MMQ_ERR_STATE, "mmq_get_count_moments: no count moments (call mmq_count_moments_begin first)");
+  if (which < 0 || which > 2) return mmq_fail(h, MMQ_ERR_ARG, "mmq_get_count_moments: which must be 0, 1 or 2");
+  const int64_t r0 = which == 0 ? 0 : which == 1 ? h->n : h->n + h->cnt_ident;
+  const int64_t rows = which == 0 ? h->n : which == 1 ? h->cnt_ident : h->cnt_groups - h->cnt_ident;
+  MMQ_CUDA(h, cudaSetDevice(h->device));
+  if (sweeps) *sweeps = (int64_t)h->cnt_sweeps;
+  if (rows > 0 && sum)
+    MMQ_CUDA(h, cudaMemcpyAsync(sum, h->cnt_sum + r0, sizeof(uint64_t) * (size_t)rows, cudaMemcpyDeviceToHost, h->stream));
+  std::vector<unsigned __int128> sq;
+  if (rows > 0 && (sumsq_lo || sumsq_hi)) {
+    sq.resize((size_t)rows);
+    MMQ_CUDA(h, cudaMemcpyAsync(sq.data(), h->cnt_sq + r0, sizeof(unsigned __int128) * (size_t)rows, cudaMemcpyDeviceToHost, h->stream));
+  }
+  MMQ_CUDA(h, cudaStreamSynchronize(h->stream));
+  for (size_t r = 0; r < sq.size(); ++r) {
+    if (sumsq_lo) sumsq_lo[r] = (uint64_t)sq[r];
+    if (sumsq_hi) sumsq_hi[r] = (uint64_t)(sq[r] >> 64);
+  }
+  return MMQ_OK;
+}
+
+/* One E-step at the current mu (src/mmseq.cpp:781-794): acc = the EM accumulation of all shards, out = mu * acc. */
+int mmq_expected_counts(mmq_handle* h, double* out) {
+  if (!h || !out) return mmq_fail(h, MMQ_ERR_ARG, "mmq_expected_counts: NULL argument");
+  MMQ_CUDA(h, cudaSetDevice(h->device));
+  int rc = build_transpose(h);
+  if (rc) return rc;
+  if ((rc = launch_rowterm(h, h->mu))) return rc; /* rterm = k / D(mu) */
+  const int grid_w = mmq_grid_for(h->n * 32, 256, h->num_sms * 8);
+  if (h->has_w) k_em_acc<true><<<grid_w, 256, 0, h->stream>>>(h->tptr, h->perm, h->trow, h->w, h->rterm, h->acc, h->n);
+  else k_em_acc<false><<<grid_w, 256, 0, h->stream>>>(h->tptr, h->perm, h->trow, h->w, h->rterm, h->acc, h->n);
+  MMQ_LAUNCHED(h);
+  if ((rc = mmq_allreduce(h, h->acc, (size_t)h->n, 1))) return rc;
+  k_mul<<<mmq_grid_for(h->n, 256, h->num_sms * 8), 256, 0, h->stream>>>(h->mu, h->acc, h->mu_tmp, h->n);
+  MMQ_LAUNCHED(h);
+  MMQ_CUDA(h, cudaMemcpyAsync(out, h->mu_tmp, sizeof(double) * (size_t)h->n, cudaMemcpyDeviceToHost, h->stream));
   MMQ_CUDA(h, cudaStreamSynchronize(h->stream));
   return MMQ_OK;
 }

@@ -155,6 +155,17 @@ struct mmq_handle {
   const double* graph_trace = nullptr;
   cudaStream_t graph_stream = nullptr;
 
+  /* posterior fragment-count moments (mmq_count_moments_begin; cnt_block null when not accumulating): one block-cache
+   * allocation holding sq (u128) and sum (u64) of rows [0, n) transcripts, [n, n + cnt_ident) identical sets and
+   * [n + cnt_ident, n + cnt_groups) genes, then cnt_group (int2[n], or none without groups) and cnt_gsum (int32[cnt_groups]) */
+  void* cnt_block = nullptr;
+  unsigned __int128* cnt_sq = nullptr;
+  unsigned long long* cnt_sum = nullptr;
+  int2* cnt_group = nullptr;
+  int32_t* cnt_gsum = nullptr;
+  int64_t cnt_ident = 0, cnt_groups = 0;
+  uint64_t cnt_sweeps = 0; /* sweeps accumulated (graph replays counted by mmq_gibbs) */
+
   /* MMQ_GIBBS_TIME_KERNELS: (start, stop) event pairs around each launch */
   std::vector<cudaEvent_t> ev_alloc, ev_gamma;
 

@@ -11,7 +11,8 @@
  * proportion summaries.  The host only parses, formats and writes.
  * Additive options: -gpus INT (shard hit classes over GPUs of this box),
  * -notraces (skip the four *.trace_gibbs.gz text dumps), -batch FILE / -per_gpu INT (many
- * samples dealt to the GPUs, independent chains: BASELINE config 5).
+ * samples dealt to the GPUs, independent chains: BASELINE config 5), -counts (posterior and EM fragment counts per
+ * transcript, identical set and gene: *.counts, *.identical.counts, *.gene.counts).
  */
 #include <unistd.h>
 #include <zlib.h>
@@ -72,6 +73,7 @@ static void printUsage(ostream& out) {
       << "  -notraces          (B200 build) do not write the *.trace_gibbs.gz text dumps" << endl
       << "  -batch FILE        (B200 build) many samples: FILE lists one \"hits_file output_base\" pair per line (no positional arguments)" << endl
       << "  -per_gpu INT       (B200 build) batch mode: samples in flight per GPU (default: 4)" << endl
+      << "  -counts            (B200 build) also write posterior and EM fragment counts (*.counts, *.identical.counts, *.gene.counts)" << endl
       << endl;
 }
 
@@ -137,6 +139,15 @@ static void write_rows(ostream& ofs, int64_t rows, const function<void(ostream&,
   for (auto& p : part) { const string blk = p.str(); ofs.write(blk.data(), (streamsize)blk.size()); }
 }
 
+/* posterior sd of a count from its moments over S sweeps: sqrt((S sum c^2 - (sum c)^2) / (S (S - 1))), the numerator
+ * exact in 128 bits (it can pass 2^64 long before the end of a chain) and the S - 1 of the sd column (src/sokal.cc:63) */
+static double count_sd(int64_t S, uint64_t sum, uint64_t sumsq_lo, uint64_t sumsq_hi) {
+  if (S < 2) return 0.0;
+  const unsigned __int128 sq = ((unsigned __int128)sumsq_hi << 64) | sumsq_lo;
+  const unsigned __int128 num = (unsigned __int128)(uint64_t)S * sq - (unsigned __int128)sum * sum;
+  return sqrt((double)num / ((double)S * (double)(S - 1)));
+}
+
 struct Shard {
   int device = 0;
   int64_t row0 = 0, row1 = 0;
@@ -160,7 +171,7 @@ struct Options {
   double alpha = 0.1, beta = 0.1, epsilon = 0.1;
   int max_em_iter = 1000, gibbs_iter = 16384, trace_length = 1024, gibbs_ss = 16384 / 1024, seed = 1234;
   vector<double> percentiles{5.0, 25.0, 50.0, 75.0, 95.0};
-  bool debug = false, notraces = false;
+  bool debug = false, notraces = false, counts = false;
   int ngpus = 1;
   string batch;     /* -batch FILE: one "hits_file output_base" pair per line */
   int per_gpu = 4;  /* -per_gpu INT: samples in flight per GPU in batch mode */
@@ -201,7 +212,7 @@ static Options parse_command_line(int argc, char** argv) {
       {"-epsilon", REAL, &o.epsilon},     {"-gibbs_iter", INT, &o.gibbs_iter}, {"-gibbs_ss", INT, &o.gibbs_ss},
       {"-seed", INT, &o.seed},            {"-percentiles", TEXT, &pct},       {"-gpus", INT, &o.ngpus},
       {"-batch", TEXT, &o.batch},         {"-per_gpu", INT, &o.per_gpu},      {"-notraces", FLAG, &o.notraces},
-      {"-debug", FLAG, &o.debug},
+      {"-debug", FLAG, &o.debug},         {"-counts", FLAG, &o.counts},
   };
   /* options come first; what is left must be the mandatory arguments (none in batch mode) */
   int i = 1;
@@ -514,6 +525,27 @@ static void run_sample(const Options& o, const string& hits_file, const string& 
     check(mmq_get_mu(H0, mu_em.data()), H0, "mmq_get_mu");
   }
 
+  /* ---- -counts: EM expected counts at mu_em (one E-step, all shards), and from here on every Gibbs sweep adds its
+   * counts of transcripts, identical sets and genes into the accumulators of every shard */
+  vector<double> em_count;
+  if (o.counts) {
+    em_count.resize((size_t)n);
+    vector<vector<double>> other((size_t)ngpus);
+    on_all([&](int g) {
+      mmq_handle* h = shards[(size_t)g].h;
+      if (g > 0) other[(size_t)g].resize((size_t)n);
+      check(mmq_expected_counts(h, g == 0 ? em_count.data() : other[(size_t)g].data()), h, "mmq_expected_counts");
+    });
+    vector<int32_t> ident_of((size_t)n, -1), gene_of((size_t)n);
+    for (int64_t s = 0; s < I; ++s)
+      for (int32_t hidx : hdr.identical[(size_t)s]) { const int32_t c = cls.hdr2col[(size_t)hidx]; if (c >= 0) ident_of[(size_t)c] = (int32_t)s; }
+    for (int64_t t = 0; t < n; ++t) gene_of[(size_t)t] = hdr.gene_of[(size_t)cls.col2hdr[(size_t)t]];
+    on_all([&](int g) {
+      mmq_handle* h = shards[(size_t)g].h;
+      check(mmq_count_moments_begin(h, ident_of.data(), I, gene_of.data(), G), h, "mmq_count_moments_begin");
+    });
+  }
+
   /* ---- Gibbs (src/mmseq.cpp:822-918) */
   {
     auto t0 = chrono::steady_clock::now();
@@ -667,6 +699,16 @@ static void run_sample(const Options& o, const string& hits_file, const string& 
   }
 
   phase("summaries");
+  /* feature id of an identical set: the member names joined by "+" (:1560-1565) */
+  auto identical_id = [&](int64_t s) {
+    string id;
+    const auto& mem = hdr.identical[(size_t)s];
+    for (size_t j = 0; j < mem.size(); ++j) {
+      id += hdr.names[(size_t)mem[j]];
+      if (hdr.names[(size_t)mem[j]].compare(hdr.names[(size_t)mem.back()]) != 0) id += "+";
+    }
+    return id;
+  };
   /* ---- trace dumps (:829-831, :911-917, :1033-1108) */
   if (!notraces) {
     vector<double> tr((size_t)n * (size_t)L);
@@ -680,13 +722,7 @@ static void run_sample(const Options& o, const string& hits_file, const string& 
     vector<string> iids((size_t)I);
     vector<char> keep((size_t)I);
     for (int64_t s = 0; s < I; ++s) {
-      string id;
-      const auto& mem = hdr.identical[(size_t)s];
-      for (size_t j = 0; j < mem.size(); ++j) {
-        id += hdr.names[(size_t)mem[j]];
-        if (hdr.names[(size_t)mem[j]].compare(hdr.names[(size_t)mem.back()]) != 0) id += "+";
-      }
-      iids[(size_t)s] = id;
+      iids[(size_t)s] = identical_id(s);
       keep[(size_t)s] = isfinite(log(itr[(size_t)s * (size_t)L])) != 0; /* :1045 */
     }
     write_trace_gz(output_base + ".identical.trace_gibbs.gz", iids, keep, itr.data(), L);
@@ -803,6 +839,40 @@ static void run_sample(const Options& o, const string& hits_file, const string& 
   });
   ofs.close(); ofs.clear();
 
+  /* ---- -counts: .counts, .identical.counts, .gene.counts — rows and ids as in the three tables above; posterior
+   * mean and sd over the chain's sweeps, EM expected count (a group's: the sum of its members').  Every shard holds
+   * the same moments. */
+  if (o.counts) {
+    auto write_counts = [&](const string& path, int which, int64_t rows, const function<string(int64_t)>& id, const function<int64_t(int64_t)>& row_of,
+                            const function<double(int64_t)>& em) {
+      int64_t S = 0;
+      const int64_t R = which == 0 ? n : which == 1 ? I : G;
+      vector<uint64_t> sum((size_t)R), lo((size_t)R), hi((size_t)R);
+      check(mmq_get_count_moments(H0, which, &S, sum.data(), lo.data(), hi.data()), H0, "mmq_get_count_moments");
+      ofs.open(path.c_str());
+      ofs << "# Mapped fragments: " << N << endl;
+      ofs << "feature_id\tposterior_mean_count\tposterior_sd_count\tem_count\n";
+      write_rows(ofs, rows, [&](ostream& ofs, int64_t r) {
+        const int64_t q = row_of(r);
+        ofs << id(r) << "\t";
+        if (q < 0 || S == 0) ofs << 0.0 << "\t" << 0.0 << "\t" << 0.0 << "\n";
+        else ofs << (double)sum[(size_t)q] / (double)S << "\t" << count_sd(S, sum[(size_t)q], lo[(size_t)q], hi[(size_t)q]) << "\t" << em(q) << "\n";
+      });
+      ofs.close(); ofs.clear();
+    };
+    auto em_group = [&](const vector<int32_t>& members) {
+      double e = 0.0;
+      for (int32_t hidx : members) { const int32_t c = cls.hdr2col[(size_t)hidx]; if (c >= 0) e += em_count[(size_t)c]; }
+      return e;
+    };
+    write_counts(output_base + ".counts", 0, T, [&](int64_t hI) { return hdr.names[(size_t)hI]; },
+                 [&](int64_t hI) { return (int64_t)cls.hdr2col[(size_t)hI]; }, [&](int64_t c) { return em_count[(size_t)c]; });
+    write_counts(output_base + ".identical.counts", 1, I, identical_id, [](int64_t s) { return s; },
+                 [&](int64_t s) { return em_group(hdr.identical[(size_t)s]); });
+    write_counts(output_base + ".gene.counts", 2, G, [&](int64_t g) { return hdr.gene_names[(size_t)g]; }, [](int64_t g) { return g; },
+                 [&](int64_t g) { return em_group(hdr.gene_members[(size_t)g]); });
+  }
+
   out << "done." << endl;
   for (auto& S : shards) mmq_destroy(S.h);
 
@@ -811,6 +881,10 @@ static void run_sample(const Options& o, const string& hits_file, const string& 
        << "  " << output_base << ".mmseq" << endl
        << "  " << output_base << ".identical.mmseq" << endl
        << "  " << output_base << ".gene.mmseq" << endl;
+  if (o.counts)
+    out << "  " << output_base << ".counts" << endl
+        << "  " << output_base << ".identical.counts" << endl
+        << "  " << output_base << ".gene.counts" << endl;
   out << "  " << output_base << ".M" << endl << "  " << output_base << ".k" << endl << endl;
   if (!notraces)
     out << "  " << output_base << ".trace_gibbs.gz" << endl
