@@ -19,6 +19,7 @@
 #include <chrono>
 #include <map>
 #include <mutex>
+#include <type_traits>
 #include <unordered_map>
 #include <cstdio>
 #include <cstring>
@@ -760,60 +761,13 @@ __global__ void k_count_groups(mmq_cnt_acc A, int64_t n, int64_t groups) {
   }
 }
 
-/* K4 (+K5 capture): mu[t] ~ Gamma(alpha + counts[t], rate beta + l[t]); counts
- * are cleared for the next sweep; trace_col (= trace + slot, or null) receives
- * mu at stride trace_len.  src/mmseq.cpp:904-917.
- * ACC: also add the counts into the moment accumulators (k_gamma_acc).  A compile-time variant: k_gamma is bound by
- * the latency of one pass and stays the same machine code. */
-template <bool ACC>
-__device__ __forceinline__ void gamma_sweep(gamma_smem& S, int32_t* __restrict__ counts, const int32_t* __restrict__ counts_base,
-                                            const double* __restrict__ len, double* __restrict__ mu, double* __restrict__ trace,
-                                            int stride, int trace_len, int64_t n, double alpha, double beta, uint32_t seed,
-                                            uint32_t sweep, int32_t* __restrict__ counts_copy, const uint32_t* __restrict__ sweep_base,
-                                            const mmq_cnt_acc& A) {
-  if (sweep_base) sweep += *sweep_base;
-  /* sweep s with s % stride == 0 is recorded in slot s / stride (src/mmseq.cpp:911-917) */
-  double* trace_col = nullptr;
-  if (trace && stride > 0 && sweep % (uint32_t)stride == 0 && sweep / (uint32_t)stride < (uint32_t)trace_len) trace_col = trace + sweep / (uint32_t)stride;
-  for (int64_t t0 = (int64_t)blockIdx.x * MMQ_GAMMA_THREADS; t0 < n; t0 += (int64_t)gridDim.x * MMQ_GAMMA_THREADS) {
-    const int64_t t = t0 + threadIdx.x < n ? t0 + threadIdx.x : -1;
-    int32_t c = 0;
-    double rate = 1.0;
-    if (t >= 0) {
-      c = counts[t];
-      counts[t] = counts_base ? counts_base[t] : 0; /* classes the allocation kernels skip (singletons) */
-      if (counts_copy) counts_copy[t] = c;
-      rate = beta + len[t];
-    }
-    if (ACC) count_acc(A, t, c);
-    const double v = gamma_block(S, t, c, rate, alpha, seed, sweep);
-    if (t >= 0) {
-      mu[t] = v;
-      if (trace_col) trace_col[t * (int64_t)trace_len] = v;
-    }
-  }
+/* The trace rule of src/mmseq.cpp:911-917: sweep s is recorded in slot s / stride when s % stride == 0 and that slot is
+ * < trace_len.  stride > 0. */
+__host__ __device__ __forceinline__ bool trace_recorded(uint32_t sweep, int stride, int trace_len) {
+  return sweep % (uint32_t)stride == 0 && sweep / (uint32_t)stride < (uint32_t)trace_len;
 }
 
-__global__ void __launch_bounds__(MMQ_GAMMA_THREADS, 5)
-k_gamma(int32_t* __restrict__ counts, const int32_t* __restrict__ counts_base, const double* __restrict__ len,
-        double* __restrict__ mu, double* __restrict__ trace, int stride, int trace_len, int64_t n,
-        double alpha, double beta, uint32_t seed, uint32_t sweep, int32_t* __restrict__ counts_copy,
-        const uint32_t* __restrict__ sweep_base) {
-  __shared__ gamma_smem S;
-  gamma_sweep<false>(S, counts, counts_base, len, mu, trace, stride, trace_len, n, alpha, beta, seed, sweep, counts_copy, sweep_base,
-                     mmq_cnt_acc{});
-}
-
-__global__ void __launch_bounds__(MMQ_GAMMA_THREADS, 5)
-k_gamma_acc(int32_t* __restrict__ counts, const int32_t* __restrict__ counts_base, const double* __restrict__ len,
-            double* __restrict__ mu, double* __restrict__ trace, int stride, int trace_len, int64_t n,
-            double alpha, double beta, uint32_t seed, uint32_t sweep, int32_t* __restrict__ counts_copy,
-            const uint32_t* __restrict__ sweep_base, mmq_cnt_acc A) {
-  __shared__ gamma_smem S;
-  gamma_sweep<true>(S, counts, counts_base, len, mu, trace, stride, trace_len, n, alpha, beta, seed, sweep, counts_copy, sweep_base, A);
-}
-
-/* ---- K3 + K4 fused over NVLink peer memory -------------------------------------------------------
+/* ---- peer memory (NVLink) ----------------------------------------------------------------------
  * Every rank owns a peer-mapped block (mmq_internal.h: MMQ_P2P_*): two flag arrays, the two parity
  * buffers of its count vector and its mu vector.  Flags are written with st.release.sys into the
  * peers' blocks and polled locally with ld.acquire.sys. */
@@ -834,39 +788,67 @@ struct mmq_p2p_args {
   const int32_t* epoch_base;
 };
 
-/* Debug / parity variant (mmq_sweep_debug): a full all-reduce — every rank reads the count vectors of
- * ALL ranks, draws every Gamma variate and keeps the summed counts.  One barrier.
- * ACC (k_gamma_p2p_acc): every rank adds the summed counts into its own accumulators. */
-template <bool ACC>
-__device__ __forceinline__ void gamma_p2p_sweep(gamma_smem& S, mmq_p2p_args a, const int32_t* __restrict__ counts_base,
-                                                const double* __restrict__ len, double* __restrict__ mu, double* __restrict__ trace,
-                                                int stride, int trace_len, int64_t n, double alpha, double beta, uint32_t seed,
-                                                uint32_t sweep, int32_t* __restrict__ counts_copy, const uint32_t* __restrict__ sweep_base,
-                                                const mmq_cnt_acc& A) {
-  if (sweep_base) sweep += *sweep_base;
-  const int32_t epoch = a.epoch + (a.epoch_base ? *a.epoch_base : 0);
+/* The exchange's barrier at the start of a Gamma kernel: block 0 tells every rank that this rank's allocation of the
+ * epoch is done, and every block waits for the peers'.  One thread per peer polls that peer's flag (own allocation is
+ * complete by stream order: no wait on self): the waits overlap instead of one system-scope round trip after the
+ * other; the block barrier orders everybody else's loads behind them.  (& rather than &&: one predicate, and
+ * threadIdx.x is read once for both tests.) */
+__device__ __forceinline__ void p2p_arrive_and_wait(const mmq_p2p_args& a, int32_t epoch) {
   int32_t* own = reinterpret_cast<int32_t*>(a.base[a.rank]);
-  if (blockIdx.x == 0 && threadIdx.x < a.nranks)
+  if ((blockIdx.x == 0) & (threadIdx.x < a.nranks))
     p2p_publish(reinterpret_cast<int32_t*>(a.base[threadIdx.x]) + MMQ_P2P_FLAG_ALLOC + 8 * a.rank, epoch);
-  /* one thread per peer polls that peer's flag (own allocation is complete by stream order: no wait on self): the waits
-   * overlap instead of one system-scope round trip after the other; the block barrier orders everybody else's loads behind them */
   if (threadIdx.x < a.nranks && (int)threadIdx.x != a.rank) p2p_wait(own + MMQ_P2P_FLAG_ALLOC + 8 * threadIdx.x, epoch);
   __syncthreads();
+}
+
+/* transcript t's count summed over the ranks: all ranks' counts in flight at once — with a run-time trip count the adds
+ * serialise the peer loads, one NVLink round trip after the other */
+__device__ __forceinline__ int32_t p2p_count(const mmq_p2p_args& a, int64_t t) {
+  int32_t v[MMQ_P2P_MAX];
+#pragma unroll
+  for (int r = 0; r < MMQ_P2P_MAX; ++r) v[r] = r < a.nranks ? __ldcv(reinterpret_cast<const int32_t*>(a.base[r] + a.off_counts) + t) : 0;
+  int32_t c = 0;
+#pragma unroll
+  for (int r = 0; r < MMQ_P2P_MAX; ++r) c += v[r];
+  return c;
+}
+
+/* K4 (+K5 capture): mu[t] ~ Gamma(alpha + counts[t], rate beta + l[t]); counts are cleared for the next sweep (to
+ * counts_base: classes the allocation kernels skip, the singletons); a recorded sweep stores mu into its trace slot.
+ * src/mmseq.cpp:904-917.  Compile-time variants (the kernel is bound by the latency of one pass, so each one is the
+ * machine code it would be on its own):
+ *   P2P: src is the peer blocks (mmq_p2p_args), the all-reduce over peer memory that multi-GPU runs use by default.
+ *        Every rank reads the count vectors of ALL ranks (parity buffer src.off_counts), draws every Gamma variate,
+ *        keeps the summed counts and clears its own other parity buffer (src.off_reset).  One barrier.
+ *        Else src is the own count vector, read and cleared in place.  One parameter whose type follows P2P, rather
+ *        than both: the parameters after it then sit at the constant-bank alignment they would have in a kernel of
+ *        either kind alone, and ptxas pairs their loads the same way.
+ *   ACC: also add the counts into the moment accumulators A (mmq_count_moments_begin).  Without ACC, A is unused. */
+template <bool ACC, bool P2P>
+__global__ void __launch_bounds__(MMQ_GAMMA_THREADS, 5)
+k_gamma(std::conditional_t<P2P, mmq_p2p_args, int32_t* __restrict__> src, const int32_t* __restrict__ counts_base,
+        const double* __restrict__ len, double* __restrict__ mu, double* __restrict__ trace, int stride, int trace_len, int64_t n,
+        double alpha, double beta, uint32_t seed, uint32_t sweep, int32_t* __restrict__ counts_copy,
+        const uint32_t* __restrict__ sweep_base, mmq_cnt_acc A) {
+  __shared__ gamma_smem S;
+  if (sweep_base) sweep += *sweep_base;
+  int32_t epoch = 0;
+  if constexpr (P2P) {
+    epoch = src.epoch + (src.epoch_base ? *src.epoch_base : 0);
+    p2p_arrive_and_wait(src, epoch);
+  }
   double* trace_col = nullptr;
-  if (trace && stride > 0 && sweep % (uint32_t)stride == 0 && sweep / (uint32_t)stride < (uint32_t)trace_len) trace_col = trace + sweep / (uint32_t)stride;
-  int32_t* reset = reinterpret_cast<int32_t*>(a.base[a.rank] + a.off_reset);
+  if (trace && stride > 0 && trace_recorded(sweep, stride, trace_len)) trace_col = trace + sweep / (uint32_t)stride;
+  int32_t* reset;
+  if constexpr (P2P) reset = reinterpret_cast<int32_t*>(src.base[src.rank] + src.off_reset);
+  else reset = src;
   for (int64_t t0 = (int64_t)blockIdx.x * MMQ_GAMMA_THREADS; t0 < n; t0 += (int64_t)gridDim.x * MMQ_GAMMA_THREADS) {
     const int64_t t = t0 + threadIdx.x < n ? t0 + threadIdx.x : -1;
     int32_t c = 0;
     double rate = 1.0;
     if (t >= 0) {
-      /* all ranks' counts in flight at once: with a run-time trip count the adds serialise the peer loads, one NVLink round
-       * trip after the other */
-      int32_t v[MMQ_P2P_MAX];
-#pragma unroll
-      for (int r = 0; r < MMQ_P2P_MAX; ++r) v[r] = r < a.nranks ? __ldcv(reinterpret_cast<const int32_t*>(a.base[r] + a.off_counts) + t) : 0;
-#pragma unroll
-      for (int r = 0; r < MMQ_P2P_MAX; ++r) c += v[r];
+      if constexpr (P2P) c = p2p_count(src, t);
+      else c = src[t];
       reset[t] = counts_base ? counts_base[t] : 0;
       if (counts_copy) counts_copy[t] = c;
       rate = beta + len[t];
@@ -880,30 +862,13 @@ __device__ __forceinline__ void gamma_p2p_sweep(gamma_smem& S, mmq_p2p_args a, c
   }
   /* the mu flags advance too, so that a later k_gamma_rs (which waits for them) sees a monotone epoch: every rank
    * wrote its own mu, nothing to wait for */
-  if (blockIdx.x == 0 && threadIdx.x < a.nranks)
-    p2p_publish(reinterpret_cast<int32_t*>(a.base[threadIdx.x]) + MMQ_P2P_FLAG_MU + 8 * a.rank, epoch);
+  if constexpr (P2P)
+    if (blockIdx.x == 0 && threadIdx.x < src.nranks)
+      p2p_publish(reinterpret_cast<int32_t*>(src.base[threadIdx.x]) + MMQ_P2P_FLAG_MU + 8 * src.rank, epoch);
 }
 
-__global__ void __launch_bounds__(MMQ_GAMMA_THREADS, 5)
-k_gamma_p2p(mmq_p2p_args a, const int32_t* __restrict__ counts_base, const double* __restrict__ len,
-            double* __restrict__ mu, double* __restrict__ trace, int stride, int trace_len, int64_t n,
-            double alpha, double beta, uint32_t seed, uint32_t sweep, int32_t* __restrict__ counts_copy,
-            const uint32_t* __restrict__ sweep_base) {
-  __shared__ gamma_smem S;
-  gamma_p2p_sweep<false>(S, a, counts_base, len, mu, trace, stride, trace_len, n, alpha, beta, seed, sweep, counts_copy, sweep_base,
-                         mmq_cnt_acc{});
-}
-
-__global__ void __launch_bounds__(MMQ_GAMMA_THREADS, 5)
-k_gamma_p2p_acc(mmq_p2p_args a, const int32_t* __restrict__ counts_base, const double* __restrict__ len,
-                double* __restrict__ mu, double* __restrict__ trace, int stride, int trace_len, int64_t n,
-                double alpha, double beta, uint32_t seed, uint32_t sweep, int32_t* __restrict__ counts_copy,
-                const uint32_t* __restrict__ sweep_base, mmq_cnt_acc A) {
-  __shared__ gamma_smem S;
-  gamma_p2p_sweep<true>(S, a, counts_base, len, mu, trace, stride, trace_len, n, alpha, beta, seed, sweep, counts_copy, sweep_base, A);
-}
-
-/* Production variant: reduce-scatter + Gamma + all-gather in ONE kernel.  Rank r owns the transcripts
+/* The reduce-scatter alternative to k_gamma<ACC, true> (mmq_tune knob 6; the all-reduce is the default, DESIGN §7):
+ * reduce-scatter + Gamma + all-gather in ONE kernel.  Rank r owns the transcripts
  * [n r / N, n (r+1) / N): after the "allocation done" barrier it sums the N count vectors for its slice
  * only ((N-1) 4n/N bytes over NVLink instead of (N-1) 4n), draws n/N Gamma variates instead of n, and
  * stores each new mu into the mu vector of EVERY rank (P2P stores).  The last block to finish publishes
@@ -917,23 +882,14 @@ k_gamma_rs(mmq_p2p_args a, const int32_t* __restrict__ counts_base, const double
   if (sweep_base) sweep += *sweep_base;
   const int32_t epoch = a.epoch + (a.epoch_base ? *a.epoch_base : 0);
   int32_t* own = reinterpret_cast<int32_t*>(a.base[a.rank]);
-  if (blockIdx.x == 0 && threadIdx.x < a.nranks)
-    p2p_publish(reinterpret_cast<int32_t*>(a.base[threadIdx.x]) + MMQ_P2P_FLAG_ALLOC + 8 * a.rank, epoch);
-  /* one thread per peer polls that peer's flag (own allocation is complete by stream order: no wait on self): the waits
-   * overlap instead of one system-scope round trip after the other; the block barrier orders everybody else's loads behind them */
-  if (threadIdx.x < a.nranks && (int)threadIdx.x != a.rank) p2p_wait(own + MMQ_P2P_FLAG_ALLOC + 8 * threadIdx.x, epoch);
-  __syncthreads();
+  p2p_arrive_and_wait(a, epoch);
   const int64_t s0 = n * a.rank / a.nranks, s1 = n * (a.rank + 1) / a.nranks;
   for (int64_t t0 = s0 + (int64_t)blockIdx.x * MMQ_GAMMA_THREADS; t0 < s1; t0 += (int64_t)gridDim.x * MMQ_GAMMA_THREADS) {
     const int64_t t = t0 + threadIdx.x < s1 ? t0 + threadIdx.x : -1;
     int32_t c = 0;
     double rate = 1.0;
     if (t >= 0) {
-      int32_t v[MMQ_P2P_MAX];
-#pragma unroll
-      for (int r = 0; r < MMQ_P2P_MAX; ++r) v[r] = r < a.nranks ? __ldcv(reinterpret_cast<const int32_t*>(a.base[r] + a.off_counts) + t) : 0;
-#pragma unroll
-      for (int r = 0; r < MMQ_P2P_MAX; ++r) c += v[r];
+      c = p2p_count(a, t);
       rate = beta + len[t];
     }
     const double v = gamma_block(S, t, c, rate, alpha, seed, sweep);
@@ -964,7 +920,7 @@ k_gamma_rs(mmq_p2p_args a, const int32_t* __restrict__ counts_base, const double
 __global__ void k_trace_capture(const double* __restrict__ mu, double* __restrict__ trace, int stride, int trace_len, int64_t n,
                                 uint32_t sweep, const uint32_t* __restrict__ sweep_base) {
   if (sweep_base) sweep += *sweep_base;
-  if (sweep % (uint32_t)stride != 0 || sweep / (uint32_t)stride >= (uint32_t)trace_len) return;
+  if (!trace_recorded(sweep, stride, trace_len)) return;
   double* col = trace + sweep / (uint32_t)stride;
   for (int64_t t = blockIdx.x * (int64_t)blockDim.x + threadIdx.x; t < n; t += (int64_t)gridDim.x * blockDim.x)
     col[t * (int64_t)trace_len] = mu[t];
@@ -1580,6 +1536,64 @@ static int count_groups_step(mmq_handle* h, const uint32_t* sweep_base) {
   MMQ_LAUNCHED(h);
   return MMQ_OK;
 }
+/* K4 of a sweep: the k_gamma instantiation for the handle (accumulating or not, own counts or the peers' in a), or the
+ * reduce-scatter kernel and its trace capture. */
+static int launch_gamma(mmq_handle* h, const mmq_p2p_args& a, uint32_t seed, uint32_t sweep, int stride, int32_t* counts_copy,
+                        const uint32_t* sweep_base) {
+  const bool p2p = h->p2p_n > 1;
+  if (p2p && !counts_copy && h->exchange_rs == 1) { /* mmq_tune(h, 6, 1): reduce-scatter + Gamma + all-gather */
+    /* the all-reduce is the default: the Gamma kernel is bound by the latency of one pass, not by throughput, so
+     * drawing n / N variates instead of n saves nothing, while this variant pays a second barrier and the peer stores
+     * (DESIGN §7) */
+    const int64_t slice = (h->n + h->p2p_n - 1) / h->p2p_n;
+    k_gamma_rs<<<mmq_grid_for(std::max<int64_t>(slice, h->n / 8), MMQ_GAMMA_THREADS, h->num_sms * 4), MMQ_GAMMA_THREADS, 0, h->stream>>>(a, h->seg_base, h->len, h->n, h->alpha, h->beta, seed, sweep, sweep_base);
+    MMQ_LAUNCHED(h);
+    /* is this sweep recorded?  plain launch: the host knows; graph capture: sweep = j, the replays start at
+     * sweeps congruent to capture_phase modulo the stride (the kernel re-checks against the real sweep number) */
+    if (stride > 0 && h->trace &&
+        (sweep_base ? ((uint32_t)h->capture_phase + sweep) % (uint32_t)stride == 0 : trace_recorded(sweep, stride, h->trace_len))) {
+      k_trace_capture<<<mmq_grid_for(h->n, 256, h->num_sms * 4), 256, 0, h->stream>>>(h->mu, h->trace, stride, h->trace_len, h->n, sweep, sweep_base);
+      MMQ_LAUNCHED(h);
+    }
+    return MMQ_OK;
+  }
+  const int grid = mmq_grid_for(h->n, MMQ_GAMMA_THREADS, h->num_sms * 5);
+  auto go = [&](auto kernel, const auto& src) {
+    kernel<<<grid, MMQ_GAMMA_THREADS, 0, h->stream>>>(src, h->seg_base, h->len, h->mu, stride > 0 ? h->trace : nullptr, stride, h->trace_len, h->n,
+                                                      h->alpha, h->beta, seed, sweep, counts_copy, sweep_base, count_args(h));
+  };
+  if (p2p) h->cnt_block ? go(k_gamma<true, true>, a) : go(k_gamma<false, true>, a);
+  else h->cnt_block ? go(k_gamma<true, false>, h->counts) : go(k_gamma<false, false>, h->counts);
+  MMQ_LAUNCHED(h);
+  return count_groups_step(h, sweep_base);
+}
+/* The peer-memory exchange of the next sweep: this epoch's parity buffers; advances the epoch. */
+static mmq_p2p_args p2p_args(mmq_handle* h, const int32_t* epoch_base) {
+  const int b = h->p2p_epoch & 1;
+  mmq_p2p_args a;
+  for (int r = 0; r < MMQ_P2P_MAX; ++r) a.base[r] = r < h->p2p_n ? h->p2p_base[r] : nullptr;
+  a.off_counts = (int64_t)p2p_off_counts(h, b);
+  a.off_reset = (int64_t)p2p_off_counts(h, b ^ 1);
+  a.off_mu = (int64_t)p2p_off_mu(h);
+  a.nranks = h->p2p_n; a.rank = h->p2p_rank;
+  ++h->p2p_epoch;
+  /* inside a graph capture the epoch is relative to the device counter that the graph advances */
+  a.epoch = epoch_base ? (int32_t)(h->p2p_epoch - h->graph_epoch0) : (int32_t)h->p2p_epoch;
+  a.epoch_base = epoch_base;
+  return a;
+}
+/* K2 on the per-fragment layout without multiplicities (k_alloc_cat); it visits the singletons itself. */
+template <bool HAS_W>
+static int launch_alloc_cat(mmq_handle* h, uint32_t seed, uint32_t sweep, const uint32_t* sweep_base) {
+  constexpr int SLAB = HAS_W ? MMQ_CAT_SLAB_W : MMQ_CAT_SLAB;
+  constexpr int SM = MMQ_CAT_WARPS * (16 + 2 * SLAB * 4 * (HAS_W ? 2 : 1));
+  MMQ_CUDA(h, cudaFuncSetAttribute(k_alloc_cat<HAS_W, SLAB>, cudaFuncAttributeMaxDynamicSharedMemorySize, SM));
+  const int64_t n_chunks = (h->m + MMQ_CAT_ROWS - 1) / MMQ_CAT_ROWS;
+  const int cgrid = (int)std::min<int64_t>((n_chunks + MMQ_CAT_WARPS - 1) / MMQ_CAT_WARPS, (int64_t)h->num_sms * 3);
+  k_alloc_cat<HAS_W, SLAB><<<cgrid, MMQ_CAT_WARPS * 32, SM, h->stream>>>(h->row_ptr, h->col, h->w, h->mu, h->counts, h->m, n_chunks, seed, sweep,
+                                                                       h->class_id_base, (int32_t)h->n, sweep_base);
+  return MMQ_OK;
+}
 extern "C" {
 
 /* State a sweep builds on first use (synchronising copies, allocations): done ahead of a graph capture. */
@@ -1597,7 +1611,7 @@ static int prepare_sweep(mmq_handle* h, int flags) {
   return MMQ_OK;
 }
 
-/* One sweep on the stream.  trace_col = device address of trace[0*L + slot] or null. */
+/* One sweep on the stream: the allocation launch, the count exchange, the Gamma launch. */
 static int enqueue_sweep(mmq_handle* h, uint32_t seed, uint32_t sweep, int flags, int stride, int32_t* counts_copy, const uint32_t* sweep_base,
                          const int32_t* epoch_base = nullptr) {
   const bool transposed = (flags & MMQ_GIBBS_TRANSPOSED) != 0;
@@ -1631,19 +1645,7 @@ static int enqueue_sweep(mmq_handle* h, uint32_t seed, uint32_t sweep, int flags
         g_mmq_launches.fetch_sub(1, std::memory_order_relaxed); /* counted inside; MMQ_LAUNCHED below adds one */
       } else if (!h->has_k && !(flags & MMQ_GIBBS_GENERIC_KERNEL)) {
         if ((rc = mmq_seg_add_base(h, false))) return rc; /* this kernel visits the singletons itself */
-        const int64_t n_chunks = (h->m + MMQ_CAT_ROWS - 1) / MMQ_CAT_ROWS;
-        const int64_t want = (n_chunks + MMQ_CAT_WARPS - 1) / MMQ_CAT_WARPS;
-        if (h->has_w) {
-          constexpr int SM = MMQ_CAT_WARPS * (16 + 2 * MMQ_CAT_SLAB_W * 4 * 2);
-          MMQ_CUDA(h, cudaFuncSetAttribute(k_alloc_cat<true, MMQ_CAT_SLAB_W>, cudaFuncAttributeMaxDynamicSharedMemorySize, SM));
-          const int cgrid = (int)std::min<int64_t>(want, (int64_t)h->num_sms * 3);
-          k_alloc_cat<true, MMQ_CAT_SLAB_W><<<cgrid, MMQ_CAT_WARPS * 32, SM, h->stream>>>(h->row_ptr, h->col, h->w, h->mu, h->counts, h->m, n_chunks, seed, sweep, h->class_id_base, (int32_t)h->n, sweep_base);
-        } else {
-          constexpr int SM = MMQ_CAT_WARPS * (16 + 2 * MMQ_CAT_SLAB * 4);
-          MMQ_CUDA(h, cudaFuncSetAttribute(k_alloc_cat<false, MMQ_CAT_SLAB>, cudaFuncAttributeMaxDynamicSharedMemorySize, SM));
-          const int cgrid = (int)std::min<int64_t>(want, (int64_t)h->num_sms * 3);
-          k_alloc_cat<false, MMQ_CAT_SLAB><<<cgrid, MMQ_CAT_WARPS * 32, SM, h->stream>>>(h->row_ptr, h->col, h->w, h->mu, h->counts, h->m, n_chunks, seed, sweep, h->class_id_base, (int32_t)h->n, sweep_base);
-        }
+        if ((rc = h->has_w ? launch_alloc_cat<true>(h, seed, sweep, sweep_base) : launch_alloc_cat<false>(h, seed, sweep, sweep_base))) return rc;
       } else {
         if ((rc = mmq_seg_add_base(h, false))) return rc;
         launch_alloc_t<false>(h, grid, seed, sweep, sweep_base);
@@ -1652,64 +1654,16 @@ static int enqueue_sweep(mmq_handle* h, uint32_t seed, uint32_t sweep, int flags
       mark(h->ev_alloc);
     }
   }
-  if (h->p2p_n > 1) { /* count exchange and Gamma update fused over peer memory */
-    const int b = h->p2p_epoch & 1;
-    mmq_p2p_args a;
-    for (int r = 0; r < MMQ_P2P_MAX; ++r) a.base[r] = r < h->p2p_n ? h->p2p_base[r] : nullptr;
-    a.off_counts = (int64_t)p2p_off_counts(h, b);
-    a.off_reset = (int64_t)p2p_off_counts(h, b ^ 1);
-    a.off_mu = (int64_t)p2p_off_mu(h);
-    a.nranks = h->p2p_n; a.rank = h->p2p_rank;
-    ++h->p2p_epoch;
-    /* inside a graph capture the epoch is relative to the device counter that the graph advances */
-    a.epoch = epoch_base ? (int32_t)(h->p2p_epoch - h->graph_epoch0) : (int32_t)h->p2p_epoch;
-    a.epoch_base = epoch_base;
-    mark(h->ev_gamma);
-    if (counts_copy || h->exchange_rs != 1) {
-      /* default: every rank reads the count vectors of all ranks and draws every Gamma variate — ONE barrier per sweep.
-       * (The Gamma kernel is bound by the latency of one pass, not by throughput, so drawing n / N variates instead of
-       * n saves nothing, while the reduce-scatter variant below pays a second barrier and the peer stores: measured at
-       * N = 2, 36 us against 24 us per sweep.) */
-      const int ggrid = mmq_grid_for(h->n, MMQ_GAMMA_THREADS, h->num_sms * 5);
-      if (h->cnt_block)
-        k_gamma_p2p_acc<<<ggrid, MMQ_GAMMA_THREADS, 0, h->stream>>>(a, h->seg_base, h->len, h->mu, stride > 0 ? h->trace : nullptr, stride,
-                                                                    h->trace_len, h->n, h->alpha, h->beta, seed, sweep, counts_copy, sweep_base, count_args(h));
-      else
-        k_gamma_p2p<<<ggrid, MMQ_GAMMA_THREADS, 0, h->stream>>>(a, h->seg_base, h->len, h->mu, stride > 0 ? h->trace : nullptr, stride,
-                                                                h->trace_len, h->n, h->alpha, h->beta, seed, sweep, counts_copy, sweep_base);
-      MMQ_LAUNCHED(h);
-      if ((rc = count_groups_step(h, sweep_base))) return rc;
-    } else { /* mmq_tune(h, 6, 1): reduce-scatter + Gamma + all-gather */
-      const int64_t slice = (h->n + h->p2p_n - 1) / h->p2p_n;
-      k_gamma_rs<<<mmq_grid_for(std::max<int64_t>(slice, h->n / 8), MMQ_GAMMA_THREADS, h->num_sms * 4), MMQ_GAMMA_THREADS, 0, h->stream>>>(a, h->seg_base, h->len, h->n, h->alpha, h->beta, seed, sweep, sweep_base);
-      MMQ_LAUNCHED(h);
-      /* is this sweep recorded?  plain launch: the host knows; graph capture: sweep = j, the replays start at
-       * sweeps congruent to capture_phase modulo the stride (the kernel re-checks against the real sweep number) */
-      const bool recorded = sweep_base ? (((uint32_t)h->capture_phase + sweep) % (uint32_t)std::max(stride, 1) == 0)
-                                       : (sweep % (uint32_t)std::max(stride, 1) == 0 && sweep / (uint32_t)std::max(stride, 1) < (uint32_t)h->trace_len);
-      if (stride > 0 && h->trace && recorded) {
-        k_trace_capture<<<mmq_grid_for(h->n, 256, h->num_sms * 4), 256, 0, h->stream>>>(h->mu, h->trace, stride, h->trace_len, h->n, sweep, sweep_base);
-        MMQ_LAUNCHED(h);
-      }
-    }
-    mark(h->ev_gamma);
-    h->counts = h->p2p_counts[h->p2p_epoch & 1]; /* the next sweep reduces into the other parity buffer */
-    if (h->seg_base) h->seg_base_in_counts = true;
-    return MMQ_OK;
-  }
-  if ((rc = mmq_allreduce(h, h->counts, (size_t)h->n, 0))) return rc;
+  /* the count exchange: fused into the Gamma kernel over peer memory, else an all-reduce (a no-op on one GPU) */
+  const bool p2p = h->p2p_n > 1;
+  mmq_p2p_args a{};
+  if (p2p) a = p2p_args(h, epoch_base);
+  else if ((rc = mmq_allreduce(h, h->counts, (size_t)h->n, 0))) return rc;
   mark(h->ev_gamma);
-  const int ggrid = mmq_grid_for(h->n, MMQ_GAMMA_THREADS, h->num_sms * 5);
-  if (h->cnt_block)
-    k_gamma_acc<<<ggrid, MMQ_GAMMA_THREADS, 0, h->stream>>>(h->counts, h->seg_base, h->len, h->mu, stride > 0 ? h->trace : nullptr, stride, h->trace_len, h->n,
-                                                            h->alpha, h->beta, seed, sweep, counts_copy, sweep_base, count_args(h));
-  else
-    k_gamma<<<ggrid, MMQ_GAMMA_THREADS, 0, h->stream>>>(h->counts, h->seg_base, h->len, h->mu, stride > 0 ? h->trace : nullptr, stride, h->trace_len, h->n,
-                                                        h->alpha, h->beta, seed, sweep, counts_copy, sweep_base);
-  MMQ_LAUNCHED(h);
-  if ((rc = count_groups_step(h, sweep_base))) return rc;
+  if ((rc = launch_gamma(h, a, seed, sweep, stride, counts_copy, sweep_base))) return rc;
   mark(h->ev_gamma);
-  if (h->seg_base) h->seg_base_in_counts = true; /* k_gamma restarted counts[] from seg_base */
+  if (p2p) h->counts = h->p2p_counts[h->p2p_epoch & 1]; /* the next sweep reduces into the other parity buffer */
+  if (h->seg_base) h->seg_base_in_counts = true; /* the Gamma kernel restarted counts[] from seg_base */
   return MMQ_OK;
 }
 

@@ -75,8 +75,8 @@ def test_two_ranks_reproduce_single_gpu_chain(use_p2p):
 
 
 # padded: the length array has 3 x 189,440 + 77 transcripts, most of them without hits, so that the fused Gamma kernels
-# loop: k_gamma_p2p runs min(n / 256, 5 sms) CTAs and k_gamma_rs min(max(n / ranks, n / 8) / 256, 4 sms) CTAs of 256
-# threads (mmq_core.cu:1570,1575).  rs: mmq_tune knob 6, the reduce-scatter exchange (k_gamma_rs + k_trace_capture).
+# loop: k_gamma<ACC, true> runs min(n / 256, 5 sms) CTAs and k_gamma_rs min(max(n / ranks, n / 8) / 256, 4 sms) CTAs of 256
+# threads (launch_gamma in mmq_core.cu).  rs: mmq_tune knob 6, the reduce-scatter exchange (k_gamma_rs + k_trace_capture).
 @pytest.mark.parametrize("weighted,padded,rs", [(False, False, False), (True, False, False), (False, True, False), (True, True, True)],
                          ids=["False", "True", "padded", "padded-rs"])
 def test_single_process_peer_attach_matches_single_gpu(weighted, padded, rs):

@@ -227,7 +227,7 @@ def test_class_plan_kernels_many_chunks_per_warp(monkeypatch, plan, cid_base):
     assert hi >= 2.5 * sms * 5 * MMQ_CLS_WARPS, hi
     assert chain_ch >= 3 * sms * 3 * (MMQ_CHAIN_CLASSES // 32), chain_ch
     assert rest >= 2.5 * sms * 3 * MMQ_ALLOC_WARPS, rest
-    # k_gamma, mmq_core.cu:1593: min(n / 256, 5 sms) CTAs of 256 threads, one transcript per thread and pass
+    # k_gamma (launch_gamma in mmq_core.cu): min(n / 256, 5 sms) CTAs of 256 threads, one transcript per thread and pass
     assert n >= 2.5 * sms * 5 * MMQ_GAMMA_THREADS
     # init and EM accumulation (k_init_acc, k_em_acc): 8 sms CTAs of 8 warps, one warp per transcript
     assert n >= 3 * sms * 8 * 8
