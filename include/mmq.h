@@ -246,6 +246,40 @@ int mmq_prior_draws(int device, int64_t count, const int64_t* ids, const double*
 int mmq_sokal_batch(int device, int64_t rows, int len, const double* x, double* var, double* tau,
                     int32_t* win, int32_t* status);
 
+/* ---- convergence of several independent chains (none in the reference; mmseq -chains) -----------------------------
+ * Seed of chain `chain` (0 <= chain < 8) of a run with seed `seed`: chain 0 is `seed` itself; chain c >= 1 is word 0 of
+ * Philox4x32-10 at counter (c, j, 0, 0) under key (seed, 0x4348414e "CHAN") for the first j whose value differs from the
+ * seeds of chains 0 .. c-1, so the seeds of one run are distinct.  Outside the range: `seed`.  (include/mmq_sampler.h
+ * defines the same function inline for host and device code.) */
+#ifndef MMQ_SAMPLER_H
+uint32_t mmq_chain_seed(uint32_t seed, int chain);
+#endif
+/* Rank-normalised split-R-hat and bulk / tail effective sample size per feature (Vehtari, Gelman, Simpson, Carpenter,
+ * Buerkner 2021, as Stan, ArviZ and the `posterior` R package report them).  chain_dev[c] (a host array of device
+ * pointers): chain c's draws [row * L + s], the mmq_get_trace layout, all on the calling device; 2 <= nchains <= 8, L a
+ * power of two in [8, 2048], nchains * L <= 8192, else MMQ_ERR_ARG.  out_dev: fp64[5 * rows], [q * rows + row] for
+ * q = 0 rhat, 1 ess_bulk, 2 ess_tail, 3 log_mean, 4 log_sd.  Asynchronous on cuda_stream, no allocation; one CTA per
+ * feature, grid min(rows, 2 x SMs); every value is fp64 and independent of the grid and of the row order.
+ * Definitions, for one feature's draws x[c][s] (S = nchains L draws), split into M = 2 nchains chains of N = L/2,
+ * y[2c+h][i] = x[c][h N + i]:
+ *   any x NaN or +-inf: all five outputs NaN;
+ *   z(v) = Phi^-1((r - 3/8) / (S + 1/4)), r the average rank of each value among all S (ties share the mean rank);
+ *   split R-hat(y): m_j, w_j the split chains' means and variances (ddof 1; a chain of equal values: that value and 0),
+ *     W = mean w_j, B = N var(m_j, ddof 1), R-hat = sqrt(((N-1)/N W + B/N) / W), NaN when W = 0;
+ *   rhat = max(R-hat(z(x)), R-hat(z(|x - med|))), med the median of all S draws; NaN when either is NaN;
+ *   ess(y): Geyer's initial monotone sequence over the split chains' autocovariances, as Stan and ArviZ compute it
+ *     (tests/chain_reference.py spells it out), NaN when all S values of y are equal;
+ *   ess_bulk = ess(z(x)); ess_tail = min(ess(1[x <= q_0.05]), ess(1[x <= q_0.95])), q_p the type-7 quantile of all S
+ *     draws, NaN when either is NaN;
+ *   log_mean, log_sd: mean and sd (S - 1) of log x over all S draws, plain IEEE (a zero draw gives -inf / NaN). */
+int mmq_chain_diagnostics_dev(const double* const* chain_dev, int nchains, int64_t rows, int L, double* out_dev, void* cuda_stream);
+/* The same on the traces the handles recorded (mmq_gibbs with trace_len = L): which 0 transcripts, 1 identical sets,
+ * 2 genes (groups set alike on every handle, mmq_set_groups).  Runs on chains[0]'s device and stream; traces of handles
+ * on other devices are copied there (cudaMemcpyPeerAsync, a workspace of rows L 8 bytes per such chain).  Same n,
+ * trace_len and group counts on every handle, else MMQ_ERR_ARG.  Outputs fp64[rows] on the host; any may be NULL. */
+int mmq_chain_diagnostics(mmq_handle* const* chains, int nchains, int which, double* rhat, double* ess_bulk,
+                          double* ess_tail, double* log_mean, double* log_sd);
+
 /* ---- the consumer of the traces: mmcollapse's covariance step (src/mmcollapse.cpp:483-561) ----------
  * The one dense contraction of the package: tensor cores (tcgen05, bf16 split products, fp32 accumulation in
  * TMEM), everything around it fp64.  nsplit = bf16 terms per value (2: the default of the callers here).  Error in

@@ -118,6 +118,27 @@ MMQ_HD void mmq_philox4x32_10(uint32_t ctr[4], uint32_t k0, uint32_t k1) {
   ctr[0] = c0; ctr[1] = c1; ctr[2] = c2; ctr[3] = c3;
 }
 
+/* Seed of chain `chain` (0 <= chain < MMQ_CHAINS_MAX) of a run with several independent Gibbs chains (mmseq -chains):
+ * chain 0 is `seed` itself, so a single chain is the chain of the run without chains.  Chain c >= 1 takes word 0 of
+ * Philox4x32-10 at counter (c, j, 0, 0) under key (seed, MMQ_STREAM_CHAIN), for the first j = 0, 1, ... whose value
+ * differs from the seeds of chains 0 .. c-1: the seeds of one run are distinct.  A chain outside the range gets `seed`. */
+#define MMQ_STREAM_CHAIN 0x4348414eu /* "CHAN" */
+#define MMQ_CHAINS_MAX 8
+MMQ_HD uint32_t mmq_chain_seed(uint32_t seed, int chain) {
+  if (chain <= 0 || chain >= MMQ_CHAINS_MAX) return seed;
+  uint32_t s[MMQ_CHAINS_MAX];
+  s[0] = seed;
+  for (int c = 1; c <= chain; ++c)
+    for (uint32_t j = 0;; ++j) {
+      uint32_t w[4] = {(uint32_t)c, j, 0u, 0u};
+      mmq_philox4x32_10(w, seed, MMQ_STREAM_CHAIN);
+      int dup = 0;
+      for (int d = 0; d < c; ++d) dup |= w[0] == s[d];
+      if (!dup) { s[c] = w[0]; break; }
+    }
+  return s[chain];
+}
+
 /* A stream = (seed, stream tag) key and (id_lo, id_hi, sweep, block) counter.
  * Each block yields two 52-bit uniforms; `block` counts upwards from 0, so a
  * draw is a pure function of (seed, stream, id, sweep, how many uniforms the

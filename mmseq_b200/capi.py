@@ -77,6 +77,9 @@ def _load():
         "mmq_prop_summaries": (i32, [vp, vp, vp, vp, vp, vp, i32, vp, vp, vp]),
         "mmq_unique_hits_sets": (i32, [vp, vp, i64, vp]),
         "mmq_sokal_batch": (i32, [i32, i64, i32, vp, vp, vp, vp, vp]),
+        "mmq_chain_seed": (u32, [u32, i32]),
+        "mmq_chain_diagnostics_dev": (i32, [C.POINTER(vp), i32, i64, i32, vp, vp]),
+        "mmq_chain_diagnostics": (i32, [C.POINTER(vp), i32, i32, vp, vp, vp, vp, vp]),
         "mmq_prior_draws": (i32, [i32, i64, vp, vp, dbl, u32, i32, vp]),
         "mmq_trace_cov": (i32, [i32, vp, i32, i64, i32, vp]),
         "mmq_trace_cov_workspace_bytes": (i64, [i32, i64, i32]),
@@ -112,7 +115,7 @@ EXPORTS = [
     "mmq_loglik", "mmq_em", "mmq_gibbs", "mmq_sweep_debug", "mmq_kernel_times", "mmq_cls_stats", "mmq_tune", "mmq_get_trace", "mmq_trace_len",
     "mmq_count_moments_begin", "mmq_count_moments_end", "mmq_get_count_moments", "mmq_expected_counts",
     "mmq_set_groups", "mmq_summarize", "mmq_get_group_trace", "mmq_prop_summaries",
-    "mmq_unique_hits_sets", "mmq_sokal_batch", "mmq_prior_draws", "mmq_trace_cov", "mmq_trace_cov_workspace_bytes", "mmq_trace_cov_dev",
+    "mmq_unique_hits_sets", "mmq_sokal_batch", "mmq_chain_seed", "mmq_chain_diagnostics_dev", "mmq_chain_diagnostics", "mmq_prior_draws", "mmq_trace_cov", "mmq_trace_cov_workspace_bytes", "mmq_trace_cov_dev",
     "mmq_handle_trace_cov", "mmq_mean_corrs", "mmq_mean_corrs_dev", "mmq_release_cache", "mmq_launch_count", "mmq_warmup", "mmq_version",
 ]
 
@@ -157,6 +160,33 @@ def sokal_batch(x, device=0):
     if rc:
         raise MmqError("mmq_sokal_batch: " + lib().mmq_last_error(None).decode())
     return var, tau, win, status
+
+
+CHAIN_OUTPUTS = ("rhat", "ess_bulk", "ess_tail", "log_mean", "log_sd")
+
+
+def chain_seed(seed, chain):
+    """Seed of chain `chain` (0 <= chain < 8) of a run with seed `seed`; chain 0 is `seed`."""
+    return int(lib().mmq_chain_seed(seed, chain))
+
+
+def chain_diagnostics_dev(chain_ptrs, rows, L, out_ptr, stream_ptr):
+    """mmq_chain_diagnostics_dev: chain_ptrs, device pointers (ints) of each chain's [rows, L] fp64 draws; out_ptr:
+    fp64[5 * rows] on the same device.  Asynchronous on the stream."""
+    arr = (C.c_void_p * len(chain_ptrs))(*chain_ptrs)
+    _global_check(lib().mmq_chain_diagnostics_dev(arr, len(chain_ptrs), rows, L, out_ptr, stream_ptr), "mmq_chain_diagnostics_dev")
+
+
+def chain_diagnostics(handles, which=0):
+    """mmq_chain_diagnostics over the traces the handles recorded: dict of CHAIN_OUTPUTS, fp64[rows] each."""
+    h0 = handles[0]
+    rows = h0.n if which == 0 else h0._ng[which - 1]
+    out = {k: np.zeros(rows) for k in CHAIN_OUTPUTS}
+    arr = (C.c_void_p * len(handles))(*[h._h for h in handles])
+    rc = lib().mmq_chain_diagnostics(arr, len(handles), which, *[_ptr(out[k]) for k in CHAIN_OUTPUTS])
+    if rc:
+        raise MmqError(f"mmq_chain_diagnostics failed ({rc}): " + lib().mmq_last_error(h0._h).decode())
+    return out
 
 
 def _global_check(rc, what):

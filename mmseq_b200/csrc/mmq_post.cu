@@ -232,6 +232,258 @@ __global__ void k_prior(const int64_t* __restrict__ ids, const double* __restric
   }
 }
 
+/* ------------------------------------------------ convergence of several chains
+ * Rank-normalised split-R-hat and bulk / tail ESS (Vehtari, Gelman, Simpson, Carpenter, Buerkner 2021), one CTA per
+ * feature.  Definitions: include/mmq.h (mmq_chain_diagnostics_dev); tests/chain_reference.py restates them in numpy.
+ * Shared memory, P = the power of two >= S = C L draws:  key fp64[P] | z fp64[S] | idx int32[P] | run int32[S].
+ * key/idx: the (value, draw) pairs being sorted; z: the series under study, in draw order; run: the first sorted
+ * position of each value's run of ties.  The ESS step reuses key as the FFT's (re, im), idx as the summed
+ * autocovariance and run as the autocorrelation sequence: 12 (P + S) bytes in all, 192 KB at S = 8192. */
+#define MMQ_CHAIN_SMAX 8192
+
+struct mmq_chain_ptrs { const double* p[MMQ_CHAINS_MAX]; };
+
+static int chain_pow2_at_least(int s) { int p = 1; while (p < s) p <<= 1; return p; }
+static size_t chain_smem_bytes(int S) { return (size_t)12 * (size_t)(chain_pow2_at_least(S) + S); }
+
+/* draw k (< S) of the row: chain k >> lgL, sweep slot k & (L - 1) */
+__device__ __forceinline__ double chain_x(const mmq_chain_ptrs& cp, int64_t row, int lgL, int k) {
+  return cp.p[k >> lgL][(row << lgL) + (k & ((1 << lgL) - 1))];
+}
+
+/* bitonic sort of (key, idx) pairs, ascending by key then idx; P a power of two */
+__device__ __forceinline__ void chain_sort(double* key, int32_t* idx, int P) {
+  __syncthreads();
+  for (int k = 2; k <= P; k <<= 1)
+    for (int j = k >> 1; j > 0; j >>= 1) {
+      for (int i = threadIdx.x; i < P; i += blockDim.x) {
+        const int p = i ^ j;
+        if (p > i) {
+          const double a = key[i], b = key[p];
+          const int32_t ia = idx[i], ib = idx[p];
+          const bool gt = a > b || (a == b && ia > ib);
+          if (gt == ((i & k) == 0)) { key[i] = b; key[p] = a; idx[i] = ib; idx[p] = ia; }
+        }
+      }
+      __syncthreads();
+    }
+}
+
+/* z[draw] = Phi^-1((r - 3/8) / (S + 1/4)), r the average 1-based rank of the draw's value among the S sorted keys.
+ * Each thread owns a contiguous range of sorted positions; the run of ties that crosses into it from the left (right)
+ * starts (ends) at the last head (first tail) of the threads before (after) it. */
+__device__ __forceinline__ void chain_rank_normalise(const double* key, const int32_t* idx, int32_t* run, double* z, int S) {
+  __shared__ int32_t s_head[MMQ_POST_THREADS], s_tail[MMQ_POST_THREADS];
+  const int T = blockDim.x, t = threadIdx.x;
+  const int chunk = (S + T - 1) / T;
+  const int a = min(S, t * chunk), b = min(S, a + chunk);
+  auto head = [&](int i) { return i == 0 || key[i] != key[i - 1]; };
+  auto tail = [&](int i) { return i == S - 1 || key[i] != key[i + 1]; };
+  int last_head = -1, first_tail = 0x7fffffff;
+  for (int i = a; i < b; ++i) if (head(i)) last_head = i;
+  for (int i = b - 1; i >= a; --i) if (tail(i)) first_tail = i;
+  s_head[t] = last_head;
+  s_tail[t] = first_tail;
+  __syncthreads();
+  if (t == 0) { /* exclusive prefix max of the heads, exclusive suffix min of the tails */
+    int c = -1;
+    for (int u = 0; u < T; ++u) { const int v = s_head[u]; s_head[u] = c; c = max(c, v); }
+    c = 0x7fffffff;
+    for (int u = T - 1; u >= 0; --u) { const int v = s_tail[u]; s_tail[u] = c; c = min(c, v); }
+  }
+  __syncthreads();
+  int start = s_head[t];
+  for (int i = a; i < b; ++i) { if (head(i)) start = i; run[i] = start; }
+  int end = s_tail[t];
+  const double denom = (double)S + 0.25;
+  for (int i = b - 1; i >= a; --i) {
+    if (tail(i)) end = i;
+    const double r = 0.5 * (double)(run[i] + end + 2);
+    z[idx[i]] = mmq_ndtri((r - 0.375) / denom);
+  }
+  __syncthreads();
+}
+
+/* mean and variance (ddof 1) of each of the M split chains y[j N .. j N + N), one warp per chain.  A split chain whose
+ * values are all equal has exactly that mean and variance 0. */
+__device__ __forceinline__ void chain_split_moments(const double* y, int M, int N, double* s_m, double* s_w) {
+  const int lane = threadIdx.x & 31, nw = blockDim.x >> 5;
+  for (int j = threadIdx.x >> 5; j < M; j += nw) {
+    const double* q = y + (size_t)j * N;
+    const double y0 = q[0];
+    double s = 0.0;
+    bool same = true;
+    for (int i = lane; i < N; i += 32) { s += q[i]; same &= q[i] == y0; }
+    s = post_warp_sum(s);
+    same = __all_sync(0xffffffffu, same);
+    const double m = same ? y0 : __shfl_sync(0xffffffffu, s, 0) / (double)N;
+    double v = 0.0;
+    if (!same) {
+      for (int i = lane; i < N; i += 32) { const double d = q[i] - m; v += d * d; }
+      v = post_warp_sum(v);
+    }
+    if (lane == 0) { s_m[j] = m; s_w[j] = same ? 0.0 : v / (double)(N - 1); }
+  }
+  __syncthreads();
+}
+
+/* split R-hat from the split chains' moments; NaN when the within-chain variance W is 0 */
+__device__ __forceinline__ double chain_rhat(const double* s_m, const double* s_w, int M, int N) {
+  double W = 0.0, mm = 0.0, B = 0.0;
+  for (int j = 0; j < M; ++j) { W += s_w[j]; mm += s_m[j]; }
+  W /= (double)M;
+  mm /= (double)M;
+  for (int j = 0; j < M; ++j) { const double d = s_m[j] - mm; B += d * d; }
+  B = (double)N * (B / (double)(M - 1));
+  if (W == 0.0) return mmq_u2d(0x7ff8000000000000ull);
+  return sqrt((((double)(N - 1) / (double)N) * W + B / (double)N) / W);
+}
+
+/* ESS of the split chains y (moments s_m from chain_split_moments): autocovariances by FFT (zero-padded to 2N = L,
+ * as k_row_sokal), then Geyer's initial monotone sequence.  The result is valid in thread 0; NaN when `constant`. */
+__device__ __forceinline__ double chain_ess(const double* y, int M, int N, const double* s_m, bool constant, double* key, int32_t* idx_area,
+                            int32_t* run_area) {
+  const int L = 2 * N;
+  double* re = key;
+  double* im = key + L;
+  double* acc = reinterpret_cast<double*>(idx_area); /* sum over split chains of L * sum_i yc[i] yc[i + t] */
+  double* r = reinterpret_cast<double*>(run_area);
+  double out = mmq_u2d(0x7ff8000000000000ull);
+  if (constant) return out;
+  for (int t = threadIdx.x; t < N; t += blockDim.x) acc[t] = 0.0;
+  for (int j = 0; j < M; ++j) {
+    for (int i = threadIdx.x; i < L; i += blockDim.x) {
+      re[i] = i < N ? y[(size_t)j * N + i] - s_m[j] : 0.0;
+      im[i] = 0.0;
+    }
+    __syncthreads();
+    smem_fft(re, im, L, true);
+    for (int i = threadIdx.x; i < L; i += blockDim.x) {
+      re[i] = re[i] * re[i] + im[i] * im[i];
+      im[i] = 0.0;
+    }
+    __syncthreads();
+    smem_fft(re, im, L, false);
+    for (int t = threadIdx.x; t < N; t += blockDim.x) acc[t] += re[t];
+    __syncthreads();
+  }
+  if (threadIdx.x == 0) {
+    const double scale = 1.0 / ((double)M * (double)L * (double)N); /* acc -> mean over chains of acov_j */
+    double mm = 0.0, vm = 0.0;
+    for (int j = 0; j < M; ++j) mm += s_m[j];
+    mm /= (double)M;
+    for (int j = 0; j < M; ++j) { const double d = s_m[j] - mm; vm += d * d; }
+    vm /= (double)(M - 1);
+    const double mean_var = acc[0] * scale * ((double)N / (double)(N - 1));
+    const double var_plus = mean_var * ((double)(N - 1) / (double)N) + vm;
+    if (var_plus > 0.0) {
+      auto rho = [&](int t) { return 1.0 - (mean_var - acc[t] * scale) / var_plus; };
+      for (int t = 0; t < N; ++t) r[t] = 0.0;
+      r[0] = 1.0;
+      r[1] = rho(1);
+      double even = 1.0, odd = r[1];
+      int t = 1;
+      while (t < N - 3 && even + odd > 0.0) {
+        even = rho(t + 1);
+        odd = rho(t + 2);
+        if (even + odd >= 0.0) { r[t + 1] = even; r[t + 2] = odd; }
+        t += 2;
+      }
+      const int max_t = t - 2;
+      if (even > 0.0) r[max_t + 1] = even;
+      for (t = 1; t <= max_t - 2; t += 2)
+        if (r[t + 1] + r[t + 2] > r[t - 1] + r[t]) { r[t + 1] = (r[t - 1] + r[t]) / 2.0; r[t + 2] = r[t + 1]; }
+      double sum = 0.0;
+      for (t = 0; t <= max_t; ++t) sum += r[t];
+      const double SN = (double)M * (double)N;
+      double tau = -1.0 + 2.0 * sum + r[max_t + 1];
+      const double floor_tau = 1.0 / log10(SN);
+      if (tau < floor_tau) tau = floor_tau;
+      out = SN / tau;
+    }
+  }
+  __syncthreads(); /* the scratch areas are free again */
+  return out;
+}
+
+__global__ void __launch_bounds__(MMQ_POST_THREADS)
+k_chain_diag(const __grid_constant__ mmq_chain_ptrs cp, int C, int64_t rows, int lgL, double* __restrict__ out) {
+  extern __shared__ double sh[];
+  __shared__ double s_m[2 * MMQ_CHAINS_MAX], s_w[2 * MMQ_CHAINS_MAX];
+  const int L = 1 << lgL, N = L >> 1, M = 2 * C, S = C * L;
+  int P = 1;
+  while (P < S) P <<= 1;
+  double* key = sh;
+  double* z = sh + P;
+  int32_t* idx = reinterpret_cast<int32_t*>(sh + P + S);
+  int32_t* run = idx + P;
+  const double nan = mmq_u2d(0x7ff8000000000000ull), inf = mmq_u2d(0x7ff0000000000000ull);
+  for (int64_t row = blockIdx.x; row < rows; row += gridDim.x) {
+    /* finiteness and the log-scale mean */
+    double bad = 0.0, ls = 0.0;
+    for (int k = threadIdx.x; k < S; k += blockDim.x) {
+      const double x = chain_x(cp, row, lgL, k);
+      bad += isfinite(x) ? 0.0 : 1.0;
+      ls += log(x);
+    }
+    bad = post_block_sum(bad);
+    if (bad > 0.0) {
+      if (threadIdx.x == 0) for (int q = 0; q < 5; ++q) out[q * rows + row] = nan;
+      continue;
+    }
+    ls = post_block_sum(ls);
+    const double log_mean = ls / (double)S;
+    double lv = 0.0;
+    for (int k = threadIdx.x; k < S; k += blockDim.x) { const double d = log(chain_x(cp, row, lgL, k)) - log_mean; lv += d * d; }
+    lv = post_block_sum(lv);
+    const double log_sd = sqrt(lv / (double)(S - 1));
+
+    /* bulk: rank-normalised draws */
+    for (int i = threadIdx.x; i < P; i += blockDim.x) { key[i] = i < S ? chain_x(cp, row, lgL, i) : inf; idx[i] = i; }
+    chain_sort(key, idx, P);
+    const double med = 0.5 * (key[S / 2 - 1] + key[S / 2]);
+    auto quantile = [&](double p) { /* type 7 */
+      const double h = (double)(S - 1) * p, f = floor(h);
+      const int lo = (int)f;
+      return key[lo] + (h - f) * (key[lo + 1] - key[lo]);
+    };
+    const double q05 = quantile(0.05), q95 = quantile(0.95);
+    bool constant = key[0] == key[S - 1];
+    chain_rank_normalise(key, idx, run, z, S);
+    chain_split_moments(z, M, N, s_m, s_w);
+    const double rhat_bulk = chain_rhat(s_m, s_w, M, N);
+    const double ess_bulk = chain_ess(z, M, N, s_m, constant, key, idx, run);
+
+    /* folded: rank-normalised |x - median| */
+    for (int i = threadIdx.x; i < P; i += blockDim.x) { key[i] = i < S ? fabs(chain_x(cp, row, lgL, i) - med) : inf; idx[i] = i; }
+    chain_sort(key, idx, P);
+    chain_rank_normalise(key, idx, run, z, S);
+    chain_split_moments(z, M, N, s_m, s_w);
+    const double rhat_fold = chain_rhat(s_m, s_w, M, N);
+
+    /* tails: indicators of x <= q05 and x <= q95 */
+    double ess_tail = inf;
+    for (int side = 0; side < 2; ++side) {
+      const double q = side ? q95 : q05;
+      double cnt = 0.0;
+      for (int k = threadIdx.x; k < S; k += blockDim.x) { z[k] = chain_x(cp, row, lgL, k) <= q ? 1.0 : 0.0; cnt += z[k]; }
+      cnt = post_block_sum(cnt); /* also orders the writes of z */
+      constant = cnt == 0.0 || cnt == (double)S;
+      chain_split_moments(z, M, N, s_m, s_w);
+      const double e = chain_ess(z, M, N, s_m, constant, key, idx, run);
+      ess_tail = (isnan(e) || isnan(ess_tail)) ? nan : fmin(ess_tail, e);
+    }
+    if (threadIdx.x == 0) {
+      out[row] = (isnan(rhat_bulk) || isnan(rhat_fold)) ? nan : fmax(rhat_bulk, rhat_fold);
+      out[rows + row] = ess_bulk;
+      out[2 * rows + row] = ess_tail;
+      out[3 * rows + row] = log_mean;
+      out[4 * rows + row] = log_sd;
+    }
+    __syncthreads();
+  }
+}
+
 /* ------------------------------------------------------------------ host */
 
 static bool pow2_ok(int len) { return len >= 4 && len <= MMQ_MAX_ROW_LEN && (len & (len - 1)) == 0; }
@@ -474,5 +726,92 @@ int mmq_sokal_batch(int device, int64_t rows, int len, const double* x, double* 
   cudaFree(d_x);
   return ret;
 }
+
+int mmq_chain_diagnostics_dev(const double* const* chain_dev, int nchains, int64_t rows, int L, double* out_dev, void* cuda_stream) {
+  if (!chain_dev || nchains < 2 || nchains > MMQ_CHAINS_MAX || rows < 0 || L < 8 || L > MMQ_MAX_ROW_LEN || (L & (L - 1)) != 0 ||
+      nchains * L > MMQ_CHAIN_SMAX || (rows > 0 && !out_dev))
+    return mmq_fail(nullptr, MMQ_ERR_ARG, "mmq_chain_diagnostics_dev: bad arguments");
+  mmq_chain_ptrs cp = {};
+  for (int c = 0; c < nchains; ++c) {
+    if (!chain_dev[c]) return mmq_fail(nullptr, MMQ_ERR_ARG, "mmq_chain_diagnostics_dev: NULL chain");
+    cp.p[c] = chain_dev[c];
+  }
+  if (rows == 0) return MMQ_OK;
+  int dev = 0, sms = 0, lgL = 0;
+  while ((1 << lgL) < L) ++lgL;
+  const size_t smem = chain_smem_bytes(nchains * L);
+  cudaError_t e = cudaGetDevice(&dev);
+  if (e == cudaSuccess) e = cudaDeviceGetAttribute(&sms, cudaDevAttrMultiProcessorCount, dev);
+  if (e == cudaSuccess) e = cudaFuncSetAttribute(k_chain_diag, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem);
+  if (e != cudaSuccess) return mmq_cuda_fail(nullptr, e, "mmq_chain_diagnostics_dev", __FILE__, __LINE__);
+  const int grid = (int)std::min<int64_t>(rows, 2 * (int64_t)sms);
+  k_chain_diag<<<grid, MMQ_POST_THREADS, smem, (cudaStream_t)cuda_stream>>>(cp, nchains, rows, lgL, out_dev);
+  g_mmq_launches.fetch_add(1);
+  e = cudaGetLastError();
+  if (e != cudaSuccess) return mmq_cuda_fail(nullptr, e, "k_chain_diag", __FILE__, __LINE__);
+  return MMQ_OK;
+}
+
+int mmq_chain_diagnostics(mmq_handle* const* chains, int nchains, int which, double* rhat, double* ess_bulk, double* ess_tail,
+                          double* log_mean, double* log_sd) {
+  if (!chains || nchains < 2 || nchains > MMQ_CHAINS_MAX || which < 0 || which > 2)
+    return mmq_fail(chains ? chains[0] : nullptr, MMQ_ERR_ARG, "mmq_chain_diagnostics: bad arguments");
+  for (int c = 0; c < nchains; ++c)
+    if (!chains[c]) return mmq_fail(nullptr, MMQ_ERR_ARG, "mmq_chain_diagnostics: NULL handle");
+  mmq_handle* h0 = chains[0];
+  for (int c = 0; c < nchains; ++c) {
+    mmq_handle* h = chains[c];
+    if (!h->trace) return mmq_fail(h0, MMQ_ERR_STATE, "mmq_chain_diagnostics: a chain has no trace recorded");
+    if (h->n != h0->n || h->trace_len != h0->trace_len || h->groups[0].ngroups != h0->groups[0].ngroups ||
+        h->groups[1].ngroups != h0->groups[1].ngroups)
+      return mmq_fail(h0, MMQ_ERR_ARG, "mmq_chain_diagnostics: the chains differ in n, trace_len or group counts");
+  }
+  const int L = h0->trace_len;
+  const int64_t rows = which == 0 ? h0->n : h0->groups[which - 1].ngroups;
+  if (L < 8 || L > MMQ_MAX_ROW_LEN || (L & (L - 1)) != 0 || nchains * L > MMQ_CHAIN_SMAX)
+    return mmq_fail(h0, MMQ_ERR_ARG, "mmq_chain_diagnostics: trace_len must be a power of two in [8, 2048] with nchains * trace_len <= 8192");
+  if (rows == 0) return MMQ_OK;
+  /* every chain's trace complete on its own device */
+  for (int c = 0; c < nchains; ++c) {
+    mmq_handle* h = chains[c];
+    MMQ_CUDA(h0, cudaSetDevice(h->device));
+    if (which > 0) { const int rc = mmq_ensure_trace_groups(h); if (rc) return mmq_fail(h0, rc, mmq_last_error(h)); }
+    MMQ_CUDA(h0, cudaStreamSynchronize(h->stream));
+  }
+  MMQ_CUDA(h0, cudaSetDevice(h0->device));
+  const size_t tbytes = sizeof(double) * (size_t)rows * (size_t)L;
+  int remote = 0;
+  for (int c = 1; c < nchains; ++c) remote += chains[c]->device != h0->device;
+  double *ws = nullptr, *out = nullptr;
+  cudaError_t e = mmq_cache_malloc(&out, sizeof(double) * 5 * (size_t)rows);
+  if (e == cudaSuccess && remote) e = mmq_cache_malloc(&ws, tbytes * (size_t)remote);
+  const double* src[MMQ_CHAINS_MAX] = {};
+  for (int c = 0, r = 0; c < nchains && e == cudaSuccess; ++c) {
+    mmq_handle* h = chains[c];
+    const double* t = which == 0 ? h->trace : h->groups[which - 1].trace_dev;
+    if (h->device == h0->device) { src[c] = t; continue; }
+    double* dst = ws + (size_t)r++ * (size_t)rows * (size_t)L;
+    e = cudaMemcpyPeerAsync(dst, h0->device, t, h->device, tbytes, h0->stream);
+    src[c] = dst;
+  }
+  int ret = MMQ_OK;
+  if (e == cudaSuccess) {
+    ret = mmq_chain_diagnostics_dev(src, nchains, rows, L, out, h0->stream);
+    if (ret) ret = mmq_fail(h0, ret, mmq_last_error(nullptr));
+  }
+  double* dst[5] = {rhat, ess_bulk, ess_tail, log_mean, log_sd};
+  for (int q = 0; q < 5 && e == cudaSuccess && ret == MMQ_OK; ++q)
+    if (dst[q]) e = cudaMemcpyAsync(dst[q], out + (size_t)q * (size_t)rows, sizeof(double) * (size_t)rows, cudaMemcpyDeviceToHost, h0->stream);
+  const cudaError_t es = cudaStreamSynchronize(h0->stream);
+  if (e == cudaSuccess) e = es;
+  if (e != cudaSuccess && ret == MMQ_OK) ret = mmq_cuda_fail(h0, e, "mmq_chain_diagnostics", __FILE__, __LINE__);
+  mmq_cache_free(out);
+  mmq_cache_free(ws);
+  return ret;
+}
+
+/* exported under the name of include/mmq_sampler.h's inline function, which this file sees (so mmq.h does not declare it here) */
+extern "C" uint32_t mmq_chain_seed_export(uint32_t seed, int chain) __asm__("mmq_chain_seed");
+uint32_t mmq_chain_seed_export(uint32_t seed, int chain) { return mmq_chain_seed(seed, chain); }
 
 } /* extern "C" */

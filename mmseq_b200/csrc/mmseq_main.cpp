@@ -12,7 +12,9 @@
  * Additive options: -gpus INT (shard hit classes over GPUs of this box),
  * -notraces (skip the four *.trace_gibbs.gz text dumps), -batch FILE / -per_gpu INT (many
  * samples dealt to the GPUs, independent chains: BASELINE config 5), -counts (posterior and EM fragment counts per
- * transcript, identical set and gene: *.counts, *.identical.counts, *.gene.counts).
+ * transcript, identical set and gene: *.counts, *.identical.counts, *.gene.counts), -chains INT (independent chains
+ * from the EM estimate, split-R-hat and bulk / tail ESS per transcript, identical set and gene: *.convergence,
+ * *.identical.convergence, *.gene.convergence).
  */
 #include <unistd.h>
 #include <zlib.h>
@@ -74,6 +76,7 @@ static void printUsage(ostream& out) {
       << "  -batch FILE        (B200 build) many samples: FILE lists one \"hits_file output_base\" pair per line (no positional arguments)" << endl
       << "  -per_gpu INT       (B200 build) batch mode: samples in flight per GPU (default: 4)" << endl
       << "  -counts            (B200 build) also write posterior and EM fragment counts (*.counts, *.identical.counts, *.gene.counts)" << endl
+      << "  -chains INT        (B200 build) run INT independent chains (1..8, default: 1) and write split-R-hat and ESS per feature (*.convergence, *.identical.convergence, *.gene.convergence)" << endl
       << endl;
 }
 
@@ -175,6 +178,7 @@ struct Options {
   int ngpus = 1;
   string batch;     /* -batch FILE: one "hits_file output_base" pair per line */
   int per_gpu = 4;  /* -per_gpu INT: samples in flight per GPU in batch mode */
+  int chains = 1;   /* -chains INT: independent chains per sample */
   vector<string> positional;
 };
 
@@ -183,6 +187,8 @@ struct Options {
   printUsage(cerr);
   exit(1);
 }
+
+#define MMQ_CHAINS 8 /* chains per sample: the limit of mmq_chain_diagnostics */
 
 static bool is_power_of_two(int v) { return v > 0 && (v & (v - 1)) == 0; }
 
@@ -212,7 +218,7 @@ static Options parse_command_line(int argc, char** argv) {
       {"-epsilon", REAL, &o.epsilon},     {"-gibbs_iter", INT, &o.gibbs_iter}, {"-gibbs_ss", INT, &o.gibbs_ss},
       {"-seed", INT, &o.seed},            {"-percentiles", TEXT, &pct},       {"-gpus", INT, &o.ngpus},
       {"-batch", TEXT, &o.batch},         {"-per_gpu", INT, &o.per_gpu},      {"-notraces", FLAG, &o.notraces},
-      {"-debug", FLAG, &o.debug},         {"-counts", FLAG, &o.counts},
+      {"-debug", FLAG, &o.debug},         {"-counts", FLAG, &o.counts},       {"-chains", INT, &o.chains},
   };
   /* options come first; what is left must be the mandatory arguments (none in batch mode) */
   int i = 1;
@@ -246,6 +252,7 @@ static Options parse_command_line(int argc, char** argv) {
   if (o.gibbs_ss <= 0) usage_error("Error: gibbs_iter must be at least " + to_string(o.trace_length) + " (the trace length).");
   if (o.ngpus < 1) die("Error: -gpus must be >= 1.");
   if (o.per_gpu < 1) die("Error: -per_gpu must be >= 1.");
+  if (o.chains < 1 || o.chains > MMQ_CHAINS) die("Error: -chains must be in 1.." + to_string(MMQ_CHAINS) + ".");
   return o;
 }
 
@@ -257,10 +264,14 @@ static void run_sample(const Options& o, const string& hits_file, const string& 
   const int max_em_iter = o.max_em_iter, gibbs_iter = o.gibbs_iter, trace_length = o.trace_length, gibbs_ss = o.gibbs_ss, seed = o.seed;
   const vector<double>& percentiles = o.percentiles;
   const bool debug = o.debug, notraces = o.notraces;
-  const int ngpus = o.ngpus;
+  /* with several chains every chain runs whole on one GPU: chain c (0-based) on first_device + c mod o.ngpus */
+  const int nchains = o.chains;
+  const int ngpus = nchains > 1 ? 1 : o.ngpus; /* shards of chain 1 (the chain of the tables) */
+  const int ndev = nchains > 1 ? min(o.ngpus, nchains) : o.ngpus;
+  auto chain_device = [&](int c) { return first_device + c % o.ngpus; };
 
   /* the CUDA contexts come up (1-2 s) while the hits file is being parsed */
-  thread warmup([ngpus, first_device] { for (int g = 0; g < ngpus; ++g) mmq_warmup(first_device + g); });
+  thread warmup([ndev, first_device] { for (int g = 0; g < ndev; ++g) mmq_warmup(first_device + g); });
 
   /* ---- load: header + records -> hit classes (src/hitsio.cpp, src/mmseq.cpp:312-441).  A file with per-hit
    * weights (schema 2) cannot be collapsed: two fragments with the same transcript set differ in their weights.
@@ -286,7 +297,8 @@ static void run_sample(const Options& o, const string& hits_file, const string& 
        << "  gibbs_ss:      " << gibbs_ss << endl
        << "  seed[0]:       " << seed << endl
        << "  debug:         " << debug << endl
-       << "  threads:       " << ngpus << " GPU(s)" << endl;
+       << "  threads:       " << o.ngpus << " GPU(s)" << endl;
+  if (nchains > 1) out << "  chains:        " << nchains << endl;
   const int64_t T = (int64_t)hdr.names.size();
   const int64_t n = cls.n, m = cls.m; /* m: rows on the GPUs (sets, or fragments of a weighted file) */
   const int64_t N = cls.N;
@@ -318,6 +330,7 @@ static void run_sample(const Options& o, const string& hits_file, const string& 
   vector<Shard> shards((size_t)ngpus);
   vector<vector<int64_t>> shard_rp((size_t)ngpus), shard_id((size_t)ngpus);
   vector<vector<int32_t>> shard_col((size_t)ngpus), shard_k((size_t)ngpus);
+  mmq_problem whole; /* the problem of the unsharded chain 1, for chains 2.. (-chains) */
   for (int g = 0; g < ngpus; ++g) {
     Shard& S = shards[(size_t)g];
     S.device = first_device + g;
@@ -368,6 +381,7 @@ static void run_sample(const Options& o, const string& hits_file, const string& 
     S.row0 = 0; S.row1 = p.m;
     p.len = l.data();
     p.alpha = alpha; p.beta = beta;
+    if (g == 0) whole = p;
     int rc = mmq_create(&p, S.device, &S.h);
     if (rc) die(string("Error: mmq_create: ") + mmq_last_error(nullptr));
   }
@@ -546,6 +560,19 @@ static void run_sample(const Options& o, const string& hits_file, const string& 
     });
   }
 
+  /* ---- -chains: chains 2..C, each whole on its GPU from mu_em with its own seed, concurrently with chain 1 */
+  vector<mmq_handle*> chain_h((size_t)nchains, nullptr);
+  chain_h[0] = H0;
+  vector<thread> chain_th;
+  for (int c = 1; c < nchains; ++c)
+    chain_th.emplace_back([&, c] {
+      mmq_handle*& h = chain_h[(size_t)c];
+      if (mmq_create(&whole, chain_device(c), &h)) die(string("Error: mmq_create: ") + mmq_last_error(nullptr));
+      check(mmq_set_mu(h, mu_em.data()), h, "mmq_set_mu");
+      check(mmq_gibbs(h, mmq_chain_seed((uint32_t)seed, c), 0, gibbs_iter, gibbs_ss, L, MMQ_GIBBS_DEFAULT), h, "mmq_gibbs");
+      check(mmq_synchronize(h), h, "mmq_synchronize");
+    });
+
   /* ---- Gibbs (src/mmseq.cpp:822-918) */
   {
     auto t0 = chrono::steady_clock::now();
@@ -560,6 +587,7 @@ static void run_sample(const Options& o, const string& hits_file, const string& 
     err << "Gibbs: " << gibbs_iter << " sweeps in " << sec << " s (" << gibbs_iter / sec << " sweeps/s, " << (double)m * gibbs_iter / sec
          << (weighted ? " fragment allocations/s)" : " hit-class allocations/s)") << endl;
   }
+  for (auto& t : chain_th) t.join();
 
   phase("EM + Gibbs");
   out << "Amalgamating transcripts and calculating summary statistics..." << flush;
@@ -571,41 +599,44 @@ static void run_sample(const Options& o, const string& hits_file, const string& 
     if (cls.hdr2col[(size_t)hI] < 0) { unobs_slot[(size_t)hI] = (int64_t)unobs.size(); unobs.push_back(hI); }
   const int64_t U = (int64_t)unobs.size();
   vector<double> simu((size_t)U * (size_t)L);
-  {
-    vector<double> rate((size_t)U);
-    for (int64_t u = 0; u < U; ++u) rate[(size_t)u] = beta + hdr.efflen[(size_t)unobs[(size_t)u]] * (double)N / 1000000000.0;
-    if (U > 0 && mmq_prior_draws(shards[0].device, U, unobs.data(), rate.data(), alpha, (uint32_t)seed, L, simu.data()))
-      die(string("Error: mmq_prior_draws: ") + mmq_last_error(nullptr));
-  }
+  vector<double> rate((size_t)U);
+  for (int64_t u = 0; u < U; ++u) rate[(size_t)u] = beta + hdr.efflen[(size_t)unobs[(size_t)u]] * (double)N / 1000000000.0;
+  if (U > 0 && mmq_prior_draws(shards[0].device, U, unobs.data(), rate.data(), alpha, (uint32_t)seed, L, simu.data()))
+    die(string("Error: mmq_prior_draws: ") + mmq_last_error(nullptr));
 
-  /* ---- groups: identical sets (:938-954) and genes (:959-982) */
+  /* ---- groups: identical sets (:938-954) and genes (:959-982); with -chains, on every chain, the gene extras from
+   * each chain's own prior draws (built one chain at a time in one host buffer) */
   {
-    vector<int64_t> ptr{0};
-    vector<int32_t> mem;
+    vector<int64_t> iptr{0}, gptr{0};
+    vector<int32_t> imem, gmem;
     for (int64_t s = 0; s < I; ++s) {
-      for (int32_t hidx : hdr.identical[(size_t)s]) { int32_t c = cls.hdr2col[(size_t)hidx]; if (c >= 0) mem.push_back(c); }
-      ptr.push_back((int64_t)mem.size());
+      for (int32_t hidx : hdr.identical[(size_t)s]) { int32_t c = cls.hdr2col[(size_t)hidx]; if (c >= 0) imem.push_back(c); }
+      iptr.push_back((int64_t)imem.size());
     }
-    check(mmq_set_groups(H0, MMQ_GROUP_IDENTICAL, I, ptr.data(), mem.data(), nullptr), H0, "mmq_set_groups");
-  }
-  vector<char> gene_has_simu((size_t)G, 0);
-  {
-    vector<int64_t> ptr{0};
-    vector<int32_t> mem;
-    vector<double> extra((size_t)G * (size_t)L, 0.0);
     for (int64_t g = 0; g < G; ++g) {
-      for (int32_t hidx : hdr.gene_members[(size_t)g]) {
-        int32_t c = cls.hdr2col[(size_t)hidx];
-        if (c >= 0) mem.push_back(c);
-        else {
-          gene_has_simu[(size_t)g] = 1;
-          const double* sv = simu.data() + (size_t)unobs_slot[(size_t)hidx] * (size_t)L;
-          for (int i = 0; i < L; ++i) extra[(size_t)g * (size_t)L + (size_t)i] += sv[i];
-        }
-      }
-      ptr.push_back((int64_t)mem.size());
+      for (int32_t hidx : hdr.gene_members[(size_t)g]) { int32_t c = cls.hdr2col[(size_t)hidx]; if (c >= 0) gmem.push_back(c); }
+      gptr.push_back((int64_t)gmem.size());
     }
-    check(mmq_set_groups(H0, MMQ_GROUP_GENE, G, ptr.data(), mem.data(), extra.data()), H0, "mmq_set_groups");
+    vector<double> extra((size_t)G * (size_t)L), simu_c;
+    for (int c = 0; c < nchains; ++c) {
+      mmq_handle* h = chain_h[(size_t)c];
+      const double* sim = simu.data();
+      if (c > 0) {
+        simu_c.resize(simu.size());
+        if (U > 0 && mmq_prior_draws(chain_device(c), U, unobs.data(), rate.data(), alpha, mmq_chain_seed((uint32_t)seed, c), L, simu_c.data()))
+          die(string("Error: mmq_prior_draws: ") + mmq_last_error(nullptr));
+        sim = simu_c.data();
+      }
+      fill(extra.begin(), extra.end(), 0.0);
+      for (int64_t g = 0; g < G; ++g)
+        for (int32_t hidx : hdr.gene_members[(size_t)g])
+          if (cls.hdr2col[(size_t)hidx] < 0) {
+            const double* sv = sim + (size_t)unobs_slot[(size_t)hidx] * (size_t)L;
+            for (int i = 0; i < L; ++i) extra[(size_t)g * (size_t)L + (size_t)i] += sv[i];
+          }
+      check(mmq_set_groups(h, MMQ_GROUP_IDENTICAL, I, iptr.data(), imem.data(), nullptr), h, "mmq_set_groups");
+      check(mmq_set_groups(h, MMQ_GROUP_GENE, G, gptr.data(), gmem.data(), extra.data()), h, "mmq_set_groups");
+    }
   }
 
   /* ---- summaries on the device */
@@ -873,8 +904,65 @@ static void run_sample(const Options& o, const string& hits_file, const string& 
                  [&](int64_t g) { return em_group(hdr.gene_members[(size_t)g]); });
   }
 
+  /* ---- -chains: .convergence, .identical.convergence, .gene.convergence — rows and ids as in the three tables above.
+   * log_mu and sd pooled over the draws of all chains, split-R-hat and bulk / tail ESS (mmq_chain_diagnostics); a row
+   * whose `observed` column is 0 carries that table's closed-form log_mu and sd, and NA. */
+  if (nchains > 1) {
+    const char* const ext[3] = {".convergence", ".identical.convergence", ".gene.convergence"};
+    const char* const what[3] = {"transcripts", "identical sets", "genes"};
+    for (int which = 0; which < 3; ++which) {
+      const int64_t R = which == 0 ? n : which == 1 ? I : G;
+      vector<double> rh((size_t)R), eb((size_t)R), et((size_t)R), lm((size_t)R), ls((size_t)R);
+      if (R > 0)
+        check(mmq_chain_diagnostics(chain_h.data(), nchains, which, rh.data(), eb.data(), et.data(), lm.data(), ls.data()), H0,
+              "mmq_chain_diagnostics");
+      /* table row -> (diagnostics row or -1, feature id, closed-form log_mu and sd of an unobserved row) */
+      struct Row { int64_t q; string id; double log_mu, sd; };
+      auto row_of = [&](int64_t r) -> Row {
+        if (which == 0) {
+          const int32_t c = cls.hdr2col[(size_t)r];
+          return {c, hdr.names[(size_t)r], digalpha - log(beta + hdr.efflen[(size_t)r] * (double)N / 1000000000.0), sqrtpolygalpha};
+        }
+        if (which == 1) {
+          const auto& mem = hdr.identical[(size_t)r];
+          size_t jb = 0;
+          while (hdr.names[(size_t)mem[jb]].compare(hdr.names[(size_t)mem.back()]) != 0) ++jb;
+          return {isfinite(meanmu_identical[(size_t)r]) ? r : -1, identical_id(r),
+                  log(mem.size()) + digalpha - log(beta + hdr.efflen[(size_t)mem[jb]] * (double)N / 1000000000.0), sqrtpolygalpha};
+        }
+        bool obs = false;
+        for (int32_t hidx : hdr.gene_members[(size_t)r]) if (cls.hdr2col[(size_t)hidx] >= 0) { obs = true; break; }
+        return {obs ? r : -1, hdr.gene_names[(size_t)r], meanmu_gene[(size_t)r], sd_gene[(size_t)r]};
+      };
+      auto put = [](ostream& os, double v) -> ostream& { if (std::isnan(v)) os << "NA"; else os << v; return os; };
+      ofs.open((output_base + ext[which]).c_str());
+      ofs << "# Mapped fragments: " << N << endl;
+      ofs << "feature_id\tlog_mu\tsd\trhat\tess_bulk\tess_tail\n";
+      const int64_t rows = which == 0 ? T : R;
+      write_rows(ofs, rows, [&](ostream& os, int64_t r) {
+        const Row w = row_of(r);
+        os << w.id << "\t";
+        if (w.q < 0) { put(os, w.log_mu) << "\t"; put(os, w.sd) << "\tNA\tNA\tNA\n"; return; }
+        const size_t q = (size_t)w.q;
+        put(os, lm[q]) << "\t"; put(os, ls[q]) << "\t"; put(os, rh[q]) << "\t"; put(os, eb[q]) << "\t"; put(os, et[q]) << "\n";
+      });
+      ofs.close(); ofs.clear();
+      double max_rhat = NAN, min_ess = NAN;
+      int64_t over = 0;
+      for (int64_t r = 0; r < rows; ++r) {
+        const int64_t q = row_of(r).q;
+        if (q < 0) continue;
+        if (!std::isnan(rh[(size_t)q])) { max_rhat = std::isnan(max_rhat) ? rh[(size_t)q] : max(max_rhat, rh[(size_t)q]); over += rh[(size_t)q] > 1.01; }
+        if (!std::isnan(eb[(size_t)q])) min_ess = std::isnan(min_ess) ? eb[(size_t)q] : min(min_ess, eb[(size_t)q]);
+      }
+      err << "Convergence of the " << what[which] << " over " << nchains << " chains: largest rhat " << max_rhat << ", " << over
+          << " with rhat > 1.01, smallest ess_bulk " << min_ess << endl;
+    }
+  }
+
   out << "done." << endl;
   for (auto& S : shards) mmq_destroy(S.h);
+  for (int c = 1; c < nchains; ++c) mmq_destroy(chain_h[(size_t)c]);
 
   phase("tables");
   out << "Output files: " << endl
@@ -885,6 +973,10 @@ static void run_sample(const Options& o, const string& hits_file, const string& 
     out << "  " << output_base << ".counts" << endl
         << "  " << output_base << ".identical.counts" << endl
         << "  " << output_base << ".gene.counts" << endl;
+  if (nchains > 1)
+    out << "  " << output_base << ".convergence" << endl
+        << "  " << output_base << ".identical.convergence" << endl
+        << "  " << output_base << ".gene.convergence" << endl;
   out << "  " << output_base << ".M" << endl << "  " << output_base << ".k" << endl << endl;
   if (!notraces)
     out << "  " << output_base << ".trace_gibbs.gz" << endl
