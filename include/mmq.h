@@ -188,7 +188,9 @@ int mmq_count_moments_begin(mmq_handle* h, const int32_t* ident_of, int64_t n_id
 int mmq_count_moments_end(mmq_handle* h);
 /* which: 0 transcripts (n rows), 1 identical sets, 2 genes.  sweeps: sweeps accumulated (S); sum u64[rows] = sum_s c;
  * sumsq_lo / sumsq_hi u64[rows]: the low and high words of the 128-bit sum_s c^2.  Any output may be NULL.
- * Posterior mean sum / S; sd sqrt((S sumsq - sum^2) / (S (S - 1))) (the S - 1 of src/sokal.cc:63), 0 when S < 2. */
+ * Posterior mean sum / S; sd sqrt((S sumsq - sum^2) / (S (S - 1))) (the S - 1 of src/sokal.cc:63), 0 when S < 2.
+ * The moments of several chains (mmseq -chains C -pool) are their exact sums: the caller adds sweeps, sum and the
+ * 128-bit sumsq of the handles as integers and finishes with the same expressions (no library call does it). */
 int mmq_get_count_moments(mmq_handle* h, int which, int64_t* sweeps, uint64_t* sum, uint64_t* sumsq_lo, uint64_t* sumsq_hi);
 /* EM expected counts: one E-step at the current mu, src/mmseq.cpp:781-794: out[t] = mu[t] * sum_{i containing t}
  * k[i] w[i,t] / D_i with D_i = sum_{s in i} mu[s] w[i,s] (w = 1 without weights), summed over all shards (the fp64
@@ -279,6 +281,36 @@ int mmq_chain_diagnostics_dev(const double* const* chain_dev, int nchains, int64
  * trace_len and group counts on every handle, else MMQ_ERR_ARG.  Outputs fp64[rows] on the host; any may be NULL. */
 int mmq_chain_diagnostics(mmq_handle* const* chains, int nchains, int which, double* rhat, double* ess_bulk,
                           double* ess_tail, double* log_mean, double* log_sd);
+
+/* Posterior summaries over the pooled draws of several chains (none in the reference; mmseq -chains C -pool): the
+ * columns of the .mmseq tables over all S = nchains L draws of a feature instead of one chain's L.  chain_dev, nchains,
+ * L and their limits as mmq_chain_diagnostics_dev, else MMQ_ERR_ARG.  pct_idx_dev: int32[npct] on the device, indices
+ * into the S sorted draws (an index outside [0, S) gives NaN); pct_dev: fp64[rows * npct], [row * npct + j]; both may be
+ * NULL when npct = 0.  out_dev: fp64[3 * rows], [q * rows + row].  Asynchronous on cuda_stream, no allocation; one CTA
+ * per feature, grid min(rows, 2 x SMs); every value is fp64, summed in a fixed order, and independent of the grid and
+ * of the row order.  Definitions, for one feature's draws x[c][s] (tests/pool_reference.py restates them):
+ *   pct[j] = the draws sorted ascending (NaN last), at index pct_idx[j] (the host program: round(p / 100 (S - 1)));
+ *   mode 0 (draws of mu):
+ *     q = 0 log mean and q = 1 sd (S - 1) of log x over all S draws, plain IEEE (a zero draw gives -inf / NaN), NaN
+ *       when any x is NaN or +-inf: the bits of mmq_chain_diagnostics_dev's log_mean and log_sd;
+ *     q = 2 ess_mean: the ESS of mmq_chain_diagnostics_dev (Geyer's initial monotone sequence over the 2 nchains split
+ *       chains) applied to log x itself, not to its ranks; NaN when any log x is not finite or all are equal.
+ *     The tables' mcse = sd / sqrt(ess_mean) and iact = S / ess_mean (NaN with ess_mean).
+ *   mode 1 (proportion draws): q = 0 the mean of x over all S draws; q = 1, 2 are not written. */
+int mmq_pooled_summaries_dev(const double* const* chain_dev, int nchains, int64_t rows, int L, int mode, int npct,
+                             const int32_t* pct_idx_dev, double* out_dev, double* pct_dev, void* cuda_stream);
+/* The same on the traces the handles recorded (mmq_gibbs with trace_len = L), on chains[0]'s device and stream, traces of
+ * other devices copied there (cudaMemcpyPeerAsync, as mmq_chain_diagnostics).  which 0 transcripts, 1 identical sets,
+ * 2 genes: mode 0 into mean (log mean), sd and ess_mean.  which 3, the proportions of the observed transcripts: every
+ * chain's proportion draws are mu_t over that chain's own gene trace (mmq_prop_summaries' k_prop, run on each chain's
+ * device; gene_of, multi_iso as there), mode 1 into mean; sum_probit / sumsq_probit receive each chain's sum and sum of
+ * squares of the probits added in chain order (the host finishes them as src/mmseq.cpp:1260-1265 with S draws);
+ * sd and ess_mean are not written.  gene_of / multi_iso are read for which 3 only.  pct_idx host int32[npct] in [0, S),
+ * else MMQ_ERR_ARG.  Same n, trace_len and group counts on every handle, else MMQ_ERR_ARG.  Outputs fp64[rows] (pct
+ * fp64[rows * npct]) on the host; any may be NULL. */
+int mmq_pooled_summaries(mmq_handle* const* chains, int nchains, int which, const int32_t* gene_of, const uint8_t* multi_iso,
+                         int npct, const int32_t* pct_idx, double* mean, double* sd, double* ess_mean, double* sum_probit,
+                         double* sumsq_probit, double* pct);
 
 /* ---- the consumer of the traces: mmcollapse's covariance step (src/mmcollapse.cpp:483-561) ----------
  * The one dense contraction of the package: tensor cores (tcgen05, bf16 split products, fp32 accumulation in

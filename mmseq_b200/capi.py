@@ -80,6 +80,8 @@ def _load():
         "mmq_chain_seed": (u32, [u32, i32]),
         "mmq_chain_diagnostics_dev": (i32, [C.POINTER(vp), i32, i64, i32, vp, vp]),
         "mmq_chain_diagnostics": (i32, [C.POINTER(vp), i32, i32, vp, vp, vp, vp, vp]),
+        "mmq_pooled_summaries_dev": (i32, [C.POINTER(vp), i32, i64, i32, i32, i32, vp, vp, vp, vp]),
+        "mmq_pooled_summaries": (i32, [C.POINTER(vp), i32, i32, vp, vp, i32, vp, vp, vp, vp, vp, vp, vp]),
         "mmq_prior_draws": (i32, [i32, i64, vp, vp, dbl, u32, i32, vp]),
         "mmq_trace_cov": (i32, [i32, vp, i32, i64, i32, vp]),
         "mmq_trace_cov_workspace_bytes": (i64, [i32, i64, i32]),
@@ -115,7 +117,8 @@ EXPORTS = [
     "mmq_loglik", "mmq_em", "mmq_gibbs", "mmq_sweep_debug", "mmq_kernel_times", "mmq_cls_stats", "mmq_tune", "mmq_get_trace", "mmq_trace_len",
     "mmq_count_moments_begin", "mmq_count_moments_end", "mmq_get_count_moments", "mmq_expected_counts",
     "mmq_set_groups", "mmq_summarize", "mmq_get_group_trace", "mmq_prop_summaries",
-    "mmq_unique_hits_sets", "mmq_sokal_batch", "mmq_chain_seed", "mmq_chain_diagnostics_dev", "mmq_chain_diagnostics", "mmq_prior_draws", "mmq_trace_cov", "mmq_trace_cov_workspace_bytes", "mmq_trace_cov_dev",
+    "mmq_unique_hits_sets", "mmq_sokal_batch", "mmq_chain_seed", "mmq_chain_diagnostics_dev", "mmq_chain_diagnostics",
+    "mmq_pooled_summaries_dev", "mmq_pooled_summaries", "mmq_prior_draws", "mmq_trace_cov", "mmq_trace_cov_workspace_bytes", "mmq_trace_cov_dev",
     "mmq_handle_trace_cov", "mmq_mean_corrs", "mmq_mean_corrs_dev", "mmq_release_cache", "mmq_launch_count", "mmq_warmup", "mmq_version",
 ]
 
@@ -186,6 +189,35 @@ def chain_diagnostics(handles, which=0):
     rc = lib().mmq_chain_diagnostics(arr, len(handles), which, *[_ptr(out[k]) for k in CHAIN_OUTPUTS])
     if rc:
         raise MmqError(f"mmq_chain_diagnostics failed ({rc}): " + lib().mmq_last_error(h0._h).decode())
+    return out
+
+
+POOL_OUTPUTS = ("mean", "sd", "ess_mean")
+
+
+def pooled_summaries_dev(chain_ptrs, rows, L, mode, npct, pct_idx_ptr, out_ptr, pct_ptr, stream_ptr):
+    """mmq_pooled_summaries_dev: chain_ptrs, device pointers (ints) of each chain's [rows, L] fp64 draws; pct_idx_ptr:
+    int32[npct], out_ptr: fp64[3 * rows], pct_ptr: fp64[rows * npct], all on the same device.  Asynchronous on the
+    stream."""
+    arr = (C.c_void_p * len(chain_ptrs))(*chain_ptrs)
+    _global_check(lib().mmq_pooled_summaries_dev(arr, len(chain_ptrs), rows, L, mode, npct, pct_idx_ptr, out_ptr, pct_ptr, stream_ptr),
+                  "mmq_pooled_summaries_dev")
+
+
+def pooled_summaries(handles, which=0, pct_idx=None, gene_of=None, multi_iso=None):
+    """mmq_pooled_summaries over the traces the handles recorded: dict of POOL_OUTPUTS (fp64[rows]; sd and ess_mean stay
+    NaN for which 3), pct (rows, npct) and, for which 3, sum_probit and sumsq_probit added over the chains."""
+    h0 = handles[0]
+    rows = h0.n if which in (0, 3) else h0._ng[which - 1]
+    out = {k: np.full(rows, np.nan) for k in POOL_OUTPUTS + ("sum_probit", "sumsq_probit")}
+    pct_idx = _c(pct_idx if pct_idx is not None else [], np.int32)
+    out["pct"] = np.zeros((rows, len(pct_idx)))
+    gene_of = _c(gene_of, np.int32); multi_iso = _c(multi_iso, np.uint8)
+    arr = (C.c_void_p * len(handles))(*[h._h for h in handles])
+    rc = lib().mmq_pooled_summaries(arr, len(handles), which, _ptr(gene_of), _ptr(multi_iso), len(pct_idx), _ptr(pct_idx),
+                                    *[_ptr(out[k]) for k in POOL_OUTPUTS + ("sum_probit", "sumsq_probit", "pct")])
+    if rc:
+        raise MmqError(f"mmq_pooled_summaries failed ({rc}): " + lib().mmq_last_error(h0._h).decode())
     return out
 
 

@@ -9,10 +9,13 @@
  *   k_row_percentiles  src/mmseq.cpp:1111-1172 (sort each trace, pick indices)
  *   k_prop             src/mmseq.cpp:985-1008, :1236-1257
  *   k_uh_sets          src/uh.cpp:3-26 restated O(nnz)
+ * and, with no reference counterpart, the diagnostics of several chains (k_chain_diag) and the summaries of their
+ * pooled draws (k_pool_summ).
  * All traces are [row * trace_len + slot] (the reference's mu_trace layout).
  */
 #include <algorithm>
 #include <cstdio>
+#include <vector>
 
 #include "../../include/mmq_sampler.h"
 #include "mmq_internal.h"
@@ -245,6 +248,12 @@ struct mmq_chain_ptrs { const double* p[MMQ_CHAINS_MAX]; };
 
 static int chain_pow2_at_least(int s) { int p = 1; while (p < s) p <<= 1; return p; }
 static size_t chain_smem_bytes(int S) { return (size_t)12 * (size_t)(chain_pow2_at_least(S) + S); }
+/* The caps on dynamic shared memory that k_chain_diag and k_pool_summ are given: the largest request of any accepted
+ * shape (S = 8192; for k_pool_summ with L = 2048).  The cap is a per-device property of the function that any host thread
+ * can change between another thread's set and its launch, so it never depends on the call: a cap sized to one call's
+ * request could be lowered under a concurrent larger one, whose launch would then fail. */
+#define MMQ_CHAIN_DIAG_SMEM_CAP (12 * (8192 + 8192))
+#define MMQ_POOL_SMEM_CAP (8 * (8192 + 8192 + 2048))
 
 /* draw k (< S) of the row: chain k >> lgL, sweep slot k & (L - 1) */
 __device__ __forceinline__ double chain_x(const mmq_chain_ptrs& cp, int64_t row, int lgL, int k) {
@@ -340,14 +349,14 @@ __device__ __forceinline__ double chain_rhat(const double* s_m, const double* s_
 }
 
 /* ESS of the split chains y (moments s_m from chain_split_moments): autocovariances by FFT (zero-padded to 2N = L,
- * as k_row_sokal), then Geyer's initial monotone sequence.  The result is valid in thread 0; NaN when `constant`. */
-__device__ __forceinline__ double chain_ess(const double* y, int M, int N, const double* s_m, bool constant, double* key, int32_t* idx_area,
-                            int32_t* run_area) {
+ * as k_row_sokal), then Geyer's initial monotone sequence.  The result is valid in thread 0; NaN when `constant`.
+ * Shared scratch: key fp64[2 L], the FFT's (re, im); acc fp64[N], the sum over split chains of L * sum_i yc[i] yc[i + t];
+ * r fp64[N], the autocorrelation sequence. */
+__device__ __forceinline__ double chain_ess(const double* y, int M, int N, const double* s_m, bool constant, double* key, double* acc,
+                            double* r) {
   const int L = 2 * N;
   double* re = key;
   double* im = key + L;
-  double* acc = reinterpret_cast<double*>(idx_area); /* sum over split chains of L * sum_i yc[i] yc[i + t] */
-  double* r = reinterpret_cast<double*>(run_area);
   double out = mmq_u2d(0x7ff8000000000000ull);
   if (constant) return out;
   for (int t = threadIdx.x; t < N; t += blockDim.x) acc[t] = 0.0;
@@ -452,7 +461,8 @@ k_chain_diag(const __grid_constant__ mmq_chain_ptrs cp, int C, int64_t rows, int
     chain_rank_normalise(key, idx, run, z, S);
     chain_split_moments(z, M, N, s_m, s_w);
     const double rhat_bulk = chain_rhat(s_m, s_w, M, N);
-    const double ess_bulk = chain_ess(z, M, N, s_m, constant, key, idx, run);
+    /* the idx and run areas (4 P and 4 S bytes) hold the N fp64 of acc and of r */
+    const double ess_bulk = chain_ess(z, M, N, s_m, constant, key, reinterpret_cast<double*>(idx), reinterpret_cast<double*>(run));
 
     /* folded: rank-normalised |x - median| */
     for (int i = threadIdx.x; i < P; i += blockDim.x) { key[i] = i < S ? fabs(chain_x(cp, row, lgL, i) - med) : inf; idx[i] = i; }
@@ -470,7 +480,7 @@ k_chain_diag(const __grid_constant__ mmq_chain_ptrs cp, int C, int64_t rows, int
       cnt = post_block_sum(cnt); /* also orders the writes of z */
       constant = cnt == 0.0 || cnt == (double)S;
       chain_split_moments(z, M, N, s_m, s_w);
-      const double e = chain_ess(z, M, N, s_m, constant, key, idx, run);
+      const double e = chain_ess(z, M, N, s_m, constant, key, reinterpret_cast<double*>(idx), reinterpret_cast<double*>(run));
       ess_tail = (isnan(e) || isnan(ess_tail)) ? nan : fmin(ess_tail, e);
     }
     if (threadIdx.x == 0) {
@@ -479,6 +489,90 @@ k_chain_diag(const __grid_constant__ mmq_chain_ptrs cp, int C, int64_t rows, int
       out[2 * rows + row] = ess_tail;
       out[3 * rows + row] = log_mean;
       out[4 * rows + row] = log_sd;
+    }
+    __syncthreads();
+  }
+}
+
+/* ------------------------------------------------ summaries of the pooled draws of several chains
+ * The posterior columns of the tables over all S = C L draws of a feature (mmseq -pool), one CTA per feature.
+ * Definitions: include/mmq.h (mmq_pooled_summaries_dev); tests/pool_reference.py restates them in numpy.
+ * mode 0: log mean and sd (the sums of k_chain_diag, in its order, so the bits equal its log_mean / log_sd), the sorted
+ * draws at the percentile indices, and the ESS of the split chains of log x.  mode 1 (proportion draws): plain mean and
+ * percentiles.  Shared memory: key fp64[P] | y fp64[S] | acc fp64[L/2] | r fp64[L/2], 8 (P + S + L) bytes, 144 KB at
+ * S = 8192 (mode 1: key only).  key holds the values being sorted (padded with NaN, which sorts last), then the
+ * FFT's (re, im); y is log x in draw order. */
+__global__ void __launch_bounds__(MMQ_POST_THREADS)
+k_pool_summ(const __grid_constant__ mmq_chain_ptrs cp, int C, int64_t rows, int lgL, int mode, int npct,
+            const int32_t* __restrict__ pct_idx, double* __restrict__ out, double* __restrict__ pct) {
+  extern __shared__ double sh[];
+  __shared__ double s_m[2 * MMQ_CHAINS_MAX], s_w[2 * MMQ_CHAINS_MAX];
+  const int L = 1 << lgL, N = L >> 1, M = 2 * C, S = C * L;
+  int P = 1;
+  while (P < S) P <<= 1;
+  double* key = sh;
+  double* y = sh + P;
+  double* acc = y + S;
+  double* r = acc + N;
+  const double nan = mmq_u2d(0x7ff8000000000000ull);
+  for (int64_t row = blockIdx.x; row < rows; row += gridDim.x) {
+    double mean = nan, sd = nan, ess = nan;
+    bool logs_finite = false;
+    if (mode == 0) {
+      double bad = 0.0, badlog = 0.0, ls = 0.0;
+      for (int k = threadIdx.x; k < S; k += blockDim.x) {
+        const double x = chain_x(cp, row, lgL, k), lx = log(x);
+        bad += isfinite(x) ? 0.0 : 1.0;
+        badlog += isfinite(lx) ? 0.0 : 1.0;
+        ls += lx;
+        y[k] = lx;
+      }
+      bad = post_block_sum(bad);
+      badlog = post_block_sum(badlog);
+      ls = post_block_sum(ls);
+      if (bad == 0.0) {
+        mean = ls / (double)S;
+        double lv = 0.0;
+        for (int k = threadIdx.x; k < S; k += blockDim.x) { const double d = y[k] - mean; lv += d * d; }
+        lv = post_block_sum(lv);
+        sd = sqrt(lv / (double)(S - 1));
+      }
+      logs_finite = badlog == 0.0;
+    } else {
+      double s = 0.0;
+      for (int k = threadIdx.x; k < S; k += blockDim.x) s += chain_x(cp, row, lgL, k);
+      mean = post_block_sum(s) / (double)S;
+    }
+
+    /* percentiles: bitonic sort of the values, NaN last */
+    for (int i = threadIdx.x; i < P; i += blockDim.x) key[i] = i < S ? chain_x(cp, row, lgL, i) : nan;
+    __syncthreads();
+    for (int k = 2; k <= P; k <<= 1)
+      for (int j = k >> 1; j > 0; j >>= 1) {
+        for (int i = threadIdx.x; i < P; i += blockDim.x) {
+          const int p = i ^ j;
+          if (p > i) {
+            const double a = key[i], b = key[p];
+            const bool gt = a > b || (isnan(a) && !isnan(b));
+            if (gt == ((i & k) == 0)) { key[i] = b; key[p] = a; }
+          }
+        }
+        __syncthreads();
+      }
+    for (int j = threadIdx.x; j < npct; j += blockDim.x) {
+      const int q = pct_idx[j];
+      pct[row * npct + j] = q >= 0 && q < S ? key[q] : nan;
+    }
+
+    /* ESS of log x over the 2C split chains */
+    if (logs_finite) {
+      const bool constant = key[0] == key[S - 1];
+      chain_split_moments(y, M, N, s_m, s_w); /* its barrier also ends the reads of key above */
+      ess = chain_ess(y, M, N, s_m, constant, key, acc, r);
+    }
+    if (threadIdx.x == 0) {
+      out[row] = mean;
+      if (mode == 0) { out[rows + row] = sd; out[2 * rows + row] = ess; }
     }
     __syncthreads();
   }
@@ -742,7 +836,7 @@ int mmq_chain_diagnostics_dev(const double* const* chain_dev, int nchains, int64
   const size_t smem = chain_smem_bytes(nchains * L);
   cudaError_t e = cudaGetDevice(&dev);
   if (e == cudaSuccess) e = cudaDeviceGetAttribute(&sms, cudaDevAttrMultiProcessorCount, dev);
-  if (e == cudaSuccess) e = cudaFuncSetAttribute(k_chain_diag, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem);
+  if (e == cudaSuccess) e = cudaFuncSetAttribute(k_chain_diag, cudaFuncAttributeMaxDynamicSharedMemorySize, MMQ_CHAIN_DIAG_SMEM_CAP);
   if (e != cudaSuccess) return mmq_cuda_fail(nullptr, e, "mmq_chain_diagnostics_dev", __FILE__, __LINE__);
   const int grid = (int)std::min<int64_t>(rows, 2 * (int64_t)sms);
   k_chain_diag<<<grid, MMQ_POST_THREADS, smem, (cudaStream_t)cuda_stream>>>(cp, nchains, rows, lgL, out_dev);
@@ -752,24 +846,53 @@ int mmq_chain_diagnostics_dev(const double* const* chain_dev, int nchains, int64
   return MMQ_OK;
 }
 
+/* The checks of the handle forms (fn: the caller's name): no NULL handle, a trace on every chain, the same n, trace_len
+ * and group counts, and a trace_len within the limits of the kernels. */
+static int chain_handles_check(mmq_handle* const* chains, int nchains, const char* fn) {
+  auto fail = [&](mmq_handle* h, int code, const char* what) { return mmq_fail(h, code, std::string(fn) + ": " + what); };
+  for (int c = 0; c < nchains; ++c)
+    if (!chains[c]) return fail(nullptr, MMQ_ERR_ARG, "NULL handle");
+  mmq_handle* h0 = chains[0];
+  for (int c = 0; c < nchains; ++c) {
+    mmq_handle* h = chains[c];
+    if (!h->trace) return fail(h0, MMQ_ERR_STATE, "a chain has no trace recorded");
+    if (h->n != h0->n || h->trace_len != h0->trace_len || h->groups[0].ngroups != h0->groups[0].ngroups ||
+        h->groups[1].ngroups != h0->groups[1].ngroups)
+      return fail(h0, MMQ_ERR_ARG, "the chains differ in n, trace_len or group counts");
+  }
+  const int L = h0->trace_len;
+  if (L < 8 || L > MMQ_MAX_ROW_LEN || (L & (L - 1)) != 0 || nchains * L > MMQ_CHAIN_SMAX)
+    return fail(h0, MMQ_ERR_ARG, "trace_len must be a power of two in [8, 2048] with nchains * trace_len <= 8192");
+  return MMQ_OK;
+}
+
+/* Chain c's draws t[c] (rows x L, on chains[c]'s device) as pointers src[c] on chains[0]'s device: read in place there,
+ * copied from other devices with cudaMemcpyPeerAsync on chains[0]'s stream into *ws, a block-cache workspace of rows L 8
+ * bytes per such chain that the caller frees.  Runs with chains[0]'s device current. */
+static cudaError_t chain_gather(mmq_handle* const* chains, int nchains, const double* const* t, int64_t rows, int L, double** ws,
+                                const double** src) {
+  mmq_handle* h0 = chains[0];
+  const size_t tbytes = sizeof(double) * (size_t)rows * (size_t)L;
+  int remote = 0;
+  for (int c = 1; c < nchains; ++c) remote += chains[c]->device != h0->device;
+  cudaError_t e = remote ? mmq_cache_malloc(ws, tbytes * (size_t)remote) : cudaSuccess;
+  for (int c = 0, r = 0; c < nchains && e == cudaSuccess; ++c) {
+    if (chains[c]->device == h0->device) { src[c] = t[c]; continue; }
+    double* dst = *ws + (size_t)r++ * (size_t)rows * (size_t)L;
+    e = cudaMemcpyPeerAsync(dst, h0->device, t[c], chains[c]->device, tbytes, h0->stream);
+    src[c] = dst;
+  }
+  return e;
+}
+
 int mmq_chain_diagnostics(mmq_handle* const* chains, int nchains, int which, double* rhat, double* ess_bulk, double* ess_tail,
                           double* log_mean, double* log_sd) {
   if (!chains || nchains < 2 || nchains > MMQ_CHAINS_MAX || which < 0 || which > 2)
     return mmq_fail(chains ? chains[0] : nullptr, MMQ_ERR_ARG, "mmq_chain_diagnostics: bad arguments");
-  for (int c = 0; c < nchains; ++c)
-    if (!chains[c]) return mmq_fail(nullptr, MMQ_ERR_ARG, "mmq_chain_diagnostics: NULL handle");
+  if (const int rc = chain_handles_check(chains, nchains, "mmq_chain_diagnostics")) return rc;
   mmq_handle* h0 = chains[0];
-  for (int c = 0; c < nchains; ++c) {
-    mmq_handle* h = chains[c];
-    if (!h->trace) return mmq_fail(h0, MMQ_ERR_STATE, "mmq_chain_diagnostics: a chain has no trace recorded");
-    if (h->n != h0->n || h->trace_len != h0->trace_len || h->groups[0].ngroups != h0->groups[0].ngroups ||
-        h->groups[1].ngroups != h0->groups[1].ngroups)
-      return mmq_fail(h0, MMQ_ERR_ARG, "mmq_chain_diagnostics: the chains differ in n, trace_len or group counts");
-  }
   const int L = h0->trace_len;
   const int64_t rows = which == 0 ? h0->n : h0->groups[which - 1].ngroups;
-  if (L < 8 || L > MMQ_MAX_ROW_LEN || (L & (L - 1)) != 0 || nchains * L > MMQ_CHAIN_SMAX)
-    return mmq_fail(h0, MMQ_ERR_ARG, "mmq_chain_diagnostics: trace_len must be a power of two in [8, 2048] with nchains * trace_len <= 8192");
   if (rows == 0) return MMQ_OK;
   /* every chain's trace complete on its own device */
   for (int c = 0; c < nchains; ++c) {
@@ -779,21 +902,11 @@ int mmq_chain_diagnostics(mmq_handle* const* chains, int nchains, int which, dou
     MMQ_CUDA(h0, cudaStreamSynchronize(h->stream));
   }
   MMQ_CUDA(h0, cudaSetDevice(h0->device));
-  const size_t tbytes = sizeof(double) * (size_t)rows * (size_t)L;
-  int remote = 0;
-  for (int c = 1; c < nchains; ++c) remote += chains[c]->device != h0->device;
   double *ws = nullptr, *out = nullptr;
+  const double *t[MMQ_CHAINS_MAX] = {}, *src[MMQ_CHAINS_MAX] = {};
+  for (int c = 0; c < nchains; ++c) t[c] = which == 0 ? chains[c]->trace : chains[c]->groups[which - 1].trace_dev;
   cudaError_t e = mmq_cache_malloc(&out, sizeof(double) * 5 * (size_t)rows);
-  if (e == cudaSuccess && remote) e = mmq_cache_malloc(&ws, tbytes * (size_t)remote);
-  const double* src[MMQ_CHAINS_MAX] = {};
-  for (int c = 0, r = 0; c < nchains && e == cudaSuccess; ++c) {
-    mmq_handle* h = chains[c];
-    const double* t = which == 0 ? h->trace : h->groups[which - 1].trace_dev;
-    if (h->device == h0->device) { src[c] = t; continue; }
-    double* dst = ws + (size_t)r++ * (size_t)rows * (size_t)L;
-    e = cudaMemcpyPeerAsync(dst, h0->device, t, h->device, tbytes, h0->stream);
-    src[c] = dst;
-  }
+  if (e == cudaSuccess) e = chain_gather(chains, nchains, t, rows, L, &ws, src);
   int ret = MMQ_OK;
   if (e == cudaSuccess) {
     ret = mmq_chain_diagnostics_dev(src, nchains, rows, L, out, h0->stream);
@@ -807,6 +920,132 @@ int mmq_chain_diagnostics(mmq_handle* const* chains, int nchains, int which, dou
   if (e != cudaSuccess && ret == MMQ_OK) ret = mmq_cuda_fail(h0, e, "mmq_chain_diagnostics", __FILE__, __LINE__);
   mmq_cache_free(out);
   mmq_cache_free(ws);
+  return ret;
+}
+
+int mmq_pooled_summaries_dev(const double* const* chain_dev, int nchains, int64_t rows, int L, int mode, int npct,
+                             const int32_t* pct_idx_dev, double* out_dev, double* pct_dev, void* cuda_stream) {
+  if (!chain_dev || nchains < 2 || nchains > MMQ_CHAINS_MAX || rows < 0 || L < 8 || L > MMQ_MAX_ROW_LEN || (L & (L - 1)) != 0 ||
+      nchains * L > MMQ_CHAIN_SMAX || (mode != 0 && mode != 1) || npct < 0 || (rows > 0 && !out_dev) ||
+      (rows > 0 && npct > 0 && (!pct_idx_dev || !pct_dev)))
+    return mmq_fail(nullptr, MMQ_ERR_ARG, "mmq_pooled_summaries_dev: bad arguments");
+  mmq_chain_ptrs cp = {};
+  for (int c = 0; c < nchains; ++c) {
+    if (!chain_dev[c]) return mmq_fail(nullptr, MMQ_ERR_ARG, "mmq_pooled_summaries_dev: NULL chain");
+    cp.p[c] = chain_dev[c];
+  }
+  if (rows == 0) return MMQ_OK;
+  int dev = 0, sms = 0, lgL = 0;
+  while ((1 << lgL) < L) ++lgL;
+  const int S = nchains * L, P = chain_pow2_at_least(S);
+  const size_t smem = sizeof(double) * (size_t)(mode == 0 ? P + S + L : P);
+  cudaError_t e = cudaGetDevice(&dev);
+  if (e == cudaSuccess) e = cudaDeviceGetAttribute(&sms, cudaDevAttrMultiProcessorCount, dev);
+  if (e == cudaSuccess) e = cudaFuncSetAttribute(k_pool_summ, cudaFuncAttributeMaxDynamicSharedMemorySize, MMQ_POOL_SMEM_CAP);
+  if (e != cudaSuccess) return mmq_cuda_fail(nullptr, e, "mmq_pooled_summaries_dev", __FILE__, __LINE__);
+  const int grid = (int)std::min<int64_t>(rows, 2 * (int64_t)sms);
+  k_pool_summ<<<grid, MMQ_POST_THREADS, smem, (cudaStream_t)cuda_stream>>>(cp, nchains, rows, lgL, mode, npct, pct_idx_dev, out_dev, pct_dev);
+  g_mmq_launches.fetch_add(1);
+  e = cudaGetLastError();
+  if (e != cudaSuccess) return mmq_cuda_fail(nullptr, e, "k_pool_summ", __FILE__, __LINE__);
+  return MMQ_OK;
+}
+
+int mmq_pooled_summaries(mmq_handle* const* chains, int nchains, int which, const int32_t* gene_of, const uint8_t* multi_iso,
+                         int npct, const int32_t* pct_idx, double* mean, double* sd, double* ess_mean, double* sum_probit,
+                         double* sumsq_probit, double* pct) {
+  if (!chains || nchains < 2 || nchains > MMQ_CHAINS_MAX || which < 0 || which > 3 || npct < 0 || (npct > 0 && (!pct_idx || !pct)) ||
+      (which == 3 && (!gene_of || !multi_iso)))
+    return mmq_fail(chains ? chains[0] : nullptr, MMQ_ERR_ARG, "mmq_pooled_summaries: bad arguments");
+  if (const int rc = chain_handles_check(chains, nchains, "mmq_pooled_summaries")) return rc;
+  mmq_handle* h0 = chains[0];
+  const int L = h0->trace_len;
+  const int64_t n = h0->n;
+  const int64_t rows = which == 0 || which == 3 ? n : h0->groups[which - 1].ngroups;
+  for (int j = 0; j < npct; ++j)
+    if (pct_idx[j] < 0 || pct_idx[j] >= nchains * L) return mmq_fail(h0, MMQ_ERR_ARG, "mmq_pooled_summaries: percentile index out of range");
+  if (which == 3) {
+    if (h0->groups[MMQ_GROUP_GENE].ngroups == 0) return mmq_fail(h0, MMQ_ERR_STATE, "mmq_pooled_summaries: gene groups not set");
+    for (int64_t t = 0; t < n; ++t)
+      if (gene_of[t] < 0 || gene_of[t] >= h0->groups[MMQ_GROUP_GENE].ngroups)
+        return mmq_fail(h0, MMQ_ERR_ARG, "mmq_pooled_summaries: gene index out of range");
+  }
+  if (rows == 0) return MMQ_OK;
+  const size_t tbytes = sizeof(double) * (size_t)rows * (size_t)L;
+  /* every chain's draws complete on its own device; proportions: k_prop on each chain's device, into prop[c] */
+  double* prop[MMQ_CHAINS_MAX] = {};
+  double* part[MMQ_CHAINS_MAX] = {}; /* per chain: mean, sum and sum of squares of the probits, fp64[3 n] */
+  int32_t* gdev[MMQ_CHAINS_MAX] = {};
+  uint8_t* mdev[MMQ_CHAINS_MAX] = {};
+  std::vector<double> sums(which == 3 ? (size_t)nchains * 3 * (size_t)n : 0);
+  cudaError_t e = cudaSuccess;
+  int ret = MMQ_OK;
+  for (int c = 0; c < nchains && e == cudaSuccess && ret == MMQ_OK; ++c) {
+    mmq_handle* h = chains[c];
+    e = cudaSetDevice(h->device);
+    if (e != cudaSuccess) break;
+    if (which > 0) { const int rc = mmq_ensure_trace_groups(h); if (rc) { ret = mmq_fail(h0, rc, mmq_last_error(h)); break; } }
+    if (which == 3) {
+      e = mmq_cache_malloc(&prop[c], tbytes);
+      if (e == cudaSuccess) e = mmq_cache_malloc(&part[c], sizeof(double) * 3 * (size_t)n);
+      if (e == cudaSuccess) e = mmq_cache_malloc(&gdev[c], sizeof(int32_t) * (size_t)n);
+      if (e == cudaSuccess) e = mmq_cache_malloc(&mdev[c], (size_t)n);
+      if (e == cudaSuccess) e = cudaMemcpyAsync(gdev[c], gene_of, sizeof(int32_t) * (size_t)n, cudaMemcpyHostToDevice, h->stream);
+      if (e == cudaSuccess) e = cudaMemcpyAsync(mdev[c], multi_iso, (size_t)n, cudaMemcpyHostToDevice, h->stream);
+      if (e == cudaSuccess) {
+        const int grid = (int)std::min<int64_t>(n, (int64_t)h->num_sms * 8);
+        k_prop<<<grid, MMQ_POST_THREADS, 0, h->stream>>>(h->trace, h->groups[MMQ_GROUP_GENE].trace_dev, gdev[c], mdev[c], n, L, prop[c],
+                                                          part[c], part[c] + n, part[c] + 2 * n);
+        g_mmq_launches.fetch_add(1);
+        e = cudaGetLastError();
+      }
+      if (e == cudaSuccess) e = cudaMemcpyAsync(sums.data() + (size_t)c * 3 * (size_t)n, part[c], sizeof(double) * 3 * (size_t)n,
+                                                cudaMemcpyDeviceToHost, h->stream);
+    }
+    if (e == cudaSuccess) e = cudaStreamSynchronize(h->stream);
+  }
+  double *ws = nullptr, *out = nullptr, *d_pct = nullptr;
+  int32_t* d_idx = nullptr;
+  const double *t[MMQ_CHAINS_MAX] = {}, *src[MMQ_CHAINS_MAX] = {};
+  for (int c = 0; c < nchains; ++c) t[c] = which == 3 ? prop[c] : which == 0 ? chains[c]->trace : chains[c]->groups[which - 1].trace_dev;
+  if (e == cudaSuccess && ret == MMQ_OK) e = cudaSetDevice(h0->device);
+  if (e == cudaSuccess && ret == MMQ_OK) e = mmq_cache_malloc(&out, sizeof(double) * 3 * (size_t)rows);
+  if (e == cudaSuccess && ret == MMQ_OK && npct > 0) {
+    e = mmq_cache_malloc(&d_pct, sizeof(double) * (size_t)rows * (size_t)npct);
+    if (e == cudaSuccess) e = mmq_cache_malloc(&d_idx, sizeof(int32_t) * (size_t)npct);
+    if (e == cudaSuccess) e = cudaMemcpyAsync(d_idx, pct_idx, sizeof(int32_t) * (size_t)npct, cudaMemcpyHostToDevice, h0->stream);
+  }
+  if (e == cudaSuccess && ret == MMQ_OK) e = chain_gather(chains, nchains, t, rows, L, &ws, src);
+  if (e == cudaSuccess && ret == MMQ_OK) {
+    ret = mmq_pooled_summaries_dev(src, nchains, rows, L, which == 3 ? 1 : 0, npct, d_idx, out, d_pct, h0->stream);
+    if (ret) ret = mmq_fail(h0, ret, mmq_last_error(nullptr));
+  }
+  double* dst[3] = {mean, which == 3 ? nullptr : sd, which == 3 ? nullptr : ess_mean};
+  for (int q = 0; q < 3 && e == cudaSuccess && ret == MMQ_OK; ++q)
+    if (dst[q]) e = cudaMemcpyAsync(dst[q], out + (size_t)q * (size_t)rows, sizeof(double) * (size_t)rows, cudaMemcpyDeviceToHost, h0->stream);
+  if (e == cudaSuccess && ret == MMQ_OK && npct > 0)
+    e = cudaMemcpyAsync(pct, d_pct, sizeof(double) * (size_t)rows * (size_t)npct, cudaMemcpyDeviceToHost, h0->stream);
+  const cudaError_t es = cudaStreamSynchronize(h0->stream);
+  if (e == cudaSuccess) e = es;
+  if (e != cudaSuccess && ret == MMQ_OK) ret = mmq_cuda_fail(h0, e, "mmq_pooled_summaries", __FILE__, __LINE__);
+  /* the probit sums of the chains, added in chain order */
+  if (ret == MMQ_OK && which == 3)
+    for (int64_t t = 0; t < n; ++t) {
+      double s = 0.0, ss = 0.0;
+      for (int c = 0; c < nchains; ++c) {
+        s += sums[((size_t)c * 3 + 1) * (size_t)n + (size_t)t];
+        ss += sums[((size_t)c * 3 + 2) * (size_t)n + (size_t)t];
+      }
+      if (sum_probit) sum_probit[t] = s;
+      if (sumsq_probit) sumsq_probit[t] = ss;
+    }
+  mmq_cache_free(out); mmq_cache_free(ws); mmq_cache_free(d_pct); mmq_cache_free(d_idx);
+  for (int c = 0; c < nchains; ++c) { /* into the cache of the device each block came from */
+    if (!prop[c] && !part[c] && !gdev[c] && !mdev[c]) continue;
+    cudaSetDevice(chains[c]->device);
+    mmq_cache_free(prop[c]); mmq_cache_free(part[c]); mmq_cache_free(gdev[c]); mmq_cache_free(mdev[c]);
+  }
+  cudaSetDevice(h0->device);
   return ret;
 }
 

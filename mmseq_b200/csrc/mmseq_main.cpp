@@ -14,7 +14,8 @@
  * samples dealt to the GPUs, independent chains: BASELINE config 5), -counts (posterior and EM fragment counts per
  * transcript, identical set and gene: *.counts, *.identical.counts, *.gene.counts), -chains INT (independent chains
  * from the EM estimate, split-R-hat and bulk / tail ESS per transcript, identical set and gene: *.convergence,
- * *.identical.convergence, *.gene.convergence).
+ * *.identical.convergence, *.gene.convergence), -pool (with -chains: the three tables and the -counts files over the draws
+ * of all chains).
  */
 #include <unistd.h>
 #include <zlib.h>
@@ -77,6 +78,7 @@ static void printUsage(ostream& out) {
       << "  -per_gpu INT       (B200 build) batch mode: samples in flight per GPU (default: 4)" << endl
       << "  -counts            (B200 build) also write posterior and EM fragment counts (*.counts, *.identical.counts, *.gene.counts)" << endl
       << "  -chains INT        (B200 build) run INT independent chains (1..8, default: 1) and write split-R-hat and ESS per feature (*.convergence, *.identical.convergence, *.gene.convergence)" << endl
+      << "  -pool              (B200 build) with -chains 2 or more: the *.mmseq tables and -counts files summarise the draws of all chains (default: chain 1's); trace files stay chain 1's" << endl
       << endl;
 }
 
@@ -175,6 +177,7 @@ struct Options {
   int max_em_iter = 1000, gibbs_iter = 16384, trace_length = 1024, gibbs_ss = 16384 / 1024, seed = 1234;
   vector<double> percentiles{5.0, 25.0, 50.0, 75.0, 95.0};
   bool debug = false, notraces = false, counts = false;
+  bool pool = false; /* -pool: the tables and -counts over the draws of all chains */
   int ngpus = 1;
   string batch;     /* -batch FILE: one "hits_file output_base" pair per line */
   int per_gpu = 4;  /* -per_gpu INT: samples in flight per GPU in batch mode */
@@ -219,6 +222,7 @@ static Options parse_command_line(int argc, char** argv) {
       {"-seed", INT, &o.seed},            {"-percentiles", TEXT, &pct},       {"-gpus", INT, &o.ngpus},
       {"-batch", TEXT, &o.batch},         {"-per_gpu", INT, &o.per_gpu},      {"-notraces", FLAG, &o.notraces},
       {"-debug", FLAG, &o.debug},         {"-counts", FLAG, &o.counts},       {"-chains", INT, &o.chains},
+      {"-pool", FLAG, &o.pool},
   };
   /* options come first; what is left must be the mandatory arguments (none in batch mode) */
   int i = 1;
@@ -253,6 +257,7 @@ static Options parse_command_line(int argc, char** argv) {
   if (o.ngpus < 1) die("Error: -gpus must be >= 1.");
   if (o.per_gpu < 1) die("Error: -per_gpu must be >= 1.");
   if (o.chains < 1 || o.chains > MMQ_CHAINS) die("Error: -chains must be in 1.." + to_string(MMQ_CHAINS) + ".");
+  if (o.pool && o.chains < 2) die("Error: -pool needs -chains 2 or more.");
   return o;
 }
 
@@ -299,6 +304,7 @@ static void run_sample(const Options& o, const string& hits_file, const string& 
        << "  debug:         " << debug << endl
        << "  threads:       " << o.ngpus << " GPU(s)" << endl;
   if (nchains > 1) out << "  chains:        " << nchains << endl;
+  if (o.pool) out << "  pooled:        yes" << endl;
   const int64_t T = (int64_t)hdr.names.size();
   const int64_t n = cls.n, m = cls.m; /* m: rows on the GPUs (sets, or fragments of a weighted file) */
   const int64_t N = cls.N;
@@ -540,8 +546,9 @@ static void run_sample(const Options& o, const string& hits_file, const string& 
   }
 
   /* ---- -counts: EM expected counts at mu_em (one E-step, all shards), and from here on every Gibbs sweep adds its
-   * counts of transcripts, identical sets and genes into the accumulators of every shard */
+   * counts of transcripts, identical sets and genes into the accumulators of every shard (with -pool, of every chain) */
   vector<double> em_count;
+  vector<int32_t> ident_of, gene_of;
   if (o.counts) {
     em_count.resize((size_t)n);
     vector<vector<double>> other((size_t)ngpus);
@@ -550,7 +557,8 @@ static void run_sample(const Options& o, const string& hits_file, const string& 
       if (g > 0) other[(size_t)g].resize((size_t)n);
       check(mmq_expected_counts(h, g == 0 ? em_count.data() : other[(size_t)g].data()), h, "mmq_expected_counts");
     });
-    vector<int32_t> ident_of((size_t)n, -1), gene_of((size_t)n);
+    ident_of.assign((size_t)n, -1);
+    gene_of.resize((size_t)n);
     for (int64_t s = 0; s < I; ++s)
       for (int32_t hidx : hdr.identical[(size_t)s]) { const int32_t c = cls.hdr2col[(size_t)hidx]; if (c >= 0) ident_of[(size_t)c] = (int32_t)s; }
     for (int64_t t = 0; t < n; ++t) gene_of[(size_t)t] = hdr.gene_of[(size_t)cls.col2hdr[(size_t)t]];
@@ -569,6 +577,7 @@ static void run_sample(const Options& o, const string& hits_file, const string& 
       mmq_handle*& h = chain_h[(size_t)c];
       if (mmq_create(&whole, chain_device(c), &h)) die(string("Error: mmq_create: ") + mmq_last_error(nullptr));
       check(mmq_set_mu(h, mu_em.data()), h, "mmq_set_mu");
+      if (o.counts && o.pool) check(mmq_count_moments_begin(h, ident_of.data(), I, gene_of.data(), G), h, "mmq_count_moments_begin");
       check(mmq_gibbs(h, mmq_chain_seed((uint32_t)seed, c), 0, gibbs_iter, gibbs_ss, L, MMQ_GIBBS_DEFAULT), h, "mmq_gibbs");
       check(mmq_synchronize(h), h, "mmq_synchronize");
     });
@@ -605,7 +614,9 @@ static void run_sample(const Options& o, const string& hits_file, const string& 
     die(string("Error: mmq_prior_draws: ") + mmq_last_error(nullptr));
 
   /* ---- groups: identical sets (:938-954) and genes (:959-982); with -chains, on every chain, the gene extras from
-   * each chain's own prior draws (built one chain at a time in one host buffer) */
+   * each chain's own prior draws (built one chain at a time in one host buffer; kept under -pool for the hit-less
+   * isoforms' pooled columns) */
+  vector<vector<double>> simu_pool((size_t)nchains); /* [c >= 1]: chain c's prior draws, under -pool */
   {
     vector<int64_t> iptr{0}, gptr{0};
     vector<int32_t> imem, gmem;
@@ -622,10 +633,11 @@ static void run_sample(const Options& o, const string& hits_file, const string& 
       mmq_handle* h = chain_h[(size_t)c];
       const double* sim = simu.data();
       if (c > 0) {
-        simu_c.resize(simu.size());
-        if (U > 0 && mmq_prior_draws(chain_device(c), U, unobs.data(), rate.data(), alpha, mmq_chain_seed((uint32_t)seed, c), L, simu_c.data()))
+        vector<double>& dst = o.pool ? simu_pool[(size_t)c] : simu_c;
+        dst.resize(simu.size());
+        if (U > 0 && mmq_prior_draws(chain_device(c), U, unobs.data(), rate.data(), alpha, mmq_chain_seed((uint32_t)seed, c), L, dst.data()))
           die(string("Error: mmq_prior_draws: ") + mmq_last_error(nullptr));
-        sim = simu_c.data();
+        sim = dst.data();
       }
       fill(extra.begin(), extra.end(), 0.0);
       for (int64_t g = 0; g < G; ++g)
@@ -648,7 +660,7 @@ static void run_sample(const Options& o, const string& hits_file, const string& 
     Summ S;
     S.mean.resize((size_t)rows); S.var.resize((size_t)rows); S.tau.resize((size_t)rows);
     S.win.resize((size_t)rows); S.status.resize((size_t)rows); S.pct.resize((size_t)rows * NP);
-    if (rows > 0)
+    if (rows > 0 && !(o.pool && which == 0)) /* -pool: every transcript row comes from mmq_pooled_summaries below */
       check(mmq_summarize(H0, which, S.mean.data(), S.var.data(), S.tau.data(), S.win.data(), S.status.data(), (int)NP, pidx.data(), S.pct.data()), H0, "mmq_summarize");
     return S;
   };
@@ -667,6 +679,39 @@ static void run_sample(const Options& o, const string& hits_file, const string& 
   finish(St, sd, mumcse, iact);
   finish(Si, sd_identical, mumcse_identical, iact_identical);
   finish(Sg, sd_gene, mumcse_gene, iact_gene);
+  /* observed rows of the identical-set and gene tables (:1567, :1625-1628) */
+  vector<char> ident_obs((size_t)I), gene_obs((size_t)G, 0);
+  for (int64_t s = 0; s < I; ++s) ident_obs[(size_t)s] = isfinite(Si.mean[(size_t)s]) != 0;
+  for (int64_t g = 0; g < G; ++g)
+    for (int32_t hidx : hdr.gene_members[(size_t)g]) if (cls.hdr2col[(size_t)hidx] >= 0) { gene_obs[(size_t)g] = 1; break; }
+  /* -pool: the draws of all chains, `draws` of them per feature; the percentile rule of :1113 with draws for the trace
+   * length.  The stochastic columns of observed rows come from mmq_pooled_summaries: mcse = sd / sqrt(ess_mean),
+   * iact = draws / ess_mean.  What survives of chain 1's summaries: the unobserved rows of the identical-set and gene
+   * tables (as in the .convergence files) and the identical sets' observed test (ident_obs). */
+  const int npool = o.pool ? nchains : 1;
+  const int64_t draws = (int64_t)npool * L;
+  vector<int32_t> pidx_all(NP);
+  for (size_t i = 0; i < NP; i++) pidx_all[i] = static_cast<int>(round(percentiles[i] / 100.0 * (draws - 1)));
+  if (o.pool) {
+    auto pooled = [&](int which, int64_t rows, Summ& Sm, vector<double>& sdv, vector<double>& mcse, vector<double>& iactv,
+                      const function<bool(int64_t)>& observed) {
+      vector<double> mean((size_t)rows), psd((size_t)rows), ess((size_t)rows), pct((size_t)rows * NP);
+      if (rows > 0)
+        check(mmq_pooled_summaries(chain_h.data(), nchains, which, nullptr, nullptr, (int)NP, pidx_all.data(), mean.data(), psd.data(), ess.data(),
+                                   nullptr, nullptr, pct.data()), H0, "mmq_pooled_summaries");
+      for (int64_t r = 0; r < rows; ++r) {
+        if (!observed(r)) continue;
+        Sm.mean[(size_t)r] = mean[(size_t)r];
+        sdv[(size_t)r] = psd[(size_t)r];
+        mcse[(size_t)r] = psd[(size_t)r] / sqrt(ess[(size_t)r]);
+        iactv[(size_t)r] = (double)draws / ess[(size_t)r];
+        copy(pct.begin() + (ptrdiff_t)((size_t)r * NP), pct.begin() + (ptrdiff_t)((size_t)(r + 1) * NP), Sm.pct.begin() + (ptrdiff_t)((size_t)r * NP));
+      }
+    };
+    pooled(0, n, St, sd, mumcse, iact, [](int64_t) { return true; });
+    pooled(1, I, Si, sd_identical, mumcse_identical, iact_identical, [&](int64_t s) { return ident_obs[(size_t)s] != 0; });
+    pooled(2, G, Sg, sd_gene, mumcse_gene, iact_gene, [&](int64_t g) { return gene_obs[(size_t)g] != 0; });
+  }
   const vector<double>& meanmu = St.mean;
   const vector<double>& meanmu_identical = Si.mean;
   const vector<double>& meanmu_gene = Sg.mean;
@@ -683,50 +728,78 @@ static void run_sample(const Options& o, const string& hits_file, const string& 
       multi[(size_t)t] = hdr.gene_members[(size_t)g].size() > 1;
     }
     if (!notraces) prop_trace.resize((size_t)n * (size_t)L);
-    check(mmq_prop_summaries(H0, gene_of_col.data(), multi.data(), meanprop.data(), meanprobitprop.data(), ssprobitprop.data(), (int)NP, pidx.data(),
-                             pct_prop.data(), notraces ? nullptr : prop_trace.data()), H0, "mmq_prop_summaries");
+    if (!o.pool)
+      check(mmq_prop_summaries(H0, gene_of_col.data(), multi.data(), meanprop.data(), meanprobitprop.data(), ssprobitprop.data(), (int)NP, pidx.data(),
+                               pct_prop.data(), notraces ? nullptr : prop_trace.data()), H0, "mmq_prop_summaries");
+    else if (!notraces) /* chain 1's proportion trace for its trace file; the summaries come from all chains below */
+      check(mmq_prop_summaries(H0, gene_of_col.data(), multi.data(), nullptr, nullptr, nullptr, 0, nullptr, nullptr, prop_trace.data()), H0,
+            "mmq_prop_summaries");
+    if (o.pool) /* every chain's proportions over its own gene trace; the probit sums added over the chains */
+      check(mmq_pooled_summaries(chain_h.data(), nchains, 3, gene_of_col.data(), multi.data(), (int)NP, pidx_all.data(), meanprop.data(), nullptr,
+                                 nullptr, meanprobitprop.data(), ssprobitprop.data(), pct_prop.data()), H0, "mmq_pooled_summaries");
     for (int64_t t = 0; t < n; t++) /* :1260-1265, same expression order */
-      sdprobitprop[(size_t)t] = sqrt((ssprobitprop[(size_t)t] - meanprobitprop[(size_t)t] * meanprobitprop[(size_t)t] / trace_length) / (trace_length - 1.0));
-    for (int64_t t = 0; t < n; t++) meanprobitprop[(size_t)t] /= trace_length;
+      sdprobitprop[(size_t)t] = sqrt((ssprobitprop[(size_t)t] - meanprobitprop[(size_t)t] * meanprobitprop[(size_t)t] / draws) / (draws - 1.0));
+    for (int64_t t = 0; t < n; t++) meanprobitprop[(size_t)t] /= draws;
   }
 
   /* gene traces are needed on the host for the hit-less isoforms' proportions and the trace file */
   vector<double> gene_trace((size_t)G * (size_t)L);
   if (G > 0) check(mmq_get_group_trace(H0, 2, gene_trace.data()), H0, "mmq_get_group_trace");
 
-  /* hit-less isoforms: percentiles of the simulated trace, proportion summaries (:1174-1192, :1267-1305) */
+  /* hit-less isoforms: percentiles of the simulated trace, proportion summaries (:1174-1192, :1267-1305); with -pool over
+   * the prior draws of all chains, each chain's proportions over its own gene trace and its probit sums added in chain
+   * order */
   vector<double> pct_simu((size_t)U * NP), pct_prop_simu((size_t)U * NP), meanprop_simu((size_t)U), meanprobitprop_simu((size_t)U), sdprobitprop_simu((size_t)U);
   {
-    vector<double> probit_in((size_t)U * (size_t)L), probit_out;
-    vector<double> prop_simu((size_t)U * (size_t)L);
-    for (int64_t u = 0; u < U; ++u) {
-      const int32_t g = hdr.gene_of[(size_t)unobs[(size_t)u]];
-      const double* sv = simu.data() + (size_t)u * (size_t)L;
-      vector<double> v(sv, sv + L);
-      sort(v.begin(), v.end());
-      for (size_t j = 0; j < NP; ++j) pct_simu[(size_t)u * NP + j] = v[(size_t)pidx[j]];
-      for (int i = 0; i < L; ++i) prop_simu[(size_t)u * (size_t)L + (size_t)i] = sv[i] / gene_trace[(size_t)g * (size_t)L + (size_t)i];
-      copy(prop_simu.begin() + (ptrdiff_t)((size_t)u * (size_t)L), prop_simu.begin() + (ptrdiff_t)((size_t)(u + 1) * (size_t)L), v.begin());
-      sort(v.begin(), v.end());
-      for (size_t j = 0; j < NP; ++j) pct_prop_simu[(size_t)u * NP + j] = v[(size_t)pidx[j]];
+    vector<const double*> sim_c((size_t)npool), gtr_c((size_t)npool);
+    vector<vector<double>> gtr_other((size_t)npool);
+    for (int c = 0; c < npool; ++c) {
+      sim_c[(size_t)c] = c == 0 ? simu.data() : simu_pool[(size_t)c].data();
+      if (c == 0) { gtr_c[0] = gene_trace.data(); continue; }
+      gtr_other[(size_t)c].resize((size_t)G * (size_t)L);
+      if (U > 0) check(mmq_get_group_trace(chain_h[(size_t)c], 2, gtr_other[(size_t)c].data()), chain_h[(size_t)c], "mmq_get_group_trace");
+      gtr_c[(size_t)c] = gtr_other[(size_t)c].data();
     }
-    for (int64_t u = 0; u < U; ++u) {
-      const int32_t g = hdr.gene_of[(size_t)unobs[(size_t)u]];
-      const bool multi = hdr.gene_members[(size_t)g].size() > 1;
-      double mp = 0.0, s1 = 0.0, s2 = 0.0;
-      for (int i = 0; i < L; ++i) {
-        const double p = prop_simu[(size_t)u * (size_t)L + (size_t)i];
-        mp += p;
-        double temp;
-        if (multi) temp = mmq_host_ndtri(min(max(p, 0.000000001), 0.999999999));
-        else temp = numeric_limits<double>::infinity();
-        s1 += temp;
-        s2 += temp * temp;
+    /* isoforms u0 .. u1 - 1; every isoform's values are its own, so the host threads split the isoforms freely */
+    auto isoforms = [&](int64_t u0, int64_t u1) {
+      vector<double> v((size_t)draws), pv((size_t)draws);
+      for (int64_t u = u0; u < u1; ++u) {
+        const int32_t g = hdr.gene_of[(size_t)unobs[(size_t)u]];
+        const bool multi = hdr.gene_members[(size_t)g].size() > 1;
+        double mp = 0.0, s1 = 0.0, s2 = 0.0;
+        for (int c = 0; c < npool; ++c) {
+          const double* sv = sim_c[(size_t)c] + (size_t)u * (size_t)L;
+          const double* gt = gtr_c[(size_t)c] + (size_t)g * (size_t)L;
+          double c1 = 0.0, c2 = 0.0;
+          for (int i = 0; i < L; ++i) {
+            const double p = sv[i] / gt[i];
+            v[(size_t)c * (size_t)L + (size_t)i] = sv[i];
+            pv[(size_t)c * (size_t)L + (size_t)i] = p;
+            mp += p;
+            double temp;
+            if (multi) temp = mmq_host_ndtri(min(max(p, 0.000000001), 0.999999999));
+            else temp = numeric_limits<double>::infinity();
+            c1 += temp;
+            c2 += temp * temp;
+          }
+          s1 = c == 0 ? c1 : s1 + c1;
+          s2 = c == 0 ? c2 : s2 + c2;
+        }
+        sort(v.begin(), v.end());
+        sort(pv.begin(), pv.end());
+        for (size_t j = 0; j < NP; ++j) {
+          pct_simu[(size_t)u * NP + j] = v[(size_t)pidx_all[j]];
+          pct_prop_simu[(size_t)u * NP + j] = pv[(size_t)pidx_all[j]];
+        }
+        meanprop_simu[(size_t)u] = mp / draws;
+        sdprobitprop_simu[(size_t)u] = sqrt((s2 - s1 * s1 / draws) / (draws - 1.0));
+        meanprobitprop_simu[(size_t)u] = s1 / draws;
       }
-      meanprop_simu[(size_t)u] = mp / trace_length;
-      sdprobitprop_simu[(size_t)u] = sqrt((s2 - s1 * s1 / trace_length) / (trace_length - 1.0));
-      meanprobitprop_simu[(size_t)u] = s1 / trace_length;
-    }
+    };
+    const int nt = (int)max<int64_t>(1, min<int64_t>(min(32u, max(1u, thread::hardware_concurrency())), U * npool / 256));
+    vector<thread> th;
+    for (int t = 0; t < nt; ++t) th.emplace_back(isoforms, U * t / nt, U * (t + 1) / nt);
+    for (auto& x : th) x.join();
   }
 
   phase("summaries");
@@ -825,7 +898,7 @@ static void run_sample(const Options& o, const string& hits_file, const string& 
     const auto& mem = hdr.identical[(size_t)s];
     const string& backname = hdr.names[(size_t)mem.back()];
     const int32_t first = mem.front();
-    if (isfinite(meanmu_identical[(size_t)s])) {
+    if (ident_obs[(size_t)s]) {
       for (size_t j = 0; j < mem.size(); ++j) {
         const string& nm = hdr.names[(size_t)mem[j]];
         ofs << nm;
@@ -872,7 +945,7 @@ static void run_sample(const Options& o, const string& hits_file, const string& 
 
   /* ---- -counts: .counts, .identical.counts, .gene.counts — rows and ids as in the three tables above; posterior
    * mean and sd over the chain's sweeps, EM expected count (a group's: the sum of its members').  Every shard holds
-   * the same moments. */
+   * the same moments.  With -pool the moments of all chains are added exactly: sweeps, sums and 128-bit sums of squares. */
   if (o.counts) {
     auto write_counts = [&](const string& path, int which, int64_t rows, const function<string(int64_t)>& id, const function<int64_t(int64_t)>& row_of,
                             const function<double(int64_t)>& em) {
@@ -880,6 +953,19 @@ static void run_sample(const Options& o, const string& hits_file, const string& 
       const int64_t R = which == 0 ? n : which == 1 ? I : G;
       vector<uint64_t> sum((size_t)R), lo((size_t)R), hi((size_t)R);
       check(mmq_get_count_moments(H0, which, &S, sum.data(), lo.data(), hi.data()), H0, "mmq_get_count_moments");
+      for (int c = 1; c < npool; ++c) {
+        mmq_handle* h = chain_h[(size_t)c];
+        int64_t Sc = 0;
+        vector<uint64_t> sc((size_t)R), lc((size_t)R), hc((size_t)R);
+        check(mmq_get_count_moments(h, which, &Sc, sc.data(), lc.data(), hc.data()), h, "mmq_get_count_moments");
+        S += Sc;
+        for (size_t q = 0; q < (size_t)R; ++q) {
+          sum[q] += sc[q];
+          const uint64_t l = lo[q] + lc[q];
+          hi[q] += hc[q] + (l < lo[q]);
+          lo[q] = l;
+        }
+      }
       ofs.open(path.c_str());
       ofs << "# Mapped fragments: " << N << endl;
       ofs << "feature_id\tposterior_mean_count\tposterior_sd_count\tem_count\n";
@@ -927,7 +1013,7 @@ static void run_sample(const Options& o, const string& hits_file, const string& 
           const auto& mem = hdr.identical[(size_t)r];
           size_t jb = 0;
           while (hdr.names[(size_t)mem[jb]].compare(hdr.names[(size_t)mem.back()]) != 0) ++jb;
-          return {isfinite(meanmu_identical[(size_t)r]) ? r : -1, identical_id(r),
+          return {ident_obs[(size_t)r] ? r : -1, identical_id(r),
                   log(mem.size()) + digalpha - log(beta + hdr.efflen[(size_t)mem[jb]] * (double)N / 1000000000.0), sqrtpolygalpha};
         }
         bool obs = false;
