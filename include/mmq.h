@@ -312,6 +312,48 @@ int mmq_pooled_summaries(mmq_handle* const* chains, int nchains, int which, cons
                          int npct, const int32_t* pct_idx, double* mean, double* sd, double* ess_mean, double* sum_probit,
                          double* sumsq_probit, double* pct);
 
+/* ---- transcripts per million (none in the reference; mmseq -tpm) ------------------------------------------------------
+ * The abundance unit Salmon, kallisto and RSEM report, with its posterior over the recorded draws.  mu is a rate per
+ * scaled length (l_t = efflen_t N / 1e9, so exp(log_mu) is on the FPKM scale), and TPM is mu normalised within each draw.
+ * tests/tpm_reference.py restates these definitions in numpy.  x_c[t][s]: chain c's recorded draw of mu for observed
+ * transcript t < n at slot s < L (the mmq_get_trace layout [t * L + s]); C chains, S = C L draws per feature.
+ *   1. Totals: D_c[s] = sum_{t < n} x_c[t][s] in fp64 over the observed transcripts only (hit-less isoforms' prior draws
+ *      are not included).  Order: tiles of 512 rows, each summed in row order per slot from 0.0, then the tile sums in
+ *      tile order from 0.0.  It depends on (n, L) only, so the bits are the same on any grid, device or repeat, and the
+ *      relative error is at most about (512 + n / 512) eps: within 1e-12 of the exact sum of positive draws.
+ *   2. Draws of a feature: its members are itself (a transcript) or its observed members in the CSR order given to
+ *      mmq_set_groups (an identical set or a gene; the group's `extra` is NOT added).  Per draw, w = the sum of the
+ *      members' draws in that order from 0.0, and tpm_c[s] = (w / D_c[s]) * 1e6, in plain IEEE in exactly that order.  A
+ *      feature without members has w = 0 and so TPM 0 in every draw.  Sum over transcripts, or over genes, is 1e6.
+ *   3. Over the S draws: mean = sum tpm / S (fixed order); sd = sqrt(sum (tpm - mean)^2 / (S - 1)), two-pass; both NaN
+ *      when any draw is not finite.  pct[j] = the draws sorted ascending (NaN last) at index pct_idx[j]; an index outside
+ *      [0, S) gives NaN (the host program: round(p / 100 (S - 1)), as -pool).
+ *   4. EM (computed by the caller): tpm_em_f = (sum_{members} mu_em[t] / sum_{t < n} mu_em[t]) * 1e6, both sums in index
+ *      order; 0 for a feature without members.
+ * Limits: 1 <= nchains <= 8, L a power of two in [4, 2048], nchains L <= 8192; otherwise MMQ_ERR_ARG. */
+/* Bytes of workspace mmq_draw_totals_dev needs for a trace of `rows` rows (8 L ceil(rows / 512); 0 for bad arguments). */
+int64_t mmq_draw_totals_workspace_bytes(int64_t rows, int L);
+/* totals_dev fp64[L] = D[s] of definition 1 over the trace trace_dev [row * L + s] (rows >= 0; rows = 0 gives 0.0).
+ * Asynchronous on cuda_stream, no allocation: workspace_dev holds mmq_draw_totals_workspace_bytes(rows, L) bytes. */
+int mmq_draw_totals_dev(const double* trace_dev, int64_t rows, int L, double* totals_dev, void* workspace_dev, void* cuda_stream);
+/* Summaries 2-3 per feature.  chain_dev[c] (a host array of device pointers): chain c's transcript trace [t * L + s];
+ * totals_dev fp64[nchains L], chain-major (chain c's D at [c L + s]); group_ptr_dev int64[rows + 1] / members_dev int32
+ * both given (feature r = members[group_ptr[r] .. group_ptr[r + 1]) ) or both NULL (feature r = transcript r).  out_dev
+ * fp64[2 rows]: [r] mean, [rows + r] sd; pct_dev fp64[rows npct], [r npct + j]; pct_idx_dev int32[npct] (both may be NULL
+ * when npct = 0).  All on the calling device; asynchronous on cuda_stream, no allocation; one CTA per feature, grid
+ * min(rows, 2 x SMs); results independent of the grid and of the row order. */
+int mmq_tpm_summaries_dev(const double* const* chain_dev, const double* totals_dev, int nchains, int64_t rows, int L,
+                          const int64_t* group_ptr_dev, const int32_t* members_dev, int npct, const int32_t* pct_idx_dev,
+                          double* out_dev, double* pct_dev, void* cuda_stream);
+/* The same on the traces the handles recorded (mmq_gibbs with trace_len = L): which 0 transcripts, 1 identical sets,
+ * 2 genes, with the groups of chains[0] (mmq_set_groups).  Each chain is normalised by its own totals.  Runs on
+ * chains[0]'s device and stream; transcript traces of handles on other devices are copied there (cudaMemcpyPeerAsync,
+ * as mmq_chain_diagnostics); the workspace comes from the block cache.  Same n, trace_len and group counts on every
+ * handle, and pct_idx (host int32[npct]) in [0, S), else MMQ_ERR_ARG.  mean, sd fp64[rows], pct fp64[rows npct] and
+ * totals_out fp64[nchains L] (the D_c, chain-major) on the host; any may be NULL. */
+int mmq_tpm_summaries(mmq_handle* const* chains, int nchains, int which, int npct, const int32_t* pct_idx, double* mean, double* sd,
+                      double* pct, double* totals_out);
+
 /* ---- the consumer of the traces: mmcollapse's covariance step (src/mmcollapse.cpp:483-561) ----------
  * The one dense contraction of the package: tensor cores (tcgen05, bf16 split products, fp32 accumulation in
  * TMEM), everything around it fp64.  nsplit = bf16 terms per value (2: the default of the callers here).  Error in

@@ -82,6 +82,10 @@ def _load():
         "mmq_chain_diagnostics": (i32, [C.POINTER(vp), i32, i32, vp, vp, vp, vp, vp]),
         "mmq_pooled_summaries_dev": (i32, [C.POINTER(vp), i32, i64, i32, i32, i32, vp, vp, vp, vp]),
         "mmq_pooled_summaries": (i32, [C.POINTER(vp), i32, i32, vp, vp, i32, vp, vp, vp, vp, vp, vp, vp]),
+        "mmq_draw_totals_workspace_bytes": (i64, [i64, i32]),
+        "mmq_draw_totals_dev": (i32, [vp, i64, i32, vp, vp, vp]),
+        "mmq_tpm_summaries_dev": (i32, [C.POINTER(vp), vp, i32, i64, i32, vp, vp, i32, vp, vp, vp, vp]),
+        "mmq_tpm_summaries": (i32, [C.POINTER(vp), i32, i32, i32, vp, vp, vp, vp, vp]),
         "mmq_prior_draws": (i32, [i32, i64, vp, vp, dbl, u32, i32, vp]),
         "mmq_trace_cov": (i32, [i32, vp, i32, i64, i32, vp]),
         "mmq_trace_cov_workspace_bytes": (i64, [i32, i64, i32]),
@@ -118,7 +122,8 @@ EXPORTS = [
     "mmq_count_moments_begin", "mmq_count_moments_end", "mmq_get_count_moments", "mmq_expected_counts",
     "mmq_set_groups", "mmq_summarize", "mmq_get_group_trace", "mmq_prop_summaries",
     "mmq_unique_hits_sets", "mmq_sokal_batch", "mmq_chain_seed", "mmq_chain_diagnostics_dev", "mmq_chain_diagnostics",
-    "mmq_pooled_summaries_dev", "mmq_pooled_summaries", "mmq_prior_draws", "mmq_trace_cov", "mmq_trace_cov_workspace_bytes", "mmq_trace_cov_dev",
+    "mmq_pooled_summaries_dev", "mmq_pooled_summaries", "mmq_draw_totals_workspace_bytes", "mmq_draw_totals_dev",
+    "mmq_tpm_summaries_dev", "mmq_tpm_summaries", "mmq_prior_draws", "mmq_trace_cov", "mmq_trace_cov_workspace_bytes", "mmq_trace_cov_dev",
     "mmq_handle_trace_cov", "mmq_mean_corrs", "mmq_mean_corrs_dev", "mmq_release_cache", "mmq_launch_count", "mmq_warmup", "mmq_version",
 ]
 
@@ -218,6 +223,41 @@ def pooled_summaries(handles, which=0, pct_idx=None, gene_of=None, multi_iso=Non
                                     *[_ptr(out[k]) for k in POOL_OUTPUTS + ("sum_probit", "sumsq_probit", "pct")])
     if rc:
         raise MmqError(f"mmq_pooled_summaries failed ({rc}): " + lib().mmq_last_error(h0._h).decode())
+    return out
+
+
+def draw_totals_workspace_bytes(rows, L):
+    return int(lib().mmq_draw_totals_workspace_bytes(rows, L))
+
+
+def draw_totals_dev(trace_ptr, rows, L, totals_ptr, ws_ptr, stream_ptr):
+    """mmq_draw_totals_dev: totals_ptr fp64[L] = the column sums of the [rows, L] fp64 trace at trace_ptr in the fixed
+    tile order; ws_ptr: draw_totals_workspace_bytes(rows, L) bytes.  Device pointers (ints); asynchronous on the stream."""
+    _global_check(lib().mmq_draw_totals_dev(trace_ptr, rows, L, totals_ptr, ws_ptr, stream_ptr), "mmq_draw_totals_dev")
+
+
+def tpm_summaries_dev(chain_ptrs, totals_ptr, rows, L, group_ptr_ptr, members_ptr, npct, pct_idx_ptr, out_ptr, pct_ptr, stream_ptr):
+    """mmq_tpm_summaries_dev: chain_ptrs, device pointers (ints) of each chain's transcript trace; totals_ptr
+    fp64[C * L] chain-major; group_ptr_ptr / members_ptr: a CSR of features over the transcripts, or both None for one
+    feature per transcript; out_ptr fp64[2 * rows] (mean, sd); pct_ptr fp64[rows * npct].  Asynchronous on the stream."""
+    arr = (C.c_void_p * len(chain_ptrs))(*chain_ptrs)
+    _global_check(lib().mmq_tpm_summaries_dev(arr, totals_ptr, len(chain_ptrs), rows, L, group_ptr_ptr, members_ptr, npct, pct_idx_ptr,
+                                              out_ptr, pct_ptr, stream_ptr), "mmq_tpm_summaries_dev")
+
+
+def tpm_summaries(handles, which=0, pct_idx=None):
+    """mmq_tpm_summaries over the traces the handles recorded: dict(mean, sd: fp64[rows]; pct: (rows, npct);
+    totals: (C, L), each chain's per-draw total of the observed transcripts)."""
+    h0 = handles[0]
+    rows = h0.n if which == 0 else getattr(h0, "_ng", {}).get(which - 1, 0)          # other values: the library refuses them
+    pct_idx = _c(pct_idx if pct_idx is not None else [], np.int32)
+    out = dict(mean=np.zeros(rows), sd=np.zeros(rows), pct=np.zeros((rows, len(pct_idx))),
+               totals=np.zeros((len(handles), h0.trace_len())))
+    arr = (C.c_void_p * len(handles))(*[h._h for h in handles])
+    rc = lib().mmq_tpm_summaries(arr, len(handles), which, len(pct_idx), _ptr(pct_idx), _ptr(out["mean"]), _ptr(out["sd"]), _ptr(out["pct"]),
+                                 _ptr(out["totals"]))
+    if rc:
+        raise MmqError(f"mmq_tpm_summaries failed ({rc}): " + lib().mmq_last_error(h0._h).decode())
     return out
 
 

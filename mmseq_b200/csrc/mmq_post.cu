@@ -494,6 +494,24 @@ k_chain_diag(const __grid_constant__ mmq_chain_ptrs cp, int C, int64_t rows, int
   }
 }
 
+/* bitonic sort of key[0 .. P) ascending with NaN last, P a power of two; opens with a barrier that orders the caller's
+ * writes of key and ends with one after the last exchange */
+__device__ __forceinline__ void sort_nan_last(double* key, int P) {
+  __syncthreads();
+  for (int k = 2; k <= P; k <<= 1)
+    for (int j = k >> 1; j > 0; j >>= 1) {
+      for (int i = threadIdx.x; i < P; i += blockDim.x) {
+        const int p = i ^ j;
+        if (p > i) {
+          const double a = key[i], b = key[p];
+          const bool gt = a > b || (isnan(a) && !isnan(b));
+          if (gt == ((i & k) == 0)) { key[i] = b; key[p] = a; }
+        }
+      }
+      __syncthreads();
+    }
+}
+
 /* ------------------------------------------------ summaries of the pooled draws of several chains
  * The posterior columns of the tables over all S = C L draws of a feature (mmseq -pool), one CTA per feature.
  * Definitions: include/mmq.h (mmq_pooled_summaries_dev); tests/pool_reference.py restates them in numpy.
@@ -546,19 +564,7 @@ k_pool_summ(const __grid_constant__ mmq_chain_ptrs cp, int C, int64_t rows, int 
 
     /* percentiles: bitonic sort of the values, NaN last */
     for (int i = threadIdx.x; i < P; i += blockDim.x) key[i] = i < S ? chain_x(cp, row, lgL, i) : nan;
-    __syncthreads();
-    for (int k = 2; k <= P; k <<= 1)
-      for (int j = k >> 1; j > 0; j >>= 1) {
-        for (int i = threadIdx.x; i < P; i += blockDim.x) {
-          const int p = i ^ j;
-          if (p > i) {
-            const double a = key[i], b = key[p];
-            const bool gt = a > b || (isnan(a) && !isnan(b));
-            if (gt == ((i & k) == 0)) { key[i] = b; key[p] = a; }
-          }
-        }
-        __syncthreads();
-      }
+    sort_nan_last(key, P);
     for (int j = threadIdx.x; j < npct; j += blockDim.x) {
       const int q = pct_idx[j];
       pct[row * npct + j] = q >= 0 && q < S ? key[q] : nan;
@@ -574,6 +580,103 @@ k_pool_summ(const __grid_constant__ mmq_chain_ptrs cp, int C, int64_t rows, int 
       out[row] = mean;
       if (mode == 0) { out[rows + row] = sd; out[2 * rows + row] = ess; }
     }
+    __syncthreads();
+  }
+}
+
+/* ------------------------------------------------ transcripts per million (mmseq -tpm)
+ * Definitions: include/mmq.h (mmq_draw_totals_dev, mmq_tpm_summaries_dev); tests/tpm_reference.py restates them in numpy.
+ * k_draw_totals + k_totals_fold: D[s] = sum over the rows of a trace [row * L + s], in a fixed order that depends on
+ * (rows, L) only: tiles of MMQ_TOTALS_TILE rows, each summed in row order per slot from 0.0, then the tile sums in tile
+ * order from 0.0.  A warp reads 32 consecutive slots of one row (the trace is row-major), so every load is coalesced;
+ * each thread keeps eight loads in flight ahead of its in-order adds. */
+#define MMQ_TOTALS_TILE 512
+#define MMQ_TOTALS_THREADS 256
+
+__global__ void __launch_bounds__(MMQ_TOTALS_THREADS)
+k_draw_totals(const double* __restrict__ trace, int64_t rows, int L, double* __restrict__ partial) {
+  const int s = blockIdx.y * blockDim.x + threadIdx.x;
+  if (s >= L) return;
+  const int64_t t0 = (int64_t)blockIdx.x * MMQ_TOTALS_TILE;
+  const int nt = rows - t0 < MMQ_TOTALS_TILE ? (int)(rows - t0) : MMQ_TOTALS_TILE;
+  const double* p = trace + t0 * L + s;
+  double acc = 0.0;
+  int t = 0;
+  for (; t + 8 <= nt; t += 8) {
+    double v[8];
+#pragma unroll
+    for (int u = 0; u < 8; ++u) v[u] = p[(int64_t)(t + u) * L];
+#pragma unroll
+    for (int u = 0; u < 8; ++u) acc += v[u];
+  }
+  for (; t < nt; ++t) acc += p[(int64_t)t * L];
+  partial[(int64_t)blockIdx.x * L + s] = acc;
+}
+
+__global__ void __launch_bounds__(MMQ_TOTALS_THREADS)
+k_totals_fold(const double* __restrict__ partial, int64_t ntiles, int L, double* __restrict__ totals) {
+  const int s = blockIdx.x * blockDim.x + threadIdx.x;
+  if (s >= L) return;
+  double acc = 0.0;
+  int64_t k = 0;
+  for (; k + 8 <= ntiles; k += 8) {
+    double v[8];
+#pragma unroll
+    for (int u = 0; u < 8; ++u) v[u] = partial[(k + u) * L + s];
+#pragma unroll
+    for (int u = 0; u < 8; ++u) acc += v[u];
+  }
+  for (; k < ntiles; ++k) acc += partial[k * L + s];
+  totals[s] = acc;
+}
+
+/* One CTA per feature, grid-capped as k_pool_summ: draw k (< S = C L) of the feature is (w / D[k]) 1e6, w the sum of its
+ * members' draws at chain k >> lgL, slot k & (L - 1) in CSR order from 0.0 (gptr NULL: the feature is row `row` alone);
+ * D chain-major, so D[k] is that chain's total at that slot.  The member sum and the normalisation happen in the load,
+ * so no TPM trace is stored anywhere.  Then the mean, the two-pass sd and the percentiles of the NaN-last sort.  Shared
+ * memory: key fp64[P], the draws in draw order padded with NaN, sorted in place; 8 P bytes, 64 KB at S = 8192. */
+#define MMQ_TPM_SMEM_CAP (8 * 8192)
+
+__global__ void __launch_bounds__(MMQ_POST_THREADS)
+k_tpm_summ(const __grid_constant__ mmq_chain_ptrs cp, const double* __restrict__ totals, int C, int64_t rows, int lgL,
+           const int64_t* __restrict__ gptr, const int32_t* __restrict__ members, int npct, const int32_t* __restrict__ pct_idx,
+           double* __restrict__ out, double* __restrict__ pct) {
+  extern __shared__ double sh[];
+  const int L = 1 << lgL, S = C * L;
+  int P = 1;
+  while (P < S) P <<= 1;
+  double* key = sh;
+  const double nan = mmq_u2d(0x7ff8000000000000ull);
+  for (int64_t row = blockIdx.x; row < rows; row += gridDim.x) {
+    const int64_t b = gptr ? gptr[row] : row, e = gptr ? gptr[row + 1] : row + 1;
+    double bad = 0.0, sum = 0.0;
+    for (int k = threadIdx.x; k < P; k += blockDim.x) {
+      double v = nan;
+      if (k < S) {
+        const double* x = cp.p[k >> lgL] + (k & (L - 1));
+        double w = 0.0;
+        for (int64_t q = b; q < e; ++q) w += x[(int64_t)(gptr ? members[q] : q) << lgL];
+        v = (w / totals[k]) * 1e6;
+        bad += isfinite(v) ? 0.0 : 1.0;
+        sum += v;
+      }
+      key[k] = v;
+    }
+    bad = post_block_sum(bad); /* also orders the writes of key */
+    sum = post_block_sum(sum);
+    double mean = nan, sd = nan;
+    if (bad == 0.0) {
+      mean = sum / (double)S;
+      double ss = 0.0;
+      for (int k = threadIdx.x; k < S; k += blockDim.x) { const double d = key[k] - mean; ss += d * d; }
+      sd = sqrt(post_block_sum(ss) / (double)(S - 1));
+    }
+    sort_nan_last(key, P);
+    for (int j = threadIdx.x; j < npct; j += blockDim.x) {
+      const int q = pct_idx[j];
+      pct[row * npct + j] = q >= 0 && q < S ? key[q] : nan;
+    }
+    if (threadIdx.x == 0) { out[row] = mean; out[rows + row] = sd; }
     __syncthreads();
   }
 }
@@ -847,8 +950,8 @@ int mmq_chain_diagnostics_dev(const double* const* chain_dev, int nchains, int64
 }
 
 /* The checks of the handle forms (fn: the caller's name): no NULL handle, a trace on every chain, the same n, trace_len
- * and group counts, and a trace_len within the limits of the kernels. */
-static int chain_handles_check(mmq_handle* const* chains, int nchains, const char* fn) {
+ * and group counts, and a trace_len within the limits of the kernels (a power of two in [min_len, 2048]). */
+static int chain_handles_check(mmq_handle* const* chains, int nchains, const char* fn, int min_len = 8) {
   auto fail = [&](mmq_handle* h, int code, const char* what) { return mmq_fail(h, code, std::string(fn) + ": " + what); };
   for (int c = 0; c < nchains; ++c)
     if (!chains[c]) return fail(nullptr, MMQ_ERR_ARG, "NULL handle");
@@ -861,8 +964,9 @@ static int chain_handles_check(mmq_handle* const* chains, int nchains, const cha
       return fail(h0, MMQ_ERR_ARG, "the chains differ in n, trace_len or group counts");
   }
   const int L = h0->trace_len;
-  if (L < 8 || L > MMQ_MAX_ROW_LEN || (L & (L - 1)) != 0 || nchains * L > MMQ_CHAIN_SMAX)
-    return fail(h0, MMQ_ERR_ARG, "trace_len must be a power of two in [8, 2048] with nchains * trace_len <= 8192");
+  if (L < min_len || L > MMQ_MAX_ROW_LEN || (L & (L - 1)) != 0 || nchains * L > MMQ_CHAIN_SMAX)
+    return fail(h0, MMQ_ERR_ARG, ("trace_len must be a power of two in [" + std::to_string(min_len) +
+                                  ", 2048] with nchains * trace_len <= 8192").c_str());
   return MMQ_OK;
 }
 
@@ -1046,6 +1150,115 @@ int mmq_pooled_summaries(mmq_handle* const* chains, int nchains, int which, cons
     mmq_cache_free(prop[c]); mmq_cache_free(part[c]); mmq_cache_free(gdev[c]); mmq_cache_free(mdev[c]);
   }
   cudaSetDevice(h0->device);
+  return ret;
+}
+
+static bool tpm_len_ok(int nchains, int L) {
+  return nchains >= 1 && nchains <= MMQ_CHAINS_MAX && pow2_ok(L) && nchains * L <= MMQ_CHAIN_SMAX;
+}
+
+int64_t mmq_draw_totals_workspace_bytes(int64_t rows, int L) {
+  if (rows < 0 || !pow2_ok(L)) return 0;
+  const int64_t ntiles = (rows + MMQ_TOTALS_TILE - 1) / MMQ_TOTALS_TILE;
+  return (int64_t)sizeof(double) * ntiles * L;
+}
+
+int mmq_draw_totals_dev(const double* trace_dev, int64_t rows, int L, double* totals_dev, void* workspace_dev, void* cuda_stream) {
+  if (rows < 0 || !pow2_ok(L) || !totals_dev || (rows > 0 && (!trace_dev || !workspace_dev)))
+    return mmq_fail(nullptr, MMQ_ERR_ARG, "mmq_draw_totals_dev: bad arguments");
+  const cudaStream_t st = (cudaStream_t)cuda_stream;
+  const int64_t ntiles = (rows + MMQ_TOTALS_TILE - 1) / MMQ_TOTALS_TILE;
+  const int block = std::min(L, MMQ_TOTALS_THREADS), chunks = (L + block - 1) / block;
+  double* partial = static_cast<double*>(workspace_dev);
+  if (ntiles > 0) {
+    k_draw_totals<<<dim3((unsigned)ntiles, (unsigned)chunks), block, 0, st>>>(trace_dev, rows, L, partial);
+    g_mmq_launches.fetch_add(1);
+  }
+  k_totals_fold<<<chunks, block, 0, st>>>(partial, ntiles, L, totals_dev);
+  g_mmq_launches.fetch_add(1);
+  const cudaError_t e = cudaGetLastError();
+  if (e != cudaSuccess) return mmq_cuda_fail(nullptr, e, "k_draw_totals", __FILE__, __LINE__);
+  return MMQ_OK;
+}
+
+int mmq_tpm_summaries_dev(const double* const* chain_dev, const double* totals_dev, int nchains, int64_t rows, int L,
+                          const int64_t* group_ptr_dev, const int32_t* members_dev, int npct, const int32_t* pct_idx_dev,
+                          double* out_dev, double* pct_dev, void* cuda_stream) {
+  if (!chain_dev || !tpm_len_ok(nchains, L) || rows < 0 || npct < 0 || (!group_ptr_dev) != (!members_dev) ||
+      (rows > 0 && (!out_dev || !totals_dev)) || (rows > 0 && npct > 0 && (!pct_idx_dev || !pct_dev)))
+    return mmq_fail(nullptr, MMQ_ERR_ARG, "mmq_tpm_summaries_dev: bad arguments");
+  mmq_chain_ptrs cp = {};
+  for (int c = 0; c < nchains; ++c) {
+    if (!chain_dev[c]) return mmq_fail(nullptr, MMQ_ERR_ARG, "mmq_tpm_summaries_dev: NULL chain");
+    cp.p[c] = chain_dev[c];
+  }
+  if (rows == 0) return MMQ_OK;
+  int dev = 0, sms = 0, lgL = 0;
+  while ((1 << lgL) < L) ++lgL;
+  const size_t smem = sizeof(double) * (size_t)chain_pow2_at_least(nchains * L);
+  cudaError_t e = cudaGetDevice(&dev);
+  if (e == cudaSuccess) e = cudaDeviceGetAttribute(&sms, cudaDevAttrMultiProcessorCount, dev);
+  if (e == cudaSuccess) e = cudaFuncSetAttribute(k_tpm_summ, cudaFuncAttributeMaxDynamicSharedMemorySize, MMQ_TPM_SMEM_CAP);
+  if (e != cudaSuccess) return mmq_cuda_fail(nullptr, e, "mmq_tpm_summaries_dev", __FILE__, __LINE__);
+  const int grid = (int)std::min<int64_t>(rows, 2 * (int64_t)sms);
+  k_tpm_summ<<<grid, MMQ_POST_THREADS, smem, (cudaStream_t)cuda_stream>>>(cp, totals_dev, nchains, rows, lgL, group_ptr_dev, members_dev,
+                                                                          npct, pct_idx_dev, out_dev, pct_dev);
+  g_mmq_launches.fetch_add(1);
+  e = cudaGetLastError();
+  if (e != cudaSuccess) return mmq_cuda_fail(nullptr, e, "k_tpm_summ", __FILE__, __LINE__);
+  return MMQ_OK;
+}
+
+int mmq_tpm_summaries(mmq_handle* const* chains, int nchains, int which, int npct, const int32_t* pct_idx, double* mean, double* sd,
+                      double* pct, double* totals_out) {
+  if (!chains || nchains < 1 || nchains > MMQ_CHAINS_MAX || which < 0 || which > 2 || npct < 0 || (npct > 0 && !pct_idx))
+    return mmq_fail(chains ? chains[0] : nullptr, MMQ_ERR_ARG, "mmq_tpm_summaries: bad arguments");
+  if (const int rc = chain_handles_check(chains, nchains, "mmq_tpm_summaries", 4)) return rc;
+  mmq_handle* h0 = chains[0];
+  const int L = h0->trace_len;
+  const int64_t n = h0->n;
+  for (int j = 0; j < npct; ++j)
+    if (pct_idx[j] < 0 || pct_idx[j] >= nchains * L) return mmq_fail(h0, MMQ_ERR_ARG, "mmq_tpm_summaries: percentile index out of range");
+  const mmq_group_set* g = which == 0 ? nullptr : &h0->groups[which - 1];
+  const int64_t rows = which == 0 ? n : g->ngroups;
+  /* every chain's draws complete on its own device */
+  for (int c = 0; c < nchains; ++c) {
+    MMQ_CUDA(h0, cudaSetDevice(chains[c]->device));
+    MMQ_CUDA(h0, cudaStreamSynchronize(chains[c]->stream));
+  }
+  MMQ_CUDA(h0, cudaSetDevice(h0->device));
+  double *ws = nullptr, *work = nullptr, *totals = nullptr, *out = nullptr, *d_pct = nullptr;
+  int32_t* d_idx = nullptr;
+  const double *t[MMQ_CHAINS_MAX] = {}, *src[MMQ_CHAINS_MAX] = {};
+  for (int c = 0; c < nchains; ++c) t[c] = chains[c]->trace;
+  const int64_t wbytes = mmq_draw_totals_workspace_bytes(n, L);
+  cudaError_t e = mmq_cache_malloc(&work, (size_t)std::max<int64_t>(wbytes, 8));
+  if (e == cudaSuccess) e = mmq_cache_malloc(&totals, sizeof(double) * (size_t)nchains * (size_t)L);
+  if (e == cudaSuccess) e = mmq_cache_malloc(&out, sizeof(double) * 2 * (size_t)std::max<int64_t>(rows, 1));
+  if (e == cudaSuccess && npct > 0) {
+    e = mmq_cache_malloc(&d_pct, sizeof(double) * (size_t)std::max<int64_t>(rows, 1) * (size_t)npct);
+    if (e == cudaSuccess) e = mmq_cache_malloc(&d_idx, sizeof(int32_t) * (size_t)npct);
+    if (e == cudaSuccess) e = cudaMemcpyAsync(d_idx, pct_idx, sizeof(int32_t) * (size_t)npct, cudaMemcpyHostToDevice, h0->stream);
+  }
+  if (e == cudaSuccess) e = chain_gather(chains, nchains, t, n, L, &ws, src);
+  int ret = MMQ_OK;
+  for (int c = 0; c < nchains && e == cudaSuccess && ret == MMQ_OK; ++c) /* one workspace, reused in stream order */
+    ret = mmq_draw_totals_dev(src[c], n, L, totals + (size_t)c * (size_t)L, work, h0->stream);
+  if (e == cudaSuccess && ret == MMQ_OK)
+    ret = mmq_tpm_summaries_dev(src, totals, nchains, rows, L, g ? g->ptr_dev : nullptr, g ? g->members_dev : nullptr, npct, d_idx, out, d_pct,
+                                h0->stream);
+  if (ret) ret = mmq_fail(h0, ret, mmq_last_error(nullptr));
+  auto D = [&](void* dst, const void* from, size_t b) {
+    if (e == cudaSuccess && ret == MMQ_OK && dst && b) e = cudaMemcpyAsync(dst, from, b, cudaMemcpyDeviceToHost, h0->stream);
+  };
+  D(mean, out, sizeof(double) * (size_t)rows);
+  D(sd, out + rows, sizeof(double) * (size_t)rows);
+  if (npct > 0) D(pct, d_pct, sizeof(double) * (size_t)rows * (size_t)npct);
+  D(totals_out, totals, sizeof(double) * (size_t)nchains * (size_t)L);
+  const cudaError_t es = cudaStreamSynchronize(h0->stream);
+  if (e == cudaSuccess) e = es;
+  if (e != cudaSuccess && ret == MMQ_OK) ret = mmq_cuda_fail(h0, e, "mmq_tpm_summaries", __FILE__, __LINE__);
+  mmq_cache_free(ws); mmq_cache_free(work); mmq_cache_free(totals); mmq_cache_free(out); mmq_cache_free(d_pct); mmq_cache_free(d_idx);
   return ret;
 }
 

@@ -15,7 +15,8 @@
  * transcript, identical set and gene: *.counts, *.identical.counts, *.gene.counts), -chains INT (independent chains
  * from the EM estimate, split-R-hat and bulk / tail ESS per transcript, identical set and gene: *.convergence,
  * *.identical.convergence, *.gene.convergence), -pool (with -chains: the three tables and the -counts files over the draws
- * of all chains).
+ * of all chains), -tpm (posterior and EM transcripts per million per transcript, identical set and gene: *.tpm,
+ * *.identical.tpm, *.gene.tpm).
  */
 #include <unistd.h>
 #include <zlib.h>
@@ -79,6 +80,7 @@ static void printUsage(ostream& out) {
       << "  -counts            (B200 build) also write posterior and EM fragment counts (*.counts, *.identical.counts, *.gene.counts)" << endl
       << "  -chains INT        (B200 build) run INT independent chains (1..8, default: 1) and write split-R-hat and ESS per feature (*.convergence, *.identical.convergence, *.gene.convergence)" << endl
       << "  -pool              (B200 build) with -chains 2 or more: the *.mmseq tables and -counts files summarise the draws of all chains (default: chain 1's); trace files stay chain 1's" << endl
+      << "  -tpm               (B200 build) also write posterior and EM transcripts per million (*.tpm, *.identical.tpm, *.gene.tpm)" << endl
       << endl;
 }
 
@@ -178,6 +180,7 @@ struct Options {
   vector<double> percentiles{5.0, 25.0, 50.0, 75.0, 95.0};
   bool debug = false, notraces = false, counts = false;
   bool pool = false; /* -pool: the tables and -counts over the draws of all chains */
+  bool tpm = false;  /* -tpm: the .tpm files */
   int ngpus = 1;
   string batch;     /* -batch FILE: one "hits_file output_base" pair per line */
   int per_gpu = 4;  /* -per_gpu INT: samples in flight per GPU in batch mode */
@@ -222,7 +225,7 @@ static Options parse_command_line(int argc, char** argv) {
       {"-seed", INT, &o.seed},            {"-percentiles", TEXT, &pct},       {"-gpus", INT, &o.ngpus},
       {"-batch", TEXT, &o.batch},         {"-per_gpu", INT, &o.per_gpu},      {"-notraces", FLAG, &o.notraces},
       {"-debug", FLAG, &o.debug},         {"-counts", FLAG, &o.counts},       {"-chains", INT, &o.chains},
-      {"-pool", FLAG, &o.pool},
+      {"-pool", FLAG, &o.pool},           {"-tpm", FLAG, &o.tpm},
   };
   /* options come first; what is left must be the mandatory arguments (none in batch mode) */
   int i = 1;
@@ -990,6 +993,53 @@ static void run_sample(const Options& o, const string& hits_file, const string& 
                  [&](int64_t g) { return em_group(hdr.gene_members[(size_t)g]); });
   }
 
+  /* ---- -tpm: .tpm, .identical.tpm, .gene.tpm — rows and ids as in the three tables above.  Posterior mean, sd and
+   * percentiles of TPM over chain 1's draws (with -pool over every chain's, each chain normalised by its own totals;
+   * mmq_tpm_summaries), and the EM TPM from mu_em.  The totals are over the observed transcripts only, so TPM sums to 1e6
+   * over the observed features; a feature without an observed member reports 0 in every column. */
+  if (o.tpm) {
+    double em_total = 0.0;
+    for (int64_t t = 0; t < n; ++t) em_total += mu_em[(size_t)t];
+    auto em_members = [&](const vector<int32_t>& members) { /* the members' mu_em in header order (the CSR order of the groups) */
+      double w = 0.0;
+      for (int32_t hidx : members) { const int32_t c = cls.hdr2col[(size_t)hidx]; if (c >= 0) w += mu_em[(size_t)c]; }
+      return w;
+    };
+    auto observed = [&](const vector<int32_t>& members) {
+      for (int32_t hidx : members) if (cls.hdr2col[(size_t)hidx] >= 0) return true;
+      return false;
+    };
+    auto write_tpm = [&](const string& path, int which, int64_t rows, const function<string(int64_t)>& id, const function<int64_t(int64_t)>& row_of,
+                         const function<double(int64_t)>& em_sum) {
+      const int64_t R = which == 0 ? n : which == 1 ? I : G;
+      vector<double> mean((size_t)R), sdv((size_t)R), pct((size_t)R * NP);
+      if (R > 0)
+        check(mmq_tpm_summaries(chain_h.data(), npool, which, (int)NP, pidx_all.data(), mean.data(), sdv.data(), pct.data(), nullptr), H0,
+              "mmq_tpm_summaries");
+      const vector<double> zeros(NP, 0.0);
+      ofs.open(path.c_str());
+      ofs << "# Mapped fragments: " << N << endl;
+      ofs << "feature_id\tposterior_mean_tpm\tposterior_sd_tpm\tem_tpm\tpercentiles_tpm";
+      write_pcts(ofs, percentiles.data(), NP, '\n');
+      if (NP == 0) ofs << '\n';
+      write_rows(ofs, rows, [&](ostream& ofs, int64_t r) {
+        const int64_t q = row_of(r);
+        ofs << id(r) << "\t";
+        if (q < 0) ofs << 0 << "\t" << 0 << "\t" << 0 << "\t";
+        else ofs << mean[(size_t)q] << "\t" << sdv[(size_t)q] << "\t" << (em_sum(q) / em_total) * 1000000.0 << "\t";
+        write_pcts(ofs, q < 0 ? zeros.data() : pct.data() + (size_t)q * NP, NP, '\n');
+        if (NP == 0) ofs << '\n';
+      });
+      ofs.close(); ofs.clear();
+    };
+    write_tpm(output_base + ".tpm", 0, T, [&](int64_t hI) { return hdr.names[(size_t)hI]; },
+              [&](int64_t hI) { return (int64_t)cls.hdr2col[(size_t)hI]; }, [&](int64_t c) { return mu_em[(size_t)c]; });
+    write_tpm(output_base + ".identical.tpm", 1, I, identical_id, [&](int64_t s) { return observed(hdr.identical[(size_t)s]) ? s : -1; },
+              [&](int64_t s) { return em_members(hdr.identical[(size_t)s]); });
+    write_tpm(output_base + ".gene.tpm", 2, G, [&](int64_t g) { return hdr.gene_names[(size_t)g]; },
+              [&](int64_t g) { return observed(hdr.gene_members[(size_t)g]) ? g : -1; }, [&](int64_t g) { return em_members(hdr.gene_members[(size_t)g]); });
+  }
+
   /* ---- -chains: .convergence, .identical.convergence, .gene.convergence — rows and ids as in the three tables above.
    * log_mu and sd pooled over the draws of all chains, split-R-hat and bulk / tail ESS (mmq_chain_diagnostics); a row
    * whose `observed` column is 0 carries that table's closed-form log_mu and sd, and NA. */
@@ -1059,6 +1109,10 @@ static void run_sample(const Options& o, const string& hits_file, const string& 
     out << "  " << output_base << ".counts" << endl
         << "  " << output_base << ".identical.counts" << endl
         << "  " << output_base << ".gene.counts" << endl;
+  if (o.tpm)
+    out << "  " << output_base << ".tpm" << endl
+        << "  " << output_base << ".identical.tpm" << endl
+        << "  " << output_base << ".gene.tpm" << endl;
   if (nchains > 1)
     out << "  " << output_base << ".convergence" << endl
         << "  " << output_base << ".identical.convergence" << endl
