@@ -328,6 +328,25 @@ static void run_sample(const Options& o, const string& hits_file, const string& 
     if (mmq::scaled_lengths(hdr, cls, l, err)) die(err);
   }
 
+  /* ---- the groups in column space: each observed transcript's identical set (-1: none) and gene, whether that gene
+   * has other isoforms, and the observed members of every identical set and gene (CSR, in header order) */
+  vector<int32_t> ident_of((size_t)n, -1), gene_of((size_t)n);
+  vector<uint8_t> multi((size_t)n);
+  vector<int64_t> iptr{0}, gptr{0};
+  vector<int32_t> imem, gmem;
+  for (int64_t s = 0; s < I; ++s) {
+    for (int32_t hidx : hdr.identical[(size_t)s]) { const int32_t c = cls.hdr2col[(size_t)hidx]; if (c >= 0) { ident_of[(size_t)c] = (int32_t)s; imem.push_back(c); } }
+    iptr.push_back((int64_t)imem.size());
+  }
+  for (int64_t g = 0; g < G; ++g) {
+    for (int32_t hidx : hdr.gene_members[(size_t)g]) { const int32_t c = cls.hdr2col[(size_t)hidx]; if (c >= 0) gmem.push_back(c); }
+    gptr.push_back((int64_t)gmem.size());
+  }
+  for (int64_t t = 0; t < n; ++t) {
+    gene_of[(size_t)t] = hdr.gene_of[(size_t)cls.col2hdr[(size_t)t]];
+    multi[(size_t)t] = hdr.gene_members[(size_t)gene_of[(size_t)t]].size() > 1;
+  }
+
   /* ---- shards.  The library orders the classes of a shard itself (class plan, mmq_cls.cu), so the
    * host hands them over as they are: one GPU takes the loader's arrays in place; several GPUs take
    * every ngpus-th class (first-appearance order is unrelated to the cost of a class, so the deal is
@@ -421,14 +440,10 @@ static void run_sample(const Options& o, const string& hits_file, const string& 
   {
     phase("shards on the GPUs");
     err << "Counting unique hits to sets of identical transcripts...";
-    vector<int32_t> set_of((size_t)n, -1);
-    for (int64_t s = 0; s < I; ++s)
-      for (int32_t hidx : hdr.identical[(size_t)s]) { int32_t c = cls.hdr2col[(size_t)hidx]; if (c >= 0) set_of[(size_t)c] = (int32_t)s; }
-    if (I > 0) on_all([&](int g) { check(mmq_unique_hits_sets(shards[(size_t)g].h, set_of.data(), I, g == 0 ? identical_unique_hits.data() : vector<int32_t>((size_t)I).data()), shards[(size_t)g].h, "mmq_unique_hits_sets"); });
+    if (I > 0) on_all([&](int g) { check(mmq_unique_hits_sets(shards[(size_t)g].h, ident_of.data(), I, g == 0 ? identical_unique_hits.data() : vector<int32_t>((size_t)I).data()), shards[(size_t)g].h, "mmq_unique_hits_sets"); });
     err << "done." << endl;
     err << "Counting unique hits to genes...";
-    for (int64_t t = 0; t < n; ++t) set_of[(size_t)t] = hdr.gene_of[(size_t)cls.col2hdr[(size_t)t]];
-    on_all([&](int g) { check(mmq_unique_hits_sets(shards[(size_t)g].h, set_of.data(), G, g == 0 ? gene_unique_hits.data() : vector<int32_t>((size_t)G).data()), shards[(size_t)g].h, "mmq_unique_hits_sets"); });
+    on_all([&](int g) { check(mmq_unique_hits_sets(shards[(size_t)g].h, gene_of.data(), G, g == 0 ? gene_unique_hits.data() : vector<int32_t>((size_t)G).data()), shards[(size_t)g].h, "mmq_unique_hits_sets"); });
     err << "done." << endl;
   }
 
@@ -551,7 +566,6 @@ static void run_sample(const Options& o, const string& hits_file, const string& 
   /* ---- -counts: EM expected counts at mu_em (one E-step, all shards), and from here on every Gibbs sweep adds its
    * counts of transcripts, identical sets and genes into the accumulators of every shard (with -pool, of every chain) */
   vector<double> em_count;
-  vector<int32_t> ident_of, gene_of;
   if (o.counts) {
     em_count.resize((size_t)n);
     vector<vector<double>> other((size_t)ngpus);
@@ -560,11 +574,6 @@ static void run_sample(const Options& o, const string& hits_file, const string& 
       if (g > 0) other[(size_t)g].resize((size_t)n);
       check(mmq_expected_counts(h, g == 0 ? em_count.data() : other[(size_t)g].data()), h, "mmq_expected_counts");
     });
-    ident_of.assign((size_t)n, -1);
-    gene_of.resize((size_t)n);
-    for (int64_t s = 0; s < I; ++s)
-      for (int32_t hidx : hdr.identical[(size_t)s]) { const int32_t c = cls.hdr2col[(size_t)hidx]; if (c >= 0) ident_of[(size_t)c] = (int32_t)s; }
-    for (int64_t t = 0; t < n; ++t) gene_of[(size_t)t] = hdr.gene_of[(size_t)cls.col2hdr[(size_t)t]];
     on_all([&](int g) {
       mmq_handle* h = shards[(size_t)g].h;
       check(mmq_count_moments_begin(h, ident_of.data(), I, gene_of.data(), G), h, "mmq_count_moments_begin");
@@ -604,6 +613,13 @@ static void run_sample(const Options& o, const string& hits_file, const string& 
   phase("EM + Gibbs");
   out << "Amalgamating transcripts and calculating summary statistics..." << flush;
 
+  /* the Gamma prior's rate for a feature of effective length len, and the closed-form log_mu of a feature without
+   * hits (:971-978, :1372-1395) */
+  auto prior_rate = [&](double len) { return beta + len * (double)N / 1000000000.0; };
+  const double digalpha = mmq_host_digamma(alpha);
+  const double sqrtpolygalpha = sqrt(mmq_host_trigamma(alpha));
+  auto closed_log_mu = [&](double len) { return digalpha - log(prior_rate(len)); };
+
   /* ---- prior-simulated traces for isoforms without hits (src/mmseq.cpp:971-978), on the device */
   vector<int64_t> unobs;           /* header indices */
   vector<int64_t> unobs_slot((size_t)T, -1);
@@ -612,7 +628,7 @@ static void run_sample(const Options& o, const string& hits_file, const string& 
   const int64_t U = (int64_t)unobs.size();
   vector<double> simu((size_t)U * (size_t)L);
   vector<double> rate((size_t)U);
-  for (int64_t u = 0; u < U; ++u) rate[(size_t)u] = beta + hdr.efflen[(size_t)unobs[(size_t)u]] * (double)N / 1000000000.0;
+  for (int64_t u = 0; u < U; ++u) rate[(size_t)u] = prior_rate(hdr.efflen[(size_t)unobs[(size_t)u]]);
   if (U > 0 && mmq_prior_draws(shards[0].device, U, unobs.data(), rate.data(), alpha, (uint32_t)seed, L, simu.data()))
     die(string("Error: mmq_prior_draws: ") + mmq_last_error(nullptr));
 
@@ -621,16 +637,6 @@ static void run_sample(const Options& o, const string& hits_file, const string& 
    * isoforms' pooled columns) */
   vector<vector<double>> simu_pool((size_t)nchains); /* [c >= 1]: chain c's prior draws, under -pool */
   {
-    vector<int64_t> iptr{0}, gptr{0};
-    vector<int32_t> imem, gmem;
-    for (int64_t s = 0; s < I; ++s) {
-      for (int32_t hidx : hdr.identical[(size_t)s]) { int32_t c = cls.hdr2col[(size_t)hidx]; if (c >= 0) imem.push_back(c); }
-      iptr.push_back((int64_t)imem.size());
-    }
-    for (int64_t g = 0; g < G; ++g) {
-      for (int32_t hidx : hdr.gene_members[(size_t)g]) { int32_t c = cls.hdr2col[(size_t)hidx]; if (c >= 0) gmem.push_back(c); }
-      gptr.push_back((int64_t)gmem.size());
-    }
     vector<double> extra((size_t)G * (size_t)L), simu_c;
     for (int c = 0; c < nchains; ++c) {
       mmq_handle* h = chain_h[(size_t)c];
@@ -654,96 +660,111 @@ static void run_sample(const Options& o, const string& hits_file, const string& 
     }
   }
 
-  /* ---- summaries on the device */
-  const size_t NP = percentiles.size();
-  vector<int32_t> pidx(NP);
-  for (size_t i = 0; i < NP; i++) pidx[i] = static_cast<int>(round(percentiles[i] / 100.0 * (trace_length - 1))); /* :1113 */
-  struct Summ { vector<double> mean, var, tau, pct; vector<int32_t> win, status; };
-  auto summarize = [&](int which, int64_t rows) {
-    Summ S;
-    S.mean.resize((size_t)rows); S.var.resize((size_t)rows); S.tau.resize((size_t)rows);
-    S.win.resize((size_t)rows); S.status.resize((size_t)rows); S.pct.resize((size_t)rows * NP);
-    if (rows > 0 && !(o.pool && which == 0)) /* -pool: every transcript row comes from mmq_pooled_summaries below */
-      check(mmq_summarize(H0, which, S.mean.data(), S.var.data(), S.tau.data(), S.win.data(), S.status.data(), (int)NP, pidx.data(), S.pct.data()), H0, "mmq_summarize");
-    return S;
+  /* ---- the three levels of every per-feature output, in the order of the C ABI's `which`: transcripts (a table row
+   * per header transcript, a device row per observed one), identical sets and genes (one row per group in both) */
+  struct Summ { vector<double> mean, sd, mcse, iact, pct; }; /* the .mmseq columns of every device row */
+  Summ summ[3];
+  vector<char> ident_obs((size_t)I); /* the identical sets' `observed`: chain 1's log mean is finite (:1567) */
+  /* an identical set's columns follow its members named as the last member (:1560-1565); "+" follows the others */
+  auto named_last = [&](const vector<int32_t>& mem, size_t j) { return hdr.names[(size_t)mem[j]].compare(hdr.names[(size_t)mem.back()]) == 0; };
+  auto identical_id = [&](int64_t s) {
+    const auto& mem = hdr.identical[(size_t)s];
+    string id;
+    for (size_t j = 0; j < mem.size(); ++j) { id += hdr.names[(size_t)mem[j]]; if (!named_last(mem, j)) id += "+"; }
+    return id;
   };
-  Summ St = summarize(0, n), Si = summarize(1, I), Sg = summarize(2, G);
-  /* sd, mcse, iact (:1308-1363) */
-  auto finish = [&](const Summ& S, vector<double>& sd, vector<double>& mcse, vector<double>& iact) {
-    const size_t R = S.mean.size();
-    sd.resize(R); mcse.resize(R); iact.resize(R);
-    for (size_t r = 0; r < R; ++r) {
-      if (S.status[r] != 0) { mcse[r] = trace_length; iact[r] = NAN; }
-      else { mcse[r] = sqrt(S.tau[r] * S.var[r] / trace_length); iact[r] = S.tau[r]; }
-      sd[r] = sqrt(S.var[r]);
+  struct Level {
+    const char* suffix;         /* of the level's output files */
+    const char* name;
+    int which;
+    int64_t rows, dev_rows;     /* table rows, device rows */
+    const vector<int64_t>* ptr; /* groups: the observed members of each (iptr / imem, gptr / gmem) */
+    const vector<int32_t>* mem;
+    function<string(int64_t)> id;       /* table row -> feature id */
+    function<int64_t(int64_t)> dev_row; /* table row -> device row, -1 for a transcript without hits */
+    function<bool(int64_t)> observed;   /* device row -> the `observed` column of the .mmseq and .convergence tables */
+    function<pair<double, double>(int64_t)> unobserved; /* table row -> log_mu and sd of a row that is not observed */
+    bool has_hits(int64_t q) const { return !ptr || (*ptr)[(size_t)q + 1] > (*ptr)[(size_t)q]; }
+    double sum(int64_t q, const vector<double>& x) const { /* a group's: its members' in header order */
+      if (!ptr) return x[(size_t)q];
+      double s = 0.0;
+      for (int64_t k = (*ptr)[(size_t)q]; k < (*ptr)[(size_t)q + 1]; ++k) s += x[(size_t)(*mem)[(size_t)k]];
+      return s;
     }
   };
-  vector<double> sd, mumcse, iact, sd_identical, mumcse_identical, iact_identical, sd_gene, mumcse_gene, iact_gene;
-  finish(St, sd, mumcse, iact);
-  finish(Si, sd_identical, mumcse_identical, iact_identical);
-  finish(Sg, sd_gene, mumcse_gene, iact_gene);
-  /* observed rows of the identical-set and gene tables (:1567, :1625-1628) */
-  vector<char> ident_obs((size_t)I), gene_obs((size_t)G, 0);
-  for (int64_t s = 0; s < I; ++s) ident_obs[(size_t)s] = isfinite(Si.mean[(size_t)s]) != 0;
-  for (int64_t g = 0; g < G; ++g)
-    for (int32_t hidx : hdr.gene_members[(size_t)g]) if (cls.hdr2col[(size_t)hidx] >= 0) { gene_obs[(size_t)g] = 1; break; }
-  /* -pool: the draws of all chains, `draws` of them per feature; the percentile rule of :1113 with draws for the trace
-   * length.  The stochastic columns of observed rows come from mmq_pooled_summaries: mcse = sd / sqrt(ess_mean),
-   * iact = draws / ess_mean.  What survives of chain 1's summaries: the unobserved rows of the identical-set and gene
-   * tables (as in the .convergence files) and the identical sets' observed test (ident_obs). */
+  auto same_row = [](int64_t r) { return r; };
+  const Level levels[3] = {
+      {"", "transcripts", 0, T, n, nullptr, nullptr, [&](int64_t hI) { return hdr.names[(size_t)hI]; },
+       [&](int64_t hI) { return (int64_t)cls.hdr2col[(size_t)hI]; }, [](int64_t) { return true; },
+       [&](int64_t hI) { return make_pair(closed_log_mu(hdr.efflen[(size_t)hI]), sqrtpolygalpha); }},
+      {".identical", "identical sets", 1, I, I, &iptr, &imem, identical_id, same_row, [&](int64_t s) { return ident_obs[(size_t)s] != 0; },
+       [&](int64_t s) {
+         const auto& mem = hdr.identical[(size_t)s];
+         size_t j = 0;
+         while (!named_last(mem, j)) ++j;
+         return make_pair(log(mem.size()) + digalpha - log(prior_rate(hdr.efflen[(size_t)mem[j]])), sqrtpolygalpha);
+       }},
+      {".gene", "genes", 2, G, G, &gptr, &gmem, [&](int64_t g) { return hdr.gene_names[(size_t)g]; }, same_row,
+       [&](int64_t g) { return gptr[(size_t)g + 1] > gptr[(size_t)g]; },
+       [&](int64_t g) { return make_pair(summ[2].mean[(size_t)g], summ[2].sd[(size_t)g]); }}, /* chain 1's, as the reference */
+  };
+
+  /* ---- summaries on the device: chain 1's (sd, mcse, iact: :1308-1363).  With -pool the observed rows come from
+   * mmq_pooled_summaries over the draws of all chains, `draws` of them per feature, with the percentile rule of :1113
+   * for `draws` draws: mcse = sd / sqrt(ess_mean), iact = draws / ess_mean.  What survives of chain 1's summaries: the
+   * unobserved rows of the identical-set and gene tables (as in the .convergence files) and ident_obs. */
+  const size_t NP = percentiles.size();
   const int npool = o.pool ? nchains : 1;
   const int64_t draws = (int64_t)npool * L;
-  vector<int32_t> pidx_all(NP);
-  for (size_t i = 0; i < NP; i++) pidx_all[i] = static_cast<int>(round(percentiles[i] / 100.0 * (draws - 1)));
-  if (o.pool) {
-    auto pooled = [&](int which, int64_t rows, Summ& Sm, vector<double>& sdv, vector<double>& mcse, vector<double>& iactv,
-                      const function<bool(int64_t)>& observed) {
-      vector<double> mean((size_t)rows), psd((size_t)rows), ess((size_t)rows), pct((size_t)rows * NP);
-      if (rows > 0)
-        check(mmq_pooled_summaries(chain_h.data(), nchains, which, nullptr, nullptr, (int)NP, pidx_all.data(), mean.data(), psd.data(), ess.data(),
-                                   nullptr, nullptr, pct.data()), H0, "mmq_pooled_summaries");
-      for (int64_t r = 0; r < rows; ++r) {
-        if (!observed(r)) continue;
-        Sm.mean[(size_t)r] = mean[(size_t)r];
-        sdv[(size_t)r] = psd[(size_t)r];
-        mcse[(size_t)r] = psd[(size_t)r] / sqrt(ess[(size_t)r]);
-        iactv[(size_t)r] = (double)draws / ess[(size_t)r];
-        copy(pct.begin() + (ptrdiff_t)((size_t)r * NP), pct.begin() + (ptrdiff_t)((size_t)(r + 1) * NP), Sm.pct.begin() + (ptrdiff_t)((size_t)r * NP));
-      }
-    };
-    pooled(0, n, St, sd, mumcse, iact, [](int64_t) { return true; });
-    pooled(1, I, Si, sd_identical, mumcse_identical, iact_identical, [&](int64_t s) { return ident_obs[(size_t)s] != 0; });
-    pooled(2, G, Sg, sd_gene, mumcse_gene, iact_gene, [&](int64_t g) { return gene_obs[(size_t)g] != 0; });
+  vector<int32_t> pidx(NP), pidx_all(NP);
+  for (size_t i = 0; i < NP; i++) {
+    pidx[i] = static_cast<int>(round(percentiles[i] / 100.0 * (trace_length - 1))); /* :1113 */
+    pidx_all[i] = static_cast<int>(round(percentiles[i] / 100.0 * (draws - 1)));
   }
-  const vector<double>& meanmu = St.mean;
-  const vector<double>& meanmu_identical = Si.mean;
-  const vector<double>& meanmu_gene = Sg.mean;
+  for (const Level& lv : levels) {
+    Summ& S = summ[lv.which];
+    const size_t R = (size_t)lv.dev_rows;
+    vector<double> var(R), tau(R);
+    vector<int32_t> win(R), status(R);
+    S.mean.resize(R); S.sd.resize(R); S.mcse.resize(R); S.iact.resize(R); S.pct.resize(R * NP);
+    if (R > 0 && !(o.pool && lv.which == 0)) /* -pool: every transcript row comes from mmq_pooled_summaries */
+      check(mmq_summarize(H0, lv.which, S.mean.data(), var.data(), tau.data(), win.data(), status.data(), (int)NP, pidx.data(), S.pct.data()), H0, "mmq_summarize");
+    for (size_t r = 0; r < R; ++r) {
+      if (status[r] != 0) { S.mcse[r] = trace_length; S.iact[r] = NAN; }
+      else { S.mcse[r] = sqrt(tau[r] * var[r] / trace_length); S.iact[r] = tau[r]; }
+      S.sd[r] = sqrt(var[r]);
+    }
+    if (lv.which == 1) for (size_t s = 0; s < R; ++s) ident_obs[s] = isfinite(S.mean[s]) != 0;
+    if (!o.pool || R == 0) continue;
+    vector<double> mean(R), psd(R), ess(R), pct(R * NP);
+    check(mmq_pooled_summaries(chain_h.data(), nchains, lv.which, nullptr, nullptr, (int)NP, pidx_all.data(), mean.data(), psd.data(), ess.data(),
+                               nullptr, nullptr, pct.data()), H0, "mmq_pooled_summaries");
+    for (size_t r = 0; r < R; ++r) {
+      if (!lv.observed((int64_t)r)) continue;
+      S.mean[r] = mean[r];
+      S.sd[r] = psd[r];
+      S.mcse[r] = psd[r] / sqrt(ess[r]);
+      S.iact[r] = (double)draws / ess[r];
+      copy(pct.begin() + (ptrdiff_t)(r * NP), pct.begin() + (ptrdiff_t)((r + 1) * NP), S.pct.begin() + (ptrdiff_t)(r * NP));
+    }
+  }
 
   /* proportions of observed transcripts (:985-1008, :1236-1265) */
   vector<double> meanprop((size_t)n), meanprobitprop((size_t)n), ssprobitprop((size_t)n), sdprobitprop((size_t)n), pct_prop((size_t)n * NP);
   vector<double> prop_trace;
-  {
-    vector<int32_t> gene_of_col((size_t)n);
-    vector<uint8_t> multi((size_t)n);
-    for (int64_t t = 0; t < n; ++t) {
-      const int32_t g = hdr.gene_of[(size_t)cls.col2hdr[(size_t)t]];
-      gene_of_col[(size_t)t] = g;
-      multi[(size_t)t] = hdr.gene_members[(size_t)g].size() > 1;
-    }
-    if (!notraces) prop_trace.resize((size_t)n * (size_t)L);
-    if (!o.pool)
-      check(mmq_prop_summaries(H0, gene_of_col.data(), multi.data(), meanprop.data(), meanprobitprop.data(), ssprobitprop.data(), (int)NP, pidx.data(),
-                               pct_prop.data(), notraces ? nullptr : prop_trace.data()), H0, "mmq_prop_summaries");
-    else if (!notraces) /* chain 1's proportion trace for its trace file; the summaries come from all chains below */
-      check(mmq_prop_summaries(H0, gene_of_col.data(), multi.data(), nullptr, nullptr, nullptr, 0, nullptr, nullptr, prop_trace.data()), H0,
-            "mmq_prop_summaries");
-    if (o.pool) /* every chain's proportions over its own gene trace; the probit sums added over the chains */
-      check(mmq_pooled_summaries(chain_h.data(), nchains, 3, gene_of_col.data(), multi.data(), (int)NP, pidx_all.data(), meanprop.data(), nullptr,
-                                 nullptr, meanprobitprop.data(), ssprobitprop.data(), pct_prop.data()), H0, "mmq_pooled_summaries");
-    for (int64_t t = 0; t < n; t++) /* :1260-1265, same expression order */
-      sdprobitprop[(size_t)t] = sqrt((ssprobitprop[(size_t)t] - meanprobitprop[(size_t)t] * meanprobitprop[(size_t)t] / draws) / (draws - 1.0));
-    for (int64_t t = 0; t < n; t++) meanprobitprop[(size_t)t] /= draws;
-  }
+  if (!notraces) prop_trace.resize((size_t)n * (size_t)L);
+  if (!o.pool)
+    check(mmq_prop_summaries(H0, gene_of.data(), multi.data(), meanprop.data(), meanprobitprop.data(), ssprobitprop.data(), (int)NP, pidx.data(),
+                             pct_prop.data(), notraces ? nullptr : prop_trace.data()), H0, "mmq_prop_summaries");
+  else if (!notraces) /* chain 1's proportion trace for its trace file; the summaries come from all chains below */
+    check(mmq_prop_summaries(H0, gene_of.data(), multi.data(), nullptr, nullptr, nullptr, 0, nullptr, nullptr, prop_trace.data()), H0,
+          "mmq_prop_summaries");
+  if (o.pool) /* every chain's proportions over its own gene trace; the probit sums added over the chains */
+    check(mmq_pooled_summaries(chain_h.data(), nchains, 3, gene_of.data(), multi.data(), (int)NP, pidx_all.data(), meanprop.data(), nullptr,
+                               nullptr, meanprobitprop.data(), ssprobitprop.data(), pct_prop.data()), H0, "mmq_pooled_summaries");
+  for (int64_t t = 0; t < n; t++) /* :1260-1265, same expression order */
+    sdprobitprop[(size_t)t] = sqrt((ssprobitprop[(size_t)t] - meanprobitprop[(size_t)t] * meanprobitprop[(size_t)t] / draws) / (draws - 1.0));
+  for (int64_t t = 0; t < n; t++) meanprobitprop[(size_t)t] /= draws;
 
   /* gene traces are needed on the host for the hit-less isoforms' proportions and the trace file */
   vector<double> gene_trace((size_t)G * (size_t)L);
@@ -768,7 +789,7 @@ static void run_sample(const Options& o, const string& hits_file, const string& 
       vector<double> v((size_t)draws), pv((size_t)draws);
       for (int64_t u = u0; u < u1; ++u) {
         const int32_t g = hdr.gene_of[(size_t)unobs[(size_t)u]];
-        const bool multi = hdr.gene_members[(size_t)g].size() > 1;
+        const bool multi_iso = hdr.gene_members[(size_t)g].size() > 1;
         double mp = 0.0, s1 = 0.0, s2 = 0.0;
         for (int c = 0; c < npool; ++c) {
           const double* sv = sim_c[(size_t)c] + (size_t)u * (size_t)L;
@@ -780,7 +801,7 @@ static void run_sample(const Options& o, const string& hits_file, const string& 
             pv[(size_t)c * (size_t)L + (size_t)i] = p;
             mp += p;
             double temp;
-            if (multi) temp = mmq_host_ndtri(min(max(p, 0.000000001), 0.999999999));
+            if (multi_iso) temp = mmq_host_ndtri(min(max(p, 0.000000001), 0.999999999));
             else temp = numeric_limits<double>::infinity();
             c1 += temp;
             c2 += temp * temp;
@@ -806,16 +827,6 @@ static void run_sample(const Options& o, const string& hits_file, const string& 
   }
 
   phase("summaries");
-  /* feature id of an identical set: the member names joined by "+" (:1560-1565) */
-  auto identical_id = [&](int64_t s) {
-    string id;
-    const auto& mem = hdr.identical[(size_t)s];
-    for (size_t j = 0; j < mem.size(); ++j) {
-      id += hdr.names[(size_t)mem[j]];
-      if (hdr.names[(size_t)mem[j]].compare(hdr.names[(size_t)mem.back()]) != 0) id += "+";
-    }
-    return id;
-  };
   /* ---- trace dumps (:829-831, :911-917, :1033-1108) */
   if (!notraces) {
     vector<double> tr((size_t)n * (size_t)L);
@@ -839,22 +850,21 @@ static void run_sample(const Options& o, const string& hits_file, const string& 
   }
 
   phase("trace files");
-  /* ---- closed forms for unobserved features and gene lengths (:1372-1395) */
-  const double digalpha = mmq_host_digamma(alpha);
-  const double sqrtpolygalpha = sqrt(mmq_host_trigamma(alpha));
+  const Summ &St = summ[0], &Si = summ[1], &Sg = summ[2];
+  /* ---- gene lengths (:1372-1395) */
   vector<double> gene_lengths((size_t)G, 0.0);
   for (int64_t g = 0; g < G; ++g) {
-    if (isfinite(meanmu_gene[(size_t)g]) != 0) {
+    if (isfinite(Sg.mean[(size_t)g]) != 0) {
       double sum = 0;
       for (int32_t hidx : hdr.gene_members[(size_t)g]) {
         const int32_t c = cls.hdr2col[(size_t)hidx];
         const double len = hdr.efflen[(size_t)hidx];
         if (c >= 0) {
-          gene_lengths[(size_t)g] += len * exp(meanmu[(size_t)c]);
-          sum += exp(meanmu[(size_t)c]);
+          gene_lengths[(size_t)g] += len * exp(St.mean[(size_t)c]);
+          sum += exp(St.mean[(size_t)c]);
         } else {
-          gene_lengths[(size_t)g] += len * exp((digalpha - log(beta + len * (double)N / 1000000000.0)));
-          sum += exp((digalpha - log(beta + len * (double)N / 1000000000.0)));
+          gene_lengths[(size_t)g] += len * exp(closed_log_mu(len));
+          sum += exp(closed_log_mu(len));
         }
       }
       gene_lengths[(size_t)g] /= sum;
@@ -874,7 +884,7 @@ static void run_sample(const Options& o, const string& hits_file, const string& 
     const int32_t c = cls.hdr2col[(size_t)hI];
     const size_t ntr = hdr.gene_members[(size_t)hdr.gene_of[(size_t)hI]].size();
     if (c >= 0) {
-      ofs << name << "\t" << meanmu[(size_t)c] << "\t" << sd[(size_t)c] << "\t" << mumcse[(size_t)c] << "\t" << iact[(size_t)c] << "\t"
+      ofs << name << "\t" << St.mean[(size_t)c] << "\t" << St.sd[(size_t)c] << "\t" << St.mcse[(size_t)c] << "\t" << St.iact[(size_t)c] << "\t"
           << hdr.efflen[(size_t)hI] << "\t" << hdr.truelen[(size_t)hI] << "\t" << unique_hits[(size_t)c] << "\t" << meanprop[(size_t)c] << "\t"
           << meanprobitprop[(size_t)c] << "\t" << sdprobitprop[(size_t)c] << "\t" << log(mu_em[(size_t)c]) << "\t"
           << "1" << "\t" << ntr << "\t";
@@ -882,7 +892,7 @@ static void run_sample(const Options& o, const string& hits_file, const string& 
       write_pcts(ofs, pct_prop.data() + (size_t)c * NP, NP, '\n');
     } else {
       const size_t u = (size_t)unobs_slot[(size_t)hI];
-      ofs << name << "\t" << digalpha - log(beta + hdr.efflen[(size_t)hI] * (double)N / 1000000000.0) << "\t" << sqrtpolygalpha << "\t"
+      ofs << name << "\t" << closed_log_mu(hdr.efflen[(size_t)hI]) << "\t" << sqrtpolygalpha << "\t"
           << "0" << "\t" << "1" << "\t" << hdr.efflen[(size_t)hI] << "\t" << hdr.truelen[(size_t)hI] << "\t" << 0 << "\t" << meanprop_simu[u] << "\t"
           << meanprobitprop_simu[u] << "\t" << sdprobitprop_simu[u] << "\t" << "NA" << "\t" << "0" << "\t" << ntr << "\t";
       write_pcts(ofs, pct_simu.data() + u * NP, NP, '\t');
@@ -899,29 +909,18 @@ static void run_sample(const Options& o, const string& hits_file, const string& 
   write_pcts(ofs, percentiles.data(), NP, '\n');
   for (int64_t s = 0; s < I; ++s) {
     const auto& mem = hdr.identical[(size_t)s];
-    const string& backname = hdr.names[(size_t)mem.back()];
     const int32_t first = mem.front();
-    if (ident_obs[(size_t)s]) {
-      for (size_t j = 0; j < mem.size(); ++j) {
-        const string& nm = hdr.names[(size_t)mem[j]];
-        ofs << nm;
-        if (nm.compare(backname) != 0) ofs << "+";
-        else ofs << "\t" << meanmu_identical[(size_t)s] << "\t" << sd_identical[(size_t)s] << "\t" << mumcse_identical[(size_t)s] << "\t"
-                 << iact_identical[(size_t)s] << "\t" << hdr.efflen[(size_t)first] << "\t" << hdr.truelen[(size_t)first] << "\t"
-                 << identical_unique_hits[(size_t)s] << "\t" << "1" << "\t" << mem.size() << "\t";
-      }
-      write_pcts(ofs, Si.pct.data() + (size_t)s * NP, NP, '\n');
-    } else {
-      for (size_t j = 0; j < mem.size(); ++j) {
-        const string& nm = hdr.names[(size_t)mem[j]];
-        ofs << nm;
-        if (nm.compare(backname) != 0) ofs << "+";
-        else ofs << "\t" << log(mem.size()) + digalpha - log(beta + hdr.efflen[(size_t)mem[j]] * (double)N / 1000000000.0) << "\t" << sqrtpolygalpha
-                 << "\t" << "0" << "\t" << "NA" << "\t" << hdr.efflen[(size_t)first] << "\t" << hdr.truelen[(size_t)first] << "\t" << 0 << "\t"
-                 << "0" << "\t" << mem.size() << "\t";
-      }
-      for (size_t i = 0; i < NP; i++) ofs << "NA" << (i == NP - 1 ? "\n" : ",");
+    const bool obs = ident_obs[(size_t)s] != 0;
+    for (size_t j = 0; j < mem.size(); ++j) {
+      ofs << hdr.names[(size_t)mem[j]];
+      if (!named_last(mem, j)) { ofs << "+"; continue; }
+      if (obs) ofs << "\t" << Si.mean[(size_t)s] << "\t" << Si.sd[(size_t)s] << "\t" << Si.mcse[(size_t)s] << "\t" << Si.iact[(size_t)s];
+      else { const auto u = levels[1].unobserved(s); ofs << "\t" << u.first << "\t" << u.second << "\t" << "0" << "\t" << "NA"; }
+      ofs << "\t" << hdr.efflen[(size_t)first] << "\t" << hdr.truelen[(size_t)first] << "\t" << (obs ? identical_unique_hits[(size_t)s] : 0) << "\t"
+          << (obs ? "1" : "0") << "\t" << mem.size() << "\t";
     }
+    if (obs) write_pcts(ofs, Si.pct.data() + (size_t)s * NP, NP, '\n');
+    else for (size_t i = 0; i < NP; i++) ofs << "NA" << (i == NP - 1 ? "\n" : ",");
   }
   ofs.close(); ofs.clear();
 
@@ -932,198 +931,125 @@ static void run_sample(const Options& o, const string& hits_file, const string& 
   ofs << "percentiles";
   write_pcts(ofs, percentiles.data(), NP, '\n');
   write_rows(ofs, G, [&](ostream& ofs, int64_t g) {
-    bool obs = false;
-    for (int32_t hidx : hdr.gene_members[(size_t)g]) if (cls.hdr2col[(size_t)hidx] >= 0) { obs = true; break; }
-    if (obs) {
-      ofs << hdr.gene_names[(size_t)g] << "\t" << meanmu_gene[(size_t)g] << "\t" << sd_gene[(size_t)g] << "\t" << mumcse_gene[(size_t)g] << "\t"
-          << iact_gene[(size_t)g] << "\t" << gene_lengths[(size_t)g] << "\t" << "NA" << "\t" << gene_unique_hits[(size_t)g] << "\t"
-          << hdr.gene_members[(size_t)g].size() << "\t" << "1" << "\t";
-    } else {
-      ofs << hdr.gene_names[(size_t)g] << "\t" << meanmu_gene[(size_t)g] << "\t" << sd_gene[(size_t)g] << "\t" << sd_gene[(size_t)g] / sqrt(trace_length)
-          << "\t" << 1 << "\t" << gene_lengths[(size_t)g] << "\t" << "NA" << "\t" << "0" << "\t" << hdr.gene_members[(size_t)g].size() << "\t" << "0" << "\t";
-    }
+    const size_t ntr = hdr.gene_members[(size_t)g].size();
+    ofs << hdr.gene_names[(size_t)g] << "\t" << Sg.mean[(size_t)g] << "\t" << Sg.sd[(size_t)g] << "\t";
+    if (levels[2].observed(g))
+      ofs << Sg.mcse[(size_t)g] << "\t" << Sg.iact[(size_t)g] << "\t" << gene_lengths[(size_t)g] << "\t" << "NA" << "\t" << gene_unique_hits[(size_t)g] << "\t"
+          << ntr << "\t" << "1" << "\t";
+    else
+      ofs << Sg.sd[(size_t)g] / sqrt(trace_length) << "\t" << 1 << "\t" << gene_lengths[(size_t)g] << "\t" << "NA" << "\t" << "0" << "\t" << ntr << "\t" << "0" << "\t";
     write_pcts(ofs, Sg.pct.data() + (size_t)g * NP, NP, '\n');
   });
   ofs.close(); ofs.clear();
 
-  /* ---- -counts: .counts, .identical.counts, .gene.counts — rows and ids as in the three tables above; posterior
-   * mean and sd over the chain's sweeps, EM expected count (a group's: the sum of its members').  Every shard holds
-   * the same moments.  With -pool the moments of all chains are added exactly: sweeps, sums and 128-bit sums of squares. */
-  if (o.counts) {
-    auto write_counts = [&](const string& path, int which, int64_t rows, const function<string(int64_t)>& id, const function<int64_t(int64_t)>& row_of,
-                            const function<double(int64_t)>& em) {
+  /* output_base + suffix + ext of a level: the mapped-fragments line, `head`, then one line per table row: its id and
+   * cols(table row, device row) */
+  auto write_level = [&](const Level& lv, const char* ext, const string& head, const function<void(ostream&, int64_t, int64_t)>& cols) {
+    ofs.open((output_base + lv.suffix + ext).c_str());
+    ofs << "# Mapped fragments: " << N << endl << head;
+    write_rows(ofs, lv.rows, [&](ostream& os, int64_t r) { os << lv.id(r) << "\t"; cols(os, r, lv.dev_row(r)); });
+    ofs.close(); ofs.clear();
+  };
+
+  /* ---- -counts: .counts, .identical.counts, .gene.counts — posterior mean and sd over the chain's sweeps, EM expected
+   * count (a group's: the sum of its members').  Every shard holds the same moments.  With -pool the moments of all
+   * chains are added exactly: sweeps, sums and 128-bit sums of squares. */
+  if (o.counts)
+    for (const Level& lv : levels) {
       int64_t S = 0;
-      const int64_t R = which == 0 ? n : which == 1 ? I : G;
-      vector<uint64_t> sum((size_t)R), lo((size_t)R), hi((size_t)R);
-      check(mmq_get_count_moments(H0, which, &S, sum.data(), lo.data(), hi.data()), H0, "mmq_get_count_moments");
+      const size_t R = (size_t)lv.dev_rows;
+      vector<uint64_t> sum(R), lo(R), hi(R);
+      check(mmq_get_count_moments(H0, lv.which, &S, sum.data(), lo.data(), hi.data()), H0, "mmq_get_count_moments");
       for (int c = 1; c < npool; ++c) {
         mmq_handle* h = chain_h[(size_t)c];
         int64_t Sc = 0;
-        vector<uint64_t> sc((size_t)R), lc((size_t)R), hc((size_t)R);
-        check(mmq_get_count_moments(h, which, &Sc, sc.data(), lc.data(), hc.data()), h, "mmq_get_count_moments");
+        vector<uint64_t> sc(R), lc(R), hc(R);
+        check(mmq_get_count_moments(h, lv.which, &Sc, sc.data(), lc.data(), hc.data()), h, "mmq_get_count_moments");
         S += Sc;
-        for (size_t q = 0; q < (size_t)R; ++q) {
+        for (size_t q = 0; q < R; ++q) {
           sum[q] += sc[q];
           const uint64_t l = lo[q] + lc[q];
           hi[q] += hc[q] + (l < lo[q]);
           lo[q] = l;
         }
       }
-      ofs.open(path.c_str());
-      ofs << "# Mapped fragments: " << N << endl;
-      ofs << "feature_id\tposterior_mean_count\tposterior_sd_count\tem_count\n";
-      write_rows(ofs, rows, [&](ostream& ofs, int64_t r) {
-        const int64_t q = row_of(r);
-        ofs << id(r) << "\t";
-        if (q < 0 || S == 0) ofs << 0.0 << "\t" << 0.0 << "\t" << 0.0 << "\n";
-        else ofs << (double)sum[(size_t)q] / (double)S << "\t" << count_sd(S, sum[(size_t)q], lo[(size_t)q], hi[(size_t)q]) << "\t" << em(q) << "\n";
+      write_level(lv, ".counts", "feature_id\tposterior_mean_count\tposterior_sd_count\tem_count\n", [&](ostream& os, int64_t, int64_t q) {
+        if (q < 0 || S == 0) os << 0.0 << "\t" << 0.0 << "\t" << 0.0 << "\n";
+        else os << (double)sum[(size_t)q] / (double)S << "\t" << count_sd(S, sum[(size_t)q], lo[(size_t)q], hi[(size_t)q]) << "\t" << lv.sum(q, em_count) << "\n";
       });
-      ofs.close(); ofs.clear();
-    };
-    auto em_group = [&](const vector<int32_t>& members) {
-      double e = 0.0;
-      for (int32_t hidx : members) { const int32_t c = cls.hdr2col[(size_t)hidx]; if (c >= 0) e += em_count[(size_t)c]; }
-      return e;
-    };
-    write_counts(output_base + ".counts", 0, T, [&](int64_t hI) { return hdr.names[(size_t)hI]; },
-                 [&](int64_t hI) { return (int64_t)cls.hdr2col[(size_t)hI]; }, [&](int64_t c) { return em_count[(size_t)c]; });
-    write_counts(output_base + ".identical.counts", 1, I, identical_id, [](int64_t s) { return s; },
-                 [&](int64_t s) { return em_group(hdr.identical[(size_t)s]); });
-    write_counts(output_base + ".gene.counts", 2, G, [&](int64_t g) { return hdr.gene_names[(size_t)g]; }, [](int64_t g) { return g; },
-                 [&](int64_t g) { return em_group(hdr.gene_members[(size_t)g]); });
-  }
+    }
 
-  /* ---- -tpm: .tpm, .identical.tpm, .gene.tpm — rows and ids as in the three tables above.  Posterior mean, sd and
-   * percentiles of TPM over chain 1's draws (with -pool over every chain's, each chain normalised by its own totals;
-   * mmq_tpm_summaries), and the EM TPM from mu_em.  The totals are over the observed transcripts only, so TPM sums to 1e6
-   * over the observed features; a feature without an observed member reports 0 in every column. */
+  /* ---- -tpm: .tpm, .identical.tpm, .gene.tpm — posterior mean, sd and percentiles of TPM over chain 1's draws (with
+   * -pool over every chain's, each chain normalised by its own totals; mmq_tpm_summaries), and the EM TPM from mu_em.
+   * The totals are over the observed transcripts only, so TPM sums to 1e6 over the observed features; a feature without
+   * an observed member reports 0 in every column. */
   if (o.tpm) {
     double em_total = 0.0;
     for (int64_t t = 0; t < n; ++t) em_total += mu_em[(size_t)t];
-    auto em_members = [&](const vector<int32_t>& members) { /* the members' mu_em in header order (the CSR order of the groups) */
-      double w = 0.0;
-      for (int32_t hidx : members) { const int32_t c = cls.hdr2col[(size_t)hidx]; if (c >= 0) w += mu_em[(size_t)c]; }
-      return w;
-    };
-    auto observed = [&](const vector<int32_t>& members) {
-      for (int32_t hidx : members) if (cls.hdr2col[(size_t)hidx] >= 0) return true;
-      return false;
-    };
-    auto write_tpm = [&](const string& path, int which, int64_t rows, const function<string(int64_t)>& id, const function<int64_t(int64_t)>& row_of,
-                         const function<double(int64_t)>& em_sum) {
-      const int64_t R = which == 0 ? n : which == 1 ? I : G;
-      vector<double> mean((size_t)R), sdv((size_t)R), pct((size_t)R * NP);
+    ostringstream head;
+    head << "feature_id\tposterior_mean_tpm\tposterior_sd_tpm\tem_tpm\tpercentiles_tpm";
+    write_pcts(head, percentiles.data(), NP, '\n');
+    if (NP == 0) head << '\n';
+    const vector<double> zeros(NP, 0.0);
+    for (const Level& lv : levels) {
+      const size_t R = (size_t)lv.dev_rows;
+      vector<double> mean(R), sdv(R), pct(R * NP);
       if (R > 0)
-        check(mmq_tpm_summaries(chain_h.data(), npool, which, (int)NP, pidx_all.data(), mean.data(), sdv.data(), pct.data(), nullptr), H0,
+        check(mmq_tpm_summaries(chain_h.data(), npool, lv.which, (int)NP, pidx_all.data(), mean.data(), sdv.data(), pct.data(), nullptr), H0,
               "mmq_tpm_summaries");
-      const vector<double> zeros(NP, 0.0);
-      ofs.open(path.c_str());
-      ofs << "# Mapped fragments: " << N << endl;
-      ofs << "feature_id\tposterior_mean_tpm\tposterior_sd_tpm\tem_tpm\tpercentiles_tpm";
-      write_pcts(ofs, percentiles.data(), NP, '\n');
-      if (NP == 0) ofs << '\n';
-      write_rows(ofs, rows, [&](ostream& ofs, int64_t r) {
-        const int64_t q = row_of(r);
-        ofs << id(r) << "\t";
-        if (q < 0) ofs << 0 << "\t" << 0 << "\t" << 0 << "\t";
-        else ofs << mean[(size_t)q] << "\t" << sdv[(size_t)q] << "\t" << (em_sum(q) / em_total) * 1000000.0 << "\t";
-        write_pcts(ofs, q < 0 ? zeros.data() : pct.data() + (size_t)q * NP, NP, '\n');
-        if (NP == 0) ofs << '\n';
+      write_level(lv, ".tpm", head.str(), [&](ostream& os, int64_t, int64_t q) {
+        const bool obs = q >= 0 && lv.has_hits(q);
+        if (!obs) os << 0 << "\t" << 0 << "\t" << 0 << "\t";
+        else os << mean[(size_t)q] << "\t" << sdv[(size_t)q] << "\t" << (lv.sum(q, mu_em) / em_total) * 1000000.0 << "\t";
+        write_pcts(os, obs ? pct.data() + (size_t)q * NP : zeros.data(), NP, '\n');
+        if (NP == 0) os << '\n';
       });
-      ofs.close(); ofs.clear();
-    };
-    write_tpm(output_base + ".tpm", 0, T, [&](int64_t hI) { return hdr.names[(size_t)hI]; },
-              [&](int64_t hI) { return (int64_t)cls.hdr2col[(size_t)hI]; }, [&](int64_t c) { return mu_em[(size_t)c]; });
-    write_tpm(output_base + ".identical.tpm", 1, I, identical_id, [&](int64_t s) { return observed(hdr.identical[(size_t)s]) ? s : -1; },
-              [&](int64_t s) { return em_members(hdr.identical[(size_t)s]); });
-    write_tpm(output_base + ".gene.tpm", 2, G, [&](int64_t g) { return hdr.gene_names[(size_t)g]; },
-              [&](int64_t g) { return observed(hdr.gene_members[(size_t)g]) ? g : -1; }, [&](int64_t g) { return em_members(hdr.gene_members[(size_t)g]); });
+    }
   }
 
-  /* ---- -chains: .convergence, .identical.convergence, .gene.convergence — rows and ids as in the three tables above.
-   * log_mu and sd pooled over the draws of all chains, split-R-hat and bulk / tail ESS (mmq_chain_diagnostics); a row
-   * whose `observed` column is 0 carries that table's closed-form log_mu and sd, and NA. */
-  if (nchains > 1) {
-    const char* const ext[3] = {".convergence", ".identical.convergence", ".gene.convergence"};
-    const char* const what[3] = {"transcripts", "identical sets", "genes"};
-    for (int which = 0; which < 3; ++which) {
-      const int64_t R = which == 0 ? n : which == 1 ? I : G;
-      vector<double> rh((size_t)R), eb((size_t)R), et((size_t)R), lm((size_t)R), ls((size_t)R);
+  /* ---- -chains: .convergence, .identical.convergence, .gene.convergence — log_mu and sd pooled over the draws of all
+   * chains, split-R-hat and bulk / tail ESS (mmq_chain_diagnostics); a row whose `observed` column is 0 in the tables
+   * above carries that table's closed-form log_mu and sd, and NA. */
+  if (nchains > 1)
+    for (const Level& lv : levels) {
+      const size_t R = (size_t)lv.dev_rows;
+      vector<double> rh(R), eb(R), et(R), lm(R), ls(R);
       if (R > 0)
-        check(mmq_chain_diagnostics(chain_h.data(), nchains, which, rh.data(), eb.data(), et.data(), lm.data(), ls.data()), H0,
+        check(mmq_chain_diagnostics(chain_h.data(), nchains, lv.which, rh.data(), eb.data(), et.data(), lm.data(), ls.data()), H0,
               "mmq_chain_diagnostics");
-      /* table row -> (diagnostics row or -1, feature id, closed-form log_mu and sd of an unobserved row) */
-      struct Row { int64_t q; string id; double log_mu, sd; };
-      auto row_of = [&](int64_t r) -> Row {
-        if (which == 0) {
-          const int32_t c = cls.hdr2col[(size_t)r];
-          return {c, hdr.names[(size_t)r], digalpha - log(beta + hdr.efflen[(size_t)r] * (double)N / 1000000000.0), sqrtpolygalpha};
-        }
-        if (which == 1) {
-          const auto& mem = hdr.identical[(size_t)r];
-          size_t jb = 0;
-          while (hdr.names[(size_t)mem[jb]].compare(hdr.names[(size_t)mem.back()]) != 0) ++jb;
-          return {ident_obs[(size_t)r] ? r : -1, identical_id(r),
-                  log(mem.size()) + digalpha - log(beta + hdr.efflen[(size_t)mem[jb]] * (double)N / 1000000000.0), sqrtpolygalpha};
-        }
-        bool obs = false;
-        for (int32_t hidx : hdr.gene_members[(size_t)r]) if (cls.hdr2col[(size_t)hidx] >= 0) { obs = true; break; }
-        return {obs ? r : -1, hdr.gene_names[(size_t)r], meanmu_gene[(size_t)r], sd_gene[(size_t)r]};
-      };
       auto put = [](ostream& os, double v) -> ostream& { if (std::isnan(v)) os << "NA"; else os << v; return os; };
-      ofs.open((output_base + ext[which]).c_str());
-      ofs << "# Mapped fragments: " << N << endl;
-      ofs << "feature_id\tlog_mu\tsd\trhat\tess_bulk\tess_tail\n";
-      const int64_t rows = which == 0 ? T : R;
-      write_rows(ofs, rows, [&](ostream& os, int64_t r) {
-        const Row w = row_of(r);
-        os << w.id << "\t";
-        if (w.q < 0) { put(os, w.log_mu) << "\t"; put(os, w.sd) << "\tNA\tNA\tNA\n"; return; }
-        const size_t q = (size_t)w.q;
-        put(os, lm[q]) << "\t"; put(os, ls[q]) << "\t"; put(os, rh[q]) << "\t"; put(os, eb[q]) << "\t"; put(os, et[q]) << "\n";
+      write_level(lv, ".convergence", "feature_id\tlog_mu\tsd\trhat\tess_bulk\tess_tail\n", [&](ostream& os, int64_t r, int64_t q) {
+        if (q < 0 || !lv.observed(q)) { const auto u = lv.unobserved(r); put(os, u.first) << "\t"; put(os, u.second) << "\tNA\tNA\tNA\n"; return; }
+        put(os, lm[(size_t)q]) << "\t"; put(os, ls[(size_t)q]) << "\t"; put(os, rh[(size_t)q]) << "\t"; put(os, eb[(size_t)q]) << "\t"; put(os, et[(size_t)q]) << "\n";
       });
-      ofs.close(); ofs.clear();
       double max_rhat = NAN, min_ess = NAN;
       int64_t over = 0;
-      for (int64_t r = 0; r < rows; ++r) {
-        const int64_t q = row_of(r).q;
-        if (q < 0) continue;
+      for (int64_t r = 0; r < lv.rows; ++r) {
+        const int64_t q = lv.dev_row(r);
+        if (q < 0 || !lv.observed(q)) continue;
         if (!std::isnan(rh[(size_t)q])) { max_rhat = std::isnan(max_rhat) ? rh[(size_t)q] : max(max_rhat, rh[(size_t)q]); over += rh[(size_t)q] > 1.01; }
         if (!std::isnan(eb[(size_t)q])) min_ess = std::isnan(min_ess) ? eb[(size_t)q] : min(min_ess, eb[(size_t)q]);
       }
-      err << "Convergence of the " << what[which] << " over " << nchains << " chains: largest rhat " << max_rhat << ", " << over
+      err << "Convergence of the " << lv.name << " over " << nchains << " chains: largest rhat " << max_rhat << ", " << over
           << " with rhat > 1.01, smallest ess_bulk " << min_ess << endl;
     }
-  }
 
   out << "done." << endl;
   for (auto& S : shards) mmq_destroy(S.h);
   for (int c = 1; c < nchains; ++c) mmq_destroy(chain_h[(size_t)c]);
 
   phase("tables");
-  out << "Output files: " << endl
-       << "  " << output_base << ".mmseq" << endl
-       << "  " << output_base << ".identical.mmseq" << endl
-       << "  " << output_base << ".gene.mmseq" << endl;
-  if (o.counts)
-    out << "  " << output_base << ".counts" << endl
-        << "  " << output_base << ".identical.counts" << endl
-        << "  " << output_base << ".gene.counts" << endl;
-  if (o.tpm)
-    out << "  " << output_base << ".tpm" << endl
-        << "  " << output_base << ".identical.tpm" << endl
-        << "  " << output_base << ".gene.tpm" << endl;
-  if (nchains > 1)
-    out << "  " << output_base << ".convergence" << endl
-        << "  " << output_base << ".identical.convergence" << endl
-        << "  " << output_base << ".gene.convergence" << endl;
+  out << "Output files: " << endl;
+  auto list = [&](const char* ext) { for (const Level& lv : levels) out << "  " << output_base << lv.suffix << ext << endl; };
+  list(".mmseq");
+  if (o.counts) list(".counts");
+  if (o.tpm) list(".tpm");
+  if (nchains > 1) list(".convergence");
   out << "  " << output_base << ".M" << endl << "  " << output_base << ".k" << endl << endl;
-  if (!notraces)
-    out << "  " << output_base << ".trace_gibbs.gz" << endl
-         << "  " << output_base << ".identical.trace_gibbs.gz" << endl
-         << "  " << output_base << ".gene.trace_gibbs.gz" << endl
-         << "  " << output_base << ".prop.trace_gibbs.gz" << endl
-         << endl;
+  if (!notraces) {
+    list(".trace_gibbs.gz");
+    out << "  " << output_base << ".prop.trace_gibbs.gz" << endl << endl;
+  }
   if (debug) {
     out << endl
          << "  " << output_base << ".trace_em.gz" << endl
