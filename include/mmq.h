@@ -354,6 +354,54 @@ int mmq_tpm_summaries_dev(const double* const* chain_dev, const double* totals_d
 int mmq_tpm_summaries(mmq_handle* const* chains, int nchains, int which, int npct, const int32_t* pct_idx, double* mean, double* sd,
                       double* pct, double* totals_out);
 
+/* ---- allelic fraction of haplotype pairs (none in the reference; mmseq -allelic) ---------------------------------------
+ * A haplotype-aware reference lists every transcript twice, STEM_A and STEM_B.  The two copies share most of their
+ * fragments, so their draws are anti-correlated and the sd of a ratio cannot be formed from the .mmseq columns; these
+ * functions compute it per draw.  tests/allelic_reference.py restates the definitions in numpy.
+ *   1. Pairs (the caller's, mmseq_main.cpp): header transcripts named STEM_A and STEM_B (fixed suffixes) in one gene,
+ *      with or without hits; id STEM; in the header order of the _A copy.  A transcript named *_A / *_B whose partner is
+ *      missing or in another gene is not paired.  Genes: a gene's A side is the _A copies of the pairs inside it, its B
+ *      side their _B copies (in pair order); isoforms outside a pair are ignored.
+ *   2. Members (column space): an id m < n is observed transcript m, a row of the chain's trace; an id n + j is row j of
+ *      the caller's prior draws of that chain, laid out [j L + s] as mmq_prior_draws writes them.  The host program
+ *      passes, as prior rows, exactly the hit-less copies that belong to a pair, in header order: the draws that chain
+ *      already uses for them, the exact posterior of a copy without fragments.
+ *   3. Per draw (chain c, slot s): a = the sum of the A members' draws in CSR order from 0.0, b the same for the B
+ *      members, phi = a / (a + b) in plain IEEE.  No fraction trace is stored.
+ *   4. Over the S = C L draws: mean = sum phi / S; sd = sqrt(sum (phi - mean)^2 / (S - 1)), two-pass; prob_a =
+ *      (#{a > b} + #{a = b} / 2) / S; pct[j] = phi sorted ascending (NaN last) at index pct_idx[j] (the host program:
+ *      round(p / 100 (S - 1)), as -tpm).  If any phi is not finite (a + b = 0 in some draw, as for a unit without
+ *      members) every one of these is NaN.
+ *   5. EM (the caller's): em_fraction_a = sum_A mu_em / (sum_A mu_em + sum_B mu_em) over the observed members in index
+ *      order, hit-less copies counting 0; NaN when both sums are 0.
+ *   6. Allele-only fragments: a_only[u] = sum of k_i over the hit classes i that contain an A member of unit u and no B
+ *      member of u; b_only[u] the same with A and B swapped.  A per-fragment layout (k = NULL, also a weighted file)
+ *      counts 1 per row: set membership decides, the weights are ignored (as for unique hits).  Exact int32 counts. */
+/* unit_of int32[n]: the unit of each observed transcript or -1; side uint8[n]: 0 (A) or 1 (B).  a_only, b_only
+ * int32[nunits] on the host, all-reduced over the shards of a communicator (every rank calls it, as mmq_unique_hits_sets).
+ * A unit index outside [-1, nunits) or a side other than 0 / 1 is MMQ_ERR_ARG. */
+int mmq_allele_only_counts(mmq_handle* h, const int32_t* unit_of, const uint8_t* side, int64_t nunits, int32_t* a_only,
+                           int32_t* b_only);
+/* Summaries 3-4 per unit.  chain_dev[c] (a host array of device pointers): chain c's transcript trace [t L + s] over n
+ * observed transcripts; prior_dev[c]: chain c's nprior prior rows [j L + s] (prior_dev, or each prior_dev[c], may be NULL
+ * when nprior = 0); a_ptr_dev int64[rows + 1] / a_mem_dev int32 and b_ptr_dev / b_mem_dev: the A and B members of every
+ * unit, ids in [0, n + nprior) (not checked here: the handle form checks them).  out_dev fp64[3 rows]: [r] mean,
+ * [rows + r] sd, [2 rows + r] prob_a; pct_dev fp64[rows npct], [r npct + j].  All on the calling device; asynchronous on
+ * cuda_stream, no allocation; one CTA per unit, grid min(rows, 2 x SMs); results independent of the grid and of the row
+ * order.  Limits those of -tpm: 1 <= nchains <= 8, L a power of two in [4, 2048], nchains L <= 8192; else MMQ_ERR_ARG. */
+int mmq_allelic_summaries_dev(const double* const* chain_dev, const double* const* prior_dev, int nchains, int64_t n, int64_t nprior,
+                              int64_t rows, int L, const int64_t* a_ptr_dev, const int32_t* a_mem_dev, const int64_t* b_ptr_dev,
+                              const int32_t* b_mem_dev, int npct, const int32_t* pct_idx_dev, double* out_dev, double* pct_dev,
+                              void* cuda_stream);
+/* The same on the transcript traces the handles recorded (same n and trace_len on every handle), on chains[0]'s device
+ * and stream; traces of handles on other devices are copied there with cudaMemcpyPeerAsync, the prior rows prior_host[c]
+ * (host fp64[nprior L] per chain) and the CSRs with cudaMemcpyAsync into block-cache memory.  A member id outside
+ * [0, n + nprior), a CSR that does not start at 0 or decreases, or pct_idx outside [0, S) is MMQ_ERR_ARG.  mean, sd,
+ * prob_a fp64[rows] and pct fp64[rows npct] on the host; any may be NULL. */
+int mmq_allelic_summaries(mmq_handle* const* chains, int nchains, const double* const* prior_host, int64_t nprior, int64_t rows,
+                          const int64_t* a_ptr, const int32_t* a_mem, const int64_t* b_ptr, const int32_t* b_mem, int npct,
+                          const int32_t* pct_idx, double* mean, double* sd, double* prob_a, double* pct);
+
 /* ---- the consumer of the traces: mmcollapse's covariance step (src/mmcollapse.cpp:483-561) ----------
  * The one dense contraction of the package: tensor cores (tcgen05, bf16 split products, fp32 accumulation in
  * TMEM), everything around it fp64.  nsplit = bf16 terms per value (2: the default of the callers here).  Error in

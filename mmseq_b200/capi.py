@@ -86,6 +86,9 @@ def _load():
         "mmq_draw_totals_dev": (i32, [vp, i64, i32, vp, vp, vp]),
         "mmq_tpm_summaries_dev": (i32, [C.POINTER(vp), vp, i32, i64, i32, vp, vp, i32, vp, vp, vp, vp]),
         "mmq_tpm_summaries": (i32, [C.POINTER(vp), i32, i32, i32, vp, vp, vp, vp, vp]),
+        "mmq_allele_only_counts": (i32, [vp, vp, vp, i64, vp, vp]),
+        "mmq_allelic_summaries_dev": (i32, [C.POINTER(vp), C.POINTER(vp), i32, i64, i64, i64, i32, vp, vp, vp, vp, i32, vp, vp, vp, vp]),
+        "mmq_allelic_summaries": (i32, [C.POINTER(vp), i32, C.POINTER(vp), i64, i64, vp, vp, vp, vp, i32, vp, vp, vp, vp, vp]),
         "mmq_prior_draws": (i32, [i32, i64, vp, vp, dbl, u32, i32, vp]),
         "mmq_trace_cov": (i32, [i32, vp, i32, i64, i32, vp]),
         "mmq_trace_cov_workspace_bytes": (i64, [i32, i64, i32]),
@@ -123,7 +126,8 @@ EXPORTS = [
     "mmq_set_groups", "mmq_summarize", "mmq_get_group_trace", "mmq_prop_summaries",
     "mmq_unique_hits_sets", "mmq_sokal_batch", "mmq_chain_seed", "mmq_chain_diagnostics_dev", "mmq_chain_diagnostics",
     "mmq_pooled_summaries_dev", "mmq_pooled_summaries", "mmq_draw_totals_workspace_bytes", "mmq_draw_totals_dev",
-    "mmq_tpm_summaries_dev", "mmq_tpm_summaries", "mmq_prior_draws", "mmq_trace_cov", "mmq_trace_cov_workspace_bytes", "mmq_trace_cov_dev",
+    "mmq_tpm_summaries_dev", "mmq_tpm_summaries", "mmq_allele_only_counts", "mmq_allelic_summaries_dev", "mmq_allelic_summaries",
+    "mmq_prior_draws", "mmq_trace_cov", "mmq_trace_cov_workspace_bytes", "mmq_trace_cov_dev",
     "mmq_handle_trace_cov", "mmq_mean_corrs", "mmq_mean_corrs_dev", "mmq_release_cache", "mmq_launch_count", "mmq_warmup", "mmq_version",
 ]
 
@@ -258,6 +262,37 @@ def tpm_summaries(handles, which=0, pct_idx=None):
                                  _ptr(out["totals"]))
     if rc:
         raise MmqError(f"mmq_tpm_summaries failed ({rc}): " + lib().mmq_last_error(h0._h).decode())
+    return out
+
+
+def allelic_summaries_dev(chain_ptrs, prior_ptrs, n, nprior, rows, L, a_ptr_ptr, a_mem_ptr, b_ptr_ptr, b_mem_ptr, npct, pct_idx_ptr,
+                         out_ptr, pct_ptr, stream_ptr):
+    """mmq_allelic_summaries_dev: chain_ptrs, device pointers (ints) of each chain's transcript trace (n rows); prior_ptrs,
+    of each chain's nprior prior rows (or None); the A and B member CSRs (ids < n: trace rows, n + j: prior row j);
+    out_ptr fp64[3 * rows] (mean, sd, prob_a); pct_ptr fp64[rows * npct].  Asynchronous on the stream."""
+    arr = (C.c_void_p * len(chain_ptrs))(*chain_ptrs)
+    pri = None if prior_ptrs is None else (C.c_void_p * len(prior_ptrs))(*prior_ptrs)
+    _global_check(lib().mmq_allelic_summaries_dev(arr, pri, len(chain_ptrs), n, nprior, rows, L, a_ptr_ptr, a_mem_ptr, b_ptr_ptr, b_mem_ptr,
+                                                  npct, pct_idx_ptr, out_ptr, pct_ptr, stream_ptr), "mmq_allelic_summaries_dev")
+
+
+def allelic_summaries(handles, a_ptr, a_mem, b_ptr, b_mem, priors=None, pct_idx=None):
+    """mmq_allelic_summaries over the transcript traces the handles recorded; priors: one (nprior, L) array per chain or
+    None.  Returns dict(mean, sd, prob_a: fp64[rows]; pct: (rows, npct))."""
+    h0 = handles[0]
+    a_ptr = _c(a_ptr, np.int64); b_ptr = _c(b_ptr, np.int64)
+    a_mem = _c(a_mem, np.int32); b_mem = _c(b_mem, np.int32)
+    rows = len(a_ptr) - 1
+    pct_idx = _c(pct_idx if pct_idx is not None else [], np.int32)
+    priors = None if priors is None else [_c(p, np.float64) for p in priors]
+    nprior = 0 if priors is None else priors[0].shape[0]
+    pri = None if priors is None else (C.c_void_p * len(priors))(*[p.ctypes.data for p in priors])
+    out = dict(mean=np.zeros(rows), sd=np.zeros(rows), prob_a=np.zeros(rows), pct=np.zeros((rows, len(pct_idx))))
+    arr = (C.c_void_p * len(handles))(*[h._h for h in handles])
+    rc = lib().mmq_allelic_summaries(arr, len(handles), pri, nprior, rows, _ptr(a_ptr), _ptr(a_mem), _ptr(b_ptr), _ptr(b_mem),
+                                     len(pct_idx), _ptr(pct_idx), _ptr(out["mean"]), _ptr(out["sd"]), _ptr(out["prob_a"]), _ptr(out["pct"]))
+    if rc:
+        raise MmqError(f"mmq_allelic_summaries failed ({rc}): " + lib().mmq_last_error(h0._h).decode())
     return out
 
 
@@ -520,6 +555,13 @@ class Handle:
         self._check(lib().mmq_prop_summaries(self._h, _ptr(gene_of), _ptr(multi_iso), _ptr(mp), _ptr(sp), _ptr(ssp),
                                              len(pct_idx), _ptr(pct_idx), _ptr(pct), _ptr(tr)), "mmq_prop_summaries")
         return dict(mean_prop=mp, sum_probit=sp, sumsq_probit=ssp, pct=pct, prop_trace=tr)
+
+    def allele_only_counts(self, unit_of, side, nunits):
+        """mmq_allele_only_counts: (a_only, b_only) int32[nunits]; unit_of int32[n] (-1: none), side uint8[n] (0 A, 1 B)."""
+        unit_of = _c(unit_of, np.int32); side = _c(side, np.uint8)
+        a = np.zeros(nunits, np.int32); b = np.zeros(nunits, np.int32)
+        self._check(lib().mmq_allele_only_counts(self._h, _ptr(unit_of), _ptr(side), nunits, _ptr(a), _ptr(b)), "mmq_allele_only_counts")
+        return a, b
 
     def unique_hits_sets(self, set_of, nsets):
         set_of = _c(set_of, np.int32)

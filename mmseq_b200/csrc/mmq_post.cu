@@ -9,8 +9,9 @@
  *   k_row_percentiles  src/mmseq.cpp:1111-1172 (sort each trace, pick indices)
  *   k_prop             src/mmseq.cpp:985-1008, :1236-1257
  *   k_uh_sets          src/uh.cpp:3-26 restated O(nnz)
- * and, with no reference counterpart, the diagnostics of several chains (k_chain_diag) and the summaries of their
- * pooled draws (k_pool_summ).
+ * and, with no reference counterpart, the diagnostics of several chains (k_chain_diag), the summaries of their
+ * pooled draws (k_pool_summ), transcripts per million (k_draw_totals, k_totals_fold, k_tpm_summ) and the allelic fraction
+ * of haplotype pairs (k_allele_only, k_allelic_summ).
  * All traces are [row * trace_len + slot] (the reference's mu_trace layout).
  */
 #include <algorithm>
@@ -637,6 +638,29 @@ k_totals_fold(const double* __restrict__ partial, int64_t ntiles, int L, double*
  * memory: key fp64[P], the draws in draw order padded with NaN, sorted in place; 8 P bytes, 64 KB at S = 8192. */
 #define MMQ_TPM_SMEM_CAP (8 * 8192)
 
+/* The tail that k_tpm_summ and k_allelic_summ share.  key[0 .. P) holds the row's S draws in draw order, padded with NaN;
+ * `finite`: no draw is NaN or infinite; `sum`: the draws' block sum.  mean = sum / S and the two-pass sd (S - 1), both
+ * NaN unless `finite`; then the NaN-last sort and pct[row npct + j] = sorted[pct_idx[j]], NaN for an index outside [0, S).
+ * Every thread gets mean and sd. */
+__device__ __forceinline__ void draws_mean_sd_pct(double* key, int P, int S, bool finite, double sum, int64_t row, int npct,
+                                                  const int32_t* __restrict__ pct_idx, double* __restrict__ pct, double& mean,
+                                                  double& sd) {
+  const double nan = mmq_u2d(0x7ff8000000000000ull);
+  mean = nan;
+  sd = nan;
+  if (finite) {
+    mean = sum / (double)S;
+    double ss = 0.0;
+    for (int k = threadIdx.x; k < S; k += blockDim.x) { const double d = key[k] - mean; ss += d * d; }
+    sd = sqrt(post_block_sum(ss) / (double)(S - 1));
+  }
+  sort_nan_last(key, P);
+  for (int j = threadIdx.x; j < npct; j += blockDim.x) {
+    const int q = pct_idx[j];
+    pct[row * npct + j] = q >= 0 && q < S ? key[q] : nan;
+  }
+}
+
 __global__ void __launch_bounds__(MMQ_POST_THREADS)
 k_tpm_summ(const __grid_constant__ mmq_chain_ptrs cp, const double* __restrict__ totals, int C, int64_t rows, int lgL,
            const int64_t* __restrict__ gptr, const int32_t* __restrict__ members, int npct, const int32_t* __restrict__ pct_idx,
@@ -664,19 +688,87 @@ k_tpm_summ(const __grid_constant__ mmq_chain_ptrs cp, const double* __restrict__
     }
     bad = post_block_sum(bad); /* also orders the writes of key */
     sum = post_block_sum(sum);
-    double mean = nan, sd = nan;
-    if (bad == 0.0) {
-      mean = sum / (double)S;
-      double ss = 0.0;
-      for (int k = threadIdx.x; k < S; k += blockDim.x) { const double d = key[k] - mean; ss += d * d; }
-      sd = sqrt(post_block_sum(ss) / (double)(S - 1));
-    }
-    sort_nan_last(key, P);
-    for (int j = threadIdx.x; j < npct; j += blockDim.x) {
-      const int q = pct_idx[j];
-      pct[row * npct + j] = q >= 0 && q < S ? key[q] : nan;
-    }
+    double mean, sd;
+    draws_mean_sd_pct(key, P, S, bad == 0.0, sum, row, npct, pct_idx, pct, mean, sd);
     if (threadIdx.x == 0) { out[row] = mean; out[rows + row] = sd; }
+    __syncthreads();
+  }
+}
+
+/* ------------------------------------------------ allelic fraction of haplotype pairs (mmseq -allelic)
+ * Definitions: include/mmq.h (mmq_allele_only_counts, mmq_allelic_summaries_dev); tests/allelic_reference.py restates
+ * them in numpy.
+ * k_allele_only, the shape of k_uh_sets (one thread per hit class or fragment row, grid-capped): a row counts for side A
+ * (B) of unit u when it holds an A (B) member of u and no B (A) member of u; each (unit, side) of the row is counted once,
+ * by its first position.  The check scans the row for every member, O(len^2) on rows that are a few entries long. */
+template <bool HAS_K>
+__global__ void k_allele_only(const int64_t* __restrict__ row_ptr, const int32_t* __restrict__ col, const int32_t* __restrict__ kk,
+                              const int32_t* __restrict__ unit_of, const uint8_t* __restrict__ side, int64_t m,
+                              int32_t* __restrict__ a_only, int32_t* __restrict__ b_only) {
+  for (int64_t i = blockIdx.x * (int64_t)blockDim.x + threadIdx.x; i < m; i += (int64_t)gridDim.x * blockDim.x) {
+    const int64_t b = row_ptr[i], e = row_ptr[i + 1];
+    for (int64_t q = b; q < e; ++q) {
+      const int32_t u = unit_of[col[q]];
+      if (u < 0) continue;
+      const uint8_t s = side[col[q]];
+      bool first = true, opposite = false;
+      for (int64_t r = b; r < e && !opposite; ++r) {
+        if (r == q || unit_of[col[r]] != u) continue;
+        if (side[col[r]] != s) opposite = true;
+        else if (r < q) first = false;
+      }
+      if (first && !opposite) atomicAdd((s ? b_only : a_only) + u, HAS_K ? kk[i] : 1);
+    }
+  }
+}
+
+/* One CTA per unit, grid-capped, the layout of k_tpm_summ.  Draw k (< S = C L) is chain c = k >> lgL, slot k & (L - 1); a
+ * member id m < n is row m of chain c's trace, m >= n row m - n of chain c's prior draws.  a (b) = the sum of the A (B)
+ * members' draws in CSR order from 0.0 and phi = a / (a + b), fused into the load that fills key, so no fraction trace is
+ * stored.  Block sums: the non-finite phi, the sum of phi and 2 #{a > b} + #{a = b}.  A unit with a non-finite phi gets
+ * NaN in every output; otherwise draws_mean_sd_pct.  Shared memory: key fp64[P]; 8 P bytes, 64 KB at S = 8192. */
+#define MMQ_ALLELIC_SMEM_CAP (8 * 8192)
+
+__global__ void __launch_bounds__(MMQ_POST_THREADS)
+k_allelic_summ(const __grid_constant__ mmq_chain_ptrs cp, const __grid_constant__ mmq_chain_ptrs pp, int C, int64_t n, int64_t rows, int lgL,
+               const int64_t* __restrict__ a_ptr, const int32_t* __restrict__ a_mem, const int64_t* __restrict__ b_ptr,
+               const int32_t* __restrict__ b_mem, int npct, const int32_t* __restrict__ pct_idx, double* __restrict__ out,
+               double* __restrict__ pct) {
+  extern __shared__ double sh[];
+  const int L = 1 << lgL, S = C * L;
+  int P = 1;
+  while (P < S) P <<= 1;
+  double* key = sh;
+  const double nan = mmq_u2d(0x7ff8000000000000ull);
+  for (int64_t row = blockIdx.x; row < rows; row += gridDim.x) {
+    const int64_t ab = a_ptr[row], ae = a_ptr[row + 1], bb = b_ptr[row], be = b_ptr[row + 1];
+    double bad = 0.0, sum = 0.0, gt = 0.0;
+    for (int k = threadIdx.x; k < P; k += blockDim.x) {
+      double v = nan;
+      if (k < S) {
+        const int c = k >> lgL, s = k & (L - 1);
+        auto draw = [&](int32_t m) { return m < n ? cp.p[c][((int64_t)m << lgL) + s] : pp.p[c][(((int64_t)m - n) << lgL) + s]; };
+        double a = 0.0, b = 0.0;
+        for (int64_t q = ab; q < ae; ++q) a += draw(a_mem[q]);
+        for (int64_t q = bb; q < be; ++q) b += draw(b_mem[q]);
+        v = a / (a + b);
+        bad += isfinite(v) ? 0.0 : 1.0;
+        sum += v;
+        gt += a > b ? 2.0 : a == b ? 1.0 : 0.0;
+      }
+      key[k] = v;
+    }
+    bad = post_block_sum(bad); /* also orders the writes of key */
+    if (bad > 0.0) {
+      if (threadIdx.x == 0) { out[row] = nan; out[rows + row] = nan; out[2 * rows + row] = nan; }
+      for (int j = threadIdx.x; j < npct; j += blockDim.x) pct[row * npct + j] = nan;
+      continue;
+    }
+    sum = post_block_sum(sum);
+    gt = post_block_sum(gt);
+    double mean, sd;
+    draws_mean_sd_pct(key, P, S, true, sum, row, npct, pct_idx, pct, mean, sd);
+    if (threadIdx.x == 0) { out[row] = mean; out[rows + row] = sd; out[2 * rows + row] = gt / (2.0 * (double)S); }
     __syncthreads();
   }
 }
@@ -1259,6 +1351,145 @@ int mmq_tpm_summaries(mmq_handle* const* chains, int nchains, int which, int npc
   if (e == cudaSuccess) e = es;
   if (e != cudaSuccess && ret == MMQ_OK) ret = mmq_cuda_fail(h0, e, "mmq_tpm_summaries", __FILE__, __LINE__);
   mmq_cache_free(ws); mmq_cache_free(work); mmq_cache_free(totals); mmq_cache_free(out); mmq_cache_free(d_pct); mmq_cache_free(d_idx);
+  return ret;
+}
+
+int mmq_allele_only_counts(mmq_handle* h, const int32_t* unit_of, const uint8_t* side, int64_t nunits, int32_t* a_only, int32_t* b_only) {
+  if (!h || !unit_of || !side || !a_only || !b_only || nunits < 0) return mmq_fail(h, MMQ_ERR_ARG, "mmq_allele_only_counts: bad arguments");
+  for (int64_t t = 0; t < h->n; ++t)
+    if (unit_of[t] < -1 || unit_of[t] >= nunits || side[t] > 1)
+      return mmq_fail(h, MMQ_ERR_ARG, "mmq_allele_only_counts: unit index or side out of range");
+  if (nunits == 0) return MMQ_OK;
+  MMQ_CUDA(h, cudaSetDevice(h->device));
+  int32_t *d_unit = nullptr, *d_out = nullptr;
+  uint8_t* d_side = nullptr;
+  cudaError_t e = mmq_cache_malloc(&d_unit, sizeof(int32_t) * (size_t)std::max<int64_t>(h->n, 1));
+  if (e == cudaSuccess) e = mmq_cache_malloc(&d_side, (size_t)std::max<int64_t>(h->n, 1));
+  if (e == cudaSuccess) e = mmq_cache_malloc(&d_out, sizeof(int32_t) * 2 * (size_t)nunits);
+  if (e == cudaSuccess && h->n > 0) e = cudaMemcpyAsync(d_unit, unit_of, sizeof(int32_t) * (size_t)h->n, cudaMemcpyHostToDevice, h->stream);
+  if (e == cudaSuccess && h->n > 0) e = cudaMemcpyAsync(d_side, side, (size_t)h->n, cudaMemcpyHostToDevice, h->stream);
+  if (e == cudaSuccess) e = cudaMemsetAsync(d_out, 0, sizeof(int32_t) * 2 * (size_t)nunits, h->stream);
+  int ret = MMQ_OK;
+  if (e == cudaSuccess && h->m > 0) {
+    const int grid = mmq_grid_for(h->m, 256, h->num_sms * 8);
+    if (h->has_k) k_allele_only<true><<<grid, 256, 0, h->stream>>>(h->row_ptr, h->col, h->k, d_unit, d_side, h->m, d_out, d_out + nunits);
+    else k_allele_only<false><<<grid, 256, 0, h->stream>>>(h->row_ptr, h->col, h->k, d_unit, d_side, h->m, d_out, d_out + nunits);
+    g_mmq_launches.fetch_add(1);
+    e = cudaGetLastError();
+  }
+  if (e == cudaSuccess) ret = mmq_allreduce(h, d_out, 2 * (size_t)nunits, 0);
+  if (e == cudaSuccess && ret == MMQ_OK) e = cudaMemcpyAsync(a_only, d_out, sizeof(int32_t) * (size_t)nunits, cudaMemcpyDeviceToHost, h->stream);
+  if (e == cudaSuccess && ret == MMQ_OK) e = cudaMemcpyAsync(b_only, d_out + nunits, sizeof(int32_t) * (size_t)nunits, cudaMemcpyDeviceToHost, h->stream);
+  const cudaError_t es = cudaStreamSynchronize(h->stream);
+  if (e == cudaSuccess) e = es;
+  if (e != cudaSuccess && ret == MMQ_OK) ret = mmq_cuda_fail(h, e, "mmq_allele_only_counts", __FILE__, __LINE__);
+  mmq_cache_free(d_unit); mmq_cache_free(d_side); mmq_cache_free(d_out);
+  return ret;
+}
+
+int mmq_allelic_summaries_dev(const double* const* chain_dev, const double* const* prior_dev, int nchains, int64_t n, int64_t nprior,
+                              int64_t rows, int L, const int64_t* a_ptr_dev, const int32_t* a_mem_dev, const int64_t* b_ptr_dev,
+                              const int32_t* b_mem_dev, int npct, const int32_t* pct_idx_dev, double* out_dev, double* pct_dev,
+                              void* cuda_stream) {
+  if (!chain_dev || !tpm_len_ok(nchains, L) || n < 0 || nprior < 0 || n + nprior > INT32_MAX || rows < 0 || npct < 0 ||
+      (nprior > 0 && !prior_dev) ||
+      (rows > 0 && (!a_ptr_dev || !a_mem_dev || !b_ptr_dev || !b_mem_dev || !out_dev)) || (rows > 0 && npct > 0 && (!pct_idx_dev || !pct_dev)))
+    return mmq_fail(nullptr, MMQ_ERR_ARG, "mmq_allelic_summaries_dev: bad arguments");
+  mmq_chain_ptrs cp = {}, pp = {};
+  for (int c = 0; c < nchains; ++c) {
+    if (!chain_dev[c] || (nprior > 0 && !prior_dev[c])) return mmq_fail(nullptr, MMQ_ERR_ARG, "mmq_allelic_summaries_dev: NULL chain or prior");
+    cp.p[c] = chain_dev[c];
+    pp.p[c] = nprior > 0 ? prior_dev[c] : nullptr;
+  }
+  if (rows == 0) return MMQ_OK;
+  int dev = 0, sms = 0, lgL = 0;
+  while ((1 << lgL) < L) ++lgL;
+  const size_t smem = sizeof(double) * (size_t)chain_pow2_at_least(nchains * L);
+  cudaError_t e = cudaGetDevice(&dev);
+  if (e == cudaSuccess) e = cudaDeviceGetAttribute(&sms, cudaDevAttrMultiProcessorCount, dev);
+  if (e == cudaSuccess) e = cudaFuncSetAttribute(k_allelic_summ, cudaFuncAttributeMaxDynamicSharedMemorySize, MMQ_ALLELIC_SMEM_CAP);
+  if (e != cudaSuccess) return mmq_cuda_fail(nullptr, e, "mmq_allelic_summaries_dev", __FILE__, __LINE__);
+  const int grid = (int)std::min<int64_t>(rows, 2 * (int64_t)sms);
+  k_allelic_summ<<<grid, MMQ_POST_THREADS, smem, (cudaStream_t)cuda_stream>>>(cp, pp, nchains, n, rows, lgL, a_ptr_dev, a_mem_dev, b_ptr_dev,
+                                                                              b_mem_dev, npct, pct_idx_dev, out_dev, pct_dev);
+  g_mmq_launches.fetch_add(1);
+  e = cudaGetLastError();
+  if (e != cudaSuccess) return mmq_cuda_fail(nullptr, e, "k_allelic_summ", __FILE__, __LINE__);
+  return MMQ_OK;
+}
+
+int mmq_allelic_summaries(mmq_handle* const* chains, int nchains, const double* const* prior_host, int64_t nprior, int64_t rows,
+                          const int64_t* a_ptr, const int32_t* a_mem, const int64_t* b_ptr, const int32_t* b_mem, int npct,
+                          const int32_t* pct_idx, double* mean, double* sd, double* prob_a, double* pct) {
+  if (!chains || nchains < 1 || nchains > MMQ_CHAINS_MAX || nprior < 0 || rows < 0 || npct < 0 || (npct > 0 && !pct_idx) ||
+      (nprior > 0 && !prior_host) || (rows > 0 && (!a_ptr || !a_mem || !b_ptr || !b_mem)))
+    return mmq_fail(chains ? chains[0] : nullptr, MMQ_ERR_ARG, "mmq_allelic_summaries: bad arguments");
+  if (const int rc = chain_handles_check(chains, nchains, "mmq_allelic_summaries", 4)) return rc;
+  mmq_handle* h0 = chains[0];
+  const int L = h0->trace_len;
+  const int64_t n = h0->n;
+  auto fail = [&](const char* what) { return mmq_fail(h0, MMQ_ERR_ARG, std::string("mmq_allelic_summaries: ") + what); };
+  for (int c = 0; c < nchains; ++c)
+    if (nprior > 0 && !prior_host[c]) return fail("NULL prior draws");
+  for (int j = 0; j < npct; ++j)
+    if (pct_idx[j] < 0 || pct_idx[j] >= nchains * L) return fail("percentile index out of range");
+  if (n + nprior > INT32_MAX) return fail("too many rows");
+  if (rows == 0) return MMQ_OK;
+  if (a_ptr[0] != 0 || b_ptr[0] != 0) return fail("a unit CSR must start at 0");
+  for (int64_t r = 0; r < rows; ++r)
+    if (a_ptr[r + 1] < a_ptr[r] || b_ptr[r + 1] < b_ptr[r]) return fail("a unit CSR must not decrease");
+  const int64_t na = a_ptr[rows], nb = b_ptr[rows];
+  for (int64_t q = 0; q < na; ++q)
+    if (a_mem[q] < 0 || a_mem[q] >= n + nprior) return fail("member id out of range");
+  for (int64_t q = 0; q < nb; ++q)
+    if (b_mem[q] < 0 || b_mem[q] >= n + nprior) return fail("member id out of range");
+  /* every chain's draws complete on its own device */
+  for (int c = 0; c < nchains; ++c) {
+    MMQ_CUDA(h0, cudaSetDevice(chains[c]->device));
+    MMQ_CUDA(h0, cudaStreamSynchronize(chains[c]->stream));
+  }
+  MMQ_CUDA(h0, cudaSetDevice(h0->device));
+  double *ws = nullptr, *prior = nullptr, *out = nullptr, *d_pct = nullptr;
+  int64_t *d_aptr = nullptr, *d_bptr = nullptr;
+  int32_t *d_amem = nullptr, *d_bmem = nullptr, *d_idx = nullptr;
+  const double *t[MMQ_CHAINS_MAX] = {}, *src[MMQ_CHAINS_MAX] = {}, *pri[MMQ_CHAINS_MAX] = {};
+  for (int c = 0; c < nchains; ++c) t[c] = chains[c]->trace;
+  const size_t pbytes = sizeof(double) * (size_t)nprior * (size_t)L;
+  cudaError_t e = cudaSuccess;
+  auto A = [&](auto** p, size_t b) { if (e == cudaSuccess) e = mmq_cache_malloc(p, std::max<size_t>(b, 8)); };
+  auto H2D = [&](void* dst, const void* from, size_t b) {
+    if (e == cudaSuccess && b) e = cudaMemcpyAsync(dst, from, b, cudaMemcpyHostToDevice, h0->stream);
+  };
+  A(&prior, pbytes * (size_t)nchains);
+  A(&out, sizeof(double) * 3 * (size_t)rows);
+  A(&d_aptr, sizeof(int64_t) * (size_t)(rows + 1)); A(&d_bptr, sizeof(int64_t) * (size_t)(rows + 1));
+  A(&d_amem, sizeof(int32_t) * (size_t)na); A(&d_bmem, sizeof(int32_t) * (size_t)nb);
+  if (npct > 0) { A(&d_pct, sizeof(double) * (size_t)rows * (size_t)npct); A(&d_idx, sizeof(int32_t) * (size_t)npct); }
+  for (int c = 0; c < nchains && nprior > 0; ++c) {
+    pri[c] = prior + (size_t)c * (size_t)nprior * (size_t)L;
+    H2D(prior + (size_t)c * (size_t)nprior * (size_t)L, prior_host[c], pbytes);
+  }
+  H2D(d_aptr, a_ptr, sizeof(int64_t) * (size_t)(rows + 1)); H2D(d_bptr, b_ptr, sizeof(int64_t) * (size_t)(rows + 1));
+  H2D(d_amem, a_mem, sizeof(int32_t) * (size_t)na); H2D(d_bmem, b_mem, sizeof(int32_t) * (size_t)nb);
+  if (npct > 0) H2D(d_idx, pct_idx, sizeof(int32_t) * (size_t)npct);
+  if (e == cudaSuccess) e = chain_gather(chains, nchains, t, n, L, &ws, src);
+  int ret = MMQ_OK;
+  if (e == cudaSuccess) {
+    ret = mmq_allelic_summaries_dev(src, pri, nchains, n, nprior, rows, L, d_aptr, d_amem, d_bptr, d_bmem, npct, d_idx, out, d_pct, h0->stream);
+    if (ret) ret = mmq_fail(h0, ret, mmq_last_error(nullptr));
+  }
+  auto D = [&](void* dst, const void* from, size_t b) {
+    if (e == cudaSuccess && ret == MMQ_OK && dst && b) e = cudaMemcpyAsync(dst, from, b, cudaMemcpyDeviceToHost, h0->stream);
+  };
+  D(mean, out, sizeof(double) * (size_t)rows);
+  D(sd, out + rows, sizeof(double) * (size_t)rows);
+  D(prob_a, out + 2 * rows, sizeof(double) * (size_t)rows);
+  if (npct > 0) D(pct, d_pct, sizeof(double) * (size_t)rows * (size_t)npct);
+  const cudaError_t es = cudaStreamSynchronize(h0->stream);
+  if (e == cudaSuccess) e = es;
+  if (e != cudaSuccess && ret == MMQ_OK) ret = mmq_cuda_fail(h0, e, "mmq_allelic_summaries", __FILE__, __LINE__);
+  mmq_cache_free(ws); mmq_cache_free(prior); mmq_cache_free(out); mmq_cache_free(d_pct); mmq_cache_free(d_idx);
+  mmq_cache_free(d_aptr); mmq_cache_free(d_bptr); mmq_cache_free(d_amem); mmq_cache_free(d_bmem);
   return ret;
 }
 

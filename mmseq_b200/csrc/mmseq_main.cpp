@@ -16,7 +16,8 @@
  * from the EM estimate, split-R-hat and bulk / tail ESS per transcript, identical set and gene: *.convergence,
  * *.identical.convergence, *.gene.convergence), -pool (with -chains: the three tables and the -counts files over the draws
  * of all chains), -tpm (posterior and EM transcripts per million per transcript, identical set and gene: *.tpm,
- * *.identical.tpm, *.gene.tpm).
+ * *.identical.tpm, *.gene.tpm), -allelic (posterior and EM allelic fraction per haplotype pair STEM_A / STEM_B and gene:
+ * *.allelic, *.gene.allelic).
  */
 #include <unistd.h>
 #include <zlib.h>
@@ -37,6 +38,7 @@
 #include <sstream>
 #include <string>
 #include <thread>
+#include <unordered_map>
 #include <vector>
 
 #include "../../include/mmq.h"
@@ -81,6 +83,7 @@ static void printUsage(ostream& out) {
       << "  -chains INT        (B200 build) run INT independent chains (1..8, default: 1) and write split-R-hat and ESS per feature (*.convergence, *.identical.convergence, *.gene.convergence)" << endl
       << "  -pool              (B200 build) with -chains 2 or more: the *.mmseq tables and -counts files summarise the draws of all chains (default: chain 1's); trace files stay chain 1's" << endl
       << "  -tpm               (B200 build) also write posterior and EM transcripts per million (*.tpm, *.identical.tpm, *.gene.tpm)" << endl
+      << "  -allelic           (B200 build) also write the posterior and EM allelic fraction of every haplotype pair STEM_A / STEM_B and gene (*.allelic, *.gene.allelic)" << endl
       << endl;
 }
 
@@ -181,6 +184,7 @@ struct Options {
   bool debug = false, notraces = false, counts = false;
   bool pool = false; /* -pool: the tables and -counts over the draws of all chains */
   bool tpm = false;  /* -tpm: the .tpm files */
+  bool allelic = false; /* -allelic: the .allelic files */
   int ngpus = 1;
   string batch;     /* -batch FILE: one "hits_file output_base" pair per line */
   int per_gpu = 4;  /* -per_gpu INT: samples in flight per GPU in batch mode */
@@ -225,7 +229,7 @@ static Options parse_command_line(int argc, char** argv) {
       {"-seed", INT, &o.seed},            {"-percentiles", TEXT, &pct},       {"-gpus", INT, &o.ngpus},
       {"-batch", TEXT, &o.batch},         {"-per_gpu", INT, &o.per_gpu},      {"-notraces", FLAG, &o.notraces},
       {"-debug", FLAG, &o.debug},         {"-counts", FLAG, &o.counts},       {"-chains", INT, &o.chains},
-      {"-pool", FLAG, &o.pool},           {"-tpm", FLAG, &o.tpm},
+      {"-pool", FLAG, &o.pool},           {"-tpm", FLAG, &o.tpm},            {"-allelic", FLAG, &o.allelic},
   };
   /* options come first; what is left must be the mandatory arguments (none in batch mode) */
   int i = 1;
@@ -264,6 +268,41 @@ static Options parse_command_line(int argc, char** argv) {
   return o;
 }
 
+/* -allelic: the haplotype pairs of a header (include/mmq.h, allelic fraction): header transcripts STEM_A and STEM_B of one
+ * gene, with or without hits, in the header order of the _A copy.  `lonely` counts the transcripts named *_A / *_B whose
+ * partner is missing or in another gene. */
+struct HaploPairs {
+  vector<int32_t> a, b; /* header indices of the two copies of every pair */
+  vector<string> stem;  /* the pair's feature id */
+  vector<char> paired;  /* per header transcript */
+  int64_t lonely = 0;
+};
+
+static HaploPairs find_pairs(const mmq::HitsHeader& hdr) {
+  HaploPairs hp;
+  const int64_t T = (int64_t)hdr.names.size();
+  unordered_map<string, int32_t> index;
+  for (int64_t t = 0; t < T; ++t) index.emplace(hdr.names[(size_t)t], (int32_t)t);
+  auto named = [&](int64_t t, char copy) {
+    const string& s = hdr.names[(size_t)t];
+    return s.size() >= 2 && s[s.size() - 2] == '_' && s.back() == copy;
+  };
+  hp.paired.assign((size_t)T, 0);
+  for (int64_t t = 0; t < T; ++t) {
+    if (!named(t, 'A')) continue;
+    const string& s = hdr.names[(size_t)t];
+    const string stem = s.substr(0, s.size() - 2);
+    const auto it = index.find(stem + "_B");
+    if (it == index.end() || hdr.gene_of[(size_t)it->second] != hdr.gene_of[(size_t)t]) continue;
+    hp.a.push_back((int32_t)t);
+    hp.b.push_back(it->second);
+    hp.stem.push_back(stem);
+    hp.paired[(size_t)t] = hp.paired[(size_t)it->second] = 1;
+  }
+  for (int64_t t = 0; t < T; ++t) hp.lonely += (named(t, 'A') || named(t, 'B')) && !hp.paired[(size_t)t];
+  return hp;
+}
+
 /* One sample: hits file in, the nine output files out (src/mmseq.cpp:312-1694).  first_device: the GPU of a
  * single-GPU run, or the first of o.ngpus consecutive devices.  Messages go to out / err (the terminal for a
  * single sample, the sample's log in batch mode). */
@@ -296,6 +335,12 @@ static void run_sample(const Options& o, const string& hits_file, const string& 
   if (cls.first_zero_weight_record >= 0) /* its likelihood term is log 0: EM would turn mu into NaN */
     die("Error: fragment record " + to_string(cls.first_zero_weight_record + 1) + " of \"" + hits_file +
         "\" has per-hit weights that are all zero: its likelihood is zero whatever the abundances.");
+  HaploPairs hp;
+  if (o.allelic) {
+    hp = find_pairs(hdr);
+    if (hp.a.empty()) die("Error: -allelic found no pair of transcripts STEM_A / STEM_B in one gene.");
+    if (hp.lonely > 0) err << "Note: -allelic: " << hp.lonely << " transcripts named *_A / *_B have no partner in their gene." << endl;
+  }
   out << "Running mmseq with parameters:\n"
        << "  alpha:         " << alpha << endl
        << "  beta:          " << beta << endl
@@ -709,6 +754,57 @@ static void run_sample(const Options& o, const string& hits_file, const string& 
        [&](int64_t g) { return make_pair(summ[2].mean[(size_t)g], summ[2].sd[(size_t)g]); }}, /* chain 1's, as the reference */
   };
 
+  /* ---- the two levels of -allelic: haplotype pairs (a row per pair) and genes (a row per gene of .gene.mmseq, its A side
+   * the _A copies of the pairs inside it, its B side their _B copies, in pair order).  Members are in column space: an
+   * observed copy is its column, a hit-less copy n + j, j its row among the prior rows (the hit-less paired copies in
+   * header order).  unit_of / side: the unit of every observed copy (-1: none) and its side (0 A, 1 B). */
+  struct AlleleLevel {
+    const char* suffix; /* of the level's .allelic file */
+    int64_t rows;
+    function<string(int64_t)> id;
+    vector<int64_t> npairs, a_ptr{0}, b_ptr{0};
+    vector<int32_t> a_mem, b_mem, unit_of;
+    vector<uint8_t> side;
+    int64_t n_obs; /* member ids below it have hits */
+    bool observed(int64_t u) const { /* a member with hits on either side */
+      for (int64_t q = a_ptr[(size_t)u]; q < a_ptr[(size_t)u + 1]; ++q) if (a_mem[(size_t)q] < n_obs) return true;
+      for (int64_t q = b_ptr[(size_t)u]; q < b_ptr[(size_t)u + 1]; ++q) if (b_mem[(size_t)q] < n_obs) return true;
+      return false;
+    }
+  };
+  vector<AlleleLevel> allele_levels;
+  vector<int32_t> prior_hdr; /* header index of prior row j */
+  if (o.allelic) {
+    vector<int32_t> col_of((size_t)T);
+    for (int64_t hI = 0; hI < T; ++hI) {
+      col_of[(size_t)hI] = cls.hdr2col[(size_t)hI];
+      if (hp.paired[(size_t)hI] && col_of[(size_t)hI] < 0) { col_of[(size_t)hI] = (int32_t)(n + (int64_t)prior_hdr.size()); prior_hdr.push_back((int32_t)hI); }
+    }
+    vector<vector<int32_t>> by_gene((size_t)G);
+    const int64_t P = (int64_t)hp.a.size();
+    for (int64_t p = 0; p < P; ++p) by_gene[(size_t)hdr.gene_of[(size_t)hp.a[(size_t)p]]].push_back((int32_t)p);
+    allele_levels = {{"", P, [&](int64_t p) { return hp.stem[(size_t)p]; }}, {".gene", G, [&](int64_t g) { return hdr.gene_names[(size_t)g]; }}};
+    for (int lvl = 0; lvl < 2; ++lvl) {
+      AlleleLevel& al = allele_levels[(size_t)lvl];
+      al.n_obs = n;
+      al.unit_of.assign((size_t)n, -1);
+      al.side.assign((size_t)n, 0);
+      for (int64_t u = 0; u < al.rows; ++u) {
+        const vector<int32_t> one{(int32_t)u};
+        const vector<int32_t>& ps = lvl == 0 ? one : by_gene[(size_t)u];
+        for (int32_t p : ps)
+          for (int sd = 0; sd < 2; ++sd) {
+            const int32_t c = col_of[(size_t)(sd ? hp.b : hp.a)[(size_t)p]];
+            (sd ? al.b_mem : al.a_mem).push_back(c);
+            if (c < n) { al.unit_of[(size_t)c] = (int32_t)u; al.side[(size_t)c] = (uint8_t)sd; }
+          }
+        al.npairs.push_back((int64_t)ps.size());
+        al.a_ptr.push_back((int64_t)al.a_mem.size());
+        al.b_ptr.push_back((int64_t)al.b_mem.size());
+      }
+    }
+  }
+
   /* ---- summaries on the device: chain 1's (sd, mcse, iact: :1308-1363).  With -pool the observed rows come from
    * mmq_pooled_summaries over the draws of all chains, `draws` of them per feature, with the percentile rule of :1113
    * for `draws` draws: mcse = sd / sqrt(ess_mean), iact = draws / ess_mean.  What survives of chain 1's summaries: the
@@ -942,13 +1038,17 @@ static void run_sample(const Options& o, const string& hits_file, const string& 
   });
   ofs.close(); ofs.clear();
 
-  /* output_base + suffix + ext of a level: the mapped-fragments line, `head`, then one line per table row: its id and
+  /* output_base + suffix + ext: the mapped-fragments line, `head`, then one line per table row: its id and
    * cols(table row, device row) */
-  auto write_level = [&](const Level& lv, const char* ext, const string& head, const function<void(ostream&, int64_t, int64_t)>& cols) {
-    ofs.open((output_base + lv.suffix + ext).c_str());
+  auto write_table = [&](const string& suffix, const string& head, int64_t rows, const function<string(int64_t)>& id,
+                         const function<void(ostream&, int64_t)>& cols) {
+    ofs.open((output_base + suffix).c_str());
     ofs << "# Mapped fragments: " << N << endl << head;
-    write_rows(ofs, lv.rows, [&](ostream& os, int64_t r) { os << lv.id(r) << "\t"; cols(os, r, lv.dev_row(r)); });
+    write_rows(ofs, rows, [&](ostream& os, int64_t r) { os << id(r) << "\t"; cols(os, r); });
     ofs.close(); ofs.clear();
+  };
+  auto write_level = [&](const Level& lv, const char* ext, const string& head, const function<void(ostream&, int64_t, int64_t)>& cols) {
+    write_table(string(lv.suffix) + ext, head, lv.rows, lv.id, [&](ostream& os, int64_t r) { cols(os, r, lv.dev_row(r)); });
   };
 
   /* ---- -counts: .counts, .identical.counts, .gene.counts — posterior mean and sd over the chain's sweeps, EM expected
@@ -1007,6 +1107,57 @@ static void run_sample(const Options& o, const string& hits_file, const string& 
     }
   }
 
+  /* ---- -allelic: .allelic, .gene.allelic — per unit the fragments only one side explains (mmq_allele_only_counts, all
+   * shards), the EM fraction from mu_em, and the posterior mean, sd, P(a > b) and percentiles of phi = a / (a + b) over
+   * chain 1's draws (with -pool over every chain's; mmq_allelic_summaries).  The hit-less copies of a pair enter as the
+   * prior draws their chain already uses.  A unit without an observed member reports NA in every posterior and EM
+   * column; NaN is written NA. */
+  if (o.allelic) {
+    const int64_t nprior = (int64_t)prior_hdr.size();
+    vector<vector<double>> prior_rows((size_t)npool, vector<double>((size_t)nprior * (size_t)L));
+    vector<const double*> prior_ptr((size_t)npool);
+    for (int c = 0; c < npool; ++c) {
+      const double* sim = c == 0 ? simu.data() : simu_pool[(size_t)c].data();
+      for (int64_t j = 0; j < nprior; ++j)
+        copy_n(sim + (size_t)unobs_slot[(size_t)prior_hdr[(size_t)j]] * (size_t)L, L, prior_rows[(size_t)c].begin() + (ptrdiff_t)(j * L));
+      prior_ptr[(size_t)c] = prior_rows[(size_t)c].data();
+    }
+    ostringstream head;
+    head << "feature_id\tpairs\ta_only_fragments\tb_only_fragments\tem_fraction_a\tposterior_mean_fraction_a\tposterior_sd_fraction_a"
+            "\tprob_a_gt_b\tpercentiles_fraction_a";
+    write_pcts(head, percentiles.data(), NP, '\n');
+    if (NP == 0) head << '\n';
+    auto put = [](ostream& os, double v) -> ostream& { if (std::isnan(v)) os << "NA"; else os << v; return os; };
+    for (const AlleleLevel& al : allele_levels) {
+      const size_t R = (size_t)al.rows;
+      vector<int32_t> a_only(R), b_only(R);
+      on_all([&](int g) {
+        mmq_handle* h = shards[(size_t)g].h;
+        vector<int32_t> oa(g == 0 ? 0 : R), ob(g == 0 ? 0 : R);
+        check(mmq_allele_only_counts(h, al.unit_of.data(), al.side.data(), al.rows, g == 0 ? a_only.data() : oa.data(), g == 0 ? b_only.data() : ob.data()),
+              h, "mmq_allele_only_counts");
+      });
+      vector<double> mean(R), sdv(R), prob(R), pct(R * NP);
+      check(mmq_allelic_summaries(chain_h.data(), npool, prior_ptr.data(), nprior, al.rows, al.a_ptr.data(), al.a_mem.data(), al.b_ptr.data(),
+                                  al.b_mem.data(), (int)NP, pidx_all.data(), mean.data(), sdv.data(), prob.data(), pct.data()), H0,
+            "mmq_allelic_summaries");
+      write_table(string(al.suffix) + ".allelic", head.str(), al.rows, al.id, [&](ostream& os, int64_t u) {
+        const bool obs = al.observed(u);
+        double sa = 0.0, sb = 0.0; /* EM: the observed members in index order; a hit-less copy counts 0 */
+        for (int64_t q = al.a_ptr[(size_t)u]; q < al.a_ptr[(size_t)u + 1]; ++q) if (al.a_mem[(size_t)q] < n) sa += mu_em[(size_t)al.a_mem[(size_t)q]];
+        for (int64_t q = al.b_ptr[(size_t)u]; q < al.b_ptr[(size_t)u + 1]; ++q) if (al.b_mem[(size_t)q] < n) sb += mu_em[(size_t)al.b_mem[(size_t)q]];
+        const double na = NAN, em = sa == 0.0 && sb == 0.0 ? na : sa / (sa + sb);
+        os << al.npairs[(size_t)u] << "\t" << a_only[(size_t)u] << "\t" << b_only[(size_t)u] << "\t";
+        put(os, obs ? em : na) << "\t";
+        put(os, obs ? mean[(size_t)u] : na) << "\t";
+        put(os, obs ? sdv[(size_t)u] : na) << "\t";
+        put(os, obs ? prob[(size_t)u] : na) << "\t";
+        for (size_t j = 0; j < NP; ++j) put(os, obs ? pct[(size_t)u * NP + j] : na) << (j == NP - 1 ? '\n' : ',');
+        if (NP == 0) os << '\n';
+      });
+    }
+  }
+
   /* ---- -chains: .convergence, .identical.convergence, .gene.convergence — log_mu and sd pooled over the draws of all
    * chains, split-R-hat and bulk / tail ESS (mmq_chain_diagnostics); a row whose `observed` column is 0 in the tables
    * above carries that table's closed-form log_mu and sd, and NA. */
@@ -1044,6 +1195,7 @@ static void run_sample(const Options& o, const string& hits_file, const string& 
   list(".mmseq");
   if (o.counts) list(".counts");
   if (o.tpm) list(".tpm");
+  for (const AlleleLevel& al : allele_levels) out << "  " << output_base << al.suffix << ".allelic" << endl;
   if (nchains > 1) list(".convergence");
   out << "  " << output_base << ".M" << endl << "  " << output_base << ".k" << endl << endl;
   if (!notraces) {
