@@ -462,26 +462,33 @@ MMQ_HD double mmq_inv_small(int64_t x) { /* 1 <= x */
   return x < 64 ? mmq_inv_host[x] : 1.0 / (double)x;
 #endif
 }
-MMQ_HD int64_t mmq_binv(const mmq_rng* g, uint32_t block0, int64_t n, double p) {
+/* BINV in two parts, like BTRS below: the per-draw constants (one log and one exp among them), then one inversion per
+ * attempt.  A kernel that runs the attempts of a draw apart from its setup computes the constants once per draw. */
+typedef struct { double q, s, a, r0; } mmq_binv_par;
+MMQ_HD mmq_binv_par mmq_binv_setup(int64_t n, double p) {
+  mmq_binv_par t;
   const double dn = (double)n;
-  const double q = 1.0 - p;
-  const double s = p / q;
-  const double a = (dn + 1.0) * s;
-  const double r0 = mmq_exp(dn * mmq_log1p(-p));
-  for (uint32_t att = 0;; ++att) {
-    uint32_t w[4];
-    mmq_rng_block(g, block0 + att, w);
-    double r = r0;
-    double u = mmq_uniform52(w[0], w[1]);
-    int64_t x = 0;
-    while (u > r) {
-      u -= r;
-      x += 1;
-      if (x > n) break;
-      r *= (a * mmq_inv_small(x) - s);
-    }
-    if (x <= n) return x;
+  t.q = 1.0 - p;
+  t.s = p / t.q;
+  t.a = (dn + 1.0) * t.s;
+  t.r0 = mmq_exp(dn * mmq_log1p(-p));
+  return t;
+}
+/* one inversion from block `block`: returns 1 and *x_out when it ends at x <= n, 0 when it runs past n */
+MMQ_HD int mmq_binv_attempt(const mmq_rng* g, uint32_t block, int64_t n, const mmq_binv_par t, int64_t* x_out) {
+  uint32_t w[4];
+  mmq_rng_block(g, block, w);
+  double r = t.r0;
+  double u = mmq_uniform52(w[0], w[1]);
+  int64_t x = 0;
+  while (u > r) {
+    u -= r;
+    x += 1;
+    if (x > n) return 0;
+    r *= (t.a * mmq_inv_small(x) - t.s);
   }
+  *x_out = x;
+  return 1;
 }
 typedef struct { double dn, b, a, c, vr, r, alpha, m; } mmq_btrs_par;
 MMQ_HD mmq_btrs_par mmq_btrs_setup(int64_t n, double p) {
@@ -518,9 +525,13 @@ MMQ_HD int mmq_btrs_attempt(const mmq_rng* g, uint32_t block, const mmq_btrs_par
   return lv <= ub;
 }
 MMQ_HD int64_t mmq_binomial_half(const mmq_rng* g, uint32_t block0, int64_t n, double p) {
-  if ((double)n * p < MMQ_BINV_MEAN) return mmq_binv(g, block0, n, p);
-  const mmq_btrs_par t = mmq_btrs_setup(n, p);
   int64_t x = 0;
+  if ((double)n * p < MMQ_BINV_MEAN) {
+    const mmq_binv_par t = mmq_binv_setup(n, p);
+    for (uint32_t r = 0; !mmq_binv_attempt(g, block0 + r, n, t, &x); ++r) { }
+    return x;
+  }
+  const mmq_btrs_par t = mmq_btrs_setup(n, p);
   for (uint32_t r = 0; !mmq_btrs_attempt(g, block0 + r, t, &x); ++r) { }
   return x;
 }

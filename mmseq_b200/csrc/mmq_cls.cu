@@ -320,8 +320,10 @@ k_alloc_cls1(int chunk_begin, int chunk_end, const int32_t* __restrict__ pcol, c
 /* The chain set: classes with more than mmq_cat_limit(d) fragments — the multinomial by conditional binomials
  * (gsl_ran_multinomial, src/mmseq.cpp:880), O(d) binomials per class whatever k is, in the balanced splitting order of
  * mmq_alloc_chain (include/mmq_sampler.h): ceil(log2 d) levels, the binomials of a level independent of each other.
- * One class per lane of the block's first four warps, 32 classes of equal size per chunk (member-major like the small
- * set, so every column load of a warp is one 128-byte line), longest classes first.
+ * One class per lane of the block's first warps, 32 classes of equal size per chunk (member-major like the small set, so
+ * every column load of a warp is one 128-byte line), longest classes first.  Three instances, one per splitting depth
+ * (class sizes 5..16, 3..4 and 2), each over its contiguous chunk range: 91 % of the chain classes of the config-2
+ * sample need one or two levels and no longer carry the shared memory and the level loop of the 16-member classes.
  *
  * A binomial is a rejection sampler (BTRS above a mean of 10) or an inversion loop of data-dependent length (BINV
  * below): with every lane running its own, a warp pays for the union of the regimes and for its slowest lane — the first
@@ -332,40 +334,51 @@ k_alloc_cls1(int chunk_begin, int chunk_end, const int32_t* __restrict__ pcol, c
  * rejected ones re-queued; the inversions on the remaining threads of the first round.  Same integers as the CPU
  * replay's mmq_alloc_chain. */
 #define MMQ_CHAIN_THREADS 256 /* threads per block */
-#define MMQ_CHAIN_CLASSES 128 /* classes per block pass: the lanes of warps 0..3 (the other warps only work in the dense phases) */
 #define MMQ_CHAIN_SPEC 2      /* attempts of an open BTRS draw evaluated side by side per round */
-#define MMQ_CHAIN_NODES 8     /* nodes of a class on the last splitting level: 2^(ceil(log2 MMQ_CLS_CHAIN_DMAX) - 1) */
-#define MMQ_CHAIN_QCAP (MMQ_CHAIN_CLASSES * MMQ_CHAIN_NODES)
-struct chain_req { double p; int n; int owner; }; /* owner: thread | node << 8 | flip << 16 (x = n - x' for p > 1/2) */
+/* a queued draw, p <= 1/2; owner: class slot | node << 8 | flip << 16 (x = n - x' for p > 1/2).  BTRS draws fill the
+ * queue from the front, inversions from the back.  (Keeping each draw's BTRS / BINV constants here instead of
+ * recomputing them per attempt grows an entry from 16 to 72 bytes and did not pay: DESIGN.md, "Tried and measured out".) */
+struct chain_req { double p; int n, owner; };
+/* One instance per splitting depth: LV levels at most (class sizes up to 2^LV), C classes per block pass (the lanes of
+ * the first C / 32 warps own them; every warp works in the dense phases).  The arrays are sized by the deepest class the
+ * instance serves, so the shallow classes, most of the chain set, do not carry the footprint of the deep ones. */
+template <int LV, int C>
 struct chain_smem {
-  double p[MMQ_CLS_CHAIN_DMAX][MMQ_CHAIN_CLASSES];      /* mu of the members */
-  int cnt[2 * MMQ_CHAIN_NODES][MMQ_CHAIN_CLASSES];      /* fragments of the nodes of the current level */
-  int res[MMQ_CHAIN_NODES][MMQ_CHAIN_CLASSES];          /* left-half counts drawn on this level */
-  chain_req qt[MMQ_CHAIN_QCAP];                         /* BTRS draws of this level */
-  chain_req qi[MMQ_CHAIN_QCAP];                         /* inversions and the trivial cases */
-  int open[2][MMQ_CHAIN_QCAP];                          /* BTRS draws not yet accepted (indices into qt), ping-pong over rounds */
-  int att[MMQ_CHAIN_THREADS];                           /* this pass's attempts: x, or -1 rejected */
-  uint32_t cid[MMQ_CHAIN_CLASSES];
-  int n[4]; /* BTRS draws, inversions, open[0], open[1] */
+  static constexpr int NM = 1 << LV;         /* members of a class */
+  static constexpr int NN = 1 << (LV - 1);   /* nodes of a class on its last level */
+  static constexpr int QCAP = C * NN;        /* draws of a level */
+  double p[NM][C];                           /* mu of the members */
+  int cnt[NM][C];                            /* fragments of the nodes of the current level */
+  int res[NN][C];                            /* left-half counts drawn on this level */
+  chain_req q[QCAP];                         /* BTRS draws of this level from the front, inversions from the back */
+  int open[2][QCAP];                         /* BTRS draws not yet accepted (indices into q), ping-pong over rounds */
+  int att[MMQ_CHAIN_THREADS];                /* this pass's attempts: x, or -1 rejected */
+  uint32_t cid[C];
+  int d[C];                                  /* class size, 0 for a padding lane */
+  int n[4];                                  /* BTRS draws, inversions, open[0], open[1] */
   int dmax;
 };
-__global__ void __launch_bounds__(MMQ_CHAIN_THREADS)
-k_alloc_chain(int chunks, const int32_t* __restrict__ pcol, const int32_t* __restrict__ ck, const uint32_t* __restrict__ ccid,
+template <int LV, int C, int MINB>
+__global__ void __launch_bounds__(MMQ_CHAIN_THREADS, MINB)
+k_alloc_chain(int chunk_begin, int chunk_end, const int32_t* __restrict__ pcol, const int32_t* __restrict__ ck, const uint32_t* __restrict__ ccid,
               const unsigned long long* __restrict__ cdesc, uint32_t cid_hi, const double* __restrict__ mu,
               int32_t* __restrict__ counts, uint32_t seed, uint32_t sweep, const uint32_t* __restrict__ sweep_base) {
+  using SM = chain_smem<LV, C>;
+  constexpr int QCAP = SM::QCAP;
+  static_assert(C % 32 == 0 && C <= MMQ_CHAIN_THREADS && C <= 256, "class slots: owner warps, 8 bits of the owner word");
   extern __shared__ __align__(16) unsigned char chain_raw[];
-  chain_smem& S = *reinterpret_cast<chain_smem*>(chain_raw);
+  SM& S = *reinterpret_cast<SM*>(chain_raw);
   if (sweep_base) sweep += *sweep_base;
   const int tid = threadIdx.x, lane = tid & 31, wib = tid >> 5;
-  constexpr int CW = MMQ_CHAIN_CLASSES / 32;
+  constexpr int CW = C / 32;
   const bool owner_warp = wib < CW;
-  for (int chunk0 = blockIdx.x * CW; chunk0 < chunks; chunk0 += gridDim.x * CW) {
+  for (int chunk0 = chunk_begin + blockIdx.x * CW; chunk0 < chunk_end; chunk0 += gridDim.x * CW) {
     const int chunk = chunk0 + wib;
     int D = 0;
     const int32_t* pc = pcol;
     int kv = 0;
     uint32_t cid = 0;
-    if (owner_warp && chunk < chunks) {
+    if (owner_warp && chunk < chunk_end) {
       const unsigned long long desc = cdesc[chunk];
       D = (int)(desc & 0xffull);
       pc = pcol + (desc >> 8) + lane;
@@ -377,6 +390,7 @@ k_alloc_chain(int chunks, const int32_t* __restrict__ pcol, const int32_t* __res
     if (tid == 0) S.dmax = 0;
     if (owner_warp) {
       S.cid[tid] = cid;
+      S.d[tid] = D;
       S.cnt[0][tid] = kv;
       for (int j = 0; j < D; ++j) S.p[j][tid] = mu[ld_plan(pc + 32 * j)];
     }
@@ -388,46 +402,59 @@ k_alloc_chain(int chunks, const int32_t* __restrict__ pcol, const int32_t* __res
     __syncthreads();
     int levels = 0;
     while ((1 << levels) < S.dmax) ++levels;
-    for (int L = 0; L < levels; ++L) {
+    for (int L = 0; L < LV && L < levels; ++L) {
       const int nodes = 1 << L;
       if (tid < 4) S.n[tid] = 0;
       __syncthreads();
-      /* ---- the nodes of this level: what has to be drawn? */
-      if (owner_warp) {
-        for (int i = 0; i < nodes; ++i) {
-          bool pending = false, btrs = false;
-          double pr = 0.0;
-          int n = 0;
-          if (D > 0) {
-            const int lo = MMQ_NODE_LO(i, L, D), hi = MMQ_NODE_LO(i + 1, L, D);
-            n = S.cnt[i][tid];
-            if (hi - lo >= 2) {
-              const int mid = MMQ_NODE_LO(2 * i + 1, L + 1, D);
-              if (mid == lo) S.res[i][tid] = 0;
-              else if (mid == hi) S.res[i][tid] = n;
-              else if (n == 0) S.res[i][tid] = 0;
-              else {
-                double left = 0.0, right = 0.0;
-                for (int j = lo; j < mid; ++j) left += S.p[j][tid];
-                for (int j = mid; j < hi; ++j) right += S.p[j][tid];
-                const double tot = left + right;
-                pr = tot > 0.0 ? left / tot : 0.0;
-                if (pr > 1.0) pr = 1.0;
+      /* ---- the nodes of this level: what has to be drawn?  The (class, node) pairs are spread over all threads, 32
+       * classes of one node per warp */
+      for (int w0 = 0; w0 < C * nodes; w0 += MMQ_CHAIN_THREADS) {
+        const int w = w0 + tid, c = w % C, i = w / C;
+        bool pending = false, btrs = false;
+        double pr = 0.0;
+        int n = 0;
+        const int dc = w < C * nodes ? S.d[c] : 0;
+        if (dc > 0) {
+          const int lo = MMQ_NODE_LO(i, L, dc), hi = MMQ_NODE_LO(i + 1, L, dc);
+          n = S.cnt[i][c];
+          if (hi - lo >= 2) {
+            const int mid = MMQ_NODE_LO(2 * i + 1, L + 1, dc);
+            if (mid == lo) S.res[i][c] = 0;
+            else if (mid == hi) S.res[i][c] = n;
+            else if (n == 0) S.res[i][c] = 0;
+            else {
+              double left = 0.0, right = 0.0;
+              for (int j = lo; j < mid; ++j) left += S.p[j][c];
+              for (int j = mid; j < hi; ++j) right += S.p[j][c];
+              const double tot = left + right;
+              pr = tot > 0.0 ? left / tot : 0.0;
+              if (pr > 1.0) pr = 1.0;
+              const double ph = pr > 0.5 ? 1.0 - pr : pr;
+              if (n >= 2 && pr > 0.0 && pr < 1.0) {
                 pending = true;
-                const double ph = pr > 0.5 ? 1.0 - pr : pr;
-                btrs = n >= 2 && pr > 0.0 && pr < 1.0 && (double)n * ph >= MMQ_BINV_MEAN;
+                btrs = (double)n * ph >= MMQ_BINV_MEAN;
+              } else { /* p == 0 or 1, or a single fragment: mmq_binomial's first cases, here rather than queued */
+                int x = pr >= 1.0 ? n : 0;
+                if (n == 1 && pr > 0.0 && pr < 1.0) {
+                  uint32_t wd[4];
+                  cls_block(wd, S.cid[c], cid_hi, sweep, MMQ_CHAIN_BLOCK(nodes + i), seed);
+                  x = mmq_uniform52(wd[0], wd[1]) < pr ? 1 : 0;
+                }
+                S.res[i][c] = x;
               }
             }
           }
-          const int pt = queue_slot(&S.n[0], pending && btrs, lane);
-          if (pt >= 0) { S.qt[pt].p = pr > 0.5 ? 1.0 - pr : pr; S.qt[pt].n = n; S.qt[pt].owner = tid | (i << 8) | (pr > 0.5 ? 1 << 16 : 0); S.open[1][pt] = pt; }
-          const int pi = queue_slot(&S.n[1], pending && !btrs, lane);
-          if (pi >= 0) { S.qi[pi].p = pr; S.qi[pi].n = n; S.qi[pi].owner = tid | (i << 8); }
         }
+        const int owner = c | (i << 8) | (pr > 0.5 ? 1 << 16 : 0);
+        const double ph = pr > 0.5 ? 1.0 - pr : pr;
+        const int pt = queue_slot(&S.n[0], pending && btrs, lane);
+        if (pt >= 0) { S.q[pt] = chain_req{ph, n, owner}; S.open[1][pt] = pt; }
+        const int pi = queue_slot(&S.n[1], pending && !btrs, lane);
+        if (pi >= 0) S.q[QCAP - 1 - pi] = chain_req{ph, n, owner};
       }
       __syncthreads();
       /* ---- round r: attempts SPEC r .. SPEC r + SPEC - 1 of every open BTRS draw, one per thread; in round 0 the
-       * threads after them do the inversions (mean below 10), single fragments and p == 0 or 1 */
+       * threads after them do the inversions (mean below 10) */
       const uint32_t heap = (uint32_t)nodes;
       const int ni = S.n[1];
       int nopen = S.n[0];
@@ -442,17 +469,23 @@ k_alloc_chain(int chunks, const int32_t* __restrict__ pcol, const int32_t* __res
         for (int w0 = 0; w0 < work + extra; w0 += MMQ_CHAIN_THREADS) { /* passes of one work item per thread */
           const int wi = w0 + tid;
           if (wi < work) {
-            const chain_req q = S.qt[S.open[(rr + 1) & 1][wi / spec]];
+            const chain_req q = S.q[S.open[(rr + 1) & 1][wi / spec]];
+            const int owner = q.owner;
             mmq_rng g;
-            mmq_rng_init(&g, seed, MMQ_STREAM_ALLOC, ((uint64_t)cid_hi << 32) | S.cid[q.owner & 0xff], sweep);
+            mmq_rng_init(&g, seed, MMQ_STREAM_ALLOC, ((uint64_t)cid_hi << 32) | S.cid[owner & 0xff], sweep);
             int64_t xb = 0;
-            const bool ok = mmq_btrs_attempt(&g, MMQ_CHAIN_BLOCK(heap + ((q.owner >> 8) & 0xff)) + r + (uint32_t)(wi % spec), mmq_btrs_setup(q.n, q.p), &xb) != 0;
+            const bool ok = mmq_btrs_attempt(&g, MMQ_CHAIN_BLOCK(heap + ((owner >> 8) & 0xff)) + r + (uint32_t)(wi % spec), mmq_btrs_setup(q.n, q.p), &xb) != 0;
             S.att[tid] = ok ? (int)xb : -1;
           } else if (wi < work + extra) {
-            const chain_req q = S.qi[wi - work];
+            const chain_req q = S.q[QCAP - 1 - (wi - work)];
+            const int owner = q.owner, n = q.n;
             mmq_rng g;
-            mmq_rng_init(&g, seed, MMQ_STREAM_ALLOC, ((uint64_t)cid_hi << 32) | S.cid[q.owner & 0xff], sweep);
-            S.res[(q.owner >> 8) & 0xff][q.owner & 0xff] = (int)mmq_binomial(&g, MMQ_CHAIN_BLOCK(heap + ((q.owner >> 8) & 0xff)), q.n, q.p);
+            mmq_rng_init(&g, seed, MMQ_STREAM_ALLOC, ((uint64_t)cid_hi << 32) | S.cid[owner & 0xff], sweep);
+            const uint32_t b0 = MMQ_CHAIN_BLOCK(heap + ((owner >> 8) & 0xff));
+            int64_t x = 0;
+            const mmq_binv_par bt = mmq_binv_setup(n, q.p);
+            for (uint32_t att = 0; !mmq_binv_attempt(&g, b0 + att, n, bt, &x); ++att) { }
+            S.res[(owner >> 8) & 0xff][owner & 0xff] = (owner >> 16) ? n - (int)x : (int)x;
           }
           __syncthreads();
           /* the first thread of each draw of this pass takes the lowest accepted attempt, or re-queues the draw */
@@ -463,8 +496,10 @@ k_alloc_chain(int chunks, const int32_t* __restrict__ pcol, const int32_t* __res
               req = S.open[(rr + 1) & 1][wi / spec];
               int xa = -1;
               for (int sp = spec - 1; sp >= 0; --sp) if (S.att[tid + sp] >= 0) xa = S.att[tid + sp];
-              if (xa >= 0) { const chain_req q = S.qt[req]; S.res[(q.owner >> 8) & 0xff][q.owner & 0xff] = (q.owner >> 16) ? q.n - xa : xa; }
-              else again = true;
+              if (xa >= 0) {
+                const chain_req q = S.q[req];
+                S.res[(q.owner >> 8) & 0xff][q.owner & 0xff] = (q.owner >> 16) ? q.n - xa : xa;
+              } else again = true;
             }
             const int pos = queue_slot(&S.n[2 + (rr & 1)], again, lane);
             if (pos >= 0) S.open[rr & 1][pos] = req;
@@ -686,6 +721,7 @@ static int cls_plan_device(mmq_handle* h, const mmq_problem* p) {
   std::vector<int> first_h(MMQ_CLSB_NDP, -1), nch(MMQ_CLSB_NDP, 0);
   std::vector<clsb_run> runs(MMQ_CLSB_NDP);
   int64_t chunks = 0, packed = 0, chunks_lo = 0, chunks_gen = 0, c_chunks = 0, c_packed = 0, small_slots = 0, n_chain = 0;
+  int64_t c_end[3] = {0, 0, 0};
   if (S > 0) {
     CLSB(mmq_cache_malloc(&keys, sizeof(unsigned long long) * (size_t)S));
     CLSB(mmq_cache_malloc(&keys2, sizeof(unsigned long long) * (size_t)S));
@@ -725,6 +761,8 @@ static int cls_plan_device(mmq_handle* h, const mmq_problem* p) {
       } else {
         runs[dp].e0 = c_packed; runs[dp].chunk0 = (int)c_chunks;
         c_chunks += nc; c_packed += nc * 32 * d; n_chain += cnt[dp];
+        for (int v = 0; v < 3; ++v)
+          if (d > (4 >> v)) c_end[v] = c_chunks;
       }
     }
     if (chunks > 0x7fff0000ll) { cleanup(); mmq_dev_free(h, h->seg_base); h->seg_base = nullptr; return MMQ_OK; }
@@ -799,6 +837,7 @@ static int cls_plan_device(mmq_handle* h, const mmq_problem* p) {
   h->cls_rest = n_rest; h->cls_rest_nnz = nnz_rest; h->cls_rest_tiles = n_rest;
   h->cls_packed = packed;
   h->cls_c_chunks = c_chunks; h->cls_c_packed = c_packed; h->cls_chain = n_chain;
+  for (int v = 0; v < 3; ++v) h->cls_c_end[v] = c_end[v];
   h->cls_ready = true;
   return MMQ_OK;
 }
@@ -813,11 +852,14 @@ int mmq_cls_plan(mmq_handle* h, const mmq_problem* p) {
     MMQ_CUDA(h, cudaStreamCreateWithFlags(&h->stream3, cudaStreamNonBlocking));
     MMQ_CUDA(h, cudaStreamCreateWithFlags(&h->stream4, cudaStreamNonBlocking));
     MMQ_CUDA(h, cudaStreamCreateWithFlags(&h->stream5, cudaStreamNonBlocking));
+    MMQ_CUDA(h, cudaStreamCreateWithFlags(&h->stream6, cudaStreamNonBlocking));
     MMQ_CUDA(h, cudaEventCreateWithFlags(&h->ev_fork, cudaEventDisableTiming));
     MMQ_CUDA(h, cudaEventCreateWithFlags(&h->ev_join, cudaEventDisableTiming));
     MMQ_CUDA(h, cudaEventCreateWithFlags(&h->ev_join3, cudaEventDisableTiming));
     MMQ_CUDA(h, cudaEventCreateWithFlags(&h->ev_join4, cudaEventDisableTiming));
     MMQ_CUDA(h, cudaEventCreateWithFlags(&h->ev_join5, cudaEventDisableTiming));
+    MMQ_CUDA(h, cudaEventCreateWithFlags(&h->ev_fork6, cudaEventDisableTiming));
+    MMQ_CUDA(h, cudaEventCreateWithFlags(&h->ev_join6, cudaEventDisableTiming));
   }
   if (!host_plan) return cls_plan_device(h, p);
   mmq_cls_host_plan P;
@@ -885,6 +927,7 @@ int mmq_cls_plan(mmq_handle* h, const mmq_problem* p) {
   h->cls_c_chunks = P.c_chunks;
   h->cls_c_packed = P.c_packed;
   h->cls_chain = P.n_chain;
+  for (int v = 0; v < 3; ++v) h->cls_c_end[v] = P.c_end[v];
   h->cls_ready = true;
   return MMQ_OK;
 }
@@ -917,15 +960,29 @@ int mmq_cls_launch(mmq_handle* h, uint32_t seed, uint32_t sweep, const uint32_t*
    * one and waits for the others */
   MMQ_CUDA(h, cudaEventRecord(h->ev_fork, h->stream));
 #define MMQ_CLS_ARGS(c0, c1) (int)(c0), (int)(c1), h->cls_pcol, h->cls_pk, h->cls_pcid, h->cls_cdesc, h->cls_cid_hi, h->mu, h->counts, seed, sweep, sweep_base
-  if (do_chain) { /* the longest dependent chains: first in */
-    MMQ_CUDA(h, cudaStreamWaitEvent(h->stream4, h->ev_fork, 0));
-    constexpr int CW = MMQ_CHAIN_CLASSES / 32;
-    const int grid = (int)std::min<int64_t>((h->cls_c_chunks + CW - 1) / CW, (int64_t)h->num_sms * CHAIN_CTAS);
-    MMQ_CUDA(h, cudaFuncSetAttribute(k_alloc_chain, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)sizeof(chain_smem)));
-    k_alloc_chain<<<grid, MMQ_CHAIN_THREADS, sizeof(chain_smem), h->stream4>>>((int)h->cls_c_chunks, h->cls_c_pcol, h->cls_c_k, h->cls_c_cid, h->cls_c_desc, h->cls_cid_hi,
-                                                              h->mu, h->counts, seed, sweep, sweep_base);
+  /* the chain set: one k_alloc_chain instance per splitting depth over its contiguous chunk range */
+  auto chain = [&](auto kern, int C, size_t smem, int64_t c0, int64_t c1, cudaStream_t st) -> int {
+    const int cw = C / 32;
+    const int grid = (int)std::min<int64_t>((c1 - c0 + cw - 1) / cw, (int64_t)h->num_sms * CHAIN_CTAS);
+    MMQ_CUDA(h, cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
+    kern<<<grid, MMQ_CHAIN_THREADS, smem, st>>>((int)c0, (int)c1, h->cls_c_pcol, h->cls_c_k, h->cls_c_cid, h->cls_c_desc, h->cls_cid_hi,
+                                                 h->mu, h->counts, seed, sweep, sweep_base);
     MMQ_LAUNCHED(h);
+    return MMQ_OK;
+  };
+  const int64_t* ce = h->cls_c_end;
+  const bool do_deep = do_chain && ce[0] > 0, do_shallow = do_chain && ce[2] > ce[0];
+  if (do_deep) { /* the longest dependent chains: first in */
+    MMQ_CUDA(h, cudaStreamWaitEvent(h->stream4, h->ev_fork, 0));
+    if ((rc = chain(k_alloc_chain<4, 64, 2>, 64, sizeof(chain_smem<4, 64>), 0, ce[0], h->stream4))) return rc;
     MMQ_CUDA(h, cudaEventRecord(h->ev_join4, h->stream4));
+  }
+  if (do_shallow) { /* d 3..4, then d == 2, one after the other on their own stream */
+    MMQ_CUDA(h, cudaEventRecord(h->ev_fork6, h->stream));
+    MMQ_CUDA(h, cudaStreamWaitEvent(h->stream6, h->ev_fork6, 0));
+    if (ce[1] > ce[0] && (rc = chain(k_alloc_chain<2, 128, 3>, 128, sizeof(chain_smem<2, 128>), ce[0], ce[1], h->stream6))) return rc;
+    if (ce[2] > ce[1] && (rc = chain(k_alloc_chain<1, 128, 3>, 128, sizeof(chain_smem<1, 128>), ce[1], ce[2], h->stream6))) return rc;
+    MMQ_CUDA(h, cudaEventRecord(h->ev_join6, h->stream6));
   }
   if (do_rest) {
     MMQ_CUDA(h, cudaStreamWaitEvent(h->stream2, h->ev_fork, 0));
@@ -961,6 +1018,7 @@ int mmq_cls_launch(mmq_handle* h, uint32_t seed, uint32_t sweep, const uint32_t*
   if (do_lo) MMQ_CUDA(h, cudaStreamWaitEvent(h->stream, h->ev_join5, 0));
   if (do_hi) MMQ_CUDA(h, cudaStreamWaitEvent(h->stream, h->ev_join3, 0));
   if (do_rest) MMQ_CUDA(h, cudaStreamWaitEvent(h->stream, h->ev_join, 0));
-  if (do_chain) MMQ_CUDA(h, cudaStreamWaitEvent(h->stream, h->ev_join4, 0));
+  if (do_shallow) MMQ_CUDA(h, cudaStreamWaitEvent(h->stream, h->ev_join6, 0));
+  if (do_deep) MMQ_CUDA(h, cudaStreamWaitEvent(h->stream, h->ev_join4, 0));
   return MMQ_OK;
 }

@@ -58,6 +58,7 @@ struct mmq_cls_host_plan {
   std::vector<uint32_t> c_cid;             /* [c_chunks * 32] low word of the class id */
   std::vector<unsigned long long> c_desc;  /* [c_chunks] offset of the chunk in c_pcol << 8 | class size */
   int64_t c_chunks = 0, c_packed = 0, n_chain = 0;
+  int64_t c_end[3] = {0, 0, 0};            /* chain chunks of the classes above 4 members, above 2, all (k_alloc_chain's instances) */
   std::vector<int64_t> o_rp, o_cid, o_tiles; /* the rest: sub-CSR for the general kernel, one class per tile */
   std::vector<int32_t> o_col, o_k;
   std::vector<int32_t> s_col, s_k;           /* singleton classes: column and count */
@@ -285,6 +286,8 @@ static bool mmq_cls_build_host(int64_t n, int64_t m, const int64_t* rp, const in
       for (int64_t c = 0; c < nch; ++c) P.c_desc.push_back(((unsigned long long)(c_packed + c * 32 * d) << 8) | (unsigned long long)d);
       c_chunks += nch;
       c_packed += nch * 32 * d;
+      for (int v = 0; v < 3; ++v)
+        if (d > (4 >> v)) P.c_end[v] = c_chunks;
       a = b;
     }
     P.c_pcol.reset(new int32_t[(size_t)std::max<int64_t>(c_packed, 1)]);

@@ -1193,6 +1193,9 @@ void mmq_destroy(mmq_handle* h) {
   if (h->ev_join4) cudaEventDestroy(h->ev_join4);
   if (h->stream5) { cudaStreamSynchronize(h->stream5); cudaStreamDestroy(h->stream5); }
   if (h->ev_join5) cudaEventDestroy(h->ev_join5);
+  if (h->stream6) { cudaStreamSynchronize(h->stream6); cudaStreamDestroy(h->stream6); }
+  if (h->ev_fork6) cudaEventDestroy(h->ev_fork6);
+  if (h->ev_join6) cudaEventDestroy(h->ev_join6);
   if (h->ev_fork) cudaEventDestroy(h->ev_fork);
   if (h->ev_join) cudaEventDestroy(h->ev_join);
   if (h->ev_join3) cudaEventDestroy(h->ev_join3);

@@ -126,8 +126,10 @@ struct mmq_handle {
   uint32_t* cls_c_cid = nullptr;
   unsigned long long* cls_c_desc = nullptr;
   int64_t cls_c_chunks = 0, cls_c_packed = 0, cls_chain = 0;
-  cudaStream_t stream2 = nullptr, stream3 = nullptr, stream4 = nullptr, stream5 = nullptr;
+  int64_t cls_c_end[3] = {0, 0, 0}; /* chain chunks [0, end[0]): d > 4; [end[0], end[1]): d 3..4; [end[1], end[2]): d == 2 */
+  cudaStream_t stream2 = nullptr, stream3 = nullptr, stream4 = nullptr, stream5 = nullptr, stream6 = nullptr;
   cudaEvent_t ev_fork = nullptr, ev_join = nullptr, ev_join3 = nullptr, ev_join4 = nullptr, ev_join5 = nullptr;
+  cudaEvent_t ev_fork6 = nullptr, ev_join6 = nullptr;
 
   /* fused count exchange over peer memory: one peer-mapped block per rank, laid out as
    * [flags MMQ_P2P_HEAD bytes | counts parity 0 | counts parity 1 | mu] (offsets: p2p_off_* in mmq_core.cu) */
