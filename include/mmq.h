@@ -402,6 +402,55 @@ int mmq_allelic_summaries(mmq_handle* const* chains, int nchains, const double* 
                           const int64_t* a_ptr, const int32_t* a_mem, const int64_t* b_ptr, const int32_t* b_mem, int npct,
                           const int32_t* pct_idx, double* mean, double* sd, double* prob_a, double* pct);
 
+/* ---- isoform pairs within a gene (none in the reference; mmseq -isocorr) ------------------------------------------------
+ * Isoforms that share most of their fragments get strongly anti-correlated draws: their marginal log_mu and sd look
+ * confident while their split is not.  mmcollapse thresholds the correlation of the mu draws (src/mmcollapse.cpp:514-561);
+ * these functions give it per sample and gene, with P(first > second) and the shared fragments, without the trace files.
+ * tests/isocorr_reference.py restates the definitions in numpy.
+ *   1. Pairs: for every gene, its observed isoforms (members with hits) in the CSR order given to
+ *      mmq_set_groups(MMQ_GROUP_GENE) (the host program: header order), m_0 .. m_{k-1}.  Every (a, b) with a < b is one
+ *      pair, a-major within the gene; genes in group order.  pair_base[g] = sum_{g' < g} k'(k' - 1) / 2, and the pair
+ *      index is pair_base[g] + a (2k - a - 1) / 2 + (b - a - 1).  Hit-less isoforms (their prior draws are independent of
+ *      everything by construction) and isoforms of different genes are not pairs.
+ *   2. Draws: x_i[c, s] = chain c's recorded mu of member i at slot s, over S = C L draws; a pair's two values always come
+ *      from the same (c, s).
+ *   3. Per pair (i, j): corr_mu = sum (x_i - m_i)(x_j - m_j) / sqrt(sum (x_i - m_i)^2 sum (x_j - m_j)^2), two-pass, m the
+ *      mean over all S draws (pooled, not per chain), clamped to [-1, 1]; corr_log_mu the same on log x; prob_1_gt_2 =
+ *      (#{x_i > x_j} + #{x_i = x_j} / 2) / S.  A correlation is NaN when either member has a draw that is not finite (for
+ *      the log, also a draw <= 0) or a centred sum of squares of 0; all three are NaN when either member has a NaN draw.
+ *      Order: a member's mean and sum of squares over the draws in 32 lane-strided partial sums and a fixed shuffle tree;
+ *      a pair's cross sum in draw order (fma) by one thread.  Nothing depends on the grid, the device, the gene order or
+ *      a repeat.
+ *   4. Shared fragments: shared[p] = sum of k_r over the hit classes r that contain both members of pair p.  A
+ *      per-fragment layout (k = NULL, also a weighted file) counts 1 per row: the weights are ignored (as for unique
+ *      hits), so a weighted file gives the counts of the unweighted file with the same records.  Exact int64.
+ * Limits of the summaries those of -tpm: 1 <= nchains <= 8, L a power of two in [4, 2048], nchains L <= 8192. */
+/* gene_of / local_of int32[n]: the gene and the local index a of every observed transcript, both -1 for one whose gene
+ * has fewer than 2 observed isoforms; pair_base int64[ngenes] (definition 1; gene g's pairs end at pair_base[g + 1], the
+ * last gene's at npairs).  out int64[npairs] on the host, all-reduced over the shards of a communicator (every rank
+ * calls it, as mmq_allele_only_counts).  A gene index outside [-1, ngenes), a local index outside [0, k), a pair_base
+ * that does not start at 0, decreases, exceeds npairs or gives a gene a pair count other than k (k - 1) / 2 is
+ * MMQ_ERR_ARG. */
+int mmq_pair_shared_counts(mmq_handle* h, const int32_t* gene_of, const int32_t* local_of, const int64_t* pair_base, int64_t ngenes,
+                           int64_t npairs, int64_t* out);
+/* Bytes of workspace mmq_isocorr_summaries_dev needs: 40 nmembers + 8 (ngenes + 1) (0 for bad arguments). */
+int64_t mmq_isocorr_workspace_bytes(int64_t ngenes, int64_t nmembers);
+/* Summaries 3 per pair.  chain_dev[c] (a host array of device pointers): chain c's transcript trace [t L + s];
+ * gene_ptr_dev int64[ngenes + 1] / members_dev int32[nmembers]: every gene's observed members (trace rows, not checked
+ * here: the handle form's come from mmq_set_groups), nmembers = gene_ptr[ngenes]; pair_base_dev int64[ngenes]
+ * (definition 1, npairs in all).  out_dev fp64[3 npairs]: [p] corr_mu, [npairs + p] corr_log_mu, [2 npairs + p]
+ * prob_1_gt_2.  All on the calling device; asynchronous on cuda_stream, no allocation: workspace_dev holds
+ * mmq_isocorr_workspace_bytes(ngenes, nmembers) bytes.  Work items (gene, pair of 32-member tiles), grid
+ * min(npairs, 2 x SMs); every member's trace row is read once per item.  Bad limits are MMQ_ERR_ARG. */
+int mmq_isocorr_summaries_dev(const double* const* chain_dev, int nchains, int64_t ngenes, int64_t nmembers, int L,
+                              const int64_t* gene_ptr_dev, const int32_t* members_dev, const int64_t* pair_base_dev, int64_t npairs,
+                              double* out_dev, void* workspace_dev, void* cuda_stream);
+/* The same on the transcript traces the handles recorded (same n, trace_len and group counts on every handle), with
+ * chains[0]'s gene groups; pair_base is derived from that CSR.  Runs on chains[0]'s device and stream; traces of handles
+ * on other devices are copied there with cudaMemcpyPeerAsync; the workspace comes from the block cache.  npairs other
+ * than the groups' pair count is MMQ_ERR_ARG.  corr_mu, corr_log_mu, prob_gt fp64[npairs] on the host; any may be NULL. */
+int mmq_isocorr_summaries(mmq_handle* const* chains, int nchains, int64_t npairs, double* corr_mu, double* corr_log_mu, double* prob_gt);
+
 /* ---- the consumer of the traces: mmcollapse's covariance step (src/mmcollapse.cpp:483-561) ----------
  * The one dense contraction of the package: tensor cores (tcgen05, bf16 split products, fp32 accumulation in
  * TMEM), everything around it fp64.  nsplit = bf16 terms per value (2: the default of the callers here).  Error in

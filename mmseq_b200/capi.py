@@ -89,6 +89,10 @@ def _load():
         "mmq_allele_only_counts": (i32, [vp, vp, vp, i64, vp, vp]),
         "mmq_allelic_summaries_dev": (i32, [C.POINTER(vp), C.POINTER(vp), i32, i64, i64, i64, i32, vp, vp, vp, vp, i32, vp, vp, vp, vp]),
         "mmq_allelic_summaries": (i32, [C.POINTER(vp), i32, C.POINTER(vp), i64, i64, vp, vp, vp, vp, i32, vp, vp, vp, vp, vp]),
+        "mmq_pair_shared_counts": (i32, [vp, vp, vp, vp, i64, i64, vp]),
+        "mmq_isocorr_workspace_bytes": (i64, [i64, i64]),
+        "mmq_isocorr_summaries_dev": (i32, [C.POINTER(vp), i32, i64, i64, i32, vp, vp, vp, i64, vp, vp, vp]),
+        "mmq_isocorr_summaries": (i32, [C.POINTER(vp), i32, i64, vp, vp, vp]),
         "mmq_prior_draws": (i32, [i32, i64, vp, vp, dbl, u32, i32, vp]),
         "mmq_trace_cov": (i32, [i32, vp, i32, i64, i32, vp]),
         "mmq_trace_cov_workspace_bytes": (i64, [i32, i64, i32]),
@@ -127,6 +131,7 @@ EXPORTS = [
     "mmq_unique_hits_sets", "mmq_sokal_batch", "mmq_chain_seed", "mmq_chain_diagnostics_dev", "mmq_chain_diagnostics",
     "mmq_pooled_summaries_dev", "mmq_pooled_summaries", "mmq_draw_totals_workspace_bytes", "mmq_draw_totals_dev",
     "mmq_tpm_summaries_dev", "mmq_tpm_summaries", "mmq_allele_only_counts", "mmq_allelic_summaries_dev", "mmq_allelic_summaries",
+    "mmq_pair_shared_counts", "mmq_isocorr_workspace_bytes", "mmq_isocorr_summaries_dev", "mmq_isocorr_summaries",
     "mmq_prior_draws", "mmq_trace_cov", "mmq_trace_cov_workspace_bytes", "mmq_trace_cov_dev",
     "mmq_handle_trace_cov", "mmq_mean_corrs", "mmq_mean_corrs_dev", "mmq_release_cache", "mmq_launch_count", "mmq_warmup", "mmq_version",
 ]
@@ -293,6 +298,31 @@ def allelic_summaries(handles, a_ptr, a_mem, b_ptr, b_mem, priors=None, pct_idx=
                                      len(pct_idx), _ptr(pct_idx), _ptr(out["mean"]), _ptr(out["sd"]), _ptr(out["prob_a"]), _ptr(out["pct"]))
     if rc:
         raise MmqError(f"mmq_allelic_summaries failed ({rc}): " + lib().mmq_last_error(h0._h).decode())
+    return out
+
+
+def isocorr_workspace_bytes(ngenes, nmembers):
+    return int(lib().mmq_isocorr_workspace_bytes(ngenes, nmembers))
+
+
+def isocorr_summaries_dev(chain_ptrs, ngenes, nmembers, L, gene_ptr_ptr, members_ptr, pair_base_ptr, npairs, out_ptr, ws_ptr, stream_ptr):
+    """mmq_isocorr_summaries_dev: chain_ptrs, device pointers (ints) of each chain's transcript trace; the gene CSR
+    (int64[ngenes + 1], int32[nmembers]) and pair_base (int64[ngenes]) on the device; out_ptr fp64[3 * npairs] (corr_mu,
+    corr_log_mu, prob_1_gt_2); ws_ptr isocorr_workspace_bytes(ngenes, nmembers) bytes.  Asynchronous on the stream."""
+    arr = (C.c_void_p * len(chain_ptrs))(*chain_ptrs)
+    _global_check(lib().mmq_isocorr_summaries_dev(arr, len(chain_ptrs), ngenes, nmembers, L, gene_ptr_ptr, members_ptr, pair_base_ptr,
+                                                  npairs, out_ptr, ws_ptr, stream_ptr), "mmq_isocorr_summaries_dev")
+
+
+def isocorr_summaries(handles, npairs):
+    """mmq_isocorr_summaries over the transcript traces the handles recorded and handles[0]'s gene groups.  Returns
+    dict(corr_mu, corr_log_mu, prob_1_gt_2: fp64[npairs])."""
+    h0 = handles[0]
+    out = dict(corr_mu=np.zeros(npairs), corr_log_mu=np.zeros(npairs), prob_1_gt_2=np.zeros(npairs))
+    arr = (C.c_void_p * len(handles))(*[h._h for h in handles])
+    rc = lib().mmq_isocorr_summaries(arr, len(handles), npairs, _ptr(out["corr_mu"]), _ptr(out["corr_log_mu"]), _ptr(out["prob_1_gt_2"]))
+    if rc:
+        raise MmqError(f"mmq_isocorr_summaries failed ({rc}): " + lib().mmq_last_error(h0._h).decode())
     return out
 
 
@@ -562,6 +592,14 @@ class Handle:
         a = np.zeros(nunits, np.int32); b = np.zeros(nunits, np.int32)
         self._check(lib().mmq_allele_only_counts(self._h, _ptr(unit_of), _ptr(side), nunits, _ptr(a), _ptr(b)), "mmq_allele_only_counts")
         return a, b
+
+    def pair_shared_counts(self, gene_of, local_of, pair_base, npairs):
+        """mmq_pair_shared_counts: int64[npairs]; gene_of / local_of int32[n] (-1: no pair), pair_base int64[ngenes]."""
+        gene_of = _c(gene_of, np.int32); local_of = _c(local_of, np.int32); pair_base = _c(pair_base, np.int64)
+        out = np.zeros(npairs, np.int64)
+        self._check(lib().mmq_pair_shared_counts(self._h, _ptr(gene_of), _ptr(local_of), _ptr(pair_base), len(pair_base), npairs, _ptr(out)),
+                    "mmq_pair_shared_counts")
+        return out
 
     def unique_hits_sets(self, set_of, nsets):
         set_of = _c(set_of, np.int32)

@@ -959,9 +959,10 @@ const char* nccl_load() {
 }
 }  // namespace
 
-int mmq_allreduce(mmq_handle* h, void* buf, size_t count, int is_double) {
+int mmq_allreduce(mmq_handle* h, void* buf, size_t count, int type) {
   if (h->nranks <= 1 || !h->comm) return MMQ_OK;
-  ncclResult_t r = g_nccl.AllReduce(buf, buf, count, is_double ? ncclFloat64 : ncclInt32, ncclSum, (ncclComm_t)h->comm, h->stream);
+  const ncclDataType_t dt = type == 1 ? ncclFloat64 : type == 2 ? ncclInt64 : ncclInt32;
+  ncclResult_t r = g_nccl.AllReduce(buf, buf, count, dt, ncclSum, (ncclComm_t)h->comm, h->stream);
   if (r != ncclSuccess)
     return mmq_fail(h, MMQ_ERR_NCCL, std::string("ncclAllReduce: ") + (g_nccl.GetErrorString ? g_nccl.GetErrorString(r) : "?"));
   return MMQ_OK;

@@ -199,7 +199,8 @@ template <class T>
 static inline cudaError_t mmq_cache_malloc(T** p, size_t bytes) { return mmq_cache_malloc_raw((void**)p, bytes); }
 int mmq_dev_alloc(mmq_handle* h, void** p, size_t bytes);
 void mmq_dev_free(mmq_handle* h, void* p);
-int mmq_allreduce(mmq_handle* h, void* buf, size_t count, int is_double);
+/* in-place sum over the ranks of h's communicator (none: no-op); type 0 int32, 1 fp64, 2 int64 */
+int mmq_allreduce(mmq_handle* h, void* buf, size_t count, int type);
 int mmq_ensure_trace_groups(mmq_handle* h);
 int mmq_seg_scan(mmq_handle* h, const int64_t* row_ptr_host);
 int mmq_seg_plan(mmq_handle* h);

@@ -10,8 +10,9 @@
  *   k_prop             src/mmseq.cpp:985-1008, :1236-1257
  *   k_uh_sets          src/uh.cpp:3-26 restated O(nnz)
  * and, with no reference counterpart, the diagnostics of several chains (k_chain_diag), the summaries of their
- * pooled draws (k_pool_summ), transcripts per million (k_draw_totals, k_totals_fold, k_tpm_summ) and the allelic fraction
- * of haplotype pairs (k_allele_only, k_allelic_summ).
+ * pooled draws (k_pool_summ), transcripts per million (k_draw_totals, k_totals_fold, k_tpm_summ), the allelic fraction
+ * of haplotype pairs (k_allele_only, k_allelic_summ) and the isoform pairs within a gene (k_pair_shared, k_isocorr_prep,
+ * k_isocorr_items, k_isocorr).
  * All traces are [row * trace_len + slot] (the reference's mu_trace layout).
  */
 #include <algorithm>
@@ -773,6 +774,198 @@ k_allelic_summ(const __grid_constant__ mmq_chain_ptrs cp, const __grid_constant_
   }
 }
 
+/* ------------------------------------------------ isoform pairs within a gene (mmseq -isocorr)
+ * Definitions: include/mmq.h (mmq_pair_shared_counts, mmq_isocorr_summaries_dev); tests/isocorr_reference.py restates
+ * them in numpy.
+ * k_pair_shared, the shape of k_allele_only: one thread per hit class or fragment row, grid-capped.  Every two positions
+ * q < r of the row whose transcripts are observed isoforms of one gene add k (or 1) at the pair's index, rowbase[t_a] +
+ * local_of[t_b] with a < b the two local indices; O(len^2) on the row. */
+template <bool HAS_K>
+__global__ void k_pair_shared(const int64_t* __restrict__ row_ptr, const int32_t* __restrict__ col, const int32_t* __restrict__ kk,
+                              const int32_t* __restrict__ gene_of, const int32_t* __restrict__ local_of,
+                              const int64_t* __restrict__ rowbase, int64_t m, unsigned long long* __restrict__ out) {
+  for (int64_t i = blockIdx.x * (int64_t)blockDim.x + threadIdx.x; i < m; i += (int64_t)gridDim.x * blockDim.x) {
+    const int64_t b = row_ptr[i], e = row_ptr[i + 1];
+    const unsigned long long w = HAS_K ? (unsigned long long)kk[i] : 1ull;
+    for (int64_t q = b; q < e; ++q) {
+      const int32_t t = col[q], g = gene_of[t];
+      if (g < 0) continue;
+      for (int64_t r = q + 1; r < e; ++r) {
+        const int32_t u = col[r];
+        if (gene_of[u] != g) continue;
+        const int32_t la = local_of[t], lb = local_of[u];
+        if (la == lb) continue;
+        atomicAdd(out + (la < lb ? rowbase[t] + lb : rowbase[u] + la), w);
+      }
+    }
+  }
+}
+
+/* The pair summaries.  S = C L draws; draw k is chain k >> lgL, slot k & (L - 1).  Work in three kernels:
+ *   k_isocorr_prep   one warp per CSR position q (every gene's observed members): mean and two-pass centred sum of
+ *                    squares of x and of log x over the S draws, lanes strided by 32 in draw order, then a fixed shuffle
+ *                    tree.  st[5 q ..]: mean x (NaN if a draw is not finite), ss x, mean log x (NaN if a draw is not
+ *                    finite or <= 0), ss log x, 1.0 if a draw is NaN.
+ *   k_isocorr_items  one CTA: items[g] = the exclusive prefix of T(T + 1) / 2 over the genes, T = ceil(k / 32) tiles of a
+ *                    gene of k >= 2 members; items[ngenes] = the total.
+ *   k_isocorr        a work item is (gene, tile row ta <= tile column tb), 32 x 32 members, in a grid-capped loop.  The
+ *                    two tiles' draws, centred draws and centred logs are staged in shared memory MMQ_ISO_CHUNK draws at
+ *                    a time ([draw][member], padded to 33); each thread owns four pairs (rows i0, i0 + 8, .., column j =
+ *                    its lane) and adds their three sums in draw order.  Every member's trace row is read once per item.
+ * Nothing depends on gridDim or on the gene order, so the bits are the same on any grid, device or repeat. */
+#define MMQ_ISO_TILE 32
+#define MMQ_ISO_CHUNK 32
+#define MMQ_ISO_PAD (MMQ_ISO_TILE + 1)
+#define MMQ_ISO_SMEM (3 * 2 * MMQ_ISO_CHUNK * MMQ_ISO_PAD * 8)
+
+__global__ void __launch_bounds__(MMQ_POST_THREADS)
+k_isocorr_prep(const __grid_constant__ mmq_chain_ptrs cp, int C, int lgL, const int32_t* __restrict__ members, int64_t nmem,
+               double* __restrict__ st) {
+  const int S = C << lgL, lane = threadIdx.x & 31;
+  const int64_t warps = (int64_t)gridDim.x * (blockDim.x >> 5);
+  const double nan = mmq_u2d(0x7ff8000000000000ull);
+  auto warp_total = [&](double v) { return __shfl_sync(0xffffffffu, post_warp_sum(v), 0); };
+  for (int64_t q = blockIdx.x * (int64_t)(blockDim.x >> 5) + (threadIdx.x >> 5); q < nmem; q += warps) {
+    const int64_t row = members[q];
+    double sx = 0.0, sl = 0.0, nonfin = 0.0, badlog = 0.0, isnanv = 0.0;
+    for (int k = lane; k < S; k += 32) {
+      const double x = chain_x(cp, row, lgL, k);
+      sx += x;
+      sl += log(x);
+      nonfin += isfinite(x) ? 0.0 : 1.0;
+      badlog += isfinite(x) && x > 0.0 ? 0.0 : 1.0;
+      isnanv += isnan(x) ? 1.0 : 0.0;
+    }
+    nonfin = warp_total(nonfin);
+    badlog = warp_total(badlog);
+    isnanv = warp_total(isnanv);
+    const double mx = nonfin == 0.0 ? warp_total(sx) / (double)S : nan;
+    const double ml = badlog == 0.0 ? warp_total(sl) / (double)S : nan;
+    double ssx = 0.0, ssl = 0.0;
+    for (int k = lane; k < S; k += 32) {
+      const double x = chain_x(cp, row, lgL, k), dx = x - mx, dl = log(x) - ml;
+      ssx += dx * dx;
+      ssl += dl * dl;
+    }
+    ssx = warp_total(ssx);
+    ssl = warp_total(ssl);
+    if (lane == 0) {
+      double* o = st + 5 * q;
+      o[0] = mx; o[1] = ssx; o[2] = ml; o[3] = ssl; o[4] = isnanv > 0.0 ? 1.0 : 0.0;
+    }
+  }
+}
+
+__device__ __forceinline__ int64_t iso_items_of(int64_t k) {
+  const int64_t T = (k + MMQ_ISO_TILE - 1) / MMQ_ISO_TILE;
+  return k >= 2 ? T * (T + 1) / 2 : 0;
+}
+
+#define MMQ_ISO_SCAN 1024
+__global__ void __launch_bounds__(MMQ_ISO_SCAN)
+k_isocorr_items(const int64_t* __restrict__ gene_ptr, int64_t ngenes, int64_t* __restrict__ items) {
+  __shared__ int64_t part[MMQ_ISO_SCAN];
+  const int64_t g0 = ngenes * threadIdx.x / MMQ_ISO_SCAN, g1 = ngenes * (threadIdx.x + 1) / MMQ_ISO_SCAN;
+  int64_t s = 0;
+  for (int64_t g = g0; g < g1; ++g) s += iso_items_of(gene_ptr[g + 1] - gene_ptr[g]);
+  part[threadIdx.x] = s;
+  __syncthreads();
+  for (int d = 1; d < MMQ_ISO_SCAN; d <<= 1) { /* inclusive Hillis-Steele scan */
+    const int64_t v = threadIdx.x >= d ? part[threadIdx.x - d] : 0;
+    __syncthreads();
+    part[threadIdx.x] += v;
+    __syncthreads();
+  }
+  s = part[threadIdx.x] - s;
+  for (int64_t g = g0; g < g1; ++g) { items[g] = s; s += iso_items_of(gene_ptr[g + 1] - gene_ptr[g]); }
+  if (threadIdx.x == MMQ_ISO_SCAN - 1) items[ngenes] = s;
+}
+
+__global__ void __launch_bounds__(MMQ_POST_THREADS)
+k_isocorr(const __grid_constant__ mmq_chain_ptrs cp, int C, int lgL, int64_t ngenes, const int64_t* __restrict__ gene_ptr,
+          const int32_t* __restrict__ members, const int64_t* __restrict__ pair_base, int64_t npairs,
+          const double* __restrict__ st, const int64_t* __restrict__ items, double* __restrict__ out) {
+  extern __shared__ double sh[];
+  typedef double tile_t[MMQ_ISO_CHUNK][MMQ_ISO_PAD];
+  tile_t* X = reinterpret_cast<tile_t*>(sh);  /* [2]: the draws of tile row / tile column */
+  tile_t* D = X + 2;                          /* [2]: x - mean x */
+  tile_t* E = X + 4;                          /* [2]: log x - mean log x */
+  __shared__ int64_t s_row[2][MMQ_ISO_TILE];
+  __shared__ double s_mx[2][MMQ_ISO_TILE], s_ml[2][MMQ_ISO_TILE];
+  const int S = C << lgL, j = threadIdx.x & 31, i0 = threadIdx.x >> 5;
+  const double nan = mmq_u2d(0x7ff8000000000000ull);
+  const int64_t nitems = items[ngenes];
+  for (int64_t it = blockIdx.x; it < nitems; it += gridDim.x) {
+    int64_t lo = 0, hi = ngenes; /* items[lo] <= it < items[hi] */
+    while (hi - lo > 1) { const int64_t mid = (lo + hi) >> 1; if (items[mid] <= it) lo = mid; else hi = mid; }
+    const int64_t g = lo, q0 = gene_ptr[g], k = gene_ptr[g + 1] - q0;
+    const int T = (int)((k + MMQ_ISO_TILE - 1) / MMQ_ISO_TILE);
+    int r = (int)(it - items[g]), ta = 0;
+    while (r >= T - ta) { r -= T - ta; ++ta; }
+    const int tb = ta + r;
+    const bool diag = ta == tb;
+    const int ka = (int)min((int64_t)MMQ_ISO_TILE, k - (int64_t)ta * MMQ_ISO_TILE);
+    const int kb = (int)min((int64_t)MMQ_ISO_TILE, k - (int64_t)tb * MMQ_ISO_TILE);
+    const int64_t qa = q0 + (int64_t)ta * MMQ_ISO_TILE, qb = q0 + (int64_t)tb * MMQ_ISO_TILE;
+    const int nside = diag ? 1 : 2, B = diag ? 0 : 1;
+    __syncthreads(); /* the previous item is done with the staging arrays */
+    if (threadIdx.x < 2 * MMQ_ISO_TILE) {
+      const int sd = threadIdx.x / MMQ_ISO_TILE, i = threadIdx.x % MMQ_ISO_TILE;
+      if (sd < nside && i < (sd ? kb : ka)) {
+        const int64_t q = (sd ? qb : qa) + i;
+        s_row[sd][i] = members[q];
+        s_mx[sd][i] = st[5 * q];
+        s_ml[sd][i] = st[5 * q + 2];
+      }
+    }
+    double sxy[4] = {0.0, 0.0, 0.0, 0.0}, sll[4] = {0.0, 0.0, 0.0, 0.0}, gt[4] = {0.0, 0.0, 0.0, 0.0};
+    for (int k0 = 0; k0 < S; k0 += MMQ_ISO_CHUNK) {
+      const int cn = min(MMQ_ISO_CHUNK, S - k0);
+      __syncthreads();
+      for (int v = threadIdx.x; v < nside * MMQ_ISO_TILE * MMQ_ISO_CHUNK; v += blockDim.x) {
+        const int sd = v / (MMQ_ISO_TILE * MMQ_ISO_CHUNK), i = (v / MMQ_ISO_CHUNK) % MMQ_ISO_TILE, s = v % MMQ_ISO_CHUNK;
+        if (i < (sd ? kb : ka) && s < cn) {
+          const double x = chain_x(cp, s_row[sd][i], lgL, k0 + s);
+          X[sd][s][i] = x;
+          D[sd][s][i] = x - s_mx[sd][i];
+          E[sd][s][i] = log(x) - s_ml[sd][i];
+        }
+      }
+      __syncthreads();
+      for (int s = 0; s < cn && i0 < ka; ++s) { /* warps without a row of the tile skip the chunk */
+        const double xb = X[B][s][j], db = D[B][s][j], eb = E[B][s][j];
+#pragma unroll
+        for (int u = 0; u < 4; ++u) {
+          const int i = i0 + 8 * u;
+          if (i >= ka) break;
+          const double xa = X[0][s][i];
+          sxy[u] = fma(D[0][s][i], db, sxy[u]);
+          sll[u] = fma(E[0][s][i], eb, sll[u]);
+          gt[u] += xa > xb ? 2.0 : xa == xb ? 1.0 : 0.0;
+        }
+      }
+    }
+#pragma unroll
+    for (int u = 0; u < 4; ++u) {
+      const int i = i0 + 8 * u;
+      if (i >= ka || j >= kb || (diag && i >= j)) continue;
+      const int64_t a = (int64_t)ta * MMQ_ISO_TILE + i, b = (int64_t)tb * MMQ_ISO_TILE + j;
+      const int64_t p = pair_base[g] + a * (2 * k - a - 1) / 2 + (b - a - 1);
+      const double* sa = st + 5 * (qa + i);
+      const double* sb = st + 5 * (qb + j);
+      auto corr = [&](double sum, double m1, double ss1, double m2, double ss2) {
+        if (isnan(m1) || isnan(m2) || ss1 == 0.0 || ss2 == 0.0) return nan;
+        const double c = sum / sqrt(ss1 * ss2);
+        return c > 1.0 ? 1.0 : c < -1.0 ? -1.0 : c;
+      };
+      const bool bad = sa[4] != 0.0 || sb[4] != 0.0;
+      out[p] = bad ? nan : corr(sxy[u], sa[0], sa[1], sb[0], sb[1]);
+      out[npairs + p] = bad ? nan : corr(sll[u], sa[2], sa[3], sb[2], sb[3]);
+      out[2 * npairs + p] = bad ? nan : gt[u] / (2.0 * (double)S);
+    }
+  }
+}
+
 /* ------------------------------------------------------------------ host */
 
 static bool pow2_ok(int len) { return len >= 4 && len <= MMQ_MAX_ROW_LEN && (len & (len - 1)) == 0; }
@@ -1490,6 +1683,158 @@ int mmq_allelic_summaries(mmq_handle* const* chains, int nchains, const double* 
   if (e != cudaSuccess && ret == MMQ_OK) ret = mmq_cuda_fail(h0, e, "mmq_allelic_summaries", __FILE__, __LINE__);
   mmq_cache_free(ws); mmq_cache_free(prior); mmq_cache_free(out); mmq_cache_free(d_pct); mmq_cache_free(d_idx);
   mmq_cache_free(d_aptr); mmq_cache_free(d_bptr); mmq_cache_free(d_amem); mmq_cache_free(d_bmem);
+  return ret;
+}
+
+int mmq_pair_shared_counts(mmq_handle* h, const int32_t* gene_of, const int32_t* local_of, const int64_t* pair_base, int64_t ngenes,
+                           int64_t npairs, int64_t* out) {
+  if (!h || !gene_of || !local_of || (!out && npairs > 0) || ngenes < 0 || npairs < 0 || (ngenes > 0 && !pair_base) || (ngenes == 0 && npairs > 0))
+    return mmq_fail(h, MMQ_ERR_ARG, "mmq_pair_shared_counts: bad arguments");
+  auto fail = [&](const char* what) { return mmq_fail(h, MMQ_ERR_ARG, std::string("mmq_pair_shared_counts: ") + what); };
+  if (ngenes > 0 && pair_base[0] != 0) return fail("pair_base must start at 0");
+  std::vector<int64_t> kof((size_t)ngenes);
+  for (int64_t g = 0; g < ngenes; ++g) {
+    const int64_t end = g + 1 < ngenes ? pair_base[g + 1] : npairs, d = end - pair_base[g];
+    if (d < 0) return fail("pair_base must not decrease or exceed npairs");
+    int64_t k = (int64_t)((1.0 + std::sqrt(1.0 + 8.0 * (double)d)) / 2.0);
+    while (k * (k - 1) / 2 > d) --k;
+    while (k * (k - 1) / 2 < d) ++k;
+    if (k * (k - 1) / 2 != d) return fail("a gene's pair count is not k (k - 1) / 2");
+    kof[(size_t)g] = d == 0 ? 0 : k;
+  }
+  std::vector<int64_t> rowbase((size_t)std::max<int64_t>(h->n, 1));
+  for (int64_t t = 0; t < h->n; ++t) {
+    const int32_t g = gene_of[t];
+    if (g < -1 || g >= ngenes) return fail("gene index out of range");
+    if (g < 0) continue;
+    const int64_t a = local_of[t], k = kof[(size_t)g];
+    if (a < 0 || a >= k) return fail("local index out of range");
+    rowbase[(size_t)t] = pair_base[g] + a * (2 * k - a - 1) / 2 - a - 1;
+  }
+  if (npairs == 0) return MMQ_OK;
+  MMQ_CUDA(h, cudaSetDevice(h->device));
+  int32_t *d_gene = nullptr, *d_local = nullptr;
+  int64_t* d_base = nullptr;
+  unsigned long long* d_out = nullptr;
+  const size_t nb = (size_t)std::max<int64_t>(h->n, 1);
+  cudaError_t e = mmq_cache_malloc(&d_gene, sizeof(int32_t) * nb);
+  if (e == cudaSuccess) e = mmq_cache_malloc(&d_local, sizeof(int32_t) * nb);
+  if (e == cudaSuccess) e = mmq_cache_malloc(&d_base, sizeof(int64_t) * nb);
+  if (e == cudaSuccess) e = mmq_cache_malloc(&d_out, sizeof(int64_t) * (size_t)npairs);
+  if (e == cudaSuccess && h->n > 0) e = cudaMemcpyAsync(d_gene, gene_of, sizeof(int32_t) * (size_t)h->n, cudaMemcpyHostToDevice, h->stream);
+  if (e == cudaSuccess && h->n > 0) e = cudaMemcpyAsync(d_local, local_of, sizeof(int32_t) * (size_t)h->n, cudaMemcpyHostToDevice, h->stream);
+  if (e == cudaSuccess && h->n > 0) e = cudaMemcpyAsync(d_base, rowbase.data(), sizeof(int64_t) * (size_t)h->n, cudaMemcpyHostToDevice, h->stream);
+  if (e == cudaSuccess) e = cudaMemsetAsync(d_out, 0, sizeof(int64_t) * (size_t)npairs, h->stream);
+  int ret = MMQ_OK;
+  if (e == cudaSuccess && h->m > 0) {
+    const int grid = mmq_grid_for(h->m, 256, h->num_sms * 8);
+    if (h->has_k) k_pair_shared<true><<<grid, 256, 0, h->stream>>>(h->row_ptr, h->col, h->k, d_gene, d_local, d_base, h->m, d_out);
+    else k_pair_shared<false><<<grid, 256, 0, h->stream>>>(h->row_ptr, h->col, h->k, d_gene, d_local, d_base, h->m, d_out);
+    g_mmq_launches.fetch_add(1);
+    e = cudaGetLastError();
+  }
+  if (e == cudaSuccess) ret = mmq_allreduce(h, d_out, (size_t)npairs, 2);
+  if (e == cudaSuccess && ret == MMQ_OK) e = cudaMemcpyAsync(out, d_out, sizeof(int64_t) * (size_t)npairs, cudaMemcpyDeviceToHost, h->stream);
+  const cudaError_t es = cudaStreamSynchronize(h->stream);
+  if (e == cudaSuccess) e = es;
+  if (e != cudaSuccess && ret == MMQ_OK) ret = mmq_cuda_fail(h, e, "mmq_pair_shared_counts", __FILE__, __LINE__);
+  mmq_cache_free(d_gene); mmq_cache_free(d_local); mmq_cache_free(d_base); mmq_cache_free(d_out);
+  return ret;
+}
+
+int64_t mmq_isocorr_workspace_bytes(int64_t ngenes, int64_t nmembers) {
+  if (ngenes < 0 || nmembers < 0) return 0;
+  return (int64_t)sizeof(double) * 5 * nmembers + (int64_t)sizeof(int64_t) * (ngenes + 1);
+}
+
+int mmq_isocorr_summaries_dev(const double* const* chain_dev, int nchains, int64_t ngenes, int64_t nmembers, int L,
+                              const int64_t* gene_ptr_dev, const int32_t* members_dev, const int64_t* pair_base_dev, int64_t npairs,
+                              double* out_dev, void* workspace_dev, void* cuda_stream) {
+  if (!chain_dev || !tpm_len_ok(nchains, L) || ngenes < 0 || nmembers < 0 || npairs < 0 ||
+      (npairs > 0 && (!gene_ptr_dev || !members_dev || !pair_base_dev || !out_dev || !workspace_dev)))
+    return mmq_fail(nullptr, MMQ_ERR_ARG, "mmq_isocorr_summaries_dev: bad arguments");
+  mmq_chain_ptrs cp = {};
+  for (int c = 0; c < nchains; ++c) {
+    if (!chain_dev[c]) return mmq_fail(nullptr, MMQ_ERR_ARG, "mmq_isocorr_summaries_dev: NULL chain");
+    cp.p[c] = chain_dev[c];
+  }
+  if (npairs == 0) return MMQ_OK;
+  int dev = 0, sms = 0, lgL = 0;
+  while ((1 << lgL) < L) ++lgL;
+  cudaError_t e = cudaGetDevice(&dev);
+  if (e == cudaSuccess) e = cudaDeviceGetAttribute(&sms, cudaDevAttrMultiProcessorCount, dev);
+  if (e == cudaSuccess) e = cudaFuncSetAttribute(k_isocorr, cudaFuncAttributeMaxDynamicSharedMemorySize, MMQ_ISO_SMEM);
+  if (e != cudaSuccess) return mmq_cuda_fail(nullptr, e, "mmq_isocorr_summaries_dev", __FILE__, __LINE__);
+  const cudaStream_t st = (cudaStream_t)cuda_stream;
+  double* stats = static_cast<double*>(workspace_dev);
+  int64_t* items = reinterpret_cast<int64_t*>(stats + 5 * nmembers);
+  if (nmembers > 0) {
+    k_isocorr_prep<<<mmq_grid_for(nmembers, MMQ_POST_THREADS / 32, 8 * sms), MMQ_POST_THREADS, 0, st>>>(cp, nchains, lgL, members_dev, nmembers, stats);
+    g_mmq_launches.fetch_add(1);
+  }
+  k_isocorr_items<<<1, MMQ_ISO_SCAN, 0, st>>>(gene_ptr_dev, ngenes, items);
+  g_mmq_launches.fetch_add(1);
+  const int grid = (int)std::min<int64_t>(npairs, 2 * (int64_t)sms); /* npairs >= work items */
+  k_isocorr<<<grid, MMQ_POST_THREADS, MMQ_ISO_SMEM, st>>>(cp, nchains, lgL, ngenes, gene_ptr_dev, members_dev, pair_base_dev, npairs, stats,
+                                                          items, out_dev);
+  g_mmq_launches.fetch_add(1);
+  e = cudaGetLastError();
+  if (e != cudaSuccess) return mmq_cuda_fail(nullptr, e, "k_isocorr", __FILE__, __LINE__);
+  return MMQ_OK;
+}
+
+int mmq_isocorr_summaries(mmq_handle* const* chains, int nchains, int64_t npairs, double* corr_mu, double* corr_log_mu, double* prob_gt) {
+  if (!chains || nchains < 1 || nchains > MMQ_CHAINS_MAX || npairs < 0)
+    return mmq_fail(chains ? chains[0] : nullptr, MMQ_ERR_ARG, "mmq_isocorr_summaries: bad arguments");
+  if (const int rc = chain_handles_check(chains, nchains, "mmq_isocorr_summaries", 4)) return rc;
+  mmq_handle* h0 = chains[0];
+  const int L = h0->trace_len;
+  const mmq_group_set& G = h0->groups[MMQ_GROUP_GENE];
+  const int64_t ngenes = G.ngroups;
+  /* every chain's draws complete on its own device */
+  for (int c = 0; c < nchains; ++c) {
+    MMQ_CUDA(h0, cudaSetDevice(chains[c]->device));
+    MMQ_CUDA(h0, cudaStreamSynchronize(chains[c]->stream));
+  }
+  MMQ_CUDA(h0, cudaSetDevice(h0->device));
+  /* pair_base from the gene CSR */
+  std::vector<int64_t> gptr((size_t)ngenes + 1, 0), pb((size_t)std::max<int64_t>(ngenes, 1), 0);
+  if (ngenes > 0) {
+    MMQ_CUDA(h0, cudaMemcpyAsync(gptr.data(), G.ptr_dev, sizeof(int64_t) * (size_t)(ngenes + 1), cudaMemcpyDeviceToHost, h0->stream));
+    MMQ_CUDA(h0, cudaStreamSynchronize(h0->stream));
+  }
+  int64_t total = 0;
+  for (int64_t g = 0; g < ngenes; ++g) {
+    const int64_t k = gptr[(size_t)g + 1] - gptr[(size_t)g];
+    pb[(size_t)g] = total;
+    total += k * (k - 1) / 2;
+  }
+  if (total != npairs)
+    return mmq_fail(h0, MMQ_ERR_ARG, "mmq_isocorr_summaries: npairs is " + std::to_string(npairs) + ", the gene groups have " +
+                                         std::to_string(total) + " pairs");
+  if (npairs == 0) return MMQ_OK;
+  const int64_t n = h0->n, nmem = gptr[(size_t)ngenes];
+  double *ws = nullptr, *work = nullptr, *out = nullptr;
+  int64_t* d_pb = nullptr;
+  const double *t[MMQ_CHAINS_MAX] = {}, *src[MMQ_CHAINS_MAX] = {};
+  for (int c = 0; c < nchains; ++c) t[c] = chains[c]->trace;
+  cudaError_t e = mmq_cache_malloc(&work, (size_t)mmq_isocorr_workspace_bytes(ngenes, nmem));
+  if (e == cudaSuccess) e = mmq_cache_malloc(&out, sizeof(double) * 3 * (size_t)npairs);
+  if (e == cudaSuccess) e = mmq_cache_malloc(&d_pb, sizeof(int64_t) * (size_t)ngenes);
+  if (e == cudaSuccess) e = cudaMemcpyAsync(d_pb, pb.data(), sizeof(int64_t) * (size_t)ngenes, cudaMemcpyHostToDevice, h0->stream);
+  if (e == cudaSuccess) e = chain_gather(chains, nchains, t, n, L, &ws, src);
+  int ret = MMQ_OK;
+  if (e == cudaSuccess) {
+    ret = mmq_isocorr_summaries_dev(src, nchains, ngenes, nmem, L, G.ptr_dev, G.members_dev, d_pb, npairs, out, work, h0->stream);
+    if (ret) ret = mmq_fail(h0, ret, mmq_last_error(nullptr));
+  }
+  double* dst[3] = {corr_mu, corr_log_mu, prob_gt};
+  for (int q = 0; q < 3 && e == cudaSuccess && ret == MMQ_OK; ++q)
+    if (dst[q]) e = cudaMemcpyAsync(dst[q], out + (size_t)q * (size_t)npairs, sizeof(double) * (size_t)npairs, cudaMemcpyDeviceToHost, h0->stream);
+  const cudaError_t es = cudaStreamSynchronize(h0->stream);
+  if (e == cudaSuccess) e = es;
+  if (e != cudaSuccess && ret == MMQ_OK) ret = mmq_cuda_fail(h0, e, "mmq_isocorr_summaries", __FILE__, __LINE__);
+  mmq_cache_free(ws); mmq_cache_free(work); mmq_cache_free(out); mmq_cache_free(d_pb);
   return ret;
 }
 

@@ -17,7 +17,8 @@
  * *.identical.convergence, *.gene.convergence), -pool (with -chains: the three tables and the -counts files over the draws
  * of all chains), -tpm (posterior and EM transcripts per million per transcript, identical set and gene: *.tpm,
  * *.identical.tpm, *.gene.tpm), -allelic (posterior and EM allelic fraction per haplotype pair STEM_A / STEM_B and gene:
- * *.allelic, *.gene.allelic).
+ * *.allelic, *.gene.allelic), -isocorr (posterior correlation, P(first > second) and shared fragments of every isoform
+ * pair within a gene: *.isocorr).
  */
 #include <unistd.h>
 #include <zlib.h>
@@ -84,6 +85,7 @@ static void printUsage(ostream& out) {
       << "  -pool              (B200 build) with -chains 2 or more: the *.mmseq tables and -counts files summarise the draws of all chains (default: chain 1's); trace files stay chain 1's" << endl
       << "  -tpm               (B200 build) also write posterior and EM transcripts per million (*.tpm, *.identical.tpm, *.gene.tpm)" << endl
       << "  -allelic           (B200 build) also write the posterior and EM allelic fraction of every haplotype pair STEM_A / STEM_B and gene (*.allelic, *.gene.allelic)" << endl
+      << "  -isocorr           (B200 build) also write the posterior correlation, P(first > second) and shared fragments of every isoform pair within a gene (*.isocorr)" << endl
       << endl;
 }
 
@@ -185,6 +187,7 @@ struct Options {
   bool pool = false; /* -pool: the tables and -counts over the draws of all chains */
   bool tpm = false;  /* -tpm: the .tpm files */
   bool allelic = false; /* -allelic: the .allelic files */
+  bool isocorr = false; /* -isocorr: the .isocorr file */
   int ngpus = 1;
   string batch;     /* -batch FILE: one "hits_file output_base" pair per line */
   int per_gpu = 4;  /* -per_gpu INT: samples in flight per GPU in batch mode */
@@ -230,6 +233,7 @@ static Options parse_command_line(int argc, char** argv) {
       {"-batch", TEXT, &o.batch},         {"-per_gpu", INT, &o.per_gpu},      {"-notraces", FLAG, &o.notraces},
       {"-debug", FLAG, &o.debug},         {"-counts", FLAG, &o.counts},       {"-chains", INT, &o.chains},
       {"-pool", FLAG, &o.pool},           {"-tpm", FLAG, &o.tpm},            {"-allelic", FLAG, &o.allelic},
+      {"-isocorr", FLAG, &o.isocorr},
   };
   /* options come first; what is left must be the mandatory arguments (none in batch mode) */
   int i = 1;
@@ -754,6 +758,27 @@ static void run_sample(const Options& o, const string& hits_file, const string& 
        [&](int64_t g) { return make_pair(summ[2].mean[(size_t)g], summ[2].sd[(size_t)g]); }}, /* chain 1's, as the reference */
   };
 
+  /* ---- -isocorr: the isoform pairs of every gene (include/mmq.h, isoform pairs): a gene's observed members in the CSR
+   * order of gptr / gmem, m_0 .. m_{k-1}, and every (a, b) with a < b, a-major; genes in .gene.mmseq order.  iso_gene /
+   * iso_local: the gene and local index a of every observed isoform of a gene with two or more, else -1; pair_gene /
+   * pair_a / pair_b: the gene and the two local indices of every pair. */
+  vector<int32_t> iso_gene, iso_local, pair_gene, pair_a, pair_b;
+  vector<int64_t> pair_base;
+  if (o.isocorr) {
+    iso_gene.assign((size_t)n, -1);
+    iso_local.assign((size_t)n, -1);
+    pair_base.resize((size_t)G);
+    for (int64_t g = 0; g < G; ++g) {
+      pair_base[(size_t)g] = (int64_t)pair_gene.size();
+      const int64_t b = gptr[(size_t)g], k = gptr[(size_t)g + 1] - b;
+      for (int64_t a = 0; a < k && k >= 2; ++a) {
+        iso_gene[(size_t)gmem[(size_t)(b + a)]] = (int32_t)g;
+        iso_local[(size_t)gmem[(size_t)(b + a)]] = (int32_t)a;
+        for (int64_t c = a + 1; c < k; ++c) { pair_gene.push_back((int32_t)g); pair_a.push_back((int32_t)a); pair_b.push_back((int32_t)c); }
+      }
+    }
+  }
+
   /* ---- the two levels of -allelic: haplotype pairs (a row per pair) and genes (a row per gene of .gene.mmseq, its A side
    * the _A copies of the pairs inside it, its B side their _B copies, in pair order).  Members are in column space: an
    * observed copy is its column, a hit-less copy n + j, j its row among the prior rows (the hit-less paired copies in
@@ -1158,6 +1183,31 @@ static void run_sample(const Options& o, const string& hits_file, const string& 
     }
   }
 
+  /* ---- -isocorr: .isocorr — per isoform pair of a gene the fragments both explain (mmq_pair_shared_counts, all shards)
+   * and the correlation of mu and of log mu and P(first > second) over chain 1's draws (with -pool over every chain's;
+   * mmq_isocorr_summaries).  NaN is written NA. */
+  if (o.isocorr) {
+    const int64_t P = (int64_t)pair_gene.size();
+    vector<int64_t> shared((size_t)P);
+    on_all([&](int g) {
+      mmq_handle* h = shards[(size_t)g].h;
+      vector<int64_t> other(g == 0 ? 0 : (size_t)P);
+      check(mmq_pair_shared_counts(h, iso_gene.data(), iso_local.data(), pair_base.data(), G, P, g == 0 ? shared.data() : other.data()), h,
+            "mmq_pair_shared_counts");
+    });
+    vector<double> cmu((size_t)P), clog((size_t)P), pgt((size_t)P);
+    check(mmq_isocorr_summaries(chain_h.data(), npool, P, cmu.data(), clog.data(), pgt.data()), H0, "mmq_isocorr_summaries");
+    auto put = [](ostream& os, double v) -> ostream& { if (std::isnan(v)) os << "NA"; else os << v; return os; };
+    auto name = [&](int64_t p, int32_t a) { return hdr.names[(size_t)cls.col2hdr[(size_t)gmem[(size_t)(gptr[(size_t)pair_gene[(size_t)p]] + a)]]]; };
+    write_table(".isocorr", "gene_id\ttranscript_1\ttranscript_2\tshared_fragments\tcorr_mu\tcorr_log_mu\tprob_1_gt_2\n", P,
+                [&](int64_t p) { return hdr.gene_names[(size_t)pair_gene[(size_t)p]]; }, [&](ostream& os, int64_t p) {
+                  os << name(p, pair_a[(size_t)p]) << "\t" << name(p, pair_b[(size_t)p]) << "\t" << shared[(size_t)p] << "\t";
+                  put(os, cmu[(size_t)p]) << "\t";
+                  put(os, clog[(size_t)p]) << "\t";
+                  put(os, pgt[(size_t)p]) << "\n";
+                });
+  }
+
   /* ---- -chains: .convergence, .identical.convergence, .gene.convergence — log_mu and sd pooled over the draws of all
    * chains, split-R-hat and bulk / tail ESS (mmq_chain_diagnostics); a row whose `observed` column is 0 in the tables
    * above carries that table's closed-form log_mu and sd, and NA. */
@@ -1196,6 +1246,7 @@ static void run_sample(const Options& o, const string& hits_file, const string& 
   if (o.counts) list(".counts");
   if (o.tpm) list(".tpm");
   for (const AlleleLevel& al : allele_levels) out << "  " << output_base << al.suffix << ".allelic" << endl;
+  if (o.isocorr) out << "  " << output_base << ".isocorr" << endl;
   if (nchains > 1) list(".convergence");
   out << "  " << output_base << ".M" << endl << "  " << output_base << ".k" << endl << endl;
   if (!notraces) {
